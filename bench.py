@@ -9,6 +9,7 @@ NCCL all-reduce of the statistics when N > 1.  Weak scaling: per-GPU work is fix
     python bench.py [--gpus N] [--steps K] [--warmup W]            our arm
     python bench.py --impl reference ...                             the CPU arm (oracle on host cores)
     torchrun --nproc-per-node N bench.py --gpus N ...                N > 1
+    python bench.py ... --dump-outputs DIR                           also write the last timed step's outputs
 
 One JSON line on stdout (rank 0).  `value` = device-resident throughput; `e2e` = the same metric
 through the public host-buffer API (pinned host inputs -> H2D -> kernel -> D2H of all outputs), stated
@@ -39,6 +40,8 @@ N_GAS = 3
 FLOPS_PER_STEP = 751.0               # 163 simple + 15 exp(28) + 3 log(36) + 3 sqrt(10) + 3 div(10)
 METRIC = "ensemble member-timesteps/sec"
 CPU_SAMPLE_MEMBERS = 65536           # the CPU arm's sample, the same in both legs (cpu_baseline and --impl reference)
+DUMP_BYTES = 63_000_000              # --dump-outputs writes at most this much in all (64 MB with the .npy headers)
+DUMP_SEED = 0                        # ... and samples larger outputs with this seed
 
 
 def algorithmic_flops(gas_form, newton_iters=0):
@@ -83,7 +86,13 @@ def parse():
     ap.add_argument("--iirf-max", type=float, default=None, help="experiment: switch the iIRF ceiling on (general kernel)")
     ap.add_argument("--no-stats", action="store_true", help="experiment: integrate without histogram/moments")
     ap.add_argument("--outputs", default="C,RF,T", help="experiment: comma list of outputs written to HBM ('' = none)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy (float32 / float64, "
+                         "rank 0's members; a fixed seeded sample of members, and of steps if need be, keeps it under 64 MB)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def workload_config(args, n_gpus):
@@ -227,12 +236,15 @@ def run_reference(args):
         for _ in range(reps):
             out = run()
             co.temperature_stats(out["T"][:, :4096], -5.0, 25.0, 1024)   # histogram of a slice (serial helper; not the point)
+        return out
     for _ in range(args.warmup):
         step()
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        step()
+        out = step()
     el = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {k: out[k] for k in ("C", "RF", "T", "state")}, {})
     work = args.steps * reps * n * args.n_t
     val = work / el
     sample = ("%d members x %d steps x %d passes per step; blocked + vectorised C rendering of the loop "
@@ -271,6 +283,45 @@ def emit(line):
         sys.stdout.flush()
     else:
         os.write(_REAL_STDOUT, data)
+
+
+def dump_outputs(out_dir, per_member, per_step):
+    """--dump-outputs: write the arrays the timed path returned in its last step as out_dir/<name>.npy, float32 or
+    float64 (integer counts as float64).  per_member maps names to arrays whose last axis is the member axis, per_step
+    to arrays whose first axis is the time step; torch tensors are sampled on their device before the copy.  To stay
+    under DUMP_BYTES the per-step arrays keep at most a quarter of it (a sample of steps beyond that) and the
+    per-member arrays share the rest (a sample of members).  Samples are sorted indices drawn with DUMP_SEED, so the
+    same arguments give the same sample."""
+    rng = np.random.default_rng(DUMP_SEED)
+
+    def sample(n, k):
+        return None if k >= n else np.sort(rng.choice(n, size=max(k, 1), replace=False))
+
+    def take(x, idx, axis):
+        if idx is not None:
+            if hasattr(x, "index_select"):
+                import torch
+                x = x.index_select(axis, torch.as_tensor(idx, device=x.device))
+            else:
+                x = np.take(x, idx, axis=axis)
+        x = np.asarray(x.cpu() if hasattr(x, "cpu") else x)
+        return x if x.dtype in (np.float32, np.float64) else x.astype(np.float64)
+
+    size = lambda shape: 8 * int(np.prod(shape, dtype=np.int64))       # bytes, counted as float64
+    steps, used = None, 0
+    if per_step:
+        n_t, row = next(iter(per_step.values())).shape[0], sum(size(x.shape[1:]) for x in per_step.values())
+        steps = sample(n_t, DUMP_BYTES // 4 // row)
+        used = row * (n_t if steps is None else len(steps))
+    members = None
+    if per_member:
+        n_member, column = next(iter(per_member.values())).shape[-1], sum(size(x.shape[:-1]) for x in per_member.values())
+        members = sample(n_member, (DUMP_BYTES - used) // column)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, x in per_step.items():
+        np.save(os.path.join(out_dir, name + ".npy"), take(x, steps, 0))
+    for name, x in per_member.items():
+        np.save(os.path.join(out_dir, name + ".npy"), take(x, members, -1))
 
 
 # ------------------------------------------------------------------------------------------------
@@ -578,6 +629,9 @@ def main():
         assert bool((res.hist.sum(dim=1) == M * n_gpus).all()), "histogram rows must count every member"
     if res.T is not None:
         assert bool(torch.isfinite(res.T[-1]).all())
+    if args.dump_outputs and rank == 0:
+        pick = lambda names: {k: getattr(res, k) for k in names if getattr(res, k) is not None}
+        dump_outputs(args.dump_outputs, pick(("C", "RF", "T", "state")), pick(("hist", "moments")))
 
     line = {"metric": METRIC, "value": value, "unit": "member-timesteps/s", "n_gpus": n_gpus, "steps": args.steps,
             "warmup": args.warmup, "ms_per_step": ms_per_step, "higher_is_better": True, "scaling": "weak",

@@ -96,9 +96,10 @@ template <typename Real> static KArgs<Real> make_args(const ufair_desc* d) {
   a.stats = d->stats;
   a.newton_iters = d->newton_iters;
 #ifdef UFAIR_DEBUG_BOUNDS
-  {  // negative control of the in-kernel bounds checks: UFAIR_DEBUG_TRIP=1 must make a full-length run trap
+  {  // negative control of the in-kernel bounds checks: UFAIR_DEBUG_TRIP=1 must make a full-length run fail
     const char* trip = getenv("UFAIR_DEBUG_TRIP");
     a.dbg_cut = (trip && trip[0] == '1') ? 1 : 0;
+    a.dbg_cut_hits = nullptr;
   }
 #else
   a.dbg_cut = 0;
@@ -284,17 +285,45 @@ __global__ void __launch_bounds__(kStatsThreads)
   }
 }
 
-template <typename Real> int run_device(const ufair_desc* d, cudaStream_t stream) {
-  int rc = validate_desc(d, sizeof(Real));
-  if (rc != UFAIR_OK) return rc;
-  if (d->n_member == 0 || d->n_t == 0) return UFAIR_OK;
-  const KArgs<Real> a = make_args<Real>(d);
+template <typename Real> static int dispatch_gases(const ufair_desc* d, const KArgs<Real>& a, cudaStream_t stream) {
   switch (d->n_gas) {
     case 1: return dispatch_mode<Real, 1>(d, a, stream);
     case 2: return dispatch_mode<Real, 2>(d, a, stream);
     case 3: return dispatch_mode<Real, 3>(d, a, stream);
     default: return dispatch_mode<Real, 4>(d, a, stream);
   }
+}
+
+#ifdef UFAIR_DEBUG_BOUNDS
+// the negative control of the store check (a.dbg_cut > 0): run, then report every store the check found in the
+// rows it pretends are missing as an error of this call
+template <typename Real> static int run_cut_control(const ufair_desc* d, KArgs<Real> a, cudaStream_t stream) {
+  cudaError_t e = cudaMalloc(&a.dbg_cut_hits, sizeof(unsigned long long));
+  if (e != cudaSuccess) return cuda_error(e, "cudaMalloc(dbg_cut_hits)");
+  unsigned long long hits = 0;
+  int rc = UFAIR_OK;
+  if ((e = cudaMemsetAsync(a.dbg_cut_hits, 0, sizeof(hits), stream)) != cudaSuccess) rc = cuda_error(e, "cudaMemsetAsync(dbg_cut_hits)");
+  if (rc == UFAIR_OK) rc = dispatch_gases<Real>(d, a, stream);
+  if (rc == UFAIR_OK && (e = cudaMemcpyAsync(&hits, a.dbg_cut_hits, sizeof(hits), cudaMemcpyDeviceToHost, stream)) != cudaSuccess)
+    rc = cuda_error(e, "cudaMemcpyAsync(dbg_cut_hits)");
+  if (rc == UFAIR_OK && (e = cudaStreamSynchronize(stream)) != cudaSuccess) rc = cuda_error(e, "cudaStreamSynchronize");
+  cudaFree(a.dbg_cut_hits);
+  if (rc == UFAIR_OK && hits)
+    rc = set_error(UFAIR_ERR_ARG, "debug bounds check: %llu output stores in the last %d row(s) that UFAIR_DEBUG_TRIP cut off",
+                   hits, a.dbg_cut);
+  return rc;
+}
+#endif
+
+template <typename Real> int run_device(const ufair_desc* d, cudaStream_t stream) {
+  int rc = validate_desc(d, sizeof(Real));
+  if (rc != UFAIR_OK) return rc;
+  if (d->n_member == 0 || d->n_t == 0) return UFAIR_OK;
+  const KArgs<Real> a = make_args<Real>(d);
+#ifdef UFAIR_DEBUG_BOUNDS
+  if (a.dbg_cut) return run_cut_control<Real>(d, a, stream);
+#endif
+  return dispatch_gases<Real>(d, a, stream);
 }
 
 // ---- gas_form detection: which pools carry mass, which forcing terms exist, over all members -------

@@ -222,6 +222,9 @@ template <typename Real> struct KArgs {
   Real* oE;
   int conc_driven;  // bit g: gas g's input rows are target concentrations (INV kernels only)
   int dbg_cut;      // UFAIR_DEBUG_BOUNDS builds only: rows the store check pretends are missing (its negative control)
+#ifdef UFAIR_DEBUG_BOUNDS
+  unsigned long long* dbg_cut_hits;  // stores the check found in those rows (counted, not trapped)
+#endif
   Real* state_out;
 };
 
@@ -284,11 +287,14 @@ template <typename Real> __device__ __forceinline__ void st_stream(Real* p, Real
 // every output store must land inside its array, in a column below n_member, and every read of the
 // shared-memory rings inside the box the TMA delivered for the current stage -- otherwise the kernel traps.
 // compute-sanitizer is closed on the GPU pool this was developed on; this is the in-kernel stand-in.
+// Its negative control (dbg_cut > 0) pretends the last rows of every output array are missing: stores the
+// check finds there are counted in dbg_cut_hits and reported by the host, so the control never faults the device.
 #ifdef UFAIR_DEBUG_BOUNDS
 #define UFAIR_CHECK_ST(base, nrows, p)                                                                    \
   do {                                                                                                    \
     const long long off_ = (long long)((p) - (base));                                                     \
-    if ((base) == nullptr || off_ < 0 || off_ >= ((long long)(nrows) - a.dbg_cut) * ld || off_ % ld >= a.n_member) __trap(); \
+    if ((base) == nullptr || off_ < 0 || off_ >= (long long)(nrows) * ld || off_ % ld >= a.n_member) __trap(); \
+    if (off_ >= ((long long)(nrows) - a.dbg_cut) * ld) atomicAdd(a.dbg_cut_hits, 1ull);                \
   } while (0)
 #define UFAIR_CHECK_RING(addr, ring0, stage_bytes, box_bytes)                                             \
   do {                                                                                                    \

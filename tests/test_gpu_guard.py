@@ -231,7 +231,8 @@ def test_debug_bounds_build_never_traps_and_its_checks_are_live():
     the box the TMA delivered.  The ragged cases of this file and of the parity suite run on it in a
     subprocess (a trap poisons the CUDA context) and must pass; then the negative control: with
     UFAIR_DEBUG_TRIP=1 the store check pretends the last row of every array is missing, and the very
-    same run must die with a launch failure -- so the checks are really compiled in and reached."""
+    same run must fail with the check's error -- so the checks are really compiled in and reached.  The
+    control counts the stores it finds in the cut rows instead of trapping, so it never faults the device."""
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     env = dict(os.environ, UFAIR_LIB=_DBG, PYTHONPATH=root)
     env.pop("UFAIR_DEBUG_TRIP", None)
@@ -246,4 +247,4 @@ def test_debug_bounds_build_never_traps_and_its_checks_are_live():
     trip = subprocess.run([sys.executable, "-c", _TRIP], cwd=root, env=dict(env, UFAIR_DEBUG_TRIP="1"), capture_output=True,
                           text=True, timeout=600)
     assert trip.returncode != 0 and "completed" not in trip.stdout
-    assert "trap" in trip.stderr.lower() or "launch fail" in trip.stderr.lower() or "cuda" in trip.stderr.lower(), trip.stderr[-2000:]
+    assert "debug bounds check" in trip.stderr and "output stores in the last 1 row(s)" in trip.stderr, trip.stderr[-2000:]

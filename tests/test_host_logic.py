@@ -241,15 +241,12 @@ def test_numa_lookup_reads_sysfs(tmp_path):
 
 
 def test_vendored_reference_test_file_is_verbatim():
-    """tests/golden/ref_test_hfcs.py is the reference's tests/unit/test_hfcs.py, byte for byte (test
-    infrastructure: the GPU suite runs the FILE against this repo's U_FaIR package)."""
+    """tests/golden/ref_test_hfcs.py is the reference's tests/unit/test_hfcs.py, byte for byte, as pinned by its
+    sha256 (test infrastructure: the GPU suite runs the FILE against this repo's U_FaIR package)."""
     import hashlib
     here = os.path.dirname(os.path.abspath(__file__))
     data = open(os.path.join(here, "golden", "ref_test_hfcs.py"), "rb").read()
     assert hashlib.sha256(data).hexdigest() == "5eeed8cd25a7b55f38006f3f6e3baa3a3fb5910040da14d71b5ab49e355e1d64"
-    ref = "/root/reference/tests/unit/test_hfcs.py"
-    if os.path.exists(ref):
-        assert open(ref, "rb").read() == data
 
 
 def test_shape_validation_of_scenario_inputs():
