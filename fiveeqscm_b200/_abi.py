@@ -7,9 +7,10 @@ from __future__ import annotations
 import ctypes as C
 import os
 
-ABI_VERSION = 2
+ABI_VERSION = 3
 MAX_GAS = 4
 N_POOL = 4
+MAX_STAT_GROUPS = 256
 
 # gas_params rows (include/ufair.h UFAIR_GP_*)
 GP_A0, GP_TAU0, GP_R0, GP_RU, GP_RT, GP_RA, GP_C0, GP_EMIS2CONC, GP_F1, GP_F2, GP_F3 = (
@@ -81,6 +82,9 @@ class UfairDesc(C.Structure):
         ("gas_form", C.c_uint8 * 4),
         ("conc_driven", C.c_int32),
         ("out_E", C.c_void_p),
+        ("n_stat_groups", C.c_int32),
+        ("reserved1", C.c_int32),
+        ("stat_group", C.c_void_p),
     ]
 
     def __init__(self, **kw):

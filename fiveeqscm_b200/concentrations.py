@@ -17,6 +17,7 @@ pipeline (chunked, H2D / kernel / D2H overlapped) and numpy out.
 from __future__ import annotations
 
 import ctypes as C
+import dataclasses
 from dataclasses import dataclass
 from typing import Optional, Sequence
 
@@ -43,11 +44,16 @@ def _require_cuda():
 
 @dataclass
 class HistSpec:
-    """Per-time-step temperature histogram: `bins` equal bins on [lo, hi) (edge bins absorb outliers)."""
+    """Per-time-step temperature histogram: `bins` equal bins on [lo, hi) (edge bins absorb outliers).
+
+    ``groups`` > 0 builds one histogram and one set of moments per member label (``stat_group=`` of
+    :func:`run_ensemble`): results are then [groups][n_t][..].  0 pools every member (results [n_t][..]).
+    The private histogram scales with it: copies x groups x n_t x bins x 4 bytes on the device."""
     lo: float = -5.0
     hi: float = 25.0
     bins: int = 1024
     copies: int = 16  # privatised copies the kernel spreads its atomics over
+    groups: int = 0   # 0 = pooled; with stat_group="scenario", 0 means one group per scenario
 
 
 @dataclass
@@ -58,10 +64,11 @@ class EnsembleResult:
     alpha: object = None    # [n_gas][n_t][n_member] (diagnostic)
     E: object = None        # [n_gas][n_t][n_member] emission rates (diagnosed for concentration-driven gases)
     state: object = None    # [5 n_gas + 3][n_member]  -> pass as state_in to continue the run
-    hist: object = None     # [n_t][bins] int64 counts (this rank's members)
-    moments: object = None  # [n_t][4] float64: sum, sumsq, min, max of T over members
+    hist: object = None     # [n_t][bins] int64 counts (this rank's members); [groups][n_t][bins] when grouped
+    moments: object = None  # [n_t][4] float64: sum, sumsq, min, max of T over members; [groups][n_t][4] when grouped
     spec: Optional[HistSpec] = None
     n_member: int = 0
+    stat_group: Optional[str] = None  # what the statistics are grouped by: None (pooled), "scenario" or "labels"
 
 
 # ------------------------------------------------------------------------------------------------
@@ -144,6 +151,7 @@ def _build_desc(G, n_t, M, ld, n_scen, e_scen, fext_mode, alpha_mode, newton_ite
         d.hist_bins, d.hist_copies = int(stats.bins), int(stats.copies)
         d.hist_lo, d.hist_hi = float(stats.lo), float(stats.hi)
         d.hist_t0, d.hist_rows = 0, n_t
+        d.n_stat_groups = int(stats.groups)
     d.conc_driven = _driven_mask(conc_driven, G)
     if gas_form is not None and not isinstance(gas_form, str):
         if len(gas_form) != G:
@@ -151,6 +159,38 @@ def _build_desc(G, n_t, M, ld, n_scen, e_scen, fext_mode, alpha_mode, newton_ite
         for g, f in enumerate(gas_form):
             d.gas_form[g] = _form_byte(f)
     return d
+
+
+def _resolve_groups(stats: Optional[HistSpec], stat_group, has_scen_idx: bool, n_scen: int):
+    """(HistSpec with ``groups`` settled, source) for ``stat_group=``: source is None (pooled), "scenario" (the
+    members' scen_idx, one group per scenario unless ``groups`` says otherwise) or "labels" (an array [M]; its group
+    count is never inferred from the data, so that every rank of a multi-GPU run agrees on it)."""
+    if stats is not None and not 0 <= int(stats.groups) <= _abi.MAX_STAT_GROUPS:
+        raise ValueError(f"HistSpec.groups must be 0..{_abi.MAX_STAT_GROUPS}")
+    if stat_group is None:
+        if stats is not None and stats.groups:
+            raise ValueError("HistSpec.groups > 0 needs stat_group ('scenario' or one label per member)")
+        return stats, None
+    if stats is None:
+        raise ValueError("stat_group needs stats=HistSpec(...)")
+    if isinstance(stat_group, str):
+        if stat_group != "scenario":
+            raise ValueError("stat_group must be None, 'scenario' or one label per member")
+        if not has_scen_idx:
+            raise ValueError("stat_group='scenario' needs scen_idx")
+        groups = int(stats.groups) or int(n_scen)
+        if groups > _abi.MAX_STAT_GROUPS:
+            raise ValueError(f"{groups} scenario groups: at most {_abi.MAX_STAT_GROUPS}")
+        return dataclasses.replace(stats, groups=groups), "scenario"
+    if stats.groups < 1:
+        raise ValueError("stat_group labels need HistSpec(groups=G), G >= 1 (it is not inferred from the labels)")
+    return stats, "labels"
+
+
+def _check_labels(top: int, groups: int, name: str):
+    """The largest label must stay below the group count (negative ones mean "not counted")."""
+    if top >= groups:
+        raise ValueError(f"{name} has a label {top} >= groups {groups}")
 
 
 def _driven_mask(conc_driven, G) -> int:
@@ -239,7 +279,7 @@ def run_ensemble(emissions, gas_params, thermal_params, *, dt=1.0, scen_idx=None
                  fext_per_member=False, state_in=None, alpha_mode="exp", newton_iters=0, iirf_max=None,
                  iirf_h=100.0, t_mode="mid", outputs: Sequence[str] = ("C", "RF", "T"), stats: Optional[HistSpec] = None,
                  precision="f64", return_state=True, chunk_members=None, workspace=None, out=None,
-                 gas_form="auto", conc_driven=None) -> EnsembleResult:
+                 gas_form="auto", conc_driven=None, stat_group=None) -> EnsembleResult:
     """Integrate the 5-equation model for an ensemble (oxfair, .coveragerc:19, as one kernel launch).
 
     emissions      [G][n_t][M] per-member emission RATES, or [G][n_t][S] scenario-shared with
@@ -251,6 +291,10 @@ def run_ensemble(emissions, gas_params, thermal_params, *, dt=1.0, scen_idx=None
     state_in       optional [5G+3][M] state from a previous call's ``.state`` (resume).
     alpha_mode     "exp" | "sinh" | "newton" (``newton_iters`` fixed steps) | "one".
     outputs        any of "C", "RF", "T", "alpha".   stats: HistSpec -> per-step T histogram + moments.
+    stat_group     statistics per member group instead of pooled: "scenario" (by ``scen_idx``; one group per
+                   scenario unless ``stats.groups`` says otherwise) or labels [M] int with ``stats.groups`` = G:
+                   label g in [0, G) counts the member in group g, a negative label leaves it out of the
+                   statistics.  ``.hist`` is then [G][n_t][bins] and ``.moments`` [G][n_t][4].
     precision      "f64" (default; <= 1e-10 relative vs the float64 oracle) or "f32" (<= 1e-4 K in T).
     conc_driven    None, True (every gas) or one flag per gas: those gases' ``emissions`` rows are the
                    CONCENTRATION to reach at the end of each step; the emission rate that does so
@@ -274,10 +318,11 @@ def run_ensemble(emissions, gas_params, thermal_params, *, dt=1.0, scen_idx=None
     if on_device:
         return _run_device(torch, emissions, gas_params, thermal_params, dt, scen_idx, e_scale, f_ext,
                            fext_per_member, state_in, alpha_mode, newton_iters, iirf_max, iirf_h, t_mode,
-                           _with_E(outputs, conc_driven), stats, precision, return_state, gas_form, conc_driven)
+                           _with_E(outputs, conc_driven), stats, precision, return_state, gas_form, conc_driven,
+                           stat_group)
     return _run_host(torch, emissions, gas_params, thermal_params, dt, scen_idx, e_scale, f_ext, fext_per_member,
                      state_in, alpha_mode, newton_iters, iirf_max, iirf_h, t_mode, _with_E(outputs, conc_driven), stats,
-                     precision, return_state, chunk_members, workspace, out, gas_form, conc_driven)
+                     precision, return_state, chunk_members, workspace, out, gas_form, conc_driven, stat_group)
 
 
 def _shapes(E_shape, gp_shape, tp_shape, scen_idx, fext_shape, fext_per_member, e_scale_shape=None):
@@ -327,18 +372,19 @@ class DevicePlan:
     def __init__(self, E, gp, tp, *, dt=1.0, scen_idx=None, e_scale=None, f_ext=None, fext_per_member=False,
                  state_in=None, alpha_mode="exp", newton_iters=0, iirf_max=None, iirf_h=100.0, t_mode="mid",
                  outputs=("C", "RF", "T"), stats=None, precision="f64", return_state=True, gas_form="auto",
-                 conc_driven=None):
+                 conc_driven=None, stat_group=None):
         torch = _require_cuda()
         outputs = _with_E(outputs, conc_driven)
         self._L = _abi.lib()
         dtype = torch.float64 if precision == "f64" else torch.float32
         es = 8 if precision == "f64" else 4
         dev = E.device
-        self.device, self.precision, self.stats = dev, precision, stats
         fshape = None if f_ext is None else tuple(f_ext.shape)
         G, n_t, M, e_scen, n_scen, fext_mode = _shapes(tuple(E.shape), tuple(gp.shape), tuple(tp.shape), scen_idx,
                                                        fshape, fext_per_member,
                                                        None if e_scale is None else tuple(e_scale.shape))
+        stats, source = _resolve_groups(stats, stat_group, scen_idx is not None, n_scen)
+        self.device, self.precision, self.stats = dev, precision, stats
         self.n_gas, self.n_t, self.n_member = G, n_t, M
         self.scen_idx = None
         ld = _round_up(max(M, 1), 16 // es)
@@ -375,6 +421,21 @@ class DevicePlan:
             keep.append(si)
             d.scen_idx = si.data_ptr()
             self.scen_idx = si    # the plan's own copy: callers that re-launch may overwrite it in place
+        self.stat_group = None
+        if source == "scenario":   # the labels ARE scen_idx: no copy, and they follow in-place updates of it
+            if M:
+                _check_labels(int(si.max()), stats.groups, "scen_idx")
+            d.stat_group = d.scen_idx
+            self.stat_group = si
+        elif source == "labels":
+            lab = torch.as_tensor(stat_group, device=dev).to(torch.int32).contiguous()
+            if lab.numel() != M:
+                raise ValueError("stat_group must have one label per member")
+            if M:
+                _check_labels(int(lab.max()), stats.groups, "stat_group")
+            keep.append(lab)
+            d.stat_group = lab.data_ptr()
+            self.stat_group = lab
         if e_scale is not None:
             esd = member_rows(e_scale, "e_scale")
             keep.append(esd)
@@ -392,7 +453,7 @@ class DevicePlan:
             keep.append(sin_)
             d.state_in = sin_.data_ptr()
 
-        res = EnsembleResult(spec=stats, n_member=M)
+        res = EnsembleResult(spec=stats, n_member=M, stat_group=source)
         new = lambda *shape: torch.empty(*shape, dtype=dtype, device=dev)
         if "C" in outputs:
             buf = new(G, n_t, ld); d.out_C = buf.data_ptr(); res.C = buf[..., :M]
@@ -409,11 +470,13 @@ class DevicePlan:
         if return_state:
             buf = new(_abi.state_rows(G), ld); d.state_out = buf.data_ptr(); res.state = buf[..., :M]
         if stats is not None:
-            self._hp = torch.empty(stats.copies, n_t, stats.bins, dtype=torch.int32, device=dev)
-            self._mp = torch.empty(stats.copies, n_t, _abi.MOM_COUNT, dtype=torch.float64, device=dev)
+            lead = (stats.groups, n_t) if stats.groups else (n_t,)
+            rows = max(1, stats.groups) * n_t
+            self._hp = torch.empty(stats.copies, rows, stats.bins, dtype=torch.int32, device=dev)
+            self._mp = torch.empty(stats.copies, rows, _abi.MOM_COUNT, dtype=torch.float64, device=dev)
             d.hist_private, d.moments_private = self._hp.data_ptr(), self._mp.data_ptr()
-            res.hist = torch.empty(n_t, stats.bins, dtype=torch.int64, device=dev)
-            res.moments = torch.empty(n_t, _abi.MOM_COUNT, dtype=torch.float64, device=dev)
+            res.hist = torch.empty(*lead, stats.bins, dtype=torch.int64, device=dev)
+            res.moments = torch.empty(*lead, _abi.MOM_COUNT, dtype=torch.float64, device=dev)
         res._keep = keep  # inputs stay alive as long as the result does
         self.desc, self.result, self._keep = d, res, keep
         self._run = self._L.ufair_run_f64 if precision == "f64" else self._L.ufair_run_f32
@@ -471,12 +534,13 @@ class DevicePlan:
 
 
 def _run_device(torch, E, gp, tp, dt, scen_idx, e_scale, f_ext, fext_per_member, state_in, alpha_mode, newton_iters,
-                iirf_max, iirf_h, t_mode, outputs, stats, precision, return_state, gas_form="auto", conc_driven=None):
+                iirf_max, iirf_h, t_mode, outputs, stats, precision, return_state, gas_form="auto", conc_driven=None,
+                stat_group=None):
     return DevicePlan(E, gp, tp, dt=dt, scen_idx=scen_idx, e_scale=e_scale, f_ext=f_ext,
                       fext_per_member=fext_per_member, state_in=state_in, alpha_mode=alpha_mode,
                       newton_iters=newton_iters, iirf_max=iirf_max, iirf_h=iirf_h, t_mode=t_mode, outputs=outputs,
                       stats=stats, precision=precision, return_state=return_state, gas_form=gas_form,
-                      conc_driven=conc_driven).run()
+                      conc_driven=conc_driven, stat_group=stat_group).run()
 
 
 class Workspace:
@@ -500,7 +564,7 @@ class Workspace:
 
 def _run_host(torch, E, gp, tp, dt, scen_idx, e_scale, f_ext, fext_per_member, state_in, alpha_mode, newton_iters,
               iirf_max, iirf_h, t_mode, outputs, stats, precision, return_state, chunk_members, workspace, out=None,
-              gas_form=None, conc_driven=None):
+              gas_form=None, conc_driven=None, stat_group=None):
     L = _abi.lib()
     npdt = np.float64 if precision == "f64" else np.float32
 
@@ -515,6 +579,7 @@ def _run_host(torch, E, gp, tp, dt, scen_idx, e_scale, f_ext, fext_per_member, s
     fshape = None if f_ext is None else f_ext.shape
     G, n_t, M, e_scen, n_scen, fext_mode = _shapes(E.shape, gp.shape, tp.shape, scen_idx, fshape, fext_per_member,
                                                    None if e_scale is None else e_scale.shape)
+    stats, source = _resolve_groups(stats, stat_group, scen_idx is not None, n_scen)
     auto_form = isinstance(gas_form, str)
     if auto_form and gas_form != "auto":
         raise ValueError("gas_form must be 'auto', None or one entry per gas")
@@ -528,6 +593,19 @@ def _run_host(torch, E, gp, tp, dt, scen_idx, e_scale, f_ext, fext_per_member, s
             raise ValueError("scen_idx must have one in-range entry per member")
         keep.append(si)
         d.scen_idx = si.ctypes.data
+    if source == "scenario":   # the same host array: the pipeline stages it once per chunk for both
+        if M:
+            _check_labels(int(si.max()), stats.groups, "scen_idx")
+        d.stat_group = d.scen_idx
+    elif source == "labels":
+        lab = np.ascontiguousarray(stat_group.cpu().numpy() if isinstance(stat_group, torch.Tensor) else stat_group,
+                                   dtype=np.int32)
+        if lab.shape != (M,):
+            raise ValueError("stat_group must have one label per member")
+        if M:
+            _check_labels(int(lab.max()), stats.groups, "stat_group")
+        keep.append(lab)
+        d.stat_group = lab.ctypes.data
     if e_scale is not None:
         keep.append(e_scale)
         d.e_scale = e_scale.ctypes.data
@@ -544,7 +622,7 @@ def _run_host(torch, E, gp, tp, dt, scen_idx, e_scale, f_ext, fext_per_member, s
         for g, f in enumerate(_detect_form_host(gp, state_in)):
             d.gas_form[g] = f
     res = out if out is not None else EnsembleResult()
-    res.spec, res.n_member = stats, M
+    res.spec, res.n_member, res.stat_group = stats, M, source
 
     def host_out(name, shape, dtype):
         cur = getattr(res, name)
@@ -569,8 +647,9 @@ def _run_host(torch, E, gp, tp, dt, scen_idx, e_scale, f_ext, fext_per_member, s
         d.state_out = host_out("state", (_abi.state_rows(G), M), npdt)
     hist_p = mom_p = None
     if stats is not None:
-        hist_p = host_out("hist", (n_t, stats.bins), np.int64)
-        mom_p = host_out("moments", (n_t, _abi.MOM_COUNT), np.float64)
+        lead = (stats.groups, n_t) if stats.groups else (n_t,)
+        hist_p = host_out("hist", lead + (stats.bins,), np.int64)
+        mom_p = host_out("moments", lead + (_abi.MOM_COUNT,), np.float64)
     own = workspace is None
     if own and chunk_members is None:
         chunk_members = auto_chunk_members(G, n_t, e_member=not e_scen, fext_member=fext_mode == _abi.FEXT_MEMBER, outputs=outputs,
@@ -588,7 +667,8 @@ def _run_host(torch, E, gp, tp, dt, scen_idx, e_scale, f_ext, fext_per_member, s
 
 def pinned_result(n_gas, n_t, n_member, outputs=("C", "RF", "T"), stats: Optional[HistSpec] = None, precision="f64",
                   return_state=True) -> EnsembleResult:
-    """Page-locked host output buffers for :func:`run_ensemble` ``out=`` (D2H at full PCIe speed)."""
+    """Page-locked host output buffers for :func:`run_ensemble` ``out=`` (D2H at full PCIe speed).  Grouped
+    statistics need ``stats.groups`` set to the group count here (``HistSpec(groups=S)`` for per-scenario ones)."""
     torch = _require_cuda()
     dt = torch.float64 if precision == "f64" else torch.float32
     pin = lambda *shape, dtype=dt: torch.empty(*shape, dtype=dtype, pin_memory=True).numpy()
@@ -606,6 +686,7 @@ def pinned_result(n_gas, n_t, n_member, outputs=("C", "RF", "T"), stats: Optiona
     if return_state:
         r.state = pin(_abi.state_rows(n_gas), n_member)
     if stats is not None:
-        r.hist = pin(n_t, stats.bins, dtype=torch.int64)
-        r.moments = pin(n_t, _abi.MOM_COUNT, dtype=torch.float64)
+        lead = (stats.groups, n_t) if stats.groups else (n_t,)
+        r.hist = pin(*lead, stats.bins, dtype=torch.int64)
+        r.moments = pin(*lead, _abi.MOM_COUNT, dtype=torch.float64)
     return r

@@ -31,6 +31,19 @@ int cuda_error(cudaError_t e, const char* what) {
 // ---- descriptor validation ---------------------------------------------------------------------
 static bool misaligned(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) != 0; }
 
+// the grouped-statistics fields (shared by the run / pass validation and the statistics-buffer entry points)
+int check_stat_groups(const ufair_desc* d) {
+  if (d->n_stat_groups < 0 || d->n_stat_groups > UFAIR_MAX_STAT_GROUPS)
+    return set_error(UFAIR_ERR_ARG, "n_stat_groups %d outside 0..%d", d->n_stat_groups, UFAIR_MAX_STAT_GROUPS);
+  if (d->n_stat_groups > 1 && !d->stat_group)
+    return set_error(UFAIR_ERR_ARG, "n_stat_groups %d needs stat_group labels (NULL)", d->n_stat_groups);
+  if (d->stat_group && !d->stats) return set_error(UFAIR_ERR_ARG, "stat_group set but stats == 0");
+  if ((int64_t)stat_groups(d) * d->hist_rows > (int64_t)INT32_MAX)
+    return set_error(UFAIR_ERR_ARG, "n_stat_groups %d x hist_rows %d rows do not fit in 32 bits", d->n_stat_groups,
+                     d->hist_rows);
+  return UFAIR_OK;
+}
+
 int validate_desc(const ufair_desc* d, size_t elem) {
   if (!d) return set_error(UFAIR_ERR_ARG, "descriptor is NULL");
   if (d->struct_size != sizeof(ufair_desc))
@@ -54,6 +67,8 @@ int validate_desc(const ufair_desc* d, size_t elem) {
     return set_error(UFAIR_ERR_ARG, "newton_iters %d outside 0..8", d->newton_iters);
   if (d->n_scen < 1) return set_error(UFAIR_ERR_ARG, "n_scen must be >= 1");
   if (!(d->dt > 0.0) || !(d->iirf_h > 0.0)) return set_error(UFAIR_ERR_ARG, "dt and iirf_h must be > 0");
+  const int rc = check_stat_groups(d);
+  if (rc != UFAIR_OK) return rc;
   if (d->n_member == 0 || d->n_t == 0) return UFAIR_OK;
   if (!d->emissions || !d->gas_params || !d->thermal_params)
     return set_error(UFAIR_ERR_ARG, "emissions / gas_params / thermal_params must not be NULL");
@@ -285,6 +300,151 @@ __global__ void __launch_bounds__(kStatsThreads)
   }
 }
 
+// ---- grouped statistics (stat_group != NULL): one histogram and one set of moments per member label ----------------
+// CTA (x = t * n_tiles + z, y = c) handles member slice c of row t for the groups [z NGT, z NGT + ngt) of tile z.  The
+// tiles of one row slice are neighbours on the fastest grid axis, so they run together and all but the first find the
+// slice in L2 (with one tile, T streams past L2 as in the pooled pass, which keeps the label slice -- shared by every
+// step of slice c, and those CTAs run together -- resident).  Traversal, binning rule, NaN handling, shuffle tree and
+// warp order are those of stats_pass_kernel, one reduction per group, so one group with every label 0 reproduces the
+// pooled pass bit for bit.  The NGT groups' per-thread partials stay in registers (unrolled predicated updates).
+// Counts go to a shared-memory histogram [ngt][bins] with the per-thread run-length merging keyed by (group, bin), or,
+// when NGT x bins exceeds kStatsSmemBins, straight to the CTA's own private rows with global atomics.  A label outside
+// [0, n_groups) is counted nowhere.
+template <typename Real, int NGT>
+__global__ void __launch_bounds__(kStatsThreads)
+    stats_pass_grouped_kernel(const Real* __restrict__ T, const int32_t* __restrict__ labels, long long ld,
+                              long long n_member, int n_groups, int n_tiles, int t0_row, int rows, int bins, Real lo,
+                              Real invw, int smem_hist, unsigned int* __restrict__ hp, double* mp) {
+  using M = Math<Real>;
+  extern __shared__ unsigned int sh[];
+  const int c = blockIdx.y, copies = gridDim.y;
+  const int t = (int)(blockIdx.x / (unsigned)n_tiles), z = (int)blockIdx.x - t * n_tiles;
+  const int g0 = z * NGT, ngt = min(NGT, n_groups - g0);
+  const long long m_lo = n_member * c / copies, m_hi = n_member * (c + 1) / copies;
+  const Real* src = T + (long long)t * ld + m_lo;
+  const int32_t* lab = labels + m_lo;
+  const size_t copy_rows = (size_t)n_groups * rows, gstride = (size_t)rows * bins;  // rows per copy; one group's rows
+  unsigned int* grow = hp + ((size_t)c * copy_rows + (size_t)g0 * rows + t0_row + t) * bins;  // group g0 + j: + j gstride
+  if (smem_hist) {
+    for (int i = threadIdx.x; i < ngt * bins; i += blockDim.x) sh[i] = 0u;
+    __syncthreads();
+  }
+  const int bins_m1 = bins - 1;
+  double sm[NGT], ss[NGT], mn[NGT], mx[NGT];
+#pragma unroll
+  for (int j = 0; j < NGT; ++j) {
+    sm[j] = 0.0;
+    ss[j] = 0.0;
+    mn[j] = INFINITY;
+    mx[j] = -INFINITY;
+  }
+  const long long span = m_hi - m_lo;
+  int last_g = -1, last_b = -1;
+  unsigned run = 0;
+  auto flush = [&]() {
+    if (run) atomicAdd(smem_hist ? sh + last_g * bins + last_b : grow + last_g * gstride + last_b, run);
+  };
+  auto take = [&](Real x, int label) {
+    const int gl = label - g0;
+    const int sel = (unsigned)gl < (unsigned)ngt ? gl : -1;
+    const double v = (double)x;
+#pragma unroll
+    for (int j = 0; j < NGT; ++j) {
+      if (sel == j) {
+        sm[j] += v;
+        ss[j] = fma(v, v, ss[j]);
+        mn[j] = fmin(mn[j], v);
+        mx[j] = fmax(mx[j], v);
+      }
+    }
+    const Real q = M::bin_x(x, lo, invw);
+    const int b = (sel >= 0 && q == q) ? max(0, min(bins_m1, M::floor_to_int(q))) : -1;
+    if (b != last_b || sel != last_g) {
+      flush();
+      last_g = sel;
+      last_b = b;
+      run = 0;
+    }
+    run += (b >= 0);
+  };
+  // one tile: stream T past L2 like the pooled pass; several: keep it for the sibling tiles
+  const bool keep = n_tiles > 1;
+  auto load = [&](long long i) { return keep ? __ldg(src + i) : __ldcs(src + i); };
+  long long k = threadIdx.x;
+  for (; k + 3 * kStatsThreads < span; k += 4 * kStatsThreads) {
+    const Real x0 = load(k), x1 = load(k + kStatsThreads), x2 = load(k + 2 * kStatsThreads), x3 = load(k + 3 * kStatsThreads);
+    const int l0 = __ldg(lab + k), l1 = __ldg(lab + k + kStatsThreads), l2 = __ldg(lab + k + 2 * kStatsThreads),
+              l3 = __ldg(lab + k + 3 * kStatsThreads);
+    take(x0, l0);
+    take(x1, l1);
+    take(x2, l2);
+    take(x3, l3);
+  }
+  for (; k < span; k += kStatsThreads) take(load(k), __ldg(lab + k));
+  flush();
+#pragma unroll
+  for (int j = 0; j < NGT; ++j) {
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) {
+      sm[j] += __shfl_xor_sync(0xffffffffu, sm[j], off);
+      ss[j] += __shfl_xor_sync(0xffffffffu, ss[j], off);
+      mn[j] = fmin(mn[j], __shfl_xor_sync(0xffffffffu, mn[j], off));
+      mx[j] = fmax(mx[j], __shfl_xor_sync(0xffffffffu, mx[j], off));
+    }
+  }
+  __shared__ double red[kStatsThreads / 32][NGT][4];
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  if (lane == 0) {
+#pragma unroll
+    for (int j = 0; j < NGT; ++j) {
+      red[w][j][0] = sm[j];
+      red[w][j][1] = ss[j];
+      red[w][j][2] = mn[j];
+      red[w][j][3] = mx[j];
+    }
+  }
+  __syncthreads();
+  if (smem_hist)
+    for (int i = threadIdx.x; i < ngt * bins; i += blockDim.x)
+      if (sh[i]) grow[(size_t)(i / bins) * gstride + i % bins] += sh[i];
+  if (threadIdx.x < ngt) {  // thread j folds group g0 + j: the pooled kernel's thread-0 fold, per group
+    const int j = threadIdx.x;
+    double* o = mp + ((size_t)c * copy_rows + (size_t)(g0 + j) * rows + t0_row + t) * UFAIR_MOM_COUNT;
+    double s1 = o[UFAIR_MOM_SUM], s2 = o[UFAIR_MOM_SUMSQ], lo_ = o[UFAIR_MOM_MIN], hi_ = o[UFAIR_MOM_MAX];
+    for (int k = 0; k < (int)(blockDim.x >> 5); ++k) {
+      s1 += red[k][j][0];
+      s2 += red[k][j][1];
+      lo_ = fmin(lo_, red[k][j][2]);
+      hi_ = fmax(hi_, red[k][j][3]);
+    }
+    o[UFAIR_MOM_SUM] = s1;
+    o[UFAIR_MOM_SUMSQ] = s2;
+    o[UFAIR_MOM_MIN] = lo_;
+    o[UFAIR_MOM_MAX] = hi_;
+  }
+}
+
+template <typename Real, int NGT> static int launch_grouped_pass(const ufair_desc* d, cudaStream_t stream) {
+  const int G = stat_groups(d), n_tiles = (G + NGT - 1) / NGT;
+  if (d->hist_copies > 65535) return set_error(UFAIR_ERR_ARG, "hist_copies %d > 65535", d->hist_copies);
+  if ((int64_t)d->n_t * n_tiles > (int64_t)INT32_MAX) return set_error(UFAIR_ERR_ARG, "n_t x group tiles too large");
+  const int smem_hist = (int64_t)NGT * d->hist_bins <= kStatsSmemBins ? 1 : 0;
+  const size_t smem = smem_hist ? (size_t)NGT * d->hist_bins * sizeof(unsigned int) : 0;
+  cudaError_t e = cudaSuccess;
+  if (smem > 48 * 1024)
+    e = cudaFuncSetAttribute(stats_pass_grouped_kernel<Real, NGT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return cuda_error(e, "cudaFuncSetAttribute(stats_pass_grouped_kernel)");
+  const Real lo = (Real)d->hist_lo;
+  const Real invw = (Real)((Real)d->hist_bins / ((Real)d->hist_hi - (Real)d->hist_lo));
+  stats_pass_grouped_kernel<Real, NGT><<<dim3((unsigned)(d->n_t * n_tiles), (unsigned)d->hist_copies), kStatsThreads, smem,
+                                         stream>>>((const Real*)d->out_T, d->stat_group, d->ld_member, d->n_member, G,
+                                                   n_tiles, d->hist_t0, d->hist_rows, d->hist_bins, lo, invw, smem_hist,
+                                                   d->hist_private, d->moments_private);
+  e = cudaGetLastError();
+  if (e != cudaSuccess) return cuda_error(e, "stats_pass_grouped_kernel launch");
+  return UFAIR_OK;
+}
+
 template <typename Real> static int dispatch_gases(const ufair_desc* d, const KArgs<Real>& a, cudaStream_t stream) {
   switch (d->n_gas) {
     case 1: return dispatch_mode<Real, 1>(d, a, stream);
@@ -377,6 +537,9 @@ template <typename Real> int run_stats_pass(const ufair_desc* d, cudaStream_t st
   if (rc != UFAIR_OK) return rc;
   if (!d->stats) return set_error(UFAIR_ERR_ARG, "ufair_stats_pass: descriptor has stats == 0");
   if (d->n_member == 0 || d->n_t == 0) return UFAIR_OK;
+  // up to four groups a tile of four: half the registers and predicated updates of a tile of eight
+  if (d->stat_group)
+    return stat_groups(d) <= 4 ? launch_grouped_pass<Real, 4>(d, stream) : launch_grouped_pass<Real, 8>(d, stream);
   const int smem_hist = d->hist_bins <= kStatsSmemBins ? 1 : 0;
   const size_t smem = smem_hist ? (size_t)d->hist_bins * sizeof(unsigned int) : 0;
   cudaError_t e = cudaSuccess;
@@ -517,7 +680,7 @@ static int check_stats_desc(const ufair_desc* d) {
   if (!d || d->struct_size != sizeof(ufair_desc)) return set_error(UFAIR_ERR_ARG, "bad descriptor");
   if (d->hist_bins < 1 || d->hist_copies < 1 || d->hist_rows < 1 || !d->hist_private || !d->moments_private)
     return set_error(UFAIR_ERR_ARG, "histogram spec/buffers incomplete");
-  return UFAIR_OK;
+  return check_stat_groups(d);
 }
 
 // ---- parameter preparation ------------------------------------------------------------------------
@@ -673,7 +836,7 @@ int ufair_kernel_variant(const ufair_desc* d, int32_t elem_size, uint32_t* form,
 int ufair_stats_reset(const ufair_desc* d, void* stream) {
   int rc = check_stats_desc(d);
   if (rc != UFAIR_OK) return rc;
-  const size_t rows = (size_t)d->hist_copies * d->hist_rows;
+  const size_t rows = (size_t)d->hist_copies * stat_groups(d) * d->hist_rows;
   stats_reset_kernel<<<592, 256, 0, (cudaStream_t)stream>>>(d->hist_private, rows * d->hist_bins, d->moments_private, rows);
   cudaError_t e = cudaGetLastError();
   return e == cudaSuccess ? UFAIR_OK : cuda_error(e, "stats_reset_kernel");
@@ -684,7 +847,7 @@ int ufair_stats_finalize(const ufair_desc* d, uint64_t* hist, double* moments, v
   if (rc != UFAIR_OK) return rc;
   if (!hist || !moments) return set_error(UFAIR_ERR_ARG, "hist / moments output is NULL");
   stats_finalize_kernel<<<592, 256, 0, (cudaStream_t)stream>>>(d->hist_private, d->moments_private, d->hist_copies,
-                                                               d->hist_rows, d->hist_bins,
+                                                               stat_groups(d) * d->hist_rows, d->hist_bins,
                                                                (unsigned long long*)hist, moments);
   cudaError_t e = cudaGetLastError();
   return e == cudaSuccess ? UFAIR_OK : cuda_error(e, "stats_finalize_kernel");
@@ -695,7 +858,7 @@ int ufair_stats_finalize_packed(const ufair_desc* d, double* sums, double* ext, 
   if (rc != UFAIR_OK) return rc;
   if (!sums || !ext) return set_error(UFAIR_ERR_ARG, "sums / ext output is NULL");
   stats_finalize_packed_kernel<<<592, 256, 0, (cudaStream_t)stream>>>(d->hist_private, d->moments_private, d->hist_copies,
-                                                                      d->hist_rows, d->hist_bins, sums, ext);
+                                                                      stat_groups(d) * d->hist_rows, d->hist_bins, sums, ext);
   cudaError_t e = cudaGetLastError();
   return e == cudaSuccess ? UFAIR_OK : cuda_error(e, "stats_finalize_packed_kernel");
 }

@@ -4,7 +4,8 @@
 // cudaMemcpy2DAsync per array, integrated by the fused kernel, and copied back D2H, on three
 // streams with two device staging buffers so copy-in(c+1), kernel(c) and copy-out(c-1) overlap.
 // Scenario-shared inputs go up once.  Statistics accumulate across chunks in the private
-// histogram copies and are finalised once at the end.
+// histogram copies and are finalised once at the end; statistics labels (stat_group) are staged per
+// chunk next to scen_idx, or not at all when they are scen_idx itself.
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <string.h>
@@ -50,7 +51,7 @@ struct DevBuf {
   }
 };
 
-enum { B_E, B_FEXT, B_GP, B_TP, B_SIN, B_SCEN, B_ESC, B_OC, B_ORF, B_OT, B_OA, B_OE, B_SOUT, B_COUNT };
+enum { B_E, B_FEXT, B_GP, B_TP, B_SIN, B_SCEN, B_GRP, B_ESC, B_OC, B_ORF, B_OT, B_OA, B_OE, B_SOUT, B_COUNT };
 
 struct Stage {
   DevBuf b[B_COUNT];
@@ -92,6 +93,7 @@ static int run_chunks(ufair_workspace* ws, const ufair_desc* h, const ufair_desc
   const bool e_member = h->e_mode == UFAIR_E_MEMBER;
   const bool fx_member = h->fext_mode == UFAIR_FEXT_MEMBER;
   const bool esc_on = !e_member && h->e_scale != nullptr;
+  const bool own_labels = h->stat_group != nullptr && h->stat_group != h->scen_idx;  // else scen_idx's staging serves
   // the workspace's chunk size, cut down for long runs so that the two staging sets stay within
   // kStagingBudget bytes (rows per member grow with the step count)
   const size_t gt = (size_t)G * n_t;
@@ -146,6 +148,10 @@ static int run_chunks(ufair_workspace* ws, const ufair_desc* h, const ufair_desc
       CK(cudaDeviceSynchronize(), "cudaDeviceSynchronize");
       CK(S.b[B_SCEN].reserve((size_t)chunk * sizeof(int32_t)), "cudaMalloc(scen_idx)");
     }
+    if (own_labels && S.b[B_GRP].cap < (size_t)chunk * sizeof(int32_t)) {
+      CK(cudaDeviceSynchronize(), "cudaDeviceSynchronize");
+      CK(S.b[B_GRP].reserve((size_t)chunk * sizeof(int32_t)), "cudaMalloc(stat_group)");
+    }
     // ---- H2D
     int rc = UFAIR_OK;
     if (e_member)
@@ -164,6 +170,9 @@ static int run_chunks(ufair_workspace* ws, const ufair_desc* h, const ufair_desc
     if (h->scen_idx)
       CK(cudaMemcpyAsync(S.b[B_SCEN].p, h->scen_idx + c0, (size_t)cm * sizeof(int32_t), cudaMemcpyHostToDevice, ws->s_in),
          "H2D scen_idx");
+    if (own_labels)
+      CK(cudaMemcpyAsync(S.b[B_GRP].p, h->stat_group + c0, (size_t)cm * sizeof(int32_t), cudaMemcpyHostToDevice, ws->s_in),
+         "H2D stat_group");
     CK(cudaEventRecord(S.in_done, ws->s_in), "cudaEventRecord");
     // ---- kernel
     CK(cudaStreamWaitEvent(ws->s_run, S.in_done, 0), "cudaStreamWaitEvent");
@@ -177,6 +186,7 @@ static int run_chunks(ufair_workspace* ws, const ufair_desc* h, const ufair_desc
     k.state_in = h->state_in ? S.b[B_SIN].p : nullptr;
     k.e_scale = esc_on ? S.b[B_ESC].p : nullptr;
     k.scen_idx = h->scen_idx ? (const int32_t*)S.b[B_SCEN].p : nullptr;
+    k.stat_group = own_labels ? (const int32_t*)S.b[B_GRP].p : h->stat_group ? k.scen_idx : nullptr;
     k.out_C = S.b[B_OC].p;
     k.out_RF = S.b[B_ORF].p;
     k.out_T = S.b[B_OT].p;
@@ -227,6 +237,8 @@ template <typename Real> static int run_host(ufair_workspace* ws, const ufair_de
   if (h->n_gas < 1 || h->n_gas > UFAIR_MAX_GAS || h->n_t < 0 || h->n_member < 0 || h->ld_member < h->n_member)
     return set_error(UFAIR_ERR_ARG, "bad dimensions");
   if (h->stats && (!hist || !moments)) return set_error(UFAIR_ERR_ARG, "stats requested but hist/moments NULL");
+  const int rc0 = check_stat_groups(h);
+  if (rc0 != UFAIR_OK) return rc0;
   if (h->n_member == 0 || h->n_t == 0) return UFAIR_OK;
   if (!h->emissions || !h->gas_params || !h->thermal_params)
     return set_error(UFAIR_ERR_ARG, "emissions / gas_params / thermal_params must not be NULL");
@@ -237,6 +249,7 @@ template <typename Real> static int run_host(ufair_workspace* ws, const ufair_de
 
   const size_t es = sizeof(Real);
   const int G = h->n_gas, n_t = h->n_t;
+  const size_t out_rows = (size_t)stat_groups(h) * n_t;  // statistics rows: [groups][n_t]
   ufair_desc d = *h;
   if (h->e_mode != UFAIR_E_MEMBER) {  // scenario-shared inputs go up once
     const size_t nb = (size_t)G * n_t * h->n_scen * es;
@@ -262,11 +275,11 @@ template <typename Real> static int run_host(ufair_workspace* ws, const ufair_de
     d.hist_copies = h->hist_copies > 0 ? h->hist_copies : 16;
     d.hist_t0 = 0;
     d.hist_rows = n_t;
-    const size_t rows = (size_t)d.hist_copies * n_t;
+    const size_t rows = (size_t)d.hist_copies * out_rows;
     CKS(ws->hist_private.reserve(rows * h->hist_bins * sizeof(uint32_t)), "cudaMalloc(hist_private)");
     CKS(ws->mom_private.reserve(rows * UFAIR_MOM_COUNT * sizeof(double)), "cudaMalloc(mom_private)");
-    CKS(ws->hist_out.reserve((size_t)n_t * h->hist_bins * sizeof(uint64_t)), "cudaMalloc(hist)");
-    CKS(ws->mom_out.reserve((size_t)n_t * UFAIR_MOM_COUNT * sizeof(double)), "cudaMalloc(moments)");
+    CKS(ws->hist_out.reserve(out_rows * h->hist_bins * sizeof(uint64_t)), "cudaMalloc(hist)");
+    CKS(ws->mom_out.reserve(out_rows * UFAIR_MOM_COUNT * sizeof(double)), "cudaMalloc(moments)");
     d.hist_private = (uint32_t*)ws->hist_private.p;
     d.moments_private = (double*)ws->mom_private.p;
     int rc = ufair_stats_reset(&d, ws->s_run);
@@ -285,8 +298,8 @@ template <typename Real> static int run_host(ufair_workspace* ws, const ufair_de
   if (rc == UFAIR_OK && h->stats) {
     rc = ufair_stats_finalize(&d, (uint64_t*)ws->hist_out.p, (double*)ws->mom_out.p, ws->s_run);
     if (rc == UFAIR_OK) {
-      cudaMemcpyAsync(hist, ws->hist_out.p, (size_t)n_t * h->hist_bins * sizeof(uint64_t), cudaMemcpyDeviceToHost, ws->s_run);
-      cudaMemcpyAsync(moments, ws->mom_out.p, (size_t)n_t * UFAIR_MOM_COUNT * sizeof(double), cudaMemcpyDeviceToHost, ws->s_run);
+      cudaMemcpyAsync(hist, ws->hist_out.p, out_rows * h->hist_bins * sizeof(uint64_t), cudaMemcpyDeviceToHost, ws->s_run);
+      cudaMemcpyAsync(moments, ws->mom_out.p, out_rows * UFAIR_MOM_COUNT * sizeof(double), cudaMemcpyDeviceToHost, ws->s_run);
     }
   }
   const cudaError_t e1 = cudaStreamSynchronize(ws->s_in), e2 = cudaStreamSynchronize(ws->s_run),

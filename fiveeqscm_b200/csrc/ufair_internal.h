@@ -8,6 +8,9 @@ namespace ufair {
 int set_error(int code, const char* fmt, ...);
 int cuda_error(cudaError_t e, const char* what);
 int validate_desc(const ufair_desc* d, size_t elem);
+int check_stat_groups(const ufair_desc* d);
+// statistics groups G: every statistics buffer holds G x hist_rows rows (include/ufair.h)
+inline int stat_groups(const ufair_desc* d) { return d->n_stat_groups > 1 ? d->n_stat_groups : 1; }
 template <typename Real> int run_device(const ufair_desc* d, cudaStream_t stream);
 template <typename Real> int run_stats_pass(const ufair_desc* d, cudaStream_t stream);
 }  // namespace ufair

@@ -20,7 +20,8 @@ def shard_bounds(n_member: int, world_size: int, rank: int, align: int = 128):
 
 
 def allreduce_stats(hist, moments, group=None):
-    """In-place all-reduce of (hist int64 [n_t][bins], moments float64 [n_t][4]) across ranks, as TWO
+    """In-place all-reduce of (hist int64 [..., n_t][bins], moments float64 [..., n_t][4]; leading axes are
+    statistics groups) across ranks, as TWO
     collectives: one SUM over [counts as float64 | sum T | sum T^2] (integer counts below 2^53 add
     exactly in any order, so the reduced histogram is bitwise independent of the GPU count) and one
     MAX over [max T, -min T].  Generic torch version (any backend, CPU or CUDA tensors);
@@ -29,15 +30,15 @@ def allreduce_stats(hist, moments, group=None):
     import torch.distributed as dist
     if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) == 1:
         return hist, moments
-    bins = hist.shape[1]
-    sums = torch.cat([hist.to(torch.float64), moments[:, 0:2]], dim=1).contiguous()
-    ext = torch.stack([moments[:, 3], -moments[:, 2]], dim=1).contiguous()
+    bins = hist.shape[-1]
+    h2, m2 = hist.reshape(-1, bins), moments.reshape(-1, moments.shape[-1])
+    sums = torch.cat([h2.to(torch.float64), m2[:, 0:2]], dim=1).contiguous()
+    ext = torch.stack([m2[:, 3], -m2[:, 2]], dim=1).contiguous()
     dist.all_reduce(sums, op=dist.ReduceOp.SUM, group=group)
     dist.all_reduce(ext, op=dist.ReduceOp.MAX, group=group)
-    hist.copy_(sums[:, :bins].to(torch.int64))
-    moments[:, 0:2] = sums[:, bins:]
-    moments[:, 3] = ext[:, 0]
-    moments[:, 2] = -ext[:, 1]
+    hist.copy_(sums[:, :bins].to(torch.int64).reshape(hist.shape))
+    red = torch.stack([sums[:, bins], sums[:, bins + 1], -ext[:, 1], ext[:, 0]], dim=1)   # sum, sumsq, min, max
+    moments.copy_(red.reshape(moments.shape))
     return hist, moments
 
 
@@ -55,8 +56,9 @@ class StatsReducer:
         self.plan, self.group = plan, group
         self.world = dist.get_world_size(group) if (dist.is_available() and dist.is_initialized()) else 1
         self._k = 0
+        self._rows = plan.n_t * max(1, plan.stats.groups) if plan.stats is not None else 0   # [groups][n_t] rows
         if self.world > 1 and plan.stats is not None:
-            rows, bins = plan.n_t, plan.stats.bins
+            rows, bins = self._rows, plan.stats.bins
             dev = plan.device
             self._sums = [torch.empty(rows, bins + 2, dtype=torch.float64, device=dev) for _ in range(depth)]
             self._ext = [torch.empty(rows, 2, dtype=torch.float64, device=dev) for _ in range(depth)]
@@ -90,7 +92,7 @@ class StatsReducer:
             self._stream.wait_event(self._ready[k])
             dist.all_reduce(self._sums[k], op=dist.ReduceOp.SUM, group=self.group)
             dist.all_reduce(self._ext[k], op=dist.ReduceOp.MAX, group=self.group)
-            _abi.check(L.ufair_stats_unpack(self._sums[k].data_ptr(), self._ext[k].data_ptr(), plan.n_t, plan.stats.bins,
+            _abi.check(L.ufair_stats_unpack(self._sums[k].data_ptr(), self._ext[k].data_ptr(), self._rows, plan.stats.bins,
                                             r.hist.data_ptr(), r.moments.data_ptr(), self._stream.cuda_stream))
             ev = torch.cuda.Event()
             ev.record(self._stream)

@@ -59,22 +59,37 @@ def scenarios_from_csv(path, gases: Sequence[str] = GASES, **kw):
     return scenarios_from_frame(pd.read_csv(path), gases, **kw)
 
 
-def summary_frame(result, years, pcts: Sequence[float] = (5.0, 17.0, 50.0, 83.0, 95.0)):
+def summary_frame(result, years, pcts: Sequence[float] = (5.0, 17.0, 50.0, 83.0, 95.0), group_names=None):
     """Per-year ensemble summary of temperature from a result computed with ``stats=HistSpec(...)``
-    (after the cross-GPU all-reduce, if any): mean, std, min, max and percentiles off the histogram."""
+    (after the cross-GPU all-reduce, if any): mean, std, min, max and percentiles off the histogram.
+    Grouped statistics (``stat_group=``) give a long frame, one block of years per group, led by a
+    ``scenario`` column (grouped by scenario) or a ``group`` column (by labels) holding ``group_names[g]``
+    (default: the group index).  A group's member count is its histogram row sum."""
     import pandas as pd
     if result.hist is None or result.moments is None or result.spec is None:
         raise ValueError("summary_frame needs a result computed with stats=HistSpec(...)")
     mom = _stats._np(result.moments)
     hist = _stats._np(result.hist)
-    n = hist.sum(axis=1)
-    if not np.all(n == n[0]):
+    grouped = hist.ndim == 3
+    if not grouped:
+        hist, mom = hist[None], mom[None]
+    n = hist.sum(axis=-1)                                                                    # [groups][n_t]
+    if not np.all(n == n[:, :1]):
         raise ValueError("histogram rows count different numbers of members")
-    mean, std = _stats.mean_std(mom, int(n[0]))
+    with np.errstate(invalid="ignore", divide="ignore"):   # an empty group has no mean
+        mean, std = _stats.mean_std(mom, n)
     p = _stats.percentiles(hist, result.spec.lo, result.spec.hi, pcts)
-    data = {"year": np.asarray(years), "members": n, "T_mean": mean, "T_std": std, "T_min": mom[:, 2], "T_max": mom[:, 3]}
+    n_grp, n_t = n.shape
+    data = {"year": np.tile(np.asarray(years), n_grp), "members": n.ravel(), "T_mean": mean.ravel(),
+            "T_std": std.ravel(), "T_min": mom[..., 2].ravel(), "T_max": mom[..., 3].ravel()}
     for j, q in enumerate(pcts):
-        data[f"T_p{q:g}"] = p[:, j]
+        data[f"T_p{q:g}"] = p[..., j].ravel()
+    if grouped:
+        names = list(range(n_grp)) if group_names is None else list(group_names)
+        if len(names) != n_grp:
+            raise ValueError(f"group_names has {len(names)} entries for {n_grp} groups")
+        col = "scenario" if getattr(result, "stat_group", None) == "scenario" else "group"
+        data = {col: np.repeat(np.asarray(names, dtype=object), n_t), **data}
     return pd.DataFrame(data)
 
 

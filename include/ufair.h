@@ -40,10 +40,11 @@
 extern "C" {
 #endif
 
-#define UFAIR_ABI_VERSION 2
+#define UFAIR_ABI_VERSION 3
 
 #define UFAIR_MAX_GAS 4
 #define UFAIR_N_POOL 4
+#define UFAIR_MAX_STAT_GROUPS 256 /* cap of ufair_desc.n_stat_groups */
 
 /* rows of gas_params[n_gas][UFAIR_GP_COUNT][ld_member] */
 enum {
@@ -153,7 +154,26 @@ typedef struct ufair_desc {
    * slice c of every row into copy c of hist_private / moments_private (counts; sum, sum of
    * squares, min, max) in a fixed order.  ufair_stats_reset() initialises the private buffers
    * once; they may keep accumulating over several run + pass pairs (member chunks);
-   * ufair_stats_finalize() folds the copies. */
+   * ufair_stats_finalize() folds the copies.
+   *
+   * Grouped statistics (n_stat_groups, stat_group at the end of the struct): with stat_group != NULL
+   * every member m carries a label, and the pass builds one histogram and one set of moments per
+   * group.  Let G = max(1, n_stat_groups):
+   *   0 <= stat_group[m] < G  member m is counted in group stat_group[m];
+   *   stat_group[m] < 0       member m is counted nowhere (neither histogram nor moments);
+   *   stat_group[m] >= G      not counted either (the library does not check labels: that would
+   *                           need a synchronise; the Python layer rejects them).
+   * stat_group may be the scen_idx pointer itself: per-scenario statistics.  Group g, step t lives in
+   * row g * hist_rows + hist_t0 + t, so every statistics buffer has G times the rows:
+   *   hist_private[hist_copies][G * hist_rows][hist_bins], moments_private[hist_copies][G * hist_rows][4],
+   *   and the finalised hist / moments (and the packed sums / ext) [G][hist_rows][..].
+   * With stat_group == NULL (n_stat_groups 0 or 1) the pass is the pooled one, unchanged.
+   * The binning rule and the NaN handling are those of the pooled pass; counts are exact and the
+   * moments deterministic (fixed order, no floating-point atomics); one group with every label 0
+   * gives the pooled pass's histogram and moments bit for bit.  Memory: the private histogram is
+   * G times the pooled one (16 copies x 4 groups x 736 steps x 1024 bins x 4 B = 193 MB); fewer
+   * hist_copies reduce it.  Measured on a B200 (1000 W), T of 1.25e6 members x 736 steps f64: pooled 1.37 ms,
+   * 4 scenario groups 4.59 ms, 16 random groups 23.7 ms (DESIGN.md 4.2). */
   int32_t hist_bins;
   int32_t hist_copies;
   double hist_lo, hist_hi;
@@ -174,6 +194,11 @@ typedef struct ufair_desc {
    * the emission rate of every gas: diagnosed where the bit is set, the input otherwise. */
   int32_t conc_driven;
   void* out_E; /* [n_gas][n_t][ld_member] */
+
+  /* ---- grouped statistics (see the statistics block above; stats == 1 only) ---- */
+  int32_t n_stat_groups;      /* 0 or 1 = pooled; up to UFAIR_MAX_STAT_GROUPS */
+  int32_t reserved1;
+  const int32_t* stat_group;  /* [n_member] group labels, or NULL */
 } ufair_desc;
 
 /* ---- version / errors ---- */
@@ -214,8 +239,9 @@ int ufair_stats_reset(const ufair_desc* d, void* stream);
  * (d->out_T; same descriptor, same stream).  One call per ufair_run_* call when stats == 1. */
 int ufair_stats_pass_f64(const ufair_desc* d, void* stream);
 int ufair_stats_pass_f32(const ufair_desc* d, void* stream);
-/* Fold the private copies: hist[hist_rows][hist_bins] (uint64 counts) and
- * moments[hist_rows][UFAIR_MOM_COUNT] (sum, sumsq, min, max as doubles). */
+/* Fold the private copies: hist[G][hist_rows][hist_bins] (uint64 counts) and
+ * moments[G][hist_rows][UFAIR_MOM_COUNT] (sum, sumsq, min, max as doubles); G = max(1, n_stat_groups).
+ * Here and in ufair_stats_finalize_packed, "hist_rows" below stands for G * hist_rows. */
 int ufair_stats_finalize(const ufair_desc* d, uint64_t* hist, double* moments, void* stream);
 
 /* The same fold in the layout the cross-GPU reduction uses -- two buffers, two collectives:
