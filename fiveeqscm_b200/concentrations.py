@@ -18,6 +18,7 @@ from __future__ import annotations
 
 import ctypes as C
 import dataclasses
+import math
 from dataclasses import dataclass
 from typing import Optional, Sequence
 
@@ -54,6 +55,10 @@ class HistSpec:
     bins: int = 1024
     copies: int = 16  # privatised copies the kernel spreads its atomics over
     groups: int = 0   # 0 = pooled; with stat_group="scenario", 0 means one group per scenario
+
+    def lead_shape(self, n_t):
+        """Leading axes of every statistics array (results and private copies): [groups][n_t], or [n_t] pooled."""
+        return (self.groups, n_t) if self.groups else (n_t,)
 
 
 @dataclass
@@ -248,8 +253,7 @@ def auto_chunk_members(n_gas, n_t, *, e_member, fext_member, outputs, return_sta
     gt = n_gas * n_t
     up = (gt if e_member else 0) + (n_t if fext_member else 0) + n_gas * _abi.GP_COUNT + _abi.TP_COUNT + \
         (n_gas if e_scale else 0) + (_abi.state_rows(n_gas) if state_in else 0)
-    down = sum(gt for o in ("C", "RF", "alpha", "E") if o in outputs) + (n_t if "T" in outputs else 0) + \
-        (_abi.state_rows(n_gas) if return_state else 0)
+    down = sum(math.prod(shape) for _, _, shape, _ in _result_layout(n_gas, n_t, 1, outputs, return_state, None))
     link_ns = max(up, down) * es / 50.0                       # ns per member at 50 GB/s, the busier direction
     kernel_ns = gt * (0.010 if precision == "f64" else 0.0035)   # ns per member: 27 ms / 9 ms per 1.25e6 x 736 x 3 on B200
     return 16384 if link_ns >= kernel_ns else 131072
@@ -314,18 +318,17 @@ def run_ensemble(emissions, gas_params, thermal_params, *, dt=1.0, scen_idx=None
     torch = _require_cuda()
     if precision not in ("f64", "f32"):
         raise ValueError("precision must be 'f64' or 'f32'")
-    on_device = isinstance(emissions, torch.Tensor) and emissions.is_cuda
-    if on_device:
-        return _run_device(torch, emissions, gas_params, thermal_params, dt, scen_idx, e_scale, f_ext,
-                           fext_per_member, state_in, alpha_mode, newton_iters, iirf_max, iirf_h, t_mode,
-                           _with_E(outputs, conc_driven), stats, precision, return_state, gas_form, conc_driven,
-                           stat_group)
-    return _run_host(torch, emissions, gas_params, thermal_params, dt, scen_idx, e_scale, f_ext, fext_per_member,
-                     state_in, alpha_mode, newton_iters, iirf_max, iirf_h, t_mode, _with_E(outputs, conc_driven), stats,
-                     precision, return_state, chunk_members, workspace, out, gas_form, conc_driven, stat_group)
+    kw = dict(dt=dt, scen_idx=scen_idx, e_scale=e_scale, f_ext=f_ext, fext_per_member=fext_per_member, state_in=state_in,
+              alpha_mode=alpha_mode, newton_iters=newton_iters, iirf_max=iirf_max, iirf_h=iirf_h, t_mode=t_mode,
+              outputs=outputs, stats=stats, precision=precision, return_state=return_state, gas_form=gas_form,
+              conc_driven=conc_driven, stat_group=stat_group)
+    if isinstance(emissions, torch.Tensor) and emissions.is_cuda:
+        return DevicePlan(emissions, gas_params, thermal_params, **kw).run()
+    return _run_host(emissions, gas_params, thermal_params, chunk_members=chunk_members, workspace=workspace, out=out,
+                     **kw)
 
 
-def _shapes(E_shape, gp_shape, tp_shape, scen_idx, fext_shape, fext_per_member, e_scale_shape=None):
+def _shapes(E_shape, gp_shape, tp_shape, scen_idx, fext_shape, fext_per_member, e_scale_shape=None, state_shape=None):
     if len(E_shape) != 3 or len(gp_shape) != 3 or len(tp_shape) != 2:
         raise ValueError("emissions must be [G][n_t][M|S], gas_params [G][17][M], thermal_params [4][M]")
     G, n_t = E_shape[0], E_shape[1]
@@ -345,6 +348,8 @@ def _shapes(E_shape, gp_shape, tp_shape, scen_idx, fext_shape, fext_per_member, 
             raise ValueError("e_scale applies to scenario-shared emissions only")
         if tuple(e_scale_shape) != (G, M):
             raise ValueError(f"e_scale must be [G][M] = ({G}, {M}), got {tuple(e_scale_shape)}")
+    if state_shape is not None and tuple(state_shape) != (_abi.state_rows(G), M):
+        raise ValueError("state_in must be [5G+3][M]")
     fext_mode = _abi.FEXT_NONE
     if fext_shape is not None:
         if fext_per_member:
@@ -364,133 +369,169 @@ def _shapes(E_shape, gp_shape, tp_shape, scen_idx, fext_shape, fext_per_member, 
     return G, n_t, M, e_scen, n_scen, fext_mode
 
 
+def _result_layout(n_gas, n_t, M, outputs, return_state, stats: Optional[HistSpec]):
+    """(result field, descriptor field, shape, dtype) of every array a run returns.  dtype "real" is the run's
+    precision; hist and moments have no descriptor field (ufair_stats_finalize and ufair_run_host_* take them)."""
+    layout = [(o, "out_" + o, (n_t, M) if o == "T" else (n_gas, n_t, M), "real") for o in _OUT if o in outputs]
+    if return_state:
+        layout.append(("state", "state_out", (_abi.state_rows(n_gas), M), "real"))
+    if stats is not None:
+        lead = stats.lead_shape(n_t)
+        layout += [("hist", None, lead + (stats.bins,), "int64"), ("moments", None, lead + (_abi.MOM_COUNT,), "float64")]
+    return layout
+
+
+def _numpy(x):
+    return x.detach().cpu().numpy() if isinstance(x, _torch().Tensor) else x
+
+
+class _DeviceArrays:
+    """Places a run's arrays on `device`: tensors of the run dtype; member rows padded to a 16-byte pitch (ld) and
+    16-byte aligned, as the integrator's bulk loads need."""
+
+    def __init__(self, torch, device, dtype):
+        self.torch, self.device, self.dtype = torch, device, dtype
+
+    def ld(self, M):
+        return _round_up(max(M, 1), 16 // self.dtype.itemsize)
+
+    def array(self, x):
+        return self.torch.as_tensor(x, device=self.device).to(self.dtype).contiguous()
+
+    def rows(self, x, ld):
+        if x.shape[-1] != ld:
+            x = self.torch.nn.functional.pad(x, (0, ld - x.shape[-1]))
+        return x.clone() if x.data_ptr() % 16 else x
+
+    def labels(self, x):
+        return self.torch.as_tensor(x, device=self.device).to(self.torch.int32).contiguous().reshape(-1)
+
+    @staticmethod
+    def ptr(x):
+        return x.data_ptr()
+
+
+class _HostArrays:
+    """Places a run's arrays for the host pipeline: contiguous numpy arrays of the run dtype, row pitch ld = M."""
+
+    def __init__(self, dtype):
+        self.dtype = dtype
+
+    @staticmethod
+    def ld(M):
+        return M
+
+    def array(self, x):
+        return np.ascontiguousarray(_numpy(x), dtype=self.dtype)
+
+    @staticmethod
+    def rows(x, ld):
+        return x
+
+    @staticmethod
+    def labels(x):
+        return np.ascontiguousarray(_numpy(x), dtype=np.int32).reshape(-1)
+
+    @staticmethod
+    def ptr(x):
+        return x.ctypes.data
+
+
+def _prepare(arrays, E, gp, tp, *, dt=1.0, scen_idx=None, e_scale=None, f_ext=None, fext_per_member=False,
+             state_in=None, alpha_mode="exp", newton_iters=0, iirf_max=None, iirf_h=100.0, t_mode="mid",
+             outputs=("C", "RF", "T"), stats=None, gas_form="auto", conc_driven=None, stat_group=None):
+    """Checks a run's inputs (keywords of :func:`run_ensemble`) and places them with `arrays` (:class:`_DeviceArrays`
+    or :class:`_HostArrays`).  Returns (descriptor with every input wired, the placed arrays by descriptor field,
+    the outputs with "E" added for concentration-driven runs, the HistSpec with its group count settled, the label
+    source of :func:`_resolve_groups`).  ``gas_form="auto"`` is left to the caller: it scans the placed arrays."""
+    if isinstance(gas_form, str) and gas_form != "auto":
+        raise ValueError("gas_form must be 'auto', None or one entry per gas")
+    E, gp, tp, e_scale, f_ext, state_in = (None if x is None else arrays.array(x)
+                                           for x in (E, gp, tp, e_scale, f_ext, state_in))
+    shape = lambda x: None if x is None else tuple(x.shape)
+    G, n_t, M, e_scen, n_scen, fext_mode = _shapes(E.shape, gp.shape, tp.shape, scen_idx, shape(f_ext), fext_per_member,
+                                                   shape(e_scale), shape(state_in))
+    stats, source = _resolve_groups(stats, stat_group, scen_idx is not None, n_scen)
+    outputs = _with_E(outputs, conc_driven)
+    ld = arrays.ld(M)
+    d = _build_desc(G, n_t, M, ld, n_scen, e_scen, fext_mode, alpha_mode, newton_iters, t_mode, outputs, dt, iirf_h,
+                    iirf_max, stats, gas_form, conc_driven)
+    placed = dict(emissions=E if e_scen else arrays.rows(E, ld), gas_params=arrays.rows(gp, ld),
+                  thermal_params=arrays.rows(tp, ld))
+    if scen_idx is not None:
+        si = placed["scen_idx"] = arrays.labels(scen_idx)
+        if si.shape[0] != M:
+            raise ValueError("scen_idx must have one entry per member")
+        if M and (int(si.min()) < 0 or int(si.max()) >= n_scen):
+            raise ValueError("scen_idx out of range")
+    if source is not None:   # "scenario": the labels ARE scen_idx (no copy; they follow in-place updates of it)
+        lab = placed["stat_group"] = placed["scen_idx"] if source == "scenario" else arrays.labels(stat_group)
+        if lab.shape[0] != M:
+            raise ValueError("stat_group must have one label per member")
+        if M:
+            _check_labels(int(lab.max()), stats.groups, "scen_idx" if source == "scenario" else "stat_group")
+    if e_scale is not None:
+        placed["e_scale"] = arrays.rows(e_scale, ld)
+    if f_ext is not None:
+        if fext_per_member:
+            f_ext = arrays.rows(f_ext, ld)
+        elif math.prod(f_ext.shape) == n_t and n_scen > 1:   # [n_t] -> [n_t][S]: the one column repeated
+            f_ext = arrays.array(f_ext.reshape(n_t, 1)[:, [0] * n_scen])
+        placed["f_ext"] = f_ext
+    if state_in is not None:
+        placed["state_in"] = arrays.rows(state_in, ld)
+    for field, x in placed.items():
+        setattr(d, field, arrays.ptr(x))
+    return d, placed, outputs, stats, source
+
+
 class DevicePlan:
     """A prepared device-resident run: descriptor + buffers.  ``run_ensemble`` on CUDA tensors is
     ``plan = DevicePlan(...); plan.reset_stats(); plan.launch(); plan.finalize_stats()``; callers
-    that repeat the same run (benchmarks, time-chunked drivers) keep the plan and re-launch it."""
+    that repeat the same run (benchmarks, time-chunked drivers) keep the plan and re-launch it.
+    Keywords are those of :func:`run_ensemble` but the host pipeline's ``chunk_members``, ``workspace`` and ``out``."""
 
-    def __init__(self, E, gp, tp, *, dt=1.0, scen_idx=None, e_scale=None, f_ext=None, fext_per_member=False,
-                 state_in=None, alpha_mode="exp", newton_iters=0, iirf_max=None, iirf_h=100.0, t_mode="mid",
-                 outputs=("C", "RF", "T"), stats=None, precision="f64", return_state=True, gas_form="auto",
-                 conc_driven=None, stat_group=None):
+    def __init__(self, E, gp, tp, *, precision="f64", return_state=True, gas_form="auto", **inputs):
         torch = _require_cuda()
-        outputs = _with_E(outputs, conc_driven)
         self._L = _abi.lib()
         dtype = torch.float64 if precision == "f64" else torch.float32
-        es = 8 if precision == "f64" else 4
         dev = E.device
-        fshape = None if f_ext is None else tuple(f_ext.shape)
-        G, n_t, M, e_scen, n_scen, fext_mode = _shapes(tuple(E.shape), tuple(gp.shape), tuple(tp.shape), scen_idx,
-                                                       fshape, fext_per_member,
-                                                       None if e_scale is None else tuple(e_scale.shape))
-        stats, source = _resolve_groups(stats, stat_group, scen_idx is not None, n_scen)
+        d, placed, outputs, stats, source = _prepare(_DeviceArrays(torch, dev, dtype), E, gp, tp, gas_form=gas_form,
+                                                     **inputs)
+        G, n_t, M, ld = d.n_gas, d.n_t, d.n_member, d.ld_member
         self.device, self.precision, self.stats = dev, precision, stats
         self.n_gas, self.n_t, self.n_member = G, n_t, M
-        self.scen_idx = None
-        ld = _round_up(max(M, 1), 16 // es)
-
-        def member_rows(x, name):  # [..][M] -> contiguous [..][ld] of the run dtype, 16-byte aligned rows
-            x = torch.as_tensor(x, device=dev)
-            if x.dtype != dtype:
-                x = x.to(dtype)
-            if x.shape[-1] != M:
-                raise ValueError(f"{name}: last axis must be the member axis ({M})")
-            if ld != M:
-                x = torch.nn.functional.pad(x, (0, ld - M))
-            x = x.contiguous()
-            if x.data_ptr() % 16:
-                x = x.clone()
-            return x
-
-        def shared(x):
-            return torch.as_tensor(x, device=dev).to(dtype).contiguous()
-
-        keep = []
-        E_d = shared(E) if e_scen else member_rows(E, "emissions")
-        gp_d, tp_d = member_rows(gp, "gas_params"), member_rows(tp, "thermal_params")
-        keep += [E_d, gp_d, tp_d]
-        d = _build_desc(G, n_t, M, ld, n_scen, e_scen, fext_mode, alpha_mode, newton_iters, t_mode, outputs, dt,
-                        iirf_h, iirf_max, stats, gas_form, conc_driven)
-        d.emissions, d.gas_params, d.thermal_params = E_d.data_ptr(), gp_d.data_ptr(), tp_d.data_ptr()
-        if scen_idx is not None:
-            si = torch.as_tensor(scen_idx, device=dev).to(torch.int32).contiguous()
-            if si.numel() != M:
-                raise ValueError("scen_idx must have one entry per member")
-            if M and (int(si.min()) < 0 or int(si.max()) >= n_scen):
-                raise ValueError("scen_idx out of range")
-            keep.append(si)
-            d.scen_idx = si.data_ptr()
-            self.scen_idx = si    # the plan's own copy: callers that re-launch may overwrite it in place
-        self.stat_group = None
-        if source == "scenario":   # the labels ARE scen_idx: no copy, and they follow in-place updates of it
-            if M:
-                _check_labels(int(si.max()), stats.groups, "scen_idx")
-            d.stat_group = d.scen_idx
-            self.stat_group = si
-        elif source == "labels":
-            lab = torch.as_tensor(stat_group, device=dev).to(torch.int32).contiguous()
-            if lab.numel() != M:
-                raise ValueError("stat_group must have one label per member")
-            if M:
-                _check_labels(int(lab.max()), stats.groups, "stat_group")
-            keep.append(lab)
-            d.stat_group = lab.data_ptr()
-            self.stat_group = lab
-        if e_scale is not None:
-            esd = member_rows(e_scale, "e_scale")
-            keep.append(esd)
-            d.e_scale = esd.data_ptr()
-        if f_ext is not None:
-            fx = member_rows(f_ext, "f_ext") if fext_per_member else shared(f_ext)
-            if not fext_per_member and fx.numel() == n_t and n_scen > 1:
-                fx = fx.reshape(n_t, 1).expand(n_t, n_scen).contiguous()
-            keep.append(fx)
-            d.f_ext = fx.data_ptr()
-        if state_in is not None:
-            sin_ = member_rows(state_in, "state_in")
-            if sin_.shape[0] != _abi.state_rows(G):
-                raise ValueError("state_in must be [5G+3][M]")
-            keep.append(sin_)
-            d.state_in = sin_.data_ptr()
+        self.scen_idx = placed.get("scen_idx")   # the plan's own copy: callers that re-launch may overwrite it in place
+        self.stat_group = placed.get("stat_group")
 
         res = EnsembleResult(spec=stats, n_member=M, stat_group=source)
-        new = lambda *shape: torch.empty(*shape, dtype=dtype, device=dev)
-        if "C" in outputs:
-            buf = new(G, n_t, ld); d.out_C = buf.data_ptr(); res.C = buf[..., :M]
-        if "RF" in outputs:
-            buf = new(G, n_t, ld); d.out_RF = buf.data_ptr(); res.RF = buf[..., :M]
-        if "T" in outputs:
-            buf = new(n_t, ld); d.out_T = buf.data_ptr(); res.T = buf[..., :M]
-        elif stats is not None:  # the moments pass reads the T rows: scratch the caller never sees
-            self._t_scratch = new(n_t, ld); d.out_T = self._t_scratch.data_ptr()
-        if "alpha" in outputs:
-            buf = new(G, n_t, ld); d.out_alpha = buf.data_ptr(); res.alpha = buf[..., :M]
-        if "E" in outputs:
-            buf = new(G, n_t, ld); d.out_E = buf.data_ptr(); res.E = buf[..., :M]
-        if return_state:
-            buf = new(_abi.state_rows(G), ld); d.state_out = buf.data_ptr(); res.state = buf[..., :M]
+        for name, field, shape, kind in _result_layout(G, n_t, M, outputs, return_state, stats):
+            if field is None:
+                setattr(res, name, torch.empty(shape, dtype=getattr(torch, kind), device=dev))
+                continue
+            buf = torch.empty(shape[:-1] + (ld,), dtype=dtype, device=dev)
+            setattr(d, field, buf.data_ptr())
+            setattr(res, name, buf[..., :M])
         if stats is not None:
-            lead = (stats.groups, n_t) if stats.groups else (n_t,)
-            rows = max(1, stats.groups) * n_t
+            if "T" not in outputs:  # the moments pass reads the T rows: scratch the caller never sees
+                self._t_scratch = torch.empty(n_t, ld, dtype=dtype, device=dev)
+                d.out_T = self._t_scratch.data_ptr()
+            rows = math.prod(stats.lead_shape(n_t))
             self._hp = torch.empty(stats.copies, rows, stats.bins, dtype=torch.int32, device=dev)
             self._mp = torch.empty(stats.copies, rows, _abi.MOM_COUNT, dtype=torch.float64, device=dev)
             d.hist_private, d.moments_private = self._hp.data_ptr(), self._mp.data_ptr()
-            res.hist = torch.empty(*lead, stats.bins, dtype=torch.int64, device=dev)
-            res.moments = torch.empty(*lead, _abi.MOM_COUNT, dtype=torch.float64, device=dev)
+        keep = list(placed.values())
         res._keep = keep  # inputs stay alive as long as the result does
         self.desc, self.result, self._keep = d, res, keep
         self._run = self._L.ufair_run_f64 if precision == "f64" else self._L.ufair_run_f32
-        if isinstance(gas_form, str):
-            if gas_form != "auto":
-                raise ValueError("gas_form must be 'auto', None or one entry per gas")
-            if M:  # one scan of the parameter arrays (synchronises the current stream once, at plan time)
-                scratch = torch.empty(_abi.MAX_GAS, dtype=torch.int32, device=dev)
-                form = (C.c_uint8 * _abi.MAX_GAS)()
-                detect = self._L.ufair_detect_form_f64 if precision == "f64" else self._L.ufair_detect_form_f32
-                with torch.cuda.device(dev):
-                    _abi.check(detect(C.byref(d), scratch.data_ptr(), form, self._stream()))
-                for g in range(G):
-                    d.gas_form[g] = form[g]
+        if isinstance(gas_form, str) and M:  # "auto": one scan (synchronises the current stream once, at plan time)
+            scratch = torch.empty(_abi.MAX_GAS, dtype=torch.int32, device=dev)
+            form = (C.c_uint8 * _abi.MAX_GAS)()
+            detect = self._L.ufair_detect_form_f64 if precision == "f64" else self._L.ufair_detect_form_f32
+            with torch.cuda.device(dev):
+                _abi.check(detect(C.byref(d), scratch.data_ptr(), form, self._stream()))
+            for g in range(G):
+                d.gas_form[g] = form[g]
         self.gas_form = tuple(int(d.gas_form[g]) for g in range(G))
 
     def _stream(self):
@@ -533,16 +574,6 @@ class DevicePlan:
         return self.result
 
 
-def _run_device(torch, E, gp, tp, dt, scen_idx, e_scale, f_ext, fext_per_member, state_in, alpha_mode, newton_iters,
-                iirf_max, iirf_h, t_mode, outputs, stats, precision, return_state, gas_form="auto", conc_driven=None,
-                stat_group=None):
-    return DevicePlan(E, gp, tp, dt=dt, scen_idx=scen_idx, e_scale=e_scale, f_ext=f_ext,
-                      fext_per_member=fext_per_member, state_in=state_in, alpha_mode=alpha_mode,
-                      newton_iters=newton_iters, iirf_max=iirf_max, iirf_h=iirf_h, t_mode=t_mode, outputs=outputs,
-                      stats=stats, precision=precision, return_state=return_state, gas_form=gas_form,
-                      conc_driven=conc_driven, stat_group=stat_group).run()
-
-
 class Workspace:
     """Device staging buffers + streams of the host pipeline (reuse across calls to avoid re-allocation)."""
 
@@ -562,103 +593,39 @@ class Workspace:
             pass
 
 
-def _run_host(torch, E, gp, tp, dt, scen_idx, e_scale, f_ext, fext_per_member, state_in, alpha_mode, newton_iters,
-              iirf_max, iirf_h, t_mode, outputs, stats, precision, return_state, chunk_members, workspace, out=None,
-              gas_form=None, conc_driven=None, stat_group=None):
-    L = _abi.lib()
+def _run_host(E, gp, tp, *, precision="f64", return_state=True, gas_form="auto", chunk_members=None, workspace=None,
+              out=None, **inputs):
+    torch = _torch()
     npdt = np.float64 if precision == "f64" else np.float32
-
-    def arr(x):
-        if x is None:
-            return None
-        if isinstance(x, torch.Tensor):
-            x = x.detach().cpu().numpy()
-        return np.ascontiguousarray(x, dtype=npdt)
-
-    E, gp, tp, e_scale, f_ext, state_in = (arr(x) for x in (E, gp, tp, e_scale, f_ext, state_in))
-    fshape = None if f_ext is None else f_ext.shape
-    G, n_t, M, e_scen, n_scen, fext_mode = _shapes(E.shape, gp.shape, tp.shape, scen_idx, fshape, fext_per_member,
-                                                   None if e_scale is None else e_scale.shape)
-    stats, source = _resolve_groups(stats, stat_group, scen_idx is not None, n_scen)
-    auto_form = isinstance(gas_form, str)
-    if auto_form and gas_form != "auto":
-        raise ValueError("gas_form must be 'auto', None or one entry per gas")
-    d = _build_desc(G, n_t, M, M, n_scen, e_scen, fext_mode, alpha_mode, newton_iters, t_mode, outputs, dt, iirf_h,
-                    iirf_max, stats, gas_form, conc_driven)
-    d.emissions, d.gas_params, d.thermal_params = E.ctypes.data, gp.ctypes.data, tp.ctypes.data
-    keep = [E, gp, tp]
-    if scen_idx is not None:
-        si = np.ascontiguousarray(scen_idx.cpu().numpy() if isinstance(scen_idx, torch.Tensor) else scen_idx, dtype=np.int32)
-        if si.size != M or si.min() < 0 or si.max() >= n_scen:
-            raise ValueError("scen_idx must have one in-range entry per member")
-        keep.append(si)
-        d.scen_idx = si.ctypes.data
-    if source == "scenario":   # the same host array: the pipeline stages it once per chunk for both
-        if M:
-            _check_labels(int(si.max()), stats.groups, "scen_idx")
-        d.stat_group = d.scen_idx
-    elif source == "labels":
-        lab = np.ascontiguousarray(stat_group.cpu().numpy() if isinstance(stat_group, torch.Tensor) else stat_group,
-                                   dtype=np.int32)
-        if lab.shape != (M,):
-            raise ValueError("stat_group must have one label per member")
-        if M:
-            _check_labels(int(lab.max()), stats.groups, "stat_group")
-        keep.append(lab)
-        d.stat_group = lab.ctypes.data
-    if e_scale is not None:
-        keep.append(e_scale)
-        d.e_scale = e_scale.ctypes.data
-    if f_ext is not None:
-        if not fext_per_member and f_ext.size == n_t and n_scen > 1:
-            f_ext = np.ascontiguousarray(np.broadcast_to(f_ext.reshape(n_t, 1), (n_t, n_scen)))
-        keep.append(f_ext)
-        d.f_ext = f_ext.ctypes.data
-    if state_in is not None:
-        if state_in.shape != (_abi.state_rows(G), M):
-            raise ValueError("state_in must be [5G+3][M]")
-        d.state_in = state_in.ctypes.data
-    if auto_form and M:
-        for g, f in enumerate(_detect_form_host(gp, state_in)):
+    d, placed, outputs, stats, source = _prepare(_HostArrays(npdt), E, gp, tp, gas_form=gas_form, **inputs)
+    G, n_t, M = d.n_gas, d.n_t, d.n_member
+    if isinstance(gas_form, str) and M:
+        for g, f in enumerate(_detect_form_host(placed["gas_params"], placed.get("state_in"))):
             d.gas_form[g] = f
     res = out if out is not None else EnsembleResult()
     res.spec, res.n_member, res.stat_group = stats, M, source
-
-    def host_out(name, shape, dtype):
-        cur = getattr(res, name)
+    for name, field, shape, kind in _result_layout(G, n_t, M, outputs, return_state, stats):
+        cur = getattr(res, name)   # out= reuse: an array of the right shape and dtype is written in place
         if isinstance(cur, torch.Tensor):
             cur = cur.numpy()
+        dtype = npdt if kind == "real" else np.dtype(kind)
         if not (isinstance(cur, np.ndarray) and cur.shape == shape and cur.dtype == dtype and cur.flags.c_contiguous):
             cur = np.empty(shape, dtype=dtype)
         setattr(res, name, cur)
-        return cur.ctypes.data
-
-    if "C" in outputs:
-        d.out_C = host_out("C", (G, n_t, M), npdt)
-    if "RF" in outputs:
-        d.out_RF = host_out("RF", (G, n_t, M), npdt)
-    if "T" in outputs:
-        d.out_T = host_out("T", (n_t, M), npdt)
-    if "alpha" in outputs:
-        d.out_alpha = host_out("alpha", (G, n_t, M), npdt)
-    if "E" in outputs:
-        d.out_E = host_out("E", (G, n_t, M), npdt)
-    if return_state:
-        d.state_out = host_out("state", (_abi.state_rows(G), M), npdt)
-    hist_p = mom_p = None
-    if stats is not None:
-        lead = (stats.groups, n_t) if stats.groups else (n_t,)
-        hist_p = host_out("hist", lead + (stats.bins,), np.int64)
-        mom_p = host_out("moments", lead + (_abi.MOM_COUNT,), np.float64)
+        if field is not None:
+            setattr(d, field, cur.ctypes.data)
+    stat_out = (res.hist.ctypes.data, res.moments.ctypes.data) if stats is not None else (None, None)
     own = workspace is None
     if own and chunk_members is None:
-        chunk_members = auto_chunk_members(G, n_t, e_member=not e_scen, fext_member=fext_mode == _abi.FEXT_MEMBER, outputs=outputs,
-                                           return_state=return_state, state_in=state_in is not None,
-                                           e_scale=e_scale is not None, precision=precision)
+        chunk_members = auto_chunk_members(G, n_t, e_member=d.e_mode == _abi.E_MEMBER,
+                                           fext_member=d.fext_mode == _abi.FEXT_MEMBER, outputs=outputs,
+                                           return_state=return_state, state_in="state_in" in placed,
+                                           e_scale="e_scale" in placed, precision=precision)
     ws = Workspace(torch.cuda.current_device(), chunk_members) if own else workspace
     try:
+        L = _abi.lib()
         run = L.ufair_run_host_f64 if precision == "f64" else L.ufair_run_host_f32
-        _abi.check(run(ws._h, C.byref(d), hist_p, mom_p))
+        _abi.check(run(ws._h, C.byref(d), *stat_out))
     finally:
         if own:
             ws.close()
@@ -670,23 +637,9 @@ def pinned_result(n_gas, n_t, n_member, outputs=("C", "RF", "T"), stats: Optiona
     """Page-locked host output buffers for :func:`run_ensemble` ``out=`` (D2H at full PCIe speed).  Grouped
     statistics need ``stats.groups`` set to the group count here (``HistSpec(groups=S)`` for per-scenario ones)."""
     torch = _require_cuda()
-    dt = torch.float64 if precision == "f64" else torch.float32
-    pin = lambda *shape, dtype=dt: torch.empty(*shape, dtype=dtype, pin_memory=True).numpy()
+    real = torch.float64 if precision == "f64" else torch.float32
     r = EnsembleResult(spec=stats, n_member=n_member)
-    if "C" in outputs:
-        r.C = pin(n_gas, n_t, n_member)
-    if "RF" in outputs:
-        r.RF = pin(n_gas, n_t, n_member)
-    if "T" in outputs:
-        r.T = pin(n_t, n_member)
-    if "alpha" in outputs:
-        r.alpha = pin(n_gas, n_t, n_member)
-    if "E" in outputs:
-        r.E = pin(n_gas, n_t, n_member)
-    if return_state:
-        r.state = pin(_abi.state_rows(n_gas), n_member)
-    if stats is not None:
-        lead = (stats.groups, n_t) if stats.groups else (n_t,)
-        r.hist = pin(*lead, stats.bins, dtype=torch.int64)
-        r.moments = pin(*lead, _abi.MOM_COUNT, dtype=torch.float64)
+    for name, _, shape, kind in _result_layout(n_gas, n_t, n_member, outputs, return_state, stats):
+        dtype = real if kind == "real" else getattr(torch, kind)
+        setattr(r, name, torch.empty(shape, dtype=dtype, pin_memory=True).numpy())
     return r

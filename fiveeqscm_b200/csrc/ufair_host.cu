@@ -7,6 +7,7 @@
 // histogram copies and are finalised once at the end; statistics labels (stat_group) are staged per
 // chunk next to scen_idx, or not at all when they are scen_idx itself.
 #include <cuda_runtime.h>
+#include <stddef.h>
 #include <stdint.h>
 #include <string.h>
 #include <time.h>
@@ -51,10 +52,22 @@ struct DevBuf {
   }
 };
 
-enum { B_E, B_FEXT, B_GP, B_TP, B_SIN, B_SCEN, B_GRP, B_ESC, B_OC, B_ORF, B_OT, B_OA, B_OE, B_SOUT, B_COUNT };
+// One array the pipeline stages per chunk: `rows` rows of the chunk's members, `elem` bytes each, in a device buffer
+// that takes the place of descriptor field `field` in the chunk's descriptor.
+struct Staged {
+  size_t field;      // offsetof(ufair_desc, <the array's pointer>)
+  size_t rows;       // rows per member
+  size_t elem;       // bytes per element
+  bool in;           // copied up before the kernel; else written by the kernel
+  bool on;           // staged in this call
+  bool back;         // copied back to the caller's array after the kernel
+  bool flat;         // an [n_member] array without row pitch: one 1-D copy
+  size_t alias = 0;  // not staged but the staged array of this field instead (labels that are scen_idx itself)
+};
+constexpr int kStaged = 14;  // entries of run_chunks' table
 
 struct Stage {
-  DevBuf b[B_COUNT];
+  DevBuf b[kStaged];
   cudaEvent_t in_done = nullptr, run_done = nullptr, out_done = nullptr;
   bool used = false;
 };
@@ -77,36 +90,73 @@ namespace ufair {
     if (e__ != cudaSuccess) return cuda_error(e__, what); \
   } while (0)
 
-static int copy2d(void* dst, size_t dpitch, const void* src, size_t spitch, size_t width, size_t rows,
-                  cudaMemcpyKind kind, cudaStream_t s) {
-  if (rows == 0 || width == 0) return UFAIR_OK;
-  CK(cudaMemcpy2DAsync(dst, dpitch, src, spitch, width, rows, kind, s), "cudaMemcpy2DAsync");
+// the descriptor's pointer field at byte offset `field` (every array field is a plain pointer)
+static const void* get_field(const ufair_desc& d, size_t field) {
+  const void* p;
+  memcpy(&p, (const char*)&d + field, sizeof p);
+  return p;
+}
+static void set_field(ufair_desc& d, size_t field, const void* p) { memcpy((char*)&d + field, &p, sizeof p); }
+
+// members [c0, c0 + cm) of staged array t, between the caller's array (row pitch ld_member) and its device buffer
+// (row pitch chunk)
+static int copy_chunk(const Staged& t, const ufair_desc* h, void* dev, int64_t c0, int64_t cm, int64_t chunk,
+                      cudaMemcpyKind kind, cudaStream_t s) {
+  char* host = (char*)get_field(*h, t.field) + (size_t)c0 * t.elem;
+  const bool up = kind == cudaMemcpyHostToDevice;
+  void* dst = up ? dev : (void*)host;
+  const void* src = up ? (const void*)host : dev;
+  const size_t w = (size_t)cm * t.elem, hp = (size_t)h->ld_member * t.elem, dp = (size_t)chunk * t.elem;
+  if (t.flat) {
+    CK(cudaMemcpyAsync(dst, src, w, kind, s), "cudaMemcpyAsync");
+    return UFAIR_OK;
+  }
+  if (t.rows == 0 || w == 0) return UFAIR_OK;
+  CK(cudaMemcpy2DAsync(dst, up ? dp : hp, src, up ? hp : dp, w, t.rows, kind, s), "cudaMemcpy2DAsync");
   return UFAIR_OK;
 }
 
 template <typename Real>
 static int run_chunks(ufair_workspace* ws, const ufair_desc* h, const ufair_desc& d) {
-  const size_t es = sizeof(Real);
-  const int G = h->n_gas, n_t = h->n_t;
-  const int64_t M = h->n_member, ldh = h->ld_member;
-  const size_t srows = UFAIR_STATE_ROWS(G);
+  const size_t es = sizeof(Real), i4 = sizeof(int32_t);
+  const int G = h->n_gas, n_t = h->n_t, out = h->out_mask;
+  const int64_t M = h->n_member;
+  const size_t gt = (size_t)G * n_t, srows = UFAIR_STATE_ROWS(G);
   const bool e_member = h->e_mode == UFAIR_E_MEMBER;
-  const bool fx_member = h->fext_mode == UFAIR_FEXT_MEMBER;
-  const bool esc_on = !e_member && h->e_scale != nullptr;
-  const bool own_labels = h->stat_group != nullptr && h->stat_group != h->scen_idx;  // else scen_idx's staging serves
+  const bool labels_are_scen = h->stat_group != nullptr && h->stat_group == h->scen_idx;
+  auto want = [&](int bit) { return (out & bit) != 0; };
+  // Every array staged per chunk, in the order its copies are issued: field, rows per member, element bytes, in, on,
+  // back, flat[, alias].  Arrays that are not staged keep their field of `d`: NULL, or the scenario-shared copy
+  // run_host put on the device.
+#define F(x) offsetof(ufair_desc, x)
+  const Staged table[] = {
+      {F(emissions), gt, es, true, e_member, false, false},
+      {F(f_ext), (size_t)n_t, es, true, h->fext_mode == UFAIR_FEXT_MEMBER, false, false},
+      {F(gas_params), (size_t)G * UFAIR_GP_COUNT, es, true, true, false, false},
+      {F(thermal_params), UFAIR_TP_COUNT, es, true, true, false, false},
+      {F(state_in), srows, es, true, h->state_in != nullptr, false, false},
+      {F(e_scale), (size_t)G, es, true, !e_member && h->e_scale != nullptr, false, false},
+      {F(scen_idx), 1, i4, true, h->scen_idx != nullptr, false, true},
+      {F(stat_group), 1, i4, true, h->stat_group != nullptr && !labels_are_scen, false, true,
+       labels_are_scen ? F(scen_idx) : 0},
+      {F(out_C), gt, es, false, want(UFAIR_OUT_C), want(UFAIR_OUT_C), false},
+      {F(out_RF), gt, es, false, want(UFAIR_OUT_RF), want(UFAIR_OUT_RF), false},
+      {F(out_T), (size_t)n_t, es, false, want(UFAIR_OUT_T) || h->stats != 0, want(UFAIR_OUT_T), false},  // stats read T
+      {F(out_alpha), gt, es, false, want(UFAIR_OUT_ALPHA), want(UFAIR_OUT_ALPHA), false},
+      {F(out_E), gt, es, false, want(UFAIR_OUT_E), want(UFAIR_OUT_E), false},
+      {F(state_out), srows, es, false, h->state_out != nullptr, h->state_out != nullptr, false},
+  };
+#undef F
+  static_assert(sizeof(table) / sizeof(table[0]) == kStaged, "one staging buffer per table entry");
   // the workspace's chunk size, cut down for long runs so that the two staging sets stay within
-  // kStagingBudget bytes (rows per member grow with the step count)
-  const size_t gt = (size_t)G * n_t;
-  const size_t rows_per_member =
-      (e_member ? gt : 0) + (fx_member ? (size_t)n_t : 0) + (size_t)G * UFAIR_GP_COUNT + UFAIR_TP_COUNT +
-      (h->state_in ? srows : 0) + (esc_on ? (size_t)G : 0) + ((h->out_mask & UFAIR_OUT_C) ? gt : 0) +
-      ((h->out_mask & UFAIR_OUT_RF) ? gt : 0) + (((h->out_mask & UFAIR_OUT_T) || h->stats) ? (size_t)n_t : 0) +
-      ((h->out_mask & UFAIR_OUT_ALPHA) ? gt : 0) + ((h->out_mask & UFAIR_OUT_E) ? gt : 0) + (h->state_out ? srows : 0);
+  // kStagingBudget bytes (rows per member grow with the step count; the [n_member] label arrays are not counted)
+  size_t member_bytes = 0;
+  for (const Staged& t : table)
+    if (t.on && !t.flat) member_bytes += t.rows * t.elem;
   constexpr size_t kStagingBudget = (size_t)8 << 30;  // bytes, both staging sets together
-  int64_t fit = (int64_t)(kStagingBudget / 2 / (rows_per_member * es));
+  int64_t fit = (int64_t)(kStagingBudget / 2 / member_bytes);
   fit = fit / 256 * 256;
   const int64_t chunk = std::min<int64_t>(ws->chunk, std::max<int64_t>(fit, 256));
-  const size_t hp = (size_t)ldh * es, dp = (size_t)chunk * es;  // host / device row pitch (bytes)
 
   // Chunk schedule: the pipeline's fill time is the first chunk's copy-in (plus, when everything comes back, its
   // kernel), during which nothing else runs -- so the first chunks are short and double up to the workspace's
@@ -118,100 +168,46 @@ static int run_chunks(ufair_workspace* ws, const ufair_desc* h, const ufair_desc
   for (int64_t c = 0; c0 < M; ++c) {
     Stage& S = ws->st[c & 1];
     const int64_t cm = std::min(next, M - c0);
-    const size_t w = (size_t)cm * es;
-    auto hsrc = [&](const void* base) { return (const void*)((const char*)base + (size_t)c0 * es); };
-    auto hdst = [&](void* base) { return (void*)((char*)base + (size_t)c0 * es); };
-    struct Need { int id; size_t rows; bool on; };
-    const Need need[] = {{B_E, (size_t)G * n_t, e_member},
-                         {B_FEXT, (size_t)n_t, fx_member},
-                         {B_GP, (size_t)G * UFAIR_GP_COUNT, true},
-                         {B_TP, (size_t)UFAIR_TP_COUNT, true},
-                         {B_SIN, srows, h->state_in != nullptr},
-                         {B_ESC, (size_t)G, esc_on},
-                         {B_OC, (size_t)G * n_t, (h->out_mask & UFAIR_OUT_C) != 0},
-                         {B_ORF, (size_t)G * n_t, (h->out_mask & UFAIR_OUT_RF) != 0},
-                         {B_OT, (size_t)n_t, (h->out_mask & UFAIR_OUT_T) != 0 || h->stats != 0},  // moments pass reads T
-                         {B_OA, (size_t)G * n_t, (h->out_mask & UFAIR_OUT_ALPHA) != 0},
-                         {B_OE, (size_t)G * n_t, (h->out_mask & UFAIR_OUT_E) != 0},
-                         {B_SOUT, srows, h->state_out != nullptr}};
     if (S.used) {  // staging of chunk c-2: inputs consumed by its kernel, outputs copied out
       CK(cudaStreamWaitEvent(ws->s_in, S.run_done, 0), "cudaStreamWaitEvent");
       CK(cudaStreamWaitEvent(ws->s_run, S.out_done, 0), "cudaStreamWaitEvent");
     }
-    for (const Need& n : need) {
-      if (n.on && S.b[n.id].cap < n.rows * dp) {
+    for (int i = 0; i < kStaged; ++i) {
+      const size_t bytes = table[i].rows * (size_t)chunk * table[i].elem;
+      if (table[i].on && S.b[i].cap < bytes) {
         CK(cudaDeviceSynchronize(), "cudaDeviceSynchronize");  // growing: first call with this shape only
-        CK(S.b[n.id].reserve(n.rows * dp), "cudaMalloc(staging)");
+        CK(S.b[i].reserve(bytes), "cudaMalloc(staging)");
       }
     }
-    if (h->scen_idx && S.b[B_SCEN].cap < (size_t)chunk * sizeof(int32_t)) {
-      CK(cudaDeviceSynchronize(), "cudaDeviceSynchronize");
-      CK(S.b[B_SCEN].reserve((size_t)chunk * sizeof(int32_t)), "cudaMalloc(scen_idx)");
-    }
-    if (own_labels && S.b[B_GRP].cap < (size_t)chunk * sizeof(int32_t)) {
-      CK(cudaDeviceSynchronize(), "cudaDeviceSynchronize");
-      CK(S.b[B_GRP].reserve((size_t)chunk * sizeof(int32_t)), "cudaMalloc(stat_group)");
-    }
     // ---- H2D
-    int rc = UFAIR_OK;
-    if (e_member)
-      rc = copy2d(S.b[B_E].p, dp, hsrc(h->emissions), hp, w, (size_t)G * n_t, cudaMemcpyHostToDevice, ws->s_in);
-    if (rc == UFAIR_OK && fx_member)
-      rc = copy2d(S.b[B_FEXT].p, dp, hsrc(h->f_ext), hp, w, n_t, cudaMemcpyHostToDevice, ws->s_in);
-    if (rc == UFAIR_OK)
-      rc = copy2d(S.b[B_GP].p, dp, hsrc(h->gas_params), hp, w, (size_t)G * UFAIR_GP_COUNT, cudaMemcpyHostToDevice, ws->s_in);
-    if (rc == UFAIR_OK)
-      rc = copy2d(S.b[B_TP].p, dp, hsrc(h->thermal_params), hp, w, UFAIR_TP_COUNT, cudaMemcpyHostToDevice, ws->s_in);
-    if (rc == UFAIR_OK && h->state_in)
-      rc = copy2d(S.b[B_SIN].p, dp, hsrc(h->state_in), hp, w, srows, cudaMemcpyHostToDevice, ws->s_in);
-    if (rc == UFAIR_OK && esc_on)
-      rc = copy2d(S.b[B_ESC].p, dp, hsrc(h->e_scale), hp, w, G, cudaMemcpyHostToDevice, ws->s_in);
-    if (rc != UFAIR_OK) return rc;
-    if (h->scen_idx)
-      CK(cudaMemcpyAsync(S.b[B_SCEN].p, h->scen_idx + c0, (size_t)cm * sizeof(int32_t), cudaMemcpyHostToDevice, ws->s_in),
-         "H2D scen_idx");
-    if (own_labels)
-      CK(cudaMemcpyAsync(S.b[B_GRP].p, h->stat_group + c0, (size_t)cm * sizeof(int32_t), cudaMemcpyHostToDevice, ws->s_in),
-         "H2D stat_group");
+    for (int i = 0; i < kStaged; ++i) {
+      if (!table[i].on || !table[i].in) continue;
+      const int rc = copy_chunk(table[i], h, S.b[i].p, c0, cm, chunk, cudaMemcpyHostToDevice, ws->s_in);
+      if (rc != UFAIR_OK) return rc;
+    }
     CK(cudaEventRecord(S.in_done, ws->s_in), "cudaEventRecord");
     // ---- kernel
     CK(cudaStreamWaitEvent(ws->s_run, S.in_done, 0), "cudaStreamWaitEvent");
     ufair_desc k = d;
     k.n_member = cm;
     k.ld_member = chunk;
-    if (e_member) k.emissions = S.b[B_E].p;
-    if (fx_member) k.f_ext = S.b[B_FEXT].p;
-    k.gas_params = S.b[B_GP].p;
-    k.thermal_params = S.b[B_TP].p;
-    k.state_in = h->state_in ? S.b[B_SIN].p : nullptr;
-    k.e_scale = esc_on ? S.b[B_ESC].p : nullptr;
-    k.scen_idx = h->scen_idx ? (const int32_t*)S.b[B_SCEN].p : nullptr;
-    k.stat_group = own_labels ? (const int32_t*)S.b[B_GRP].p : h->stat_group ? k.scen_idx : nullptr;
-    k.out_C = S.b[B_OC].p;
-    k.out_RF = S.b[B_ORF].p;
-    k.out_T = S.b[B_OT].p;
-    k.out_alpha = S.b[B_OA].p;
-    k.out_E = S.b[B_OE].p;
-    k.state_out = h->state_out ? S.b[B_SOUT].p : nullptr;
-    rc = run_device<Real>(&k, ws->s_run);
+    for (int i = 0; i < kStaged; ++i) {
+      if (table[i].on)
+        set_field(k, table[i].field, S.b[i].p);
+      else if (table[i].alias)
+        set_field(k, table[i].field, get_field(k, table[i].alias));
+    }
+    int rc = run_device<Real>(&k, ws->s_run);
     if (rc == UFAIR_OK && h->stats) rc = run_stats_pass<Real>(&k, ws->s_run);
     if (rc != UFAIR_OK) return rc;
     CK(cudaEventRecord(S.run_done, ws->s_run), "cudaEventRecord");
     // ---- D2H
     CK(cudaStreamWaitEvent(ws->s_out, S.run_done, 0), "cudaStreamWaitEvent");
-    if (h->out_mask & UFAIR_OUT_C)
-      rc = copy2d(hdst(h->out_C), hp, S.b[B_OC].p, dp, w, (size_t)G * n_t, cudaMemcpyDeviceToHost, ws->s_out);
-    if (rc == UFAIR_OK && (h->out_mask & UFAIR_OUT_RF))
-      rc = copy2d(hdst(h->out_RF), hp, S.b[B_ORF].p, dp, w, (size_t)G * n_t, cudaMemcpyDeviceToHost, ws->s_out);
-    if (rc == UFAIR_OK && (h->out_mask & UFAIR_OUT_T))
-      rc = copy2d(hdst(h->out_T), hp, S.b[B_OT].p, dp, w, n_t, cudaMemcpyDeviceToHost, ws->s_out);
-    if (rc == UFAIR_OK && (h->out_mask & UFAIR_OUT_ALPHA))
-      rc = copy2d(hdst(h->out_alpha), hp, S.b[B_OA].p, dp, w, (size_t)G * n_t, cudaMemcpyDeviceToHost, ws->s_out);
-    if (rc == UFAIR_OK && (h->out_mask & UFAIR_OUT_E))
-      rc = copy2d(hdst(h->out_E), hp, S.b[B_OE].p, dp, w, (size_t)G * n_t, cudaMemcpyDeviceToHost, ws->s_out);
-    if (rc == UFAIR_OK && h->state_out)
-      rc = copy2d(hdst(h->state_out), hp, S.b[B_SOUT].p, dp, w, srows, cudaMemcpyDeviceToHost, ws->s_out);
-    if (rc != UFAIR_OK) return rc;
+    for (int i = 0; i < kStaged; ++i) {
+      if (!table[i].back) continue;
+      rc = copy_chunk(table[i], h, S.b[i].p, c0, cm, chunk, cudaMemcpyDeviceToHost, ws->s_out);
+      if (rc != UFAIR_OK) return rc;
+    }
     CK(cudaEventRecord(S.out_done, ws->s_out), "cudaEventRecord");
     S.used = true;
     c0 += cm;
@@ -349,7 +345,7 @@ int ufair_workspace_destroy(ufair_workspace* ws) {
   if (!ws) return UFAIR_OK;
   DeviceGuard guard(ws->device);
   for (int i = 0; i < 2; ++i) {
-    for (int j = 0; j < B_COUNT; ++j) ws->st[i].b[j].release();
+    for (int j = 0; j < kStaged; ++j) ws->st[i].b[j].release();
     if (ws->st[i].in_done) cudaEventDestroy(ws->st[i].in_done);
     if (ws->st[i].run_done) cudaEventDestroy(ws->st[i].run_done);
     if (ws->st[i].out_done) cudaEventDestroy(ws->st[i].out_done);

@@ -7,6 +7,8 @@ Works over any torch.distributed backend (nccl on the B200 box, gloo in the CPU 
 """
 from __future__ import annotations
 
+import math
+
 
 def shard_bounds(n_member: int, world_size: int, rank: int, align: int = 128):
     """Contiguous member block of `rank`: [lo, hi).  Block edges are multiples of `align`
@@ -56,7 +58,7 @@ class StatsReducer:
         self.plan, self.group = plan, group
         self.world = dist.get_world_size(group) if (dist.is_available() and dist.is_initialized()) else 1
         self._k = 0
-        self._rows = plan.n_t * max(1, plan.stats.groups) if plan.stats is not None else 0   # [groups][n_t] rows
+        self._rows = math.prod(plan.stats.lead_shape(plan.n_t)) if plan.stats is not None else 0
         if self.world > 1 and plan.stats is not None:
             rows, bins = self._rows, plan.stats.bins
             dev = plan.device

@@ -174,6 +174,9 @@ def test_empty_inputs(api):
     z = lambda *s: torch.zeros(*s, dtype=torch.float64, device="cuda")
     res = api.run_ensemble(z(3, 5, 0), z(3, 17, 0), z(4, 0))   # zero members
     assert res.T.shape == (5, 0)
+    res = api.run_ensemble(np.zeros((3, 5, 2)), np.zeros((3, 17, 0)), np.zeros((4, 0)),   # host pipeline, scenario inputs
+                           scen_idx=np.zeros(0, dtype=np.int32))
+    assert res.T.shape == (5, 0)
 
 
 def test_scenario_shared_emissions_and_forcing(api):

@@ -285,3 +285,51 @@ def test_any_nonzero_and_auto_chunk_choice():
     assert (full, stats_only, t_only) == (16384, 16384, 16384) and scenario == 131072 and scenario32 == 131072
     short = api.auto_chunk_members(3, 10, e_member=False, fext_member=False, outputs=(), return_state=False)
     assert short == 16384     # ten steps: the parameters going up outweigh the integration
+
+
+@pytest.mark.parametrize("where", ["host-numpy", "host-tensors", "device-rule-on-cpu"])
+def test_input_preparation_shared_by_both_paths(where):
+    """The input checks both run paths share, without a GPU: the host pipeline's placement with numpy arrays and with
+    CPU tensors, and the device placement (padded, aligned member rows) run on CPU tensors."""
+    import torch
+    host = where.startswith("host")
+    arrays = conc._HostArrays(np.float64) if host else conc._DeviceArrays(torch, torch.device("cpu"), torch.float64)
+    wrap = np.asarray if where == "host-numpy" else torch.as_tensor
+    G, n_t, M, S = 3, 6, 9, 4
+    E = wrap(np.random.default_rng(0).random((G, n_t, S)))
+    gp, tp = (wrap(x) for x in P.default_params(M))
+    scen = wrap(np.arange(M, dtype=np.int32) % S)
+    prep = lambda **kw: conc._prepare(arrays, E, gp, tp, **{"scen_idx": scen, **kw})
+    spec = conc.HistSpec(groups=3)
+    for kw, match in ((dict(scen_idx=wrap(np.zeros(M - 1, np.int32))), "scen_idx must have one entry per member"),
+                      (dict(scen_idx=wrap(np.full(M, S, np.int32))), "scen_idx out of range"),
+                      (dict(scen_idx=wrap(np.full(M, -1, np.int32))), "scen_idx out of range"),
+                      (dict(stats=spec, stat_group=wrap(np.zeros(M - 1, np.int32))), "stat_group must have one label per"),
+                      (dict(stats=spec, stat_group=wrap(np.full(M, 3, np.int32))), "stat_group has a label 3 >= groups 3"),
+                      (dict(stats=spec, stat_group="scenario"), "scen_idx has a label 3 >= groups 3"),
+                      (dict(e_scale=wrap(np.ones((G, M - 1)))), "e_scale must be"),
+                      (dict(f_ext=wrap(np.zeros(n_t + 1))), "f_ext must have n_t rows"),
+                      (dict(state_in=wrap(np.zeros((5 * G + 3, M + 1)))), "state_in must be"),
+                      (dict(gas_form="fast"), "gas_form must be"),
+                      (dict(outputs=("T", "X")), "unknown output")):
+        with pytest.raises(ValueError, match=match):
+            prep(**kw)
+    d, placed, outputs, stats, source = prep(stats=conc.HistSpec(), stat_group="scenario", conc_driven=True,
+                                             e_scale=wrap(np.ones((G, M))), f_ext=wrap(np.arange(n_t, dtype=float)))
+    assert placed["stat_group"] is placed["scen_idx"] and d.stat_group == d.scen_idx    # scen_idx serves as the labels
+    assert (stats.groups, source, outputs) == (S, "scenario", ("C", "RF", "T", "E"))
+    fx = np.asarray(placed["f_ext"])                                                   # [n_t] -> [n_t][S]
+    assert fx.shape == (n_t, S) and (fx == np.arange(n_t)[:, None]).all() and d.f_ext == arrays.ptr(placed["f_ext"])
+    ld = M if host else 10                                                             # device rows: 16-byte pitch
+    assert d.ld_member == ld and tuple(placed["gas_params"].shape) == (G, 17, ld)
+    assert tuple(placed["e_scale"].shape) == (G, ld) and tuple(placed["emissions"].shape) == (G, n_t, S)
+    if not host:
+        assert all(arrays.ptr(x) % 16 == 0 for x in placed.values())
+    # zero members with scenario inputs and labels: nothing to range-check
+    d0 = conc._prepare(arrays, E, wrap(np.zeros((G, 17, 0))), wrap(np.zeros((4, 0))), scen_idx=wrap(np.zeros(0, np.int32)),
+                       stats=spec, stat_group=wrap(np.zeros(0, np.int32)))[0]
+    assert d0.n_member == 0 and d0.n_scen == S
+    layout = conc._result_layout(G, n_t, M, ("T", "C"), True, spec)
+    assert [(name, field, shape) for name, field, shape, _ in layout] == [
+        ("C", "out_C", (G, n_t, M)), ("T", "out_T", (n_t, M)), ("state", "state_out", (5 * G + 3, M)),
+        ("hist", None, (3, n_t, spec.bins)), ("moments", None, (3, n_t, 4))]
