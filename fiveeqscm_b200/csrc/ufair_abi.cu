@@ -6,6 +6,7 @@
 #include <cuda_runtime.h>
 #include <math.h>
 #include <stdarg.h>
+#include <stddef.h>
 #include <stdio.h>
 #include <string.h>
 
@@ -201,165 +202,113 @@ static int dispatch_mode(const ufair_desc* d, const KArgs<Real>& a, cudaStream_t
 }
 
 // ---- statistics of T: second pass over the T rows the integrator just wrote ----------------------
-// CTA (c, t) handles member slice c of row t.
-//   histogram: bin = clamp(floor((T - lo) * invw), 0, bins - 1) in the run's precision (subtract and
-//   multiply rounded separately, NaN not counted); counts go to a shared-memory histogram (per-thread
-//   run-length merging in front of the atomics), then are added to hist_private[c][hist_t0 + t] -- a
-//   row this CTA alone owns, so no global atomics.  With more bins than fit in shared memory the counts go
-//   straight to that row with global atomics.
-//   moments: strided per-thread partials, shuffle tree, warps in order, merged into
-//   moments_private[c][hist_t0 + t]: no atomics, deterministic.
+// The moments of a set of values; the members are in the UFAIR_MOM_* slot order, so a Moments is one row of a moments
+// buffer and at() views a stored row as one.  take() and merge() are the only statement of the merge rule; every fold
+// applies them in a fixed order, so the moments are deterministic.
+struct Moments {
+  double sum, sumsq, min, max;
+  __device__ static Moments identity() { return {0.0, 0.0, INFINITY, -INFINITY}; }
+  __device__ static Moments& at(double* row) { return *reinterpret_cast<Moments*>(row); }
+  __device__ static const Moments& at(const double* row) { return *reinterpret_cast<const Moments*>(row); }
+  __device__ void take(double v) {
+    sum += v;
+    sumsq = fma(v, v, sumsq);
+    min = fmin(min, v);
+    max = fmax(max, v);
+  }
+  __device__ void merge(const Moments& o) {
+    sum += o.sum;
+    sumsq += o.sumsq;
+    min = fmin(min, o.min);
+    max = fmax(max, o.max);
+  }
+  __device__ Moments shfl_xor(int off) const {
+    return {__shfl_xor_sync(0xffffffffu, sum, off), __shfl_xor_sync(0xffffffffu, sumsq, off),
+            __shfl_xor_sync(0xffffffffu, min, off), __shfl_xor_sync(0xffffffffu, max, off)};
+  }
+};
+static_assert(offsetof(Moments, sum) == UFAIR_MOM_SUM * sizeof(double) &&
+                  offsetof(Moments, sumsq) == UFAIR_MOM_SUMSQ * sizeof(double) &&
+                  offsetof(Moments, min) == UFAIR_MOM_MIN * sizeof(double) &&
+                  offsetof(Moments, max) == UFAIR_MOM_MAX * sizeof(double) &&
+                  sizeof(Moments) == UFAIR_MOM_COUNT * sizeof(double),
+              "a Moments is one moments row");
+
+// CTA (x = t * n_tiles + z, y = c) handles member slice c of row t for the groups [z NGT, z NGT + ngt) of tile z.
+//   LABELS false: the pooled pass, one group, no labels read, x = t.
+//   LABELS true (stat_group, e.g. per scenario): a tile of NGT groups.  The tiles of one row slice are neighbours on the
+//   fastest grid axis, so they run together and all but the first find the slice in L2 (with one tile, T streams past
+//   L2 as in the pooled pass, which keeps the label slice -- shared by every step of slice c, and those CTAs run
+//   together -- resident).  A label outside [0, n_groups) is counted nowhere; one tile still reads the labels, so a
+//   single group skips the negative ones.
+//   histogram: bin = clamp(floor((T - lo) * invw), 0, bins - 1) in the run's precision (subtract and multiply rounded
+//   separately, NaN not counted); counts go to a shared-memory histogram [ngt][bins] (per-thread run-length merging,
+//   keyed by group and bin, in front of the atomics), then are added to row g * hist_rows + hist_t0 + t of
+//   hist_private copy c -- rows this CTA alone owns, so no global atomics.  With more than kStatsSmemBins slots the
+//   counts go straight to those rows with global atomics.
+//   moments: strided per-thread partials (per group in registers: unrolled predicated updates), shuffle tree, warps in
+//   order, merged into the same row of moments_private: no atomics, deterministic.  One group with every label 0
+//   performs the pooled pass's operations in the same order, so it reproduces the pooled pass bit for bit.
 constexpr int kStatsThreads = 256;
 constexpr int kStatsSmemBins = 16384;  // 64 KB of dynamic shared memory at most
 
-template <typename Real>
+// The label arguments come last: the pooled instantiation then keeps the pooled pass's parameter offsets, and with
+// them its instruction schedule.
+template <typename Real, int NGT, bool LABELS>
 __global__ void __launch_bounds__(kStatsThreads)
     stats_pass_kernel(const Real* __restrict__ T, long long ld, long long n_member, int t0_row, int rows, int bins,
-                      Real lo, Real invw, int smem_hist, unsigned int* __restrict__ hp, double* mp) {
-  using M = Math<Real>;
-  extern __shared__ unsigned int sh[];
-  const int c = blockIdx.y, copies = gridDim.y, t = blockIdx.x;  // t on x: no 65535 limit on the step count
-  const long long m_lo = n_member * c / copies, m_hi = n_member * (c + 1) / copies;
-  const Real* row = T + (long long)t * ld;
-  unsigned int* grow = hp + ((size_t)c * rows + t0_row + t) * bins;
-  if (smem_hist) {
-    for (int b = threadIdx.x; b < bins; b += blockDim.x) sh[b] = 0u;
-    __syncthreads();
-  }
-  unsigned int* hdst = smem_hist ? sh : grow;
-  const int bins_m1 = bins - 1;
-  double sm = 0.0, ss = 0.0, mn = INFINITY, mx = -INFINITY;
-  // four independent streaming loads in flight per thread; counts are run-length merged per thread
-  // (a thread flushes one atomic when its bin changes), so a row whose members sit in one or two bins
-  // issues almost no atomics and a spread-out row issues conflict-free ones
-  const long long span = m_hi - m_lo;
-  int last = -1;
-  unsigned run = 0;
-  auto take = [&](Real x) {
-    const double v = (double)x;
-    sm += v;
-    ss = fma(v, v, ss);
-    mn = fmin(mn, v);
-    mx = fmax(mx, v);
-    const Real q = M::bin_x(x, lo, invw);
-    const int b = (q == q) ? max(0, min(bins_m1, M::floor_to_int(q))) : -1;
-    if (b != last) {
-      if (run) atomicAdd(hdst + last, run);
-      last = b;
-      run = 0;
-    }
-    run += (b >= 0);
-  };
-  const Real* src = row + m_lo;
-  long long k = threadIdx.x;
-  for (; k + 3 * kStatsThreads < span; k += 4 * kStatsThreads) {
-    const Real x0 = __ldcs(src + k), x1 = __ldcs(src + k + kStatsThreads), x2 = __ldcs(src + k + 2 * kStatsThreads),
-               x3 = __ldcs(src + k + 3 * kStatsThreads);
-    take(x0);
-    take(x1);
-    take(x2);
-    take(x3);
-  }
-  for (; k < span; k += kStatsThreads) take(__ldcs(src + k));
-  if (run) atomicAdd(hdst + last, run);
-#pragma unroll
-  for (int off = 16; off > 0; off >>= 1) {
-    sm += __shfl_xor_sync(0xffffffffu, sm, off);
-    ss += __shfl_xor_sync(0xffffffffu, ss, off);
-    mn = fmin(mn, __shfl_xor_sync(0xffffffffu, mn, off));
-    mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, off));
-  }
-  __shared__ double red[kStatsThreads / 32][4];
-  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-  if (lane == 0) {
-    red[w][0] = sm;
-    red[w][1] = ss;
-    red[w][2] = mn;
-    red[w][3] = mx;
-  }
-  __syncthreads();
-  if (smem_hist)
-    for (int b = threadIdx.x; b < bins; b += blockDim.x)
-      if (sh[b]) grow[b] += sh[b];
-  if (threadIdx.x == 0) {
-    double* o = mp + ((size_t)c * rows + t0_row + t) * UFAIR_MOM_COUNT;
-    sm = o[UFAIR_MOM_SUM];
-    ss = o[UFAIR_MOM_SUMSQ];
-    mn = o[UFAIR_MOM_MIN];
-    mx = o[UFAIR_MOM_MAX];
-    for (int k = 0; k < (int)(blockDim.x >> 5); ++k) {
-      sm += red[k][0];
-      ss += red[k][1];
-      mn = fmin(mn, red[k][2]);
-      mx = fmax(mx, red[k][3]);
-    }
-    o[UFAIR_MOM_SUM] = sm;
-    o[UFAIR_MOM_SUMSQ] = ss;
-    o[UFAIR_MOM_MIN] = mn;
-    o[UFAIR_MOM_MAX] = mx;
-  }
-}
-
-// ---- grouped statistics (stat_group != NULL): one histogram and one set of moments per member label ----------------
-// CTA (x = t * n_tiles + z, y = c) handles member slice c of row t for the groups [z NGT, z NGT + ngt) of tile z.  The
-// tiles of one row slice are neighbours on the fastest grid axis, so they run together and all but the first find the
-// slice in L2 (with one tile, T streams past L2 as in the pooled pass, which keeps the label slice -- shared by every
-// step of slice c, and those CTAs run together -- resident).  Traversal, binning rule, NaN handling, shuffle tree and
-// warp order are those of stats_pass_kernel, one reduction per group, so one group with every label 0 reproduces the
-// pooled pass bit for bit.  The NGT groups' per-thread partials stay in registers (unrolled predicated updates).
-// Counts go to a shared-memory histogram [ngt][bins] with the per-thread run-length merging keyed by (group, bin), or,
-// when NGT x bins exceeds kStatsSmemBins, straight to the CTA's own private rows with global atomics.  A label outside
-// [0, n_groups) is counted nowhere.
-template <typename Real, int NGT>
-__global__ void __launch_bounds__(kStatsThreads)
-    stats_pass_grouped_kernel(const Real* __restrict__ T, const int32_t* __restrict__ labels, long long ld,
-                              long long n_member, int n_groups, int n_tiles, int t0_row, int rows, int bins, Real lo,
-                              Real invw, int smem_hist, unsigned int* __restrict__ hp, double* mp) {
+                      Real lo, Real invw, int smem_hist, unsigned int* __restrict__ hp, double* mp,
+                      const int32_t* __restrict__ labels, int n_groups, int n_tiles) {
+  static_assert(LABELS || NGT == 1, "without labels every member is in the one group");
   using M = Math<Real>;
   extern __shared__ unsigned int sh[];
   const int c = blockIdx.y, copies = gridDim.y;
-  const int t = (int)(blockIdx.x / (unsigned)n_tiles), z = (int)blockIdx.x - t * n_tiles;
-  const int g0 = z * NGT, ngt = min(NGT, n_groups - g0);
+  int t = blockIdx.x, g0 = 0, ngt = 1;  // t on x: no 65535 limit on the step count
+  if constexpr (LABELS) {
+    t = (int)(blockIdx.x / (unsigned)n_tiles);
+    g0 = ((int)blockIdx.x - t * n_tiles) * NGT;
+    ngt = min(NGT, n_groups - g0);
+  }
   const long long m_lo = n_member * c / copies, m_hi = n_member * (c + 1) / copies;
   const Real* src = T + (long long)t * ld + m_lo;
-  const int32_t* lab = labels + m_lo;
-  const size_t copy_rows = (size_t)n_groups * rows, gstride = (size_t)rows * bins;  // rows per copy; one group's rows
+  // rows per copy; one group's rows
+  const size_t copy_rows = (size_t)(LABELS ? n_groups : 1) * rows, gstride = (size_t)rows * bins;
   unsigned int* grow = hp + ((size_t)c * copy_rows + (size_t)g0 * rows + t0_row + t) * bins;  // group g0 + j: + j gstride
   if (smem_hist) {
     for (int i = threadIdx.x; i < ngt * bins; i += blockDim.x) sh[i] = 0u;
     __syncthreads();
   }
   const int bins_m1 = bins - 1;
-  double sm[NGT], ss[NGT], mn[NGT], mx[NGT];
+  Moments mom[NGT];
 #pragma unroll
-  for (int j = 0; j < NGT; ++j) {
-    sm[j] = 0.0;
-    ss[j] = 0.0;
-    mn[j] = INFINITY;
-    mx[j] = -INFINITY;
-  }
+  for (int j = 0; j < NGT; ++j) mom[j] = Moments::identity();
+  // four independent streaming loads in flight per thread; counts are run-length merged per thread
+  // (a thread flushes one atomic when its group or bin changes), so a row whose members sit in one or two bins
+  // issues almost no atomics and a spread-out row issues conflict-free ones
   const long long span = m_hi - m_lo;
   int last_g = -1, last_b = -1;
   unsigned run = 0;
+  unsigned int* const hdst = smem_hist ? sh : grow;  // chosen once: a choice per flush costs the pooled FP32 pass a register
   auto flush = [&]() {
-    if (run) atomicAdd(smem_hist ? sh + last_g * bins + last_b : grow + last_g * gstride + last_b, run);
+    if (!run) return;
+    if constexpr (LABELS)
+      atomicAdd(smem_hist ? sh + last_g * bins + last_b : grow + last_g * gstride + last_b, run);
+    else
+      atomicAdd(hdst + last_b, run);
   };
   auto take = [&](Real x, int label) {
-    const int gl = label - g0;
-    const int sel = (unsigned)gl < (unsigned)ngt ? gl : -1;
+    int sel = 0;  // the member's group in this tile, -1 for none
+    if constexpr (LABELS) {
+      const int gl = label - g0;
+      sel = (unsigned)gl < (unsigned)ngt ? gl : -1;
+    }
     const double v = (double)x;
 #pragma unroll
-    for (int j = 0; j < NGT; ++j) {
-      if (sel == j) {
-        sm[j] += v;
-        ss[j] = fma(v, v, ss[j]);
-        mn[j] = fmin(mn[j], v);
-        mx[j] = fmax(mx[j], v);
-      }
-    }
+    for (int j = 0; j < NGT; ++j)
+      if (sel == j) mom[j].take(v);
     const Real q = M::bin_x(x, lo, invw);
     const int b = (sel >= 0 && q == q) ? max(0, min(bins_m1, M::floor_to_int(q))) : -1;
-    if (b != last_b || sel != last_g) {
+    if (b != last_b || (LABELS && sel != last_g)) {
       flush();
       last_g = sel;
       last_b = b;
@@ -367,82 +316,69 @@ __global__ void __launch_bounds__(kStatsThreads)
     }
     run += (b >= 0);
   };
-  // one tile: stream T past L2 like the pooled pass; several: keep it for the sibling tiles
-  const bool keep = n_tiles > 1;
-  auto load = [&](long long i) { return keep ? __ldg(src + i) : __ldcs(src + i); };
+  // one tile: stream T past L2; several: keep it for the sibling tiles.  The addresses are src + k + offset: with
+  // src + (k + offset) nvcc unrolls the pooled FP64 loop differently (40 registers and 14 loads instead of 48 and 30).
+  const bool keep = LABELS && n_tiles > 1;
+  auto load = [&](const Real* p) { return keep ? __ldg(p) : __ldcs(p); };
+  auto label = [&](long long i) {
+    if constexpr (LABELS)
+      return __ldg(labels + m_lo + i);
+    else
+      return 0;
+  };
   long long k = threadIdx.x;
   for (; k + 3 * kStatsThreads < span; k += 4 * kStatsThreads) {
-    const Real x0 = load(k), x1 = load(k + kStatsThreads), x2 = load(k + 2 * kStatsThreads), x3 = load(k + 3 * kStatsThreads);
-    const int l0 = __ldg(lab + k), l1 = __ldg(lab + k + kStatsThreads), l2 = __ldg(lab + k + 2 * kStatsThreads),
-              l3 = __ldg(lab + k + 3 * kStatsThreads);
+    const Real x0 = load(src + k), x1 = load(src + k + kStatsThreads), x2 = load(src + k + 2 * kStatsThreads),
+               x3 = load(src + k + 3 * kStatsThreads);
+    const int l0 = label(k), l1 = label(k + kStatsThreads), l2 = label(k + 2 * kStatsThreads),
+              l3 = label(k + 3 * kStatsThreads);
     take(x0, l0);
     take(x1, l1);
     take(x2, l2);
     take(x3, l3);
   }
-  for (; k < span; k += kStatsThreads) take(load(k), __ldg(lab + k));
+  for (; k < span; k += kStatsThreads) take(load(src + k), label(k));
   flush();
 #pragma unroll
-  for (int j = 0; j < NGT; ++j) {
+  for (int j = 0; j < NGT; ++j)
 #pragma unroll
-    for (int off = 16; off > 0; off >>= 1) {
-      sm[j] += __shfl_xor_sync(0xffffffffu, sm[j], off);
-      ss[j] += __shfl_xor_sync(0xffffffffu, ss[j], off);
-      mn[j] = fmin(mn[j], __shfl_xor_sync(0xffffffffu, mn[j], off));
-      mx[j] = fmax(mx[j], __shfl_xor_sync(0xffffffffu, mx[j], off));
-    }
-  }
-  __shared__ double red[kStatsThreads / 32][NGT][4];
+    for (int off = 16; off > 0; off >>= 1) mom[j].merge(mom[j].shfl_xor(off));
+  __shared__ Moments red[kStatsThreads / 32][NGT];
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-  if (lane == 0) {
+  if (lane == 0)
 #pragma unroll
-    for (int j = 0; j < NGT; ++j) {
-      red[w][j][0] = sm[j];
-      red[w][j][1] = ss[j];
-      red[w][j][2] = mn[j];
-      red[w][j][3] = mx[j];
-    }
-  }
+    for (int j = 0; j < NGT; ++j) red[w][j] = mom[j];
   __syncthreads();
   if (smem_hist)
     for (int i = threadIdx.x; i < ngt * bins; i += blockDim.x)
-      if (sh[i]) grow[(size_t)(i / bins) * gstride + i % bins] += sh[i];
-  if (threadIdx.x < ngt) {  // thread j folds group g0 + j: the pooled kernel's thread-0 fold, per group
+      if (sh[i]) grow[LABELS ? (size_t)(i / bins) * gstride + i % bins : (size_t)i] += sh[i];
+  if (threadIdx.x < ngt) {  // thread j folds group g0 + j, warps in order
     const int j = threadIdx.x;
-    double* o = mp + ((size_t)c * copy_rows + (size_t)(g0 + j) * rows + t0_row + t) * UFAIR_MOM_COUNT;
-    double s1 = o[UFAIR_MOM_SUM], s2 = o[UFAIR_MOM_SUMSQ], lo_ = o[UFAIR_MOM_MIN], hi_ = o[UFAIR_MOM_MAX];
-    for (int k = 0; k < (int)(blockDim.x >> 5); ++k) {
-      s1 += red[k][j][0];
-      s2 += red[k][j][1];
-      lo_ = fmin(lo_, red[k][j][2]);
-      hi_ = fmax(hi_, red[k][j][3]);
-    }
-    o[UFAIR_MOM_SUM] = s1;
-    o[UFAIR_MOM_SUMSQ] = s2;
-    o[UFAIR_MOM_MIN] = lo_;
-    o[UFAIR_MOM_MAX] = hi_;
+    Moments& o = Moments::at(mp + ((size_t)c * copy_rows + (size_t)(g0 + j) * rows + t0_row + t) * UFAIR_MOM_COUNT);
+    Moments m = o;
+    for (int k = 0; k < (int)(blockDim.x >> 5); ++k) m.merge(red[k][j]);
+    o = m;
   }
 }
 
-template <typename Real, int NGT> static int launch_grouped_pass(const ufair_desc* d, cudaStream_t stream) {
-  const int G = stat_groups(d), n_tiles = (G + NGT - 1) / NGT;
+template <typename Real, int NGT, bool LABELS> static int launch_stats_pass(const ufair_desc* d, cudaStream_t stream) {
+  const int G = LABELS ? stat_groups(d) : 1, n_tiles = (G + NGT - 1) / NGT;
   if (d->hist_copies > 65535) return set_error(UFAIR_ERR_ARG, "hist_copies %d > 65535", d->hist_copies);
   if ((int64_t)d->n_t * n_tiles > (int64_t)INT32_MAX) return set_error(UFAIR_ERR_ARG, "n_t x group tiles too large");
   const int smem_hist = (int64_t)NGT * d->hist_bins <= kStatsSmemBins ? 1 : 0;
   const size_t smem = smem_hist ? (size_t)NGT * d->hist_bins * sizeof(unsigned int) : 0;
   cudaError_t e = cudaSuccess;
   if (smem > 48 * 1024)
-    e = cudaFuncSetAttribute(stats_pass_grouped_kernel<Real, NGT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (e != cudaSuccess) return cuda_error(e, "cudaFuncSetAttribute(stats_pass_grouped_kernel)");
+    e = cudaFuncSetAttribute(stats_pass_kernel<Real, NGT, LABELS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return cuda_error(e, "cudaFuncSetAttribute(stats_pass_kernel)");
   const Real lo = (Real)d->hist_lo;
   const Real invw = (Real)((Real)d->hist_bins / ((Real)d->hist_hi - (Real)d->hist_lo));
-  stats_pass_grouped_kernel<Real, NGT><<<dim3((unsigned)(d->n_t * n_tiles), (unsigned)d->hist_copies), kStatsThreads, smem,
-                                         stream>>>((const Real*)d->out_T, d->stat_group, d->ld_member, d->n_member, G,
-                                                   n_tiles, d->hist_t0, d->hist_rows, d->hist_bins, lo, invw, smem_hist,
-                                                   d->hist_private, d->moments_private);
+  stats_pass_kernel<Real, NGT, LABELS><<<dim3((unsigned)(d->n_t * n_tiles), (unsigned)d->hist_copies), kStatsThreads,
+                                         smem, stream>>>((const Real*)d->out_T, d->ld_member, d->n_member, d->hist_t0,
+                                                         d->hist_rows, d->hist_bins, lo, invw, smem_hist, d->hist_private,
+                                                         d->moments_private, d->stat_group, G, n_tiles);
   e = cudaGetLastError();
-  if (e != cudaSuccess) return cuda_error(e, "stats_pass_grouped_kernel launch");
-  return UFAIR_OK;
+  return e == cudaSuccess ? UFAIR_OK : cuda_error(e, "stats_pass_kernel launch");
 }
 
 template <typename Real> static int dispatch_gases(const ufair_desc* d, const KArgs<Real>& a, cudaStream_t stream) {
@@ -537,24 +473,9 @@ template <typename Real> int run_stats_pass(const ufair_desc* d, cudaStream_t st
   if (rc != UFAIR_OK) return rc;
   if (!d->stats) return set_error(UFAIR_ERR_ARG, "ufair_stats_pass: descriptor has stats == 0");
   if (d->n_member == 0 || d->n_t == 0) return UFAIR_OK;
+  if (!d->stat_group) return launch_stats_pass<Real, 1, false>(d, stream);
   // up to four groups a tile of four: half the registers and predicated updates of a tile of eight
-  if (d->stat_group)
-    return stat_groups(d) <= 4 ? launch_grouped_pass<Real, 4>(d, stream) : launch_grouped_pass<Real, 8>(d, stream);
-  const int smem_hist = d->hist_bins <= kStatsSmemBins ? 1 : 0;
-  const size_t smem = smem_hist ? (size_t)d->hist_bins * sizeof(unsigned int) : 0;
-  cudaError_t e = cudaSuccess;
-  if (smem > 48 * 1024)
-    e = cudaFuncSetAttribute(stats_pass_kernel<Real>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (e != cudaSuccess) return cuda_error(e, "cudaFuncSetAttribute(stats_pass_kernel)");
-  const Real lo = (Real)d->hist_lo;
-  const Real invw = (Real)((Real)d->hist_bins / ((Real)d->hist_hi - (Real)d->hist_lo));
-  if (d->hist_copies > 65535) return set_error(UFAIR_ERR_ARG, "hist_copies %d > 65535", d->hist_copies);
-  stats_pass_kernel<Real><<<dim3((unsigned)d->n_t, (unsigned)d->hist_copies), kStatsThreads, smem, stream>>>(
-      (const Real*)d->out_T, d->ld_member, d->n_member, d->hist_t0, d->hist_rows, d->hist_bins, lo, invw, smem_hist,
-      d->hist_private, d->moments_private);
-  e = cudaGetLastError();
-  if (e != cudaSuccess) return cuda_error(e, "stats_pass_kernel launch");
-  return UFAIR_OK;
+  return stat_groups(d) <= 4 ? launch_stats_pass<Real, 4, true>(d, stream) : launch_stats_pass<Real, 8, true>(d, stream);
 }
 template int run_stats_pass<double>(const ufair_desc*, cudaStream_t);
 template int run_stats_pass<float>(const ufair_desc*, cudaStream_t);
@@ -565,39 +486,34 @@ template int run_device<float>(const ufair_desc*, cudaStream_t);
 __global__ void stats_reset_kernel(unsigned int* hist, size_t n_hist, double* mom, size_t n_rows) {
   const size_t i0 = (size_t)blockIdx.x * blockDim.x + threadIdx.x, stride = (size_t)gridDim.x * blockDim.x;
   for (size_t i = i0; i < n_hist; i += stride) hist[i] = 0u;
-  for (size_t i = i0; i < n_rows; i += stride) {
-    double* r = mom + i * UFAIR_MOM_COUNT;
-    r[UFAIR_MOM_SUM] = 0.0;
-    r[UFAIR_MOM_SUMSQ] = 0.0;
-    r[UFAIR_MOM_MIN] = INFINITY;
-    r[UFAIR_MOM_MAX] = -INFINITY;
-  }
+  for (size_t i = i0; i < n_rows; i += stride) Moments::at(mom + i * UFAIR_MOM_COUNT) = Moments::identity();
 }
 
-__global__ void stats_finalize_kernel(const unsigned int* hp, const double* mp, int copies, int rows, int bins,
-                                      unsigned long long* hist, double* mom) {
+// The fold of the private copies, copies in order (deterministic): put_count(i, count) for every histogram slot i
+// of the [rows][bins] result, put_moments(r, moments) for every row r.  The moments merge straight from the stored
+// rows: copying each row out first reorders the unrolled loads and made the finalize kernels 14 % slower.
+template <typename PutCount, typename PutMoments>
+__device__ void fold_copies(const unsigned int* hp, const double* mp, int copies, int rows, int bins, PutCount put_count,
+                            PutMoments put_moments) {
   const size_t n = (size_t)rows * bins;
   const size_t i0 = (size_t)blockIdx.x * blockDim.x + threadIdx.x, stride = (size_t)gridDim.x * blockDim.x;
   for (size_t i = i0; i < n; i += stride) {
     unsigned long long s = 0;
     for (int c = 0; c < copies; ++c) s += hp[(size_t)c * n + i];
-    hist[i] = s;
+    put_count(i, s);
   }
   for (size_t r = i0; r < (size_t)rows; r += stride) {
-    double sm = 0.0, ss = 0.0, mn = INFINITY, mx = -INFINITY;
-    for (int c = 0; c < copies; ++c) {  // fixed order: deterministic
-      const double* p = mp + ((size_t)c * rows + r) * UFAIR_MOM_COUNT;
-      sm += p[UFAIR_MOM_SUM];
-      ss += p[UFAIR_MOM_SUMSQ];
-      mn = fmin(mn, p[UFAIR_MOM_MIN]);
-      mx = fmax(mx, p[UFAIR_MOM_MAX]);
-    }
-    double* o = mom + r * UFAIR_MOM_COUNT;
-    o[UFAIR_MOM_SUM] = sm;
-    o[UFAIR_MOM_SUMSQ] = ss;
-    o[UFAIR_MOM_MIN] = mn;
-    o[UFAIR_MOM_MAX] = mx;
+    Moments m = Moments::identity();
+    for (int c = 0; c < copies; ++c) m.merge(Moments::at(mp + ((size_t)c * rows + r) * UFAIR_MOM_COUNT));
+    put_moments(r, m);
   }
+}
+
+__global__ void stats_finalize_kernel(const unsigned int* hp, const double* mp, int copies, int rows, int bins,
+                                      unsigned long long* hist, double* mom) {
+  fold_copies(
+      hp, mp, copies, rows, bins, [&](size_t i, unsigned long long s) { hist[i] = s; },
+      [&](size_t r, const Moments& m) { Moments::at(mom + r * UFAIR_MOM_COUNT) = m; });
 }
 
 // The same fold, written in the layout the cross-GPU reduction wants: ONE buffer that is summed
@@ -607,27 +523,14 @@ __global__ void stats_finalize_kernel(const unsigned int* hp, const double* mp, 
 __global__ void stats_finalize_packed_kernel(const unsigned int* hp, const double* mp, int copies, int rows, int bins,
                                              double* sums, double* ext) {
   const int pitch = bins + 2;
-  const size_t n = (size_t)rows * bins;
-  const size_t i0 = (size_t)blockIdx.x * blockDim.x + threadIdx.x, stride = (size_t)gridDim.x * blockDim.x;
-  for (size_t i = i0; i < n; i += stride) {
-    unsigned long long s = 0;
-    for (int c = 0; c < copies; ++c) s += hp[(size_t)c * n + i];
-    sums[(i / bins) * pitch + (i % bins)] = (double)s;
-  }
-  for (size_t r = i0; r < (size_t)rows; r += stride) {
-    double sm = 0.0, ss = 0.0, mn = INFINITY, mx = -INFINITY;
-    for (int c = 0; c < copies; ++c) {  // fixed order: deterministic
-      const double* p = mp + ((size_t)c * rows + r) * UFAIR_MOM_COUNT;
-      sm += p[UFAIR_MOM_SUM];
-      ss += p[UFAIR_MOM_SUMSQ];
-      mn = fmin(mn, p[UFAIR_MOM_MIN]);
-      mx = fmax(mx, p[UFAIR_MOM_MAX]);
-    }
-    sums[r * pitch + bins] = sm;
-    sums[r * pitch + bins + 1] = ss;
-    ext[2 * r] = mx;
-    ext[2 * r + 1] = -mn;
-  }
+  fold_copies(
+      hp, mp, copies, rows, bins, [&](size_t i, unsigned long long s) { sums[(i / bins) * pitch + (i % bins)] = (double)s; },
+      [&](size_t r, const Moments& m) {
+        sums[r * pitch + bins] = m.sum;
+        sums[r * pitch + bins + 1] = m.sumsq;
+        ext[2 * r] = m.max;
+        ext[2 * r + 1] = -m.min;
+      });
 }
 
 __global__ void stats_unpack_kernel(const double* sums, const double* ext, int rows, int bins, unsigned long long* hist,

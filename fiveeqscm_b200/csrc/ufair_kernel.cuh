@@ -55,7 +55,8 @@
 //     80-byte runs; L2 merges them into full sectors (DRAM traffic 1.01x the algorithmic bytes, ncu) --
 //     nothing is re-read.
 //   * optional statistics: the per-step histogram and the moments both come from a second,
-//     HBM-speed pass over the T rows this kernel writes (stats_pass_kernel, ufair_abi.cu): block-level
+//     HBM-speed pass over the T rows this kernel writes (stats_pass_kernel, ufair_abi.cu; one kernel for
+//     pooled and per-label statistics, the pooled instantiation reading no labels): block-level
 //     shared-memory histograms behind per-thread run-length merging.  Measured: the in-loop version (one
 //     RED.ADD.U32 per member-step + the binning arithmetic in every lane) cost 2 ms of the 38 ms launch,
 //     the extra work in the pass costs 0.3 ms.

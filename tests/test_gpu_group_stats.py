@@ -79,19 +79,25 @@ def test_grouped_counts_equal_a_recount_of_the_kernels_T(api, prec, M, G, bins, 
     _check_moments(to_np(res.moments), m_ref, _abs_sums(T, lab, G))
 
 
-@pytest.mark.parametrize("prec", ["f64", "f32"])
-def test_one_group_is_the_pooled_pass_and_groups_sum_to_it(api, prec):
+@pytest.mark.parametrize("prec,bins", [pytest.param("f64", 512, id="f64"), pytest.param("f32", 512, id="f32"),
+                                       # past the 16 384-slot shared-memory budget: the pooled pass's global atomics
+                                       pytest.param("f64", 20000, id="f64-20000"),
+                                       pytest.param("f32", 20000, id="f32-20000")])
+def test_one_group_is_the_pooled_pass_and_groups_sum_to_it(api, prec, bins):
     import torch
     M, n_t = 4001, 37
-    spec = api.HistSpec(lo=-0.5, hi=3.5, bins=512, copies=5)
+    spec = api.HistSpec(lo=-0.5, hi=3.5, bins=bins, copies=5)
     pooled = _plan(api, M, n_t, prec, spec, None)[0].run()
-    one = _plan(api, M, n_t, prec, api.HistSpec(lo=-0.5, hi=3.5, bins=512, copies=5, groups=1),
+    one = _plan(api, M, n_t, prec, api.HistSpec(lo=-0.5, hi=3.5, bins=bins, copies=5, groups=1),
                 np.zeros(M, dtype=np.int32))[0].run()
     four = _plan(api, M, n_t, prec, spec, "scenario")[0].run()
     torch.cuda.synchronize()
     assert torch.equal(one.T, pooled.T)
     assert torch.equal(one.hist[0], pooled.hist) and torch.equal(one.moments[0], pooled.moments)   # bit for bit
     assert four.hist.shape[0] == 4 and torch.equal(four.hist.sum(dim=0), pooled.hist)
+    if bins > 16384:
+        h_ref, _ = grouped_temperature_stats(to_np(pooled.T), spec.lo, spec.hi, bins, np.zeros(M, dtype=np.int32), 1)
+        assert np.array_equal(to_np(pooled.hist).astype(np.uint64), h_ref[0])
 
 
 def test_moments_are_deterministic(api):
