@@ -191,16 +191,6 @@ int make_tensor_maps(const ufair_desc* d, size_t elem, int mw_members, int tile_
   return UFAIR_OK;
 }
 
-template <typename Real, int NGAS>
-static int dispatch_mode(const ufair_desc* d, const KArgs<Real>& a, cudaStream_t s) {
-  switch (d->alpha_mode) {
-    case UFAIR_ALPHA_EXP: return launch_integrate<Real, NGAS, UFAIR_ALPHA_EXP>(d, a, s);
-    case UFAIR_ALPHA_SINH: return launch_integrate<Real, NGAS, UFAIR_ALPHA_SINH>(d, a, s);
-    case UFAIR_ALPHA_NEWTON: return launch_integrate<Real, NGAS, UFAIR_ALPHA_NEWTON>(d, a, s);
-    default: return launch_integrate<Real, NGAS, UFAIR_ALPHA_ONE>(d, a, s);
-  }
-}
-
 // ---- statistics of T: second pass over the T rows the integrator just wrote ----------------------
 // The moments of a set of values; the members are in the UFAIR_MOM_* slot order, so a Moments is one row of a moments
 // buffer and at() views a stored row as one.  take() and merge() are the only statement of the merge rule; every fold
@@ -381,25 +371,30 @@ template <typename Real, int NGT, bool LABELS> static int launch_stats_pass(cons
   return e == cudaSuccess ? UFAIR_OK : cuda_error(e, "stats_pass_kernel launch");
 }
 
-template <typename Real> static int dispatch_gases(const ufair_desc* d, const KArgs<Real>& a, cudaStream_t stream) {
-  switch (d->n_gas) {
-    case 1: return dispatch_mode<Real, 1>(d, a, stream);
-    case 2: return dispatch_mode<Real, 2>(d, a, stream);
-    case 3: return dispatch_mode<Real, 3>(d, a, stream);
-    default: return dispatch_mode<Real, 4>(d, a, stream);
+// the launcher of the descriptor's gas count and alpha mode (validate_desc bounds both); v picks the kernel
+template <typename Real> static int dispatch(const ufair_desc* d, const KArgs<Real>& a, Variant v, cudaStream_t s) {
+  switch (4 * d->n_gas + d->alpha_mode) {
+#define UFAIR_GAS(G)                                                                                 \
+  case 4 * G + UFAIR_ALPHA_EXP: return launch_integrate<Real, G, UFAIR_ALPHA_EXP>(d, a, v, s);       \
+  case 4 * G + UFAIR_ALPHA_SINH: return launch_integrate<Real, G, UFAIR_ALPHA_SINH>(d, a, v, s);     \
+  case 4 * G + UFAIR_ALPHA_NEWTON: return launch_integrate<Real, G, UFAIR_ALPHA_NEWTON>(d, a, v, s); \
+  case 4 * G + UFAIR_ALPHA_ONE: return launch_integrate<Real, G, UFAIR_ALPHA_ONE>(d, a, v, s);
+    UFAIR_GAS(1) UFAIR_GAS(2) UFAIR_GAS(3) UFAIR_GAS(4)
+#undef UFAIR_GAS
   }
+  return set_error(UFAIR_ERR_UNSUPPORTED, "no integrator for %d gases in alpha mode %d", d->n_gas, d->alpha_mode);
 }
 
 #ifdef UFAIR_DEBUG_BOUNDS
 // the negative control of the store check (a.dbg_cut > 0): run, then report every store the check found in the
 // rows it pretends are missing as an error of this call
-template <typename Real> static int run_cut_control(const ufair_desc* d, KArgs<Real> a, cudaStream_t stream) {
+template <typename Real> static int run_cut_control(const ufair_desc* d, KArgs<Real> a, Variant v, cudaStream_t stream) {
   cudaError_t e = cudaMalloc(&a.dbg_cut_hits, sizeof(unsigned long long));
   if (e != cudaSuccess) return cuda_error(e, "cudaMalloc(dbg_cut_hits)");
   unsigned long long hits = 0;
   int rc = UFAIR_OK;
   if ((e = cudaMemsetAsync(a.dbg_cut_hits, 0, sizeof(hits), stream)) != cudaSuccess) rc = cuda_error(e, "cudaMemsetAsync(dbg_cut_hits)");
-  if (rc == UFAIR_OK) rc = dispatch_gases<Real>(d, a, stream);
+  if (rc == UFAIR_OK) rc = dispatch<Real>(d, a, v, stream);
   if (rc == UFAIR_OK && (e = cudaMemcpyAsync(&hits, a.dbg_cut_hits, sizeof(hits), cudaMemcpyDeviceToHost, stream)) != cudaSuccess)
     rc = cuda_error(e, "cudaMemcpyAsync(dbg_cut_hits)");
   if (rc == UFAIR_OK && (e = cudaStreamSynchronize(stream)) != cudaSuccess) rc = cuda_error(e, "cudaStreamSynchronize");
@@ -416,10 +411,11 @@ template <typename Real> int run_device(const ufair_desc* d, cudaStream_t stream
   if (rc != UFAIR_OK) return rc;
   if (d->n_member == 0 || d->n_t == 0) return UFAIR_OK;
   const KArgs<Real> a = make_args<Real>(d);
+  const Variant v = choose_variant(d, sizeof(Real));
 #ifdef UFAIR_DEBUG_BOUNDS
-  if (a.dbg_cut) return run_cut_control<Real>(d, a, stream);
+  if (a.dbg_cut) return run_cut_control<Real>(d, a, v, stream);
 #endif
-  return dispatch_gases<Real>(d, a, stream);
+  return dispatch<Real>(d, a, v, stream);
 }
 
 // ---- gas_form detection: which pools carry mass, which forcing terms exist, over all members -------
@@ -726,13 +722,11 @@ int ufair_kernel_variant(const ufair_desc* d, int32_t elem_size, uint32_t* form,
   if (elem_size != 8 && elem_size != 4) return set_error(UFAIR_ERR_ARG, "elem_size must be 8 or 4");
   const int rc = validate_desc(d, (size_t)elem_size);
   if (rc != UFAIR_OK) return rc;
-  const unsigned f = pick_form(d);
-  const int var = wants_inverse(d) ? (int)kVarInverse : plain_variant(d);
-  const int g = runtime_gases_per_lane(d, elem_size, f, var);
-  if (form) *form = f;
-  if (gpl) *gpl = g;
-  if (mw) *mw = members_per_warp(elem_size, d->n_gas, g);
-  if (loop) *loop = var;
+  const Variant v = choose_variant(d, elem_size);
+  if (form) *form = v.form;
+  if (gpl) *gpl = v.gpl;
+  if (mw) *mw = members_per_warp(elem_size, d->n_gas, v.gpl);
+  if (loop) *loop = v.loop;
   return UFAIR_OK;
 }
 

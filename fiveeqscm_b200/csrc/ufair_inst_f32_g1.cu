@@ -1,9 +1,5 @@
-// explicit instantiations of the fused integrator: float, 1 gas(es), all alpha modes, and the
-// specialised per-gas forms of the default (EXP) mode
+// the fused integrator's launchers and kernels for float, 1 gas(es): every alpha mode, loop and instantiated form
 #include "ufair_kernel.cuh"
 namespace ufair {
-UFAIR_DEFINE_LAUNCH_EXP(float, 1, UFAIR_TRY_FORM(float, 1, kForms1[0]) UFAIR_TRY_FORM(float, 1, kForms1[1]))
-UFAIR_DEFINE_LAUNCH(float, 1, UFAIR_ALPHA_SINH)
-UFAIR_DEFINE_LAUNCH(float, 1, UFAIR_ALPHA_NEWTON)
-UFAIR_DEFINE_LAUNCH(float, 1, UFAIR_ALPHA_ONE)
+UFAIR_INSTANTIATE(float, 1)
 }  // namespace ufair

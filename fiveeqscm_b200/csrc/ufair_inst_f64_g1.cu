@@ -1,9 +1,5 @@
-// explicit instantiations of the fused integrator: double, 1 gas(es), all alpha modes, and the
-// specialised per-gas forms of the default (EXP) mode
+// the fused integrator's launchers and kernels for double, 1 gas(es): every alpha mode, loop and instantiated form
 #include "ufair_kernel.cuh"
 namespace ufair {
-UFAIR_DEFINE_LAUNCH_EXP(double, 1, UFAIR_TRY_FORM(double, 1, kForms1[0]) UFAIR_TRY_FORM(double, 1, kForms1[1]))
-UFAIR_DEFINE_LAUNCH(double, 1, UFAIR_ALPHA_SINH)
-UFAIR_DEFINE_LAUNCH(double, 1, UFAIR_ALPHA_NEWTON)
-UFAIR_DEFINE_LAUNCH(double, 1, UFAIR_ALPHA_ONE)
+UFAIR_INSTANTIATE(double, 1)
 }  // namespace ufair

@@ -1,9 +1,5 @@
-// explicit instantiations of the fused integrator: double, 2 gas(es), all alpha modes, and the
-// specialised per-gas forms of the default (EXP) mode
+// the fused integrator's launchers and kernels for double, 2 gas(es): every alpha mode, loop and instantiated form
 #include "ufair_kernel.cuh"
 namespace ufair {
-UFAIR_DEFINE_LAUNCH_EXP(double, 2, UFAIR_TRY_FORM(double, 2, kForms2[0]))
-UFAIR_DEFINE_LAUNCH(double, 2, UFAIR_ALPHA_SINH)
-UFAIR_DEFINE_LAUNCH(double, 2, UFAIR_ALPHA_NEWTON)
-UFAIR_DEFINE_LAUNCH(double, 2, UFAIR_ALPHA_ONE)
+UFAIR_INSTANTIATE(double, 2)
 }  // namespace ufair

@@ -42,6 +42,8 @@
 //        569 instr per 32-member warp-step, 407 of them FP64, FP64 pipe 80 % (profiles/r2_final_summary.md).
 //   The loop body is alpha_val -> step_conc -> step_forc -> step_temp, the names the reference
 //   reserves in .coveragerc:12-19; `oxfair` is ONE launch.
+//   Which instantiation runs -- loop (VAR), lane mapping (GPL), per-gas form (FORM) -- is decided once per launch
+//   by choose_variant (end of this file); launch_integrate runs it and ufair_kernel_variant reports it.
 //
 // Memory system
 //   * per-member emissions [gas][t][member] are streamed into the warp's shared-memory ring one
@@ -64,18 +66,12 @@
 #include <cuda.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <utility>
 
 #include "../../include/ufair.h"
+#include "ufair_internal.h"
 #include "ufair_math.cuh"
 
-// 1: a lane integrates all gases of its member; 0: one gas per lane.  Round 1 measured a tie in FP64 on
-// dense parameters (35.3 vs 35.5 ms); round 2 found why -- the logarithm's special-case branch split every
-// gas into its own basic block, so the three gases of a lane never interleaved -- and with the branch-free
-// logarithm all gases per lane wins in FP64 too (31.3 -> 28.6 ms: no idle lanes, no shuffles, one thermal
-// step per member instead of three).  Small ensembles keep one gas per lane (see UFAIR_SMALL_ENSEMBLE).
-#ifndef UFAIR_GPL_ALL_F64
-#define UFAIR_GPL_ALL_F64 1
-#endif
 // FP64, default alpha mode: ensembles of at most this many members run one gas per lane (3.2x as many
 // warps: a 10^4-member ensemble fills a third of the GPU's schedulers with 32-member warps, all of them
 // with 10-member warps), larger ones all gases per lane.  Both give bit-identical results.  Measured (ms per
@@ -84,17 +80,11 @@
 #ifndef UFAIR_SMALL_ENSEMBLE
 #define UFAIR_SMALL_ENSEMBLE 100000
 #endif
-#ifndef UFAIR_GPL_ALL_F32
-#define UFAIR_GPL_ALL_F32 1
-#endif
 #ifndef UFAIR_WARPS
 #define UFAIR_WARPS 1  // warps per CTA.  A CTA is only a launch / shared-memory grouping (warps never
 #endif                 // synchronise); single-warp CTAs measured ~2 % faster than 4 (finer refill)
 #ifndef UFAIR_MINB_F64  // resident CTAs per SM the register allocator must allow, one gas per lane
 #define UFAIR_MINB_F64 (16 / UFAIR_WARPS)
-#endif
-#ifndef UFAIR_MINB_F32
-#define UFAIR_MINB_F32 (32 / UFAIR_WARPS)
 #endif
 #ifndef UFAIR_MINB_F64_GPLALL  // resident WARPS per SM, FP64 general kernel with all gases of a member in one lane:
 #define UFAIR_MINB_F64_GPLALL 8  // two per scheduler, every per-lane constant in registers (see UFAIR_REGCONST_GPLALL)
@@ -179,21 +169,27 @@ inline bool form_covers(unsigned have, unsigned want, int n_gas) {
       return false;
   return true;
 }
-// the specialised forms that are instantiated (alpha mode EXP only), most specific first
-constexpr unsigned kForms1[] = {pack_form(kGasOneLin), pack_form(kGasOneSqrt)};
-constexpr unsigned kForms2[] = {pack_form(kGasFull, kGasOneSqrt)};
-constexpr unsigned kForms3[] = {pack_form(kGasFull, kGasOneSqrt, kGasOneSqrt)};
-constexpr unsigned kForms4[] = {pack_form(kGasFull, kGasOneSqrt, kGasOneSqrt, kGasOneLin)};
-
-// gases a lane integrates: the dense kernels follow the UFAIR_GPL_ALL_* switches, a specialised
-// form always keeps a member's gases in one lane (the per-gas code differs, so it cannot share a warp
-// instruction stream across gases)
-constexpr int gases_per_lane(int elem_size, int n_gas, unsigned form = 0) {
-  return (form != 0 || (elem_size == 8 ? UFAIR_GPL_ALL_F64 : UFAIR_GPL_ALL_F32)) ? n_gas : 1;
+// the specialised forms that are instantiated, per gas count, most specific first; a row ends at its
+// first 0 (the dense kernel, never a specialised form)
+constexpr int kMaxForms = 2;
+constexpr unsigned kForms[UFAIR_MAX_GAS + 1][kMaxForms] = {
+    {},
+    {pack_form(kGasOneLin), pack_form(kGasOneSqrt)},
+    {pack_form(kGasFull, kGasOneSqrt)},
+    {pack_form(kGasFull, kGasOneSqrt, kGasOneSqrt)},
+    {pack_form(kGasFull, kGasOneSqrt, kGasOneSqrt, kGasOneLin)}};
+constexpr int n_forms(int n_gas) {
+  int n = 0;
+  while (n < kMaxForms && kForms[n_gas][n] != 0) ++n;
+  return n;
 }
-// the dense FP64 kernels of the default alpha mode also exist with one gas per lane, for small ensembles
+
+// A lane integrates all gases of its member: no idle lanes, no shuffles, one thermal step per member (with
+// the branch-free logarithm this wins in FP64 too, 31.3 -> 28.6 ms), and a specialised form must (its per-gas
+// code differs, so gases cannot share a warp's instruction stream).  The dense FP64 kernels of the default
+// alpha mode also exist with one gas per lane, for small ensembles (UFAIR_SMALL_ENSEMBLE).
 constexpr bool has_small_variant(int elem_size, int n_gas, int amode, int var) {
-  return elem_size == 8 && n_gas > 1 && UFAIR_GPL_ALL_F64 && amode == UFAIR_ALPHA_EXP && var != UFAIR_LOOP_CONC_DRIVEN;
+  return elem_size == 8 && n_gas > 1 && amode == UFAIR_ALPHA_EXP && var != UFAIR_LOOP_CONC_DRIVEN;
 }
 // members per warp: rows of MW elements must be a multiple of 16 bytes for the TMA box
 constexpr int members_per_warp(int elem_size, int n_gas, int gpl) {
@@ -374,7 +370,7 @@ template <typename Real, int NGAS, int AMODE, int GPL_, unsigned FORM = 0u> stru
 // resident CTAs per SM the register allocator must allow
 constexpr int min_blocks(int elem_size, int n_gas, int gpl, unsigned form) {
   if (form != 0) return (elem_size == 8 ? UFAIR_MINB_F64_FORM : UFAIR_MINB_F32_FORM) / UFAIR_WARPS;
-  if (elem_size == 4) return gpl == n_gas ? UFAIR_MINB_F32_GPLALL / UFAIR_WARPS : UFAIR_MINB_F32;
+  if (elem_size == 4) return UFAIR_MINB_F32_GPLALL / UFAIR_WARPS;
   return (gpl == n_gas && n_gas > 1) ? UFAIR_MINB_F64_GPLALL / UFAIR_WARPS : UFAIR_MINB_F64;
 }
 
@@ -664,12 +660,7 @@ __global__ void __launch_bounds__(kWarps * 32, min_blocks(sizeof(Real), NGAS, GP
         if (AMODE == UFAIR_ALPHA_NEWTON) {
           const Real iirf = (u - PARG(gl, WS::G_X0 + 1)) * PARG(gl, WS::G_X0);
           const Real invc = PARG(gl, WS::G_X0 + 2);
-#ifdef UFAIR_EXP_NEWTON_K  // experiment: what a compile-time (unrolled) iteration count is worth over the run-time
-#pragma unroll             // loop (measured, K = 3, configs[3] shard: 90.1 -> 87.6 ms)
-          for (int it = 0; it < UFAIR_EXP_NEWTON_K; ++it) {
-#else
           for (int it = 0; it < a.newton_iters; ++it) {
-#endif
             const Real ia = M::rcp(al);
             Real f = -iirf, fp = 0;
 #pragma unroll
@@ -847,15 +838,11 @@ __global__ void __launch_bounds__(kWarps * 32, min_blocks(sizeof(Real), NGAS, GP
 #undef SETT
 }
 
-// ---- launchers: one per (Real, NGAS, AMODE), defined in ufair_inst_*.cu ----------------------------
+// ---- the choice of instantiation, and its launch ----------------------------------------------------
 int make_tensor_maps(const ufair_desc* d, size_t elem, int mw_members, int tile_steps, CUtensorMap* tmE,
                      CUtensorMap* tmF);
-int cuda_error(cudaError_t e, const char* what);
 
-template <typename Real, int NGAS, int AMODE>
-int launch_integrate(const ufair_desc* d, const KArgs<Real>& a, cudaStream_t stream);
-
-template <typename Real, int NGAS, int AMODE, int GPL, unsigned FORM, int VAR = kVarGeneral>
+template <typename Real, int NGAS, int AMODE, int GPL, unsigned FORM, int VAR>
 int launch_variant(const ufair_desc* d, const KArgs<Real>& a, cudaStream_t stream) {
   using WS = WarpSmem<Real, NGAS, AMODE, GPL, FORM>;
   CUtensorMap tmE, tmF;  // box = WS::MW members x WS::TT steps (x NGAS gases): depends on the variant
@@ -880,73 +867,92 @@ inline unsigned requested_form(const ufair_desc* d) {
   return f;
 }
 
-// the instantiated form the dispatcher uses for this descriptor (0 = the dense kernel)
 // concentration-driven gases / the emissions output run on the INV instantiation of the general kernel
 inline bool wants_inverse(const ufair_desc* d) { return d->conc_driven != 0 || (d->out_mask & UFAIR_OUT_E) != 0; }
-// the plain configurations: no iIRF ceiling, outputs among C, RF, T only, emission-driven.  All three
-// outputs: without external forcing (kVarPlain, every alpha mode) or with it (kVarPlainFx, default
-// alpha mode); a subset of them: kVarPlainSub (default alpha mode)
-inline int plain_variant(const ufair_desc* d) {
-  if ((d->iirf_max > 0.0 && isfinite(d->iirf_max)) || d->conc_driven != 0 ||
-      (d->out_mask & (UFAIR_OUT_ALPHA | UFAIR_OUT_E)) != 0)
-    return kVarGeneral;
+
+// the loops each alpha mode has: the plain loops with external forcing (kVarPlainFx) or with a subset of
+// the outputs (kVarPlainSub) exist in the default alpha mode only ...
+constexpr bool loop_instantiated(int amode, int loop) {
+  return amode == UFAIR_ALPHA_EXP || (loop != kVarPlainFx && loop != kVarPlainSub);
+}
+// ... and so do the specialised forms, for every loop but the inverse one
+constexpr bool forms_instantiated(int amode, int loop) { return amode == UFAIR_ALPHA_EXP && loop != kVarInverse; }
+
+// which instantiation of ufair_integrate_kernel runs a descriptor (EMEM follows e_mode)
+struct Variant {
+  unsigned form;  // FORM: an entry of kForms[n_gas], 0 = the dense kernel
+  int loop;       // VAR: kVar* = UFAIR_LOOP_*
+  int gpl;        // GPL: gases per lane, 1 or n_gas
+};
+
+// The only statement of the choice: run_device launches it and ufair_kernel_variant reports it.
+inline Variant choose_variant(const ufair_desc* d, int elem_size) {
+  // the plain loops: no iIRF ceiling, outputs among C, RF, T only, emission-driven
   const int crt = UFAIR_OUT_C | UFAIR_OUT_RF | UFAIR_OUT_T;
-  if ((d->out_mask & crt) != crt) return d->alpha_mode == UFAIR_ALPHA_EXP ? kVarPlainSub : kVarGeneral;
-  if (d->fext_mode == UFAIR_FEXT_NONE) return kVarPlain;
-  return d->alpha_mode == UFAIR_ALPHA_EXP ? kVarPlainFx : kVarGeneral;
-}
-
-inline unsigned pick_form(const ufair_desc* d) {
+  int loop = wants_inverse(d) ? kVarInverse
+             : ((d->iirf_max > 0.0 && isfinite(d->iirf_max)) || (d->out_mask & UFAIR_OUT_ALPHA)) ? kVarGeneral
+             : (d->out_mask & crt) != crt ? kVarPlainSub
+             : d->fext_mode == UFAIR_FEXT_NONE ? kVarPlain
+                                              : kVarPlainFx;
+  if (!loop_instantiated(d->alpha_mode, loop)) loop = kVarGeneral;
+  unsigned form = 0;  // the first instantiated form that covers the requested one
   const unsigned want = requested_form(d);
-  if (want == 0 || d->alpha_mode != UFAIR_ALPHA_EXP || wants_inverse(d)) return 0;
-  const unsigned* tab = d->n_gas == 1 ? kForms1 : d->n_gas == 2 ? kForms2 : d->n_gas == 3 ? kForms3 : kForms4;
-  const int n = d->n_gas == 1 ? (int)(sizeof(kForms1) / sizeof(unsigned)) : 1;
-  for (int k = 0; k < n; ++k)
-    if (form_covers(tab[k], want, d->n_gas)) return tab[k];
-  return 0;
+  if (want != 0 && forms_instantiated(d->alpha_mode, loop))
+    for (int k = 0; k < n_forms(d->n_gas) && form == 0; ++k)
+      if (form_covers(kForms[d->n_gas][k], want, d->n_gas)) form = kForms[d->n_gas][k];
+  const bool small = form == 0 && has_small_variant(elem_size, d->n_gas, d->alpha_mode, loop) &&
+                     d->n_member <= UFAIR_SMALL_ENSEMBLE;
+  return {form, loop, small ? 1 : d->n_gas};
 }
 
-// dense kernels: all gases per lane, or -- small FP64 ensembles in the default alpha mode -- one gas per lane
-template <typename Real, int NGAS, int AMODE, int VAR> int launch_dense(const ufair_desc* d, const KArgs<Real>& a, cudaStream_t stream) {
-  if constexpr (has_small_variant(sizeof(Real), NGAS, AMODE, VAR)) {
-    if (d->n_member <= UFAIR_SMALL_ENSEMBLE) return launch_variant<Real, NGAS, AMODE, 1, 0u, VAR>(d, a, stream);
-  }
-  return launch_variant<Real, NGAS, AMODE, gases_per_lane(sizeof(Real), NGAS), 0u, VAR>(d, a, stream);
+// launches <GPL, FORM, LOOP> if that is v
+template <typename Real, int NGAS, int AMODE, int LOOP, int GPL, unsigned FORM>
+bool launch_if(const ufair_desc* d, const KArgs<Real>& a, Variant v, cudaStream_t stream, int& rc) {
+  if (v.loop != LOOP || v.gpl != GPL || v.form != FORM) return false;
+  rc = launch_variant<Real, NGAS, AMODE, GPL, FORM, LOOP>(d, a, stream);
+  return true;
 }
-// the lane mapping launch_integrate picks for this descriptor (ufair_kernel_variant reports it)
-inline int runtime_gases_per_lane(const ufair_desc* d, int elem_size, unsigned form, int var) {
-  if (form == 0 && has_small_variant(elem_size, d->n_gas, d->alpha_mode, var) && d->n_member <= UFAIR_SMALL_ENSEMBLE) return 1;
-  return gases_per_lane(elem_size, d->n_gas, form);
+// the instantiations of one loop: dense with one gas per lane, dense with all of them, and the forms kForms[NGAS][K]
+template <typename Real, int NGAS, int AMODE, int LOOP, size_t... K>
+bool launch_loop(const ufair_desc* d, const KArgs<Real>& a, Variant v, cudaStream_t stream, int& rc,
+                 std::index_sequence<K...>) {
+  if constexpr (loop_instantiated(AMODE, LOOP)) {
+    if constexpr (has_small_variant(sizeof(Real), NGAS, AMODE, LOOP))
+      if (launch_if<Real, NGAS, AMODE, LOOP, 1, 0u>(d, a, v, stream, rc)) return true;
+    return launch_if<Real, NGAS, AMODE, LOOP, NGAS, 0u>(d, a, v, stream, rc) ||
+           (launch_if<Real, NGAS, AMODE, LOOP, NGAS, kForms[NGAS][K]>(d, a, v, stream, rc) || ...);
+  }
+  return false;
+}
+// every instantiation of one (Real, NGAS, AMODE) in turn: exactly those choose_variant can return; one that is
+// not there is an error, never another kernel
+template <typename Real, int NGAS, int AMODE, int... LOOP>
+int launch_chosen(const ufair_desc* d, const KArgs<Real>& a, Variant v, cudaStream_t stream,
+                  std::integer_sequence<int, LOOP...>) {
+  int rc = UFAIR_OK;
+  if ((launch_loop<Real, NGAS, AMODE, LOOP>(
+           d, a, v, stream, rc, std::make_index_sequence<forms_instantiated(AMODE, LOOP) ? n_forms(NGAS) : 0>()) ||
+       ...))
+    return rc;
+  return set_error(UFAIR_ERR_UNSUPPORTED, "no integrator for %d gases, alpha mode %d, form 0x%x, %d gases per lane, loop %d",
+                   NGAS, AMODE, v.form, v.gpl, v.loop);
 }
 
-// dense launcher, and the specialised forms of the EXP alpha mode when the descriptor's gas_form allows
-#define UFAIR_TRY_FORM(Real, NGAS, F)                                                                  \
-  if (form == F) {                                                                                     \
-    if (var == kVarPlain) return launch_variant<Real, NGAS, UFAIR_ALPHA_EXP, NGAS, F, kVarPlain>(d, a, stream); \
-    if (var == kVarPlainFx) return launch_variant<Real, NGAS, UFAIR_ALPHA_EXP, NGAS, F, kVarPlainFx>(d, a, stream); \
-    if (var == kVarPlainSub) return launch_variant<Real, NGAS, UFAIR_ALPHA_EXP, NGAS, F, kVarPlainSub>(d, a, stream); \
-    return launch_variant<Real, NGAS, UFAIR_ALPHA_EXP, NGAS, F>(d, a, stream);                         \
-  }
+// The launcher of one (precision, gas count, alpha mode): runs the instantiation v names.  UFAIR_INSTANTIATE
+// defines the four of a (precision, gas count), one ufair_inst_*.cu each, so the kernels compile in parallel.
+template <typename Real, int NGAS, int AMODE>
+int launch_integrate(const ufair_desc* d, const KArgs<Real>& a, Variant v, cudaStream_t stream);
 
-#define UFAIR_DEFINE_LAUNCH_EXP(Real, NGAS, TRY_FORMS)                                                 \
-  template <> int launch_integrate<Real, NGAS, UFAIR_ALPHA_EXP>(const ufair_desc* d, const KArgs<Real>& a, \
-                                                                cudaStream_t stream) {                 \
-    const unsigned form = pick_form(d);                                                                \
-    const int var = plain_variant(d);                                                                  \
-    TRY_FORMS                                                                                          \
-    if (wants_inverse(d)) return launch_dense<Real, NGAS, UFAIR_ALPHA_EXP, kVarInverse>(d, a, stream);    \
-    if (var == kVarPlain) return launch_dense<Real, NGAS, UFAIR_ALPHA_EXP, kVarPlain>(d, a, stream);       \
-    if (var == kVarPlainFx) return launch_dense<Real, NGAS, UFAIR_ALPHA_EXP, kVarPlainFx>(d, a, stream);   \
-    if (var == kVarPlainSub) return launch_dense<Real, NGAS, UFAIR_ALPHA_EXP, kVarPlainSub>(d, a, stream); \
-    return launch_dense<Real, NGAS, UFAIR_ALPHA_EXP, kVarGeneral>(d, a, stream);                           \
+#define UFAIR_LAUNCHER(Real, NGAS, AMODE)                                                                   \
+  template <>                                                                                               \
+  int launch_integrate<Real, NGAS, AMODE>(const ufair_desc* d, const KArgs<Real>& a, Variant v, cudaStream_t s) { \
+    return launch_chosen<Real, NGAS, AMODE>(                                                                \
+        d, a, v, s, std::integer_sequence<int, kVarGeneral, kVarInverse, kVarPlain, kVarPlainFx, kVarPlainSub>()); \
   }
-
-#define UFAIR_DEFINE_LAUNCH(Real, NGAS, AMODE)                                                         \
-  template <> int launch_integrate<Real, NGAS, AMODE>(const ufair_desc* d, const KArgs<Real>& a,       \
-                                                      cudaStream_t stream) {                           \
-    if (wants_inverse(d)) return launch_dense<Real, NGAS, AMODE, kVarInverse>(d, a, stream);            \
-    if (plain_variant(d) == kVarPlain) return launch_dense<Real, NGAS, AMODE, kVarPlain>(d, a, stream); \
-    return launch_dense<Real, NGAS, AMODE, kVarGeneral>(d, a, stream);                                  \
-  }
+#define UFAIR_INSTANTIATE(Real, NGAS)                                                                       \
+  UFAIR_LAUNCHER(Real, NGAS, UFAIR_ALPHA_EXP)                                                               \
+  UFAIR_LAUNCHER(Real, NGAS, UFAIR_ALPHA_SINH)                                                              \
+  UFAIR_LAUNCHER(Real, NGAS, UFAIR_ALPHA_NEWTON)                                                            \
+  UFAIR_LAUNCHER(Real, NGAS, UFAIR_ALPHA_ONE)
 
 }  // namespace ufair

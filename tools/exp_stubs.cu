@@ -2,10 +2,9 @@
 // integrator instantiation except <double, 3 gases>, so that a tuning variant of the headline kernel
 // links in seconds.  Usage: see tools/build_variant.sh.
 #include "../fiveeqscm_b200/csrc/ufair_kernel.cuh"
-#include "../fiveeqscm_b200/csrc/ufair_internal.h"
 namespace ufair {
 #define STUB(Real, NGAS, AMODE)                                                                        \
-  template <> int launch_integrate<Real, NGAS, AMODE>(const ufair_desc*, const KArgs<Real>&, cudaStream_t) { \
+  template <> int launch_integrate<Real, NGAS, AMODE>(const ufair_desc*, const KArgs<Real>&, Variant, cudaStream_t) { \
     return set_error(UFAIR_ERR_UNSUPPORTED, "experiment build: only <double, 3 gases> is instantiated"); \
   }
 #define STUB4(Real, NGAS) STUB(Real, NGAS, UFAIR_ALPHA_EXP) STUB(Real, NGAS, UFAIR_ALPHA_SINH) STUB(Real, NGAS, UFAIR_ALPHA_NEWTON) STUB(Real, NGAS, UFAIR_ALPHA_ONE)
