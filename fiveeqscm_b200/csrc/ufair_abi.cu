@@ -158,8 +158,8 @@ static EncodeTiledFn encode_tiled() {
   return fn;
 }
 
-// emissions [n_gas][n_t][ld] -> rank-3 map, box = MW members x kTT steps x n_gas gases;
-// f_ext [n_t][ld] -> rank-2 map, box = MW x kTT.  Out-of-range parts of a box are zero-filled.
+// emissions [n_gas][n_t][ld] -> rank-3 map, box = MW members x tile_steps steps x n_gas gases;
+// f_ext [n_t][ld] -> rank-2 map, box = MW x tile_steps.  Out-of-range parts of a box are zero-filled.
 int make_tensor_maps(const ufair_desc* d, size_t elem, int mw_members, int tile_steps, CUtensorMap* tmE,
                      CUtensorMap* tmF) {
   memset(tmE, 0, sizeof(*tmE));

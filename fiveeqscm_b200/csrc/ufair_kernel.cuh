@@ -11,8 +11,9 @@
 //                                          which is what small FP64 ensembles in the default alpha mode need).
 //   Pools, cumulative emissions and the two thermal boxes stay in REGISTERS across the serial time
 //   loop.  The derived per-member constants sit in registers too where the register budget allows (all of
-//   them in the FP64 all-gases-per-lane kernels: 226-230 registers, 8 warps per SM; see UFAIR_REGCONST*), and
-//   otherwise in shared memory ([param][lane], conflict-free LDS.64 at base + immediate).
+//   them in the FP64 kernels: 226-230 registers at 8 warps per SM in the all-gases-per-lane ones), and
+//   otherwise in shared memory ([param][lane], conflict-free LDS.64 at base + immediate).  Which ones, the
+//   tile length and the occupancy target of each class of kernel are one row of kTuning; LaneConsts places them.
 //   Why: the loop is chains of dependent DFMAs (Horner polynomials); it is bound by the warp
 //   schedulers' issue rate and dependent-issue latency, not by HBM.  ncu history (profiles/):
 //     v1 thread per member, everything in regs (255), 2 warps/SMSP: FP64 pipe 35 %, IPC 0.37
@@ -83,63 +84,10 @@
 #ifndef UFAIR_WARPS
 #define UFAIR_WARPS 1  // warps per CTA.  A CTA is only a launch / shared-memory grouping (warps never
 #endif                 // synchronise); single-warp CTAs measured ~2 % faster than 4 (finer refill)
-#ifndef UFAIR_MINB_F64  // resident CTAs per SM the register allocator must allow, one gas per lane
-#define UFAIR_MINB_F64 (16 / UFAIR_WARPS)
-#endif
-#ifndef UFAIR_MINB_F64_GPLALL  // resident WARPS per SM, FP64 general kernel with all gases of a member in one lane:
-#define UFAIR_MINB_F64_GPLALL 8  // two per scheduler, every per-lane constant in registers (see UFAIR_REGCONST_GPLALL)
-#endif
-#ifndef UFAIR_MINB_F64_FORM  // resident WARPS per SM for the specialised (per-gas form) kernels
-#define UFAIR_MINB_F64_FORM 10
-#endif
-#ifndef UFAIR_MINB_F32_FORM
-#define UFAIR_MINB_F32_FORM 16
-#endif
-// which per-lane constants of the FP64 one-gas-per-lane kernels live in REGISTERS instead of shared
-// memory (bit 0: the five alpha_val constants, bit 1: the eight pool constants, bit 2: the four
-// thermal constants): fewer LDS against more registers.  Measured on the plain kernel (ms per
-// launch, [REGCONST, resident warps/SM]): [0,20] 34.5, [2,20] 34.0, [2,18] 33.8, [6,18] 33.4,
-// [3,18] 33.0, [7,18] 33.2 (spills), [7,16] 32.6 (118 registers, 229 instructions per warp-step).
-#ifndef UFAIR_REGCONST
-#define UFAIR_REGCONST 7
-#endif
-// the same switch for the FP32 general kernels (all gases of a member in one lane; their alpha_val
-// constants are in registers anyway), and the resident warps/SM their register budget is set for.
-// Measured (ms per launch, [REGCONST_F32, warps/SM]): [0,16] 9.7, [2,16] 9.7, [6,16] 9.5, [2,12] 9.3,
-// [6,12] 9.1 (128 registers, 295 instructions per 32-member warp-step).
-#ifndef UFAIR_REGCONST_F32
-#define UFAIR_REGCONST_F32 6
-#endif
-// ... and for the FP64 specialised-form kernels.  Measured (literature parameters, ms per launch,
-// [REGCONST_FORM, warps/SM]): [0,12] 19.8-20.4, [2,12] 19.6, [6,12] 19.6, [7,10] 19.0 (157 registers).
-#ifndef UFAIR_REGCONST_FORM
-#define UFAIR_REGCONST_FORM 7
-#endif
-#ifndef UFAIR_MINB_F32_GPLALL
-#define UFAIR_MINB_F32_GPLALL 12
-#endif
-// ... and for the FP64 dense kernels with all gases of a member in one lane.  Occupancy buys nothing here --
-// 16, 14, 12, 10 and 8 resident warps per SM were all measured, and what sets the time is the length of each
-// warp's own instruction stream -- so the constants go to registers as far as the 255-register limit allows.
-// Measured (ms per launch, [REGCONST, warps/SM]): [0,16] 29.5, [0,12] 29.2, [4,12] 29.1, [5,12] 28.3, [5,10] 27.5,
-// [6,8] 28.0, [7,8] 27.0 (226 registers: alpha_val, pool and thermal constants all in registers; 21 LDS per step left).
-#ifndef UFAIR_REGCONST_GPLALL
-#define UFAIR_REGCONST_GPLALL 7
-#endif
-#ifndef UFAIR_TT
-#define UFAIR_TT 8  // time steps per shared-memory tile (8 measured ~2 % faster than 4)
-#endif
-#ifndef UFAIR_TT_FORM  // ... for the specialised-form kernels (32 members per warp: their tiles are 3.2x as
-#define UFAIR_TT_FORM 2  // wide, and shared memory, not registers, would otherwise cap their occupancy)
-#endif
-#ifndef UFAIR_TT_GPLALL  // ... and for the dense FP64 kernels with all gases of a member in one lane (at 8 warps per
-#define UFAIR_TT_GPLALL 8  // SM shared memory is no constraint; measured 1 step 27.1 ms, 2: 27.2, 4: 26.8, 8: 26.5)
-#endif
 
 namespace ufair {
 
 constexpr int kWarps = UFAIR_WARPS;
-constexpr int kTT = UFAIR_TT;
 constexpr int kStages = 2;  // tile ring depth
 
 // ---- per-gas specialisation ("form"): 8 bits per gas, the descriptor's gas_form byte ------------
@@ -303,9 +251,9 @@ template <typename Real> __device__ __forceinline__ void st_stream(Real* p, Real
 #define UFAIR_CHECK_RING(addr, ring0, stage_bytes, box_bytes) ((void)0)
 #endif
 
-// per-lane derived constants.  Rows G_* exist once per gas the lane integrates; the five `hot` ones
-// (needed first in a step, on the critical path into alpha) live in registers when a lane carries
-// several gases and in shared memory otherwise.  T_* rows exist once per lane.
+// per-lane derived constants, by logical row: the G_* rows once per gas the lane integrates, the T_* rows once
+// per lane.  Where each one lives is LaneConsts' business (below).
+enum { H_RHO0 = 0, H_RHOU, H_WR, H_RHOT, H_UMAX, H_COUNT };  // u = rho0 + rhoU Gcum + wR sumR + rhoT T, capped at umax
 enum {
   G_KA0 = 0,  // c a_i tau_i: equilibrium pool per unit (E alpha)
   G_K0 = 4,   // dt / tau_i   (ALPHA_ONE: m_i = 1 - exp(-dt/tau_i))
@@ -315,32 +263,73 @@ enum {
   G_F1,
   G_F2,
   G_F3,
-  G_COLD  // = 14
+  G_HOT,                  // = 14: alpha_val's five, needed first in a step (on the critical path into alpha)
+  G_X0 = G_HOT + H_COUNT  // SINH: g0; NEWTON: g1, ln g0, 1/c
 };
-enum { H_RHO0 = 0, H_RHOU, H_WR, H_RHOT, H_UMAX, H_COUNT };  // u = rho0 + rhoU Gcum + wR sumR + rhoT T
-enum { T_QM0 = 0, T_QM1, T_DEC0, T_DEC1, T_COUNT };          // q_j (1 - e^{-dt/d_j}),  e^{-dt/d_j}
+enum { T_QM0 = 0, T_QM1, T_DEC0, T_DEC1, T_COUNT };  // q_j (1 - e^{-dt/d_j}),  e^{-dt/d_j}
+
+// ---- per-instantiation tuning: one row per class of kernel ---------------------------------------------
+// A class is a precision, dense or specialised form, and one gas or several per lane (GPL is 1 or NGAS, so the
+// one-gas kernels -- NGAS = 1, or the FP64 small-ensemble mapping -- share a row).  A row gives the time steps per
+// shared-memory tile, the resident warps per SM the register allocator must allow (__launch_bounds__), and which
+// per-lane constants live in registers instead of shared memory -- the five alpha_val ones, the eight pool ones
+// (G_KA0.., G_K0..), the four thermal ones: fewer LDS against more registers.  A tuning experiment edits one row.
+// Measurements are ms per launch at [constants in registers (a alpha_val, p pools, t thermal, - none), warps/SM].
+struct Tuning {
+  int tile_steps;
+  int warps_per_sm;
+  bool alpha_reg, pool_reg, therm_reg;
+  constexpr int min_blocks() const { return warps_per_sm / kWarps; }  // __launch_bounds__ counts CTAs
+};
+// classes by precision, then dense / specialised form, then several gases / one gas per lane
+enum { kF64Dense, kF64Dense1, kF64Form, kF64Form1, kF32Dense, kF32Dense1, kF32Form, kF32Form1, kClasses };
+constexpr int tuning_class(int elem_size, int gpl, unsigned form) {
+  return (elem_size == 8 ? 0 : 4) + (form != 0 ? 2 : 0) + (gpl == 1 ? 1 : 0);
+}
+constexpr Tuning kTuning[kClasses] = {
+    // kF64Dense: all gases of a member in one lane, 2-4 gases.  Occupancy buys nothing here -- 16, 14, 12, 10 and
+    // 8 resident warps per SM were all measured, and what sets the time is the length of each warp's own
+    // instruction stream -- so the constants go to registers as far as the 255-register limit allows: [-,16] 29.5,
+    // [-,12] 29.2, [t,12] 29.1, [at,12] 28.3, [at,10] 27.5, [pt,8] 28.0, [apt,8] 27.0 (226 registers; 21 LDS per
+    // step left).  At 8 warps per SM shared memory is no constraint on the tile: 1 step 27.1 ms, 2: 27.2, 4: 26.8,
+    // 8: 26.5.
+    {8, 8, true, true, true},
+    // kF64Dense1: one gas per lane (the small-ensemble mapping, and NGAS = 1).  Measured on the plain kernel:
+    // [-,20] 34.5, [p,20] 34.0, [p,18] 33.8, [pt,18] 33.4, [ap,18] 33.0, [apt,18] 33.2 (spills), [apt,16] 32.6
+    // (118 registers, 229 instructions per warp-step); 8-step tiles measured ~2 % faster than 4.
+    {8, 16, true, true, true},
+    // kF64Form: specialised forms, 2-4 gases.  Literature parameters: [-,12] 19.8-20.4, [p,12] 19.6, [pt,12] 19.6,
+    // [apt,10] 19.0 (157 registers).  Short tiles: with 32 members per warp they are 3.2x as wide as the one-gas-
+    // per-lane kernel's, and shared memory, not registers, would otherwise cap the occupancy.
+    {2, 10, true, true, true},
+    // kF64Form1: specialised forms of one gas: the row above with 8-step tiles (not measured on its own)
+    {8, 10, true, true, true},
+    // kF32Dense: 2-4 gases: [a,16] 9.7, [ap,16] 9.7, [apt,16] 9.5, [ap,12] 9.3, [apt,12] 9.1 (128 registers, 295
+    // instructions per 32-member warp-step)
+    {8, 12, true, true, true},
+    // kF32Dense1: one gas: every constant in shared memory (not measured on its own)
+    {8, 12, false, false, false},
+    // kF32Form: specialised forms, 2-4 gases
+    {8, 16, true, false, false},
+    // kF32Form1: specialised forms of one gas: every constant in shared memory (not measured on its own)
+    {8, 16, false, false, false}};
+constexpr Tuning tuning(int elem_size, int gpl, unsigned form) { return kTuning[tuning_class(elem_size, gpl, form)]; }
 
 constexpr int extra_rows(int amode) { return amode == UFAIR_ALPHA_NEWTON ? 3 : (amode == UFAIR_ALPHA_SINH ? 1 : 0); }
 constexpr size_t round128(size_t b) { return (b + 127) / 128 * 128; }
 
 // parameter rows of one gas when only its first `np` pools exist (the absent pools' KA / K0 rows are
-// not allocated), and the compact row of logical row k (the G_* / hot / extra numbering above)
+// not allocated), and the compact row of row k of the per-gas block (LaneConsts::slot)
 __host__ __device__ constexpr int gas_rows(int pg, int np) { return pg - 2 * (4 - np); }
 __host__ __device__ constexpr int compact_row(int np, int k) { return k < 4 ? k : (k < 8 ? np + (k - 4) : 2 * np + (k - 8)); }
 
 // per-WARP shared memory, in bytes (every piece 128-byte aligned: tensor-map TMA destinations)
-template <typename Real, int NGAS, int AMODE, int GPL_, unsigned FORM = 0u> struct WarpSmem {
-  static constexpr int GPL = GPL_;
-  // time steps per tile: short tiles wherever an FP64 lane carries several gases (32 members per warp)
-  static constexpr int TT = (sizeof(Real) == 8 && GPL_ > 1) ? (FORM != 0 ? UFAIR_TT_FORM : UFAIR_TT_GPLALL) : kTT;
-  // which constants live in registers (bit 0 alpha_val, bit 1 pools, bit 2 thermal): see UFAIR_REGCONST*
-  static constexpr int RCM = sizeof(Real) == 4 ? ((FORM == 0 && GPL_ > 1) ? UFAIR_REGCONST_F32 : 0)
-                             : (GPL_ == 1 ? UFAIR_REGCONST : (FORM != 0 ? UFAIR_REGCONST_FORM : UFAIR_REGCONST_GPLALL));
-  static constexpr bool HOT_SMEM = ((GPL == 1) || sizeof(Real) == 8) && !(RCM & 1);
+template <typename Real, int NGAS, int AMODE, int GPL, unsigned FORM = 0u> struct WarpSmem {
+  static constexpr Tuning TUNE = tuning(sizeof(Real), GPL, FORM);
+  static constexpr int TT = TUNE.tile_steps;  // time steps per tile
   static constexpr int MW = members_per_warp(sizeof(Real), NGAS, GPL);
-  static constexpr int G_HOT = G_COLD;                            // first hot row (if in smem)
-  static constexpr int G_X0 = G_COLD + (HOT_SMEM ? H_COUNT : 0);  // SINH: g0; NEWTON: g1, ln g0, 1/c
-  static constexpr int PG = G_X0 + extra_rows(AMODE);             // rows per gas
+  // rows per gas: register-resident alpha_val constants own none
+  static constexpr int PG = G_X0 - (TUNE.alpha_reg ? H_COUNT : 0) + extra_rows(AMODE);
   // first row of gas gl / of the thermal block, and the row of logical row k of gas gl
   static __host__ __device__ constexpr int gas_base(int gl) {
     int b = 0;
@@ -367,12 +356,77 @@ template <typename Real, int NGAS, int AMODE, int GPL_, unsigned FORM = 0u> stru
   static __host__ __device__ constexpr uint32_t bytes(bool fx_member) { return off_bar(fx_member) + 128u; }
 };
 
-// resident CTAs per SM the register allocator must allow
-constexpr int min_blocks(int elem_size, int n_gas, int gpl, unsigned form) {
-  if (form != 0) return (elem_size == 8 ? UFAIR_MINB_F64_FORM : UFAIR_MINB_F32_FORM) / UFAIR_WARPS;
-  if (elem_size == 4) return UFAIR_MINB_F32_GPLALL / UFAIR_WARPS;
-  return (gpl == n_gas && n_gas > 1) ? UFAIR_MINB_F64_GPLALL / UFAIR_WARPS : UFAIR_MINB_F64;
-}
+// One lane's per-lane constants: its column of the warp's parameter block ([row][lane] in shared memory) and its
+// register copies (the kernel's own arrays, declared where the compiler has always seen them).  The prologue sets
+// each gas constant once through at(), the step reads every constant through get() / get_t(), both by logical row;
+// which constants sit in registers is decided here and nowhere else:
+//   * a register-resident alpha_val constant is set directly and owns no shared-memory row;
+//   * register-resident pool and thermal constants still own a row: the prologue writes them there and load(),
+//     after the prologue's __syncwarp, reads them into registers once;
+//   * any other constant is read from its row at every use.
+// The thermal constants are written to their rows (T_BASE + k) by the prologue itself: they own a row in every
+// kernel, so there is nothing to decide, and through any helper call the FP32 specialised-form kernels compile to
+// different code.
+// A gas constant is named by a row K and an offset q inside K's block (the pool index for G_KA0 / G_K0, H_* for
+// G_HOT, the position after G_X0).  Only K decides where it lives: K is a constant at every call site, and q, a
+// loop index there, must not enter the decision -- it would stay a run-time test until the loops are unrolled
+// and change how the compiler unrolls the Newton iteration around them.  at() returns the place before the value
+// is computed, as a plain store computes its address first: a setter taking the value as an argument reorders the
+// prologue (and changes the code of the FP32 sinh kernels).
+template <typename Real, int NGAS, int AMODE, int GPL, unsigned FORM> struct LaneConsts {
+  using WS = WarpSmem<Real, NGAS, AMODE, GPL, FORM>;
+  static constexpr bool kAlphaReg = WS::TUNE.alpha_reg, kPoolReg = WS::TUNE.pool_reg, kThermReg = WS::TUNE.therm_reg;
+  uint32_t col;  // row 0 of this lane's column
+  // register copies; only the rows in_reg() names are used, and of k0 / ka only the lane's pools (q < NP)
+  Real (&hot)[GPL][H_COUNT];
+  Real (&k0)[GPL][4];
+  Real (&ka)[GPL][4];
+  Real (&t)[T_COUNT];
+
+  static __device__ __forceinline__ constexpr bool in_reg(int K) {
+    return (K == G_HOT) ? kAlphaReg : (K == G_KA0 || K == G_K0) && kPoolReg;
+  }
+  // shared-memory row of logical gas row K: without alpha_val rows the extra rows move up
+  static __device__ __forceinline__ constexpr int slot(int K) { return (kAlphaReg && K >= G_X0) ? K - H_COUNT : K; }
+  __device__ __forceinline__ uint32_t gas_addr(int gl, int K, int q) const {
+    return col + (uint32_t)WS::row(gl, slot(K) + q) * 32u * (uint32_t)sizeof(Real);
+  }
+  __device__ __forceinline__ uint32_t therm_addr(int k) const {
+    return col + (uint32_t)(WS::T_BASE + k) * 32u * (uint32_t)sizeof(Real);
+  }
+  __device__ __forceinline__ Real reg(int gl, int K, int q) const {
+    return K == G_HOT ? hot[gl][q] : K == G_KA0 ? ka[gl][q] : k0[gl][q];
+  }
+
+  struct Place {
+    Real* reg;
+    uint32_t addr;
+    template <typename V> __device__ __forceinline__ void set(V v) const {
+      if (reg)
+        *reg = (Real)v;
+      else
+        sts(addr, (Real)v);
+    }
+  };
+  __device__ __forceinline__ Place at(int gl, int K, int q = 0) {
+    return (K == G_HOT && kAlphaReg) ? Place{&hot[gl][q], 0u} : Place{nullptr, gas_addr(gl, K, q)};
+  }
+  __device__ __forceinline__ void load() {
+#pragma unroll
+    for (int gl = 0; gl < GPL; ++gl)
+#pragma unroll
+      for (int q = 0; q < 4; ++q) {
+        k0[gl][q] = (kPoolReg && q < form_pools(FORM, gl)) ? lds(gas_addr(gl, G_K0, q), Real()) : Real(0);
+        ka[gl][q] = (kPoolReg && q < form_pools(FORM, gl)) ? lds(gas_addr(gl, G_KA0, q), Real()) : Real(0);
+      }
+#pragma unroll
+    for (int k = 0; k < T_COUNT; ++k) t[k] = kThermReg ? lds(therm_addr(k), Real()) : Real(0);
+  }
+  __device__ __forceinline__ Real get(int gl, int K, int q = 0) const {
+    return in_reg(K) ? reg(gl, K, q) : lds(gas_addr(gl, K, q), Real());
+  }
+  __device__ __forceinline__ Real get_t(int k) const { return kThermReg ? t[k] : lds(therm_addr(k), Real()); }
+};
 
 // EMEM: per-member emissions (TMA-staged tile) vs scenario-shared (read-only path + register prefetch)
 // pool sum in the dense kernel's association, (R1 + R2) + (R3 + R4), without the absent pools
@@ -393,21 +447,19 @@ template <typename Real> __device__ __forceinline__ Real sum_pools(const Real (&
 // fixed before the loop; external forcing optional; default alpha mode only)
 enum { kVarGeneral = UFAIR_LOOP_GENERAL, kVarInverse = UFAIR_LOOP_CONC_DRIVEN, kVarPlain = UFAIR_LOOP_PLAIN,
        kVarPlainFx = UFAIR_LOOP_PLAIN_FEXT, kVarPlainSub = UFAIR_LOOP_PLAIN_SUBSET };
-template <typename Real, int NGAS, int AMODE, bool EMEM, int GPL_, unsigned FORM, int VAR>
-__global__ void __launch_bounds__(kWarps * 32, min_blocks(sizeof(Real), NGAS, GPL_, FORM))
+template <typename Real, int NGAS, int AMODE, bool EMEM, int GPL, unsigned FORM, int VAR>
+__global__ void __launch_bounds__(kWarps * 32, tuning(sizeof(Real), GPL, FORM).min_blocks())
     ufair_integrate_kernel(const __grid_constant__ KArgs<Real> a, const __grid_constant__ CUtensorMap tmE,
                            const __grid_constant__ CUtensorMap tmF) {
-  static_assert(FORM == 0 || GPL_ == NGAS, "a per-gas form needs all gases of a member in one lane");
+  static_assert(FORM == 0 || GPL == NGAS, "a per-gas form needs all gases of a member in one lane");
   constexpr bool INV = (VAR == kVarInverse), PLAIN = (VAR >= kVarPlain), NOFX = (VAR == kVarPlain),
                  ALLOUT = (VAR == kVarPlain || VAR == kVarPlainFx);  // C, RF and T all written: no output predicates
   using M = Math<Real>;
-  using WS = WarpSmem<Real, NGAS, AMODE, GPL_, FORM>;
-  constexpr int GPL = WS::GPL;           // gases this lane integrates
-  constexpr int kTT = WS::TT;            // time steps per tile (shadows the general kernels' constant)
+  using WS = WarpSmem<Real, NGAS, AMODE, GPL, FORM>;
+  constexpr int kTT = WS::TT;            // time steps per tile
   constexpr int GROUPS = NGAS / GPL;     // lanes per member
   constexpr int MW = WS::MW;             // members per warp
   constexpr int NACT = MW * GROUPS;      // working lanes
-  constexpr bool HOT_SMEM = WS::HOT_SMEM;
   constexpr unsigned FULL = 0xffffffffu;
   constexpr uint32_t ES = sizeof(Real);
   constexpr uint32_t GROW = (uint32_t)(kTT * MW) * ES;  // bytes between two gases inside an E stage
@@ -442,10 +494,6 @@ __global__ void __launch_bounds__(kWarps * 32, min_blocks(sizeof(Real), NGAS, GP
   pin(f_addr);
   pin(par);
   pin(tb);
-#define PARG(gl, k) lds(par + (uint32_t)WS::row(gl, k) * 32u * ES, Real())
-#define SETG(gl, k, v) sts(par + (uint32_t)WS::row(gl, k) * 32u * ES, (Real)(v))
-#define PART(k) lds(par + (uint32_t)(WS::T_BASE + (k)) * 32u * ES, Real())
-#define SETT(k, v) sts(par + (uint32_t)(WS::T_BASE + (k)) * 32u * ES, (Real)(v))
 
   const int n_tile = (n_t + kTT - 1) / kTT;
   if (lane == 0 && use_tma) {
@@ -466,7 +514,8 @@ __global__ void __launch_bounds__(kWarps * 32, min_blocks(sizeof(Real), NGAS, GP
   // (g_1 and g_0 of .coveragerc:15-16 are fused here; in FP32 they would cancel catastrophically
   // for the 10^6-year pool, so the one-off prologue always runs in FP64 and rounds once)
   Real R[GPL][4], Gcum[GPL], sumR[GPL];
-  Real hot[GPL][H_COUNT];  // used only when !HOT_SMEM (dead otherwise)
+  Real hot[GPL][H_COUNT], k0[GPL][4], ka[GPL][4], tr[T_COUNT];  // LaneConsts' register copies
+  LaneConsts<Real, NGAS, AMODE, GPL, FORM> cst{par, hot, k0, ka, tr};
   unsigned mk3[GPL];
   int nmin[GPL];  // lowest exponent alpha may take (Math::alpha_floor_exp)
   bool need_log[GPL], need_sqrt[GPL];
@@ -502,34 +551,31 @@ __global__ void __launch_bounds__(kWarps * 32, min_blocks(sizeof(Real), NGAS, GP
 #pragma unroll
     for (int q = 0; q < 4; ++q) {
       if (q < NP) {
-        SETG(gl, G_KA0 + q, c * av[q] * tau[q]);
-        SETG(gl, G_K0 + q, (AMODE == UFAIR_ALPHA_ONE) ? -expm1(-a.dt / tau[q]) : a.dt / tau[q]);
+        cst.at(gl, G_KA0, q).set(c * av[q] * tau[q]);
+        cst.at(gl, G_K0, q).set((AMODE == UFAIR_ALPHA_ONE) ? -expm1(-a.dt / tau[q]) : a.dt / tau[q]);
       }
     }
     const double hv[H_COUNT] = {r0 * inv_g1 + fold, rU * inv_g1, (rA - rU) * inv_g1 * invc, rT * inv_g1,
                                 a.clamp ? (a.iirf_max * inv_g1 + fold) : (double)INFINITY};
 #pragma unroll
-    for (int q = 0; q < H_COUNT; ++q) {
-      hot[gl][q] = (Real)hv[q];
-      if (HOT_SMEM) SETG(gl, WS::G_HOT + q, hv[q]);
-    }
+    for (int q = 0; q < H_COUNT; ++q) cst.at(gl, G_HOT, q).set(hv[q]);
     nmin[gl] = M::alpha_floor_exp(k0max, AMODE == UFAIR_ALPHA_NEWTON ? 8 : 0);
     pin(reinterpret_cast<uint32_t&>(nmin[gl]));
     const Real f1v = p[UFAIR_GP_F1 * ld], f3v = p[UFAIR_GP_F3 * ld];
-    SETG(gl, G_C0, C0d);
+    cst.at(gl, G_C0).set(C0d);
     // the logarithm's argument is 1 + sumR / C0; a gas WITHOUT the log term (f1 == 0) gets 1 / C0 := 0 here,
     // so its argument is exactly 1, its logarithm exactly 0 and the term exactly zero -- also for C0 = 0
     // gases, where 1 / C0 is infinite -- with no mask or test in the loop
-    SETG(gl, G_INVC0, f1v != Real(0) ? 1.0 / C0d : 0.0);
-    SETG(gl, G_SQRTC0, sqrt(C0d));
-    SETG(gl, G_F1, f1v);
-    SETG(gl, G_F2, p[UFAIR_GP_F2 * ld]);
-    SETG(gl, G_F3, f3v);
-    if (AMODE == UFAIR_ALPHA_SINH) SETG(gl, WS::G_X0, 1.0 / sinh(sarg));
+    cst.at(gl, G_INVC0).set(f1v != Real(0) ? 1.0 / C0d : 0.0);
+    cst.at(gl, G_SQRTC0).set(sqrt(C0d));
+    cst.at(gl, G_F1).set(f1v);
+    cst.at(gl, G_F2).set(p[UFAIR_GP_F2 * ld]);
+    cst.at(gl, G_F3).set(f3v);
+    if (AMODE == UFAIR_ALPHA_SINH) cst.at(gl, G_X0).set(1.0 / sinh(sarg));
     if (AMODE == UFAIR_ALPHA_NEWTON) {
-      SETG(gl, WS::G_X0, g1);
-      SETG(gl, WS::G_X0 + 1, lng0);
-      SETG(gl, WS::G_X0 + 2, invc);
+      cst.at(gl, G_X0).set(g1);
+      cst.at(gl, G_X0, 1).set(lng0);
+      cst.at(gl, G_X0, 2).set(invc);
     }
     // a zero forcing coefficient means a zero term; the log / sqrt is skipped only when no lane of
     // the warp needs it (voted once, outside the loop; with all gases in one lane this is per gas)
@@ -552,8 +598,9 @@ __global__ void __launch_bounds__(kWarps * 32, min_blocks(sizeof(Real), NGAS, GP
     for (int q = 0; q < 2; ++q) {
       const double qq = tp[(UFAIR_TP_Q1 + q) * ld], d = tp[(UFAIR_TP_D1 + q) * ld];
       const double mj = -expm1(-a.dt / d);
-      SETT(T_QM0 + q, qq * mj);
-      SETT(T_DEC0 + q, 1.0 - mj);
+      // the thermal rows (see LaneConsts)
+      sts(cst.col + (uint32_t)(WS::T_BASE + (T_QM0 + q)) * 32u * ES, (Real)(qq * mj));
+      sts(cst.col + (uint32_t)(WS::T_BASE + (T_DEC0 + q)) * 32u * ES, (Real)(1.0 - mj));
     }
     S0 = si ? si[(long long)(5 * NGAS + 0) * ld + m] : Real(0);
     S1 = si ? si[(long long)(5 * NGAS + 1) * ld + m] : Real(0);
@@ -561,20 +608,7 @@ __global__ void __launch_bounds__(kWarps * 32, min_blocks(sizeof(Real), NGAS, GP
   }
   Real Ssum = S0 + S1;  // carried so that the mid-step mean costs one add
   __syncwarp();
-  constexpr bool POOL_REG = (WS::RCM & 2) != 0, THERM_REG = (WS::RCM & 4) != 0;
-  Real rK0[GPL][4], rKA[GPL][4], rT[T_COUNT];  // dead unless the experiment switches ask for them
-#pragma unroll
-  for (int gl = 0; gl < GPL; ++gl)
-#pragma unroll
-    for (int q = 0; q < 4; ++q) {
-      rK0[gl][q] = (POOL_REG && q < form_pools(FORM, gl)) ? PARG(gl, G_K0 + q) : Real(0);
-      rKA[gl][q] = (POOL_REG && q < form_pools(FORM, gl)) ? PARG(gl, G_KA0 + q) : Real(0);
-    }
-#pragma unroll
-  for (int k = 0; k < T_COUNT; ++k) rT[k] = THERM_REG ? PART(k) : Real(0);
-#define PK0(gl, q) (POOL_REG ? rK0[gl][q] : PARG(gl, G_K0 + (q)))
-#define PKA(gl, q) (POOL_REG ? rKA[gl][q] : PARG(gl, G_KA0 + (q)))
-#define PTH(k) (THERM_REG ? rT[k] : PART(k))
+  cst.load();
 
   const int scen = (a.scen_idx != nullptr) ? a.scen_idx[m] : 0;
   const Real dt = (Real)a.dt;
@@ -584,14 +618,18 @@ __global__ void __launch_bounds__(kWarps * 32, min_blocks(sizeof(Real), NGAS, GP
   const Real wOld = a.w_old, wNew = a.w_new;
   const bool clamp = !PLAIN && a.clamp != 0;
 
-  // output predicates packed in one register; running output pointers (gas g0; + gl * gstride)
+  // Whether this lane stores an output this launch.  The general loops test a bit of wm, which packs all the
+  // decisions in one register on purpose.  The plain loops have no alpha or E output and keep C, RF and T as lane
+  // predicates fixed before the loop, not bits re-tested every step; in the loops that write all three those are
+  // just `active` and `owner`.  Each store site picks its form inline: through a helper lambda the compiler
+  // schedules several loops differently.
   const bool owner = active && (g0 == 0);  // the lane that owns the member's T / histogram count
   unsigned wm = (active ? (unsigned)(a.out_mask & (UFAIR_OUT_C | UFAIR_OUT_RF | UFAIR_OUT_ALPHA | (INV ? UFAIR_OUT_E : 0))) : 0u) |
                 ((owner && ((a.out_mask & UFAIR_OUT_T) || a.stats)) ? (unsigned)UFAIR_OUT_T : 0u);
-  // the plain instantiations keep the three store decisions as lane predicates, fixed before the loop
   const bool st_c = active && (a.out_mask & UFAIR_OUT_C) != 0, st_rf = active && (a.out_mask & UFAIR_OUT_RF) != 0,
              st_t = owner && ((a.out_mask & UFAIR_OUT_T) != 0 || a.stats != 0);
   pin(wm);
+  // running output pointers (gas g0; + gl * gstride)
   const long long gstride = (long long)n_t * ld;
   const long long o_gas = (long long)g0 * gstride + m_raw;
   Real* pC = a.oC + o_gas;
@@ -647,27 +685,27 @@ __global__ void __launch_bounds__(kWarps * 32, min_blocks(sizeof(Real), NGAS, GP
         alpha[gl] = Real(1);
         inva[gl] = Real(1);
       } else {
-        const Real rho0 = HOT_SMEM ? PARG(gl, WS::G_HOT + H_RHO0) : hot[gl][H_RHO0];
-        const Real rhoU = HOT_SMEM ? PARG(gl, WS::G_HOT + H_RHOU) : hot[gl][H_RHOU];
-        const Real wR = HOT_SMEM ? PARG(gl, WS::G_HOT + H_WR) : hot[gl][H_WR];
-        const Real rhoT = HOT_SMEM ? PARG(gl, WS::G_HOT + H_RHOT) : hot[gl][H_RHOT];
+        const Real rho0 = cst.get(gl, G_HOT, H_RHO0);
+        const Real rhoU = cst.get(gl, G_HOT, H_RHOU);
+        const Real wR = cst.get(gl, G_HOT, H_WR);
+        const Real rhoT = cst.get(gl, G_HOT, H_RHOT);
         Real u = fma(rhoU, Gcum[gl], fma(wR, sumR[gl], fma(rhoT, Tprev, rho0)));
         if (clamp) {  // uniform: the iIRF ceiling costs nothing when it is switched off
-          const Real umax = HOT_SMEM ? PARG(gl, WS::G_HOT + H_UMAX) : hot[gl][H_UMAX];
+          const Real umax = cst.get(gl, G_HOT, H_UMAX);
           u = (u > umax) ? umax : u;
         }
-        Real al = (AMODE == UFAIR_ALPHA_SINH) ? PARG(gl, WS::G_X0) * M::sinh_pair(u, tb, nmin[gl]) : M::exp_(u, tb, nmin[gl]);
+        Real al = (AMODE == UFAIR_ALPHA_SINH) ? cst.get(gl, G_X0) * M::sinh_pair(u, tb, nmin[gl]) : M::exp_(u, tb, nmin[gl]);
         if (AMODE == UFAIR_ALPHA_NEWTON) {
-          const Real iirf = (u - PARG(gl, WS::G_X0 + 1)) * PARG(gl, WS::G_X0);
-          const Real invc = PARG(gl, WS::G_X0 + 2);
+          const Real iirf = (u - cst.get(gl, G_X0, 1)) * cst.get(gl, G_X0);
+          const Real invc = cst.get(gl, G_X0, 2);
           for (int it = 0; it < a.newton_iters; ++it) {
             const Real ia = M::rcp(al);
             Real f = -iirf, fp = 0;
 #pragma unroll
             for (int q = 0; q < NP; ++q) {
-              const Real z = PK0(gl, q) * hdt * ia;
+              const Real z = cst.get(gl, G_K0, q) * hdt * ia;
               const Real mz = M::decay(z, tb);
-              const Real at = PKA(gl, q) * invc;  // a_i tau_i
+              const Real at = cst.get(gl, G_KA0, q) * invc;  // a_i tau_i
               f = fma(at * al, mz, f);
               fp = fma(at, mz - z * (Real(1) - mz), fp);
             }
@@ -686,7 +724,7 @@ __global__ void __launch_bounds__(kWarps * 32, min_blocks(sizeof(Real), NGAS, GP
       Real mq[4];
 #pragma unroll
       for (int q = 0; q < 4; ++q)
-        if (q < NP) mq[q] = (AMODE == UFAIR_ALPHA_ONE) ? PK0(gl, q) : M::decay(PK0(gl, q) * inva[gl], tb);
+        if (q < NP) mq[q] = (AMODE == UFAIR_ALPHA_ONE) ? cst.get(gl, G_K0, q) : M::decay(cst.get(gl, G_K0, q) * inva[gl], tb);
       if (INV) {
         // concentration-driven gas: `e` is the target C; step_conc is linear in E, so
         //   E = (C_target - C0 - sum R_i (1 - m_i)) / (alpha sum m_i c a_i tau_i)
@@ -695,9 +733,9 @@ __global__ void __launch_bounds__(kWarps * 32, min_blocks(sizeof(Real), NGAS, GP
         for (int q = 0; q < 4; ++q)
           if (q < NP) {
             keep += fma(-mq[q], R[gl][q], R[gl][q]);
-            gain = fma(mq[q], PKA(gl, q), gain);
+            gain = fma(mq[q], cst.get(gl, G_KA0, q), gain);
           }
-        const Real e_inv = ((e[gl] - PARG(gl, G_C0)) - keep) * M::rcp(gain * alpha[gl]);
+        const Real e_inv = ((e[gl] - cst.get(gl, G_C0)) - keep) * M::rcp(gain * alpha[gl]);
         if ((a.conc_driven >> (g0 + gl)) & 1) e[gl] = e_inv;
         if (wm & UFAIR_OUT_E) {
           UFAIR_CHECK_ST(a.oE, (long long)NGAS * n_t, pC + dE + gl * gstride);
@@ -707,11 +745,10 @@ __global__ void __launch_bounds__(kWarps * 32, min_blocks(sizeof(Real), NGAS, GP
       const Real ea = e[gl] * alpha[gl];
 #pragma unroll
       for (int q = 0; q < 4; ++q)
-        if (q < NP) R[gl][q] = fma(mq[q], fma(ea, PKA(gl, q), -R[gl][q]), R[gl][q]);
+        if (q < NP) R[gl][q] = fma(mq[q], fma(ea, cst.get(gl, G_KA0, q), -R[gl][q]), R[gl][q]);
       Gcum[gl] = fma(e[gl], dt, Gcum[gl]);
       sumR[gl] = sum_pools(R[gl], NP);
-      Cg[gl] = PARG(gl, G_C0) + sumR[gl];
-      // (PLAIN: the lane predicates themselves, not bits re-tested every step)
+      Cg[gl] = cst.get(gl, G_C0) + sumR[gl];
       if (ALLOUT ? active : PLAIN ? st_c : (wm & UFAIR_OUT_C) != 0) {
         UFAIR_CHECK_ST(a.oC, (long long)NGAS * n_t, pC + gl * gstride);
         st_stream(pC + gl * gstride, Cg[gl]);
@@ -729,13 +766,13 @@ __global__ void __launch_bounds__(kWarps * 32, min_blocks(sizeof(Real), NGAS, GP
 #pragma unroll
     for (int gl = 0; gl < GPL; ++gl) {
       const unsigned TERMS = form_terms(FORM, gl);
-      Real F = (TERMS & UFAIR_TERM_LIN) ? PARG(gl, G_F2) * sumR[gl] : Real(0);
+      Real F = (TERMS & UFAIR_TERM_LIN) ? cst.get(gl, G_F2) * sumR[gl] : Real(0);
       if (need_log[gl]) {
-        const Real y = fma(sumR[gl], PARG(gl, G_INVC0), Real(1));
-        F = fma(PARG(gl, G_F1), M::log_fast(y), F);
+        const Real y = fma(sumR[gl], cst.get(gl, G_INVC0), Real(1));
+        F = fma(cst.get(gl, G_F1), M::log_fast(y), F);
         bad = bad || M::not_normal(y);
       }
-      if (need_sqrt[gl]) F = fma(PARG(gl, G_F3), M::mask(M::sqrt_(Cg[gl]) - PARG(gl, G_SQRTC0), mk3[gl]), F);
+      if (need_sqrt[gl]) F = fma(cst.get(gl, G_F3), M::mask(M::sqrt_(Cg[gl]) - cst.get(gl, G_SQRTC0), mk3[gl]), F);
       Fg[gl] = F;
     }
     if (__builtin_expect(bad, 0)) {  // never on a physical trajectory: redo those gases' forcing with the special values
@@ -743,12 +780,12 @@ __global__ void __launch_bounds__(kWarps * 32, min_blocks(sizeof(Real), NGAS, GP
       for (int gl = 0; gl < GPL; ++gl) {
         const unsigned TERMS = form_terms(FORM, gl);
         if (need_log[gl]) {
-          const Real y = fma(sumR[gl], PARG(gl, G_INVC0), Real(1));
+          const Real y = fma(sumR[gl], cst.get(gl, G_INVC0), Real(1));
           if (M::not_normal(y)) {
-            Real F = (TERMS & UFAIR_TERM_LIN) ? PARG(gl, G_F2) * sumR[gl] : Real(0);
-            F = fma(PARG(gl, G_F1), M::log_special(y), F);
+            Real F = (TERMS & UFAIR_TERM_LIN) ? cst.get(gl, G_F2) * sumR[gl] : Real(0);
+            F = fma(cst.get(gl, G_F1), M::log_special(y), F);
             if (need_sqrt[gl])
-              F = fma(PARG(gl, G_F3), M::mask(M::sqrt_(PARG(gl, G_C0) + sumR[gl]) - PARG(gl, G_SQRTC0), mk3[gl]), F);
+              F = fma(cst.get(gl, G_F3), M::mask(M::sqrt_(cst.get(gl, G_C0) + sumR[gl]) - cst.get(gl, G_SQRTC0), mk3[gl]), F);
             Fg[gl] = F;
           }
         }
@@ -776,8 +813,8 @@ __global__ void __launch_bounds__(kWarps * 32, min_blocks(sizeof(Real), NGAS, GP
       Ftot += fx;
     }
     // ---- step_temp (with GROUPS > 1 computed redundantly, bit-identically, by a member's lanes)
-    const Real s0 = fma(PTH(T_QM0), Ftot, S0 * PTH(T_DEC0));
-    const Real s1 = fma(PTH(T_QM1), Ftot, S1 * PTH(T_DEC1));
+    const Real s0 = fma(cst.get_t(T_QM0), Ftot, S0 * cst.get_t(T_DEC0));
+    const Real s1 = fma(cst.get_t(T_QM1), Ftot, S1 * cst.get_t(T_DEC1));
     const Real Snew = s0 + s1;
     const Real T = fma(wNew, Snew, wOld * Ssum);
     S0 = s0;
@@ -829,13 +866,6 @@ __global__ void __launch_bounds__(kWarps * 32, min_blocks(sizeof(Real), NGAS, GP
       so[(long long)(5 * NGAS + 2) * ld + m] = Tprev;
     }
   }
-#undef PK0
-#undef PKA
-#undef PTH
-#undef PARG
-#undef SETG
-#undef PART
-#undef SETT
 }
 
 // ---- the choice of instantiation, and its launch ----------------------------------------------------
