@@ -148,7 +148,10 @@ typedef struct ufair_desc {
 
   /* ---- ensemble statistics (stats == 1) ----
    * bin(T) = clamp(floor((T - hist_lo) * (hist_bins / (hist_hi - hist_lo))), 0, hist_bins-1),
-   * evaluated in the run's precision; NaN is not counted.
+   * evaluated in the run's precision.  Non-finite T: NaN is neither counted in the histogram nor
+   * taken into min / max, but it makes its row's sum and sum of squares NaN (a mean / std computed
+   * from them flags the step); +inf and -inf are counted in the last and first bin and enter every
+   * moment.  A row with no value other than NaN keeps the min / max sentinels +inf / -inf.
    * The integrator only writes the T rows (so out_T must be non-NULL when stats == 1, whether or
    * not UFAIR_OUT_T is set); ufair_stats_pass_*() then reads them once at HBM speed and adds member
    * slice c of every row into copy c of hist_private / moments_private (counts; sum, sum of

@@ -2,25 +2,20 @@
 member / step counts (ragged tiles and warps), emission layout, external-forcing layout, alpha mode,
 clamp, temperature mode, resume state, concentration-driven gases, sparse or dense parameters
 (specialised or general kernel) that the dedicated tests only sample by hand.  Shared by the GPU
-test (the CUDA path) and a CPU test (the numpy oracle through the same harness)."""
+tests (the CUDA path, FP64 and FP32) and a CPU test (the numpy oracle through the same harness)."""
 import os
 
 import numpy as np
 
 from oracle import c_oracle as co
 from oracle import ufair_oracle as o
-from tests.util import ensemble, field_relerr
+from tests.util import TOL64, ensemble, output_relerr, slice_relerr
 
-TOL64 = 1e-10
+TOL32_T = 1e-4       # FP32: K, absolute, against the float64 oracle
+TOL32_C = 2e-5       # FP32: each gas's concentrations relative to that gas's own scale
 GASES = ("co2", "ch4", "n2o", "hfc")
 _AM = {"exp": o.ALPHA_EXP, "sinh": o.ALPHA_SINH, "newton": o.ALPHA_NEWTON, "one": o.ALPHA_ONE}
 N_CASES = int(os.environ.get("UFAIR_FUZZ_CASES", "40"))   # a one-off wider sweep: UFAIR_FUZZ_CASES=400 pytest ...
-# Forcing and temperature of a run that lasts one or two steps from pre-industrial are ~1e-6 W m-2 / K,
-# and f1 ln(C / C0) at C = C0 (1 + 1e-7) is ill-conditioned in float64 whoever evaluates it (one
-# rounding of the argument is 1e-16 / 1e-7 = 1e-9 of the result; the kernel multiplies by 1/C0 where
-# the oracle divides).  The 1e-10 criterion is therefore applied to max(field scale, 0.01 W m-2 or K):
-# an absolute 1e-12 W m-2 / K for such runs, the plain relative criterion for every run of normal length.
-FLOOR = {"RF": 1e-2, "T": 1e-2}
 
 
 def _case(seed):
@@ -38,9 +33,14 @@ def _case(seed):
     return c
 
 
-def check_case(seed, run_ensemble, HistSpec, to_dev, to_np):
-    """Build configuration `seed`, run it through `run_ensemble` (the public API's signature) and
-    check every output against the C oracle."""
+def check_case(seed, run_ensemble, HistSpec, to_dev, to_np, precision="f64"):
+    """Build configuration `seed`, run it through `run_ensemble` (the public API's signature) in `precision` and
+    check every output against the C oracle.  Returns the errors it measured, by output.
+
+    FP64: every output by the per-gas / per-state-row rule of tests.util.output_relerr, <= 1e-10.
+    FP32: T within 1e-4 K (absolute); each emission-driven gas's C within 2e-5 of that gas's own scale.  RF is
+    not checked beyond what T implies (FP32 log2 of 1 + tiny is not 2e-5-accurate in runs of a few steps), and
+    a concentration-driven gas is checked through T only (its diagnosed emissions cancel in FP32)."""
     c = _case(seed)
     G, M, n_t = c["G"], c["M"], c["n_t"]
     ens = ensemble(M, n_t=n_t, dt=c["dt"], dense=c["dense"], gases=GASES[:G], seed=seed)
@@ -85,17 +85,30 @@ def check_case(seed, run_ensemble, HistSpec, to_dev, to_np):
         kw["conc_driven"] = [bool((c["driven"] >> g) & 1) for g in range(G)]
         okw["conc_driven"] = c["driven"]
     spec = HistSpec(lo=-1.0, hi=6.0, bins=64, copies=3) if c["stats"] else None
-    res = run_ensemble(to_dev(E), to_dev(gp), to_dev(tp), dt=c["dt"], stats=spec,
+    res = run_ensemble(to_dev(E), to_dev(gp), to_dev(tp), dt=c["dt"], stats=spec, precision=precision,
                        outputs=("C", "RF", "T", "alpha"), **kw, **modes)
     ref = co.oxfair(E, gp, tp, dt=c["dt"], want_alpha=True, **okw, **omodes)
-    for k in ("C", "RF", "T", "alpha", "state"):
-        err = field_relerr(to_np(getattr(res, k)), ref[k], FLOOR.get(k, 0.0))
-        assert err < TOL64, f"{c}: {k} relative error {err:.3e}"
-    if c["driven"]:
-        for g in range(G):
-            assert field_relerr(to_np(res.E)[g], ref["E"][g]) < 1e-9, f"{c}: E[{g}]"
+    errs = {}
+    if precision == "f64":
+        for k in ("C", "RF", "T", "alpha", "state"):
+            errs[k] = output_relerr(k, to_np(getattr(res, k)), ref[k])
+            assert errs[k] < TOL64, f"{c}: {k} relative error {errs[k]:.3e}"
+        if c["driven"]:
+            errs["E"] = output_relerr("E", to_np(res.E), ref["E"])
+            assert errs["E"] < 1e-9, f"{c}: E relative error {errs['E']:.3e}"
+    else:
+        T = to_np(res.T)
+        assert T.dtype == np.float32
+        errs["T"] = float(np.max(np.abs(T.astype(np.float64) - ref["T"]))) if T.size else 0.0
+        assert errs["T"] <= TOL32_T, f"{c}: T off by {errs['T']:.3e} K"
+        emitted = [g for g in range(G) if not (c["driven"] >> g) & 1]
+        if emitted:
+            errs["C"] = slice_relerr(to_np(res.C)[emitted], ref["C"][emitted])
+            assert errs["C"] <= TOL32_C, f"{c}: C relative error {errs['C']:.3e} (gases {emitted})"
     if spec is not None:
         T = to_np(res.T)
-        hist, mom = co.temperature_stats(T, spec.lo, spec.hi, spec.bins)
+        # binned in T's own precision: the C oracle's recount casts to float64 first, so it serves FP64 only
+        hist, mom = (co if precision == "f64" else o).temperature_stats(T, spec.lo, spec.hi, spec.bins)
         assert np.array_equal(to_np(res.hist), hist.astype(np.int64)), f"{c}: histogram"
         assert np.allclose(to_np(res.moments), mom, rtol=1e-12, atol=1e-11), f"{c}: moments"
+    return errs

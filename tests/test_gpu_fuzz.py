@@ -1,4 +1,4 @@
-"""The CUDA path (through the C ABI) on the seeded random configurations of tests/fuzz.py."""
+"""The CUDA path (through the C ABI) on the seeded random configurations of tests/fuzz.py, in FP64 and in FP32."""
 import pytest
 
 from fiveeqscm_b200 import _abi
@@ -17,13 +17,22 @@ def api():
     return c
 
 
-@pytest.mark.parametrize("seed", range(fuzz.N_CASES))
-def test_random_configuration_matches_oracle(api, seed):
+def _run(api):
     import torch
 
     def run(*a, **kw):
         r = api.run_ensemble(*a, **kw)
         torch.cuda.synchronize()
         return r
+    return run
 
-    fuzz.check_case(seed, run, api.HistSpec, to_dev, to_np)
+
+@pytest.mark.parametrize("seed", range(fuzz.N_CASES))
+def test_random_configuration_matches_oracle(api, seed):
+    fuzz.check_case(seed, _run(api), api.HistSpec, to_dev, to_np)
+
+
+@pytest.mark.parametrize("seed", range(fuzz.N_CASES))
+def test_random_configuration_fp32_matches_oracle(api, seed):
+    """The same configurations on the FP32 instantiations: T within 1e-4 K, each gas's C within 2e-5."""
+    fuzz.check_case(seed, _run(api), api.HistSpec, to_dev, to_np, precision="f32")

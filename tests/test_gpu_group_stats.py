@@ -1,6 +1,6 @@
 """Grouped ensemble statistics on the device: per-group counts against a recount of the kernel's own T, the pooled
 pass reproduced by one group, determinism, sharding and the packed reduction, the host pipeline, device
-percentiles, guard bands around every grouped buffer, and argument errors."""
+percentiles, non-finite temperatures, guard bands around every grouped buffer, and argument errors."""
 import ctypes as C
 
 import numpy as np
@@ -8,7 +8,8 @@ import pytest
 
 from fiveeqscm_b200 import _abi
 from fiveeqscm_b200 import params as P
-from tests.group_stats_ref import grouped_temperature_stats
+from oracle import ufair_oracle as o
+from tests.group_stats_ref import grouped_temperature_stats, plant_non_finite
 from tests.test_gpu_guard import POISON64, _desc_and_buffers
 from tests.util import ensemble, to_dev, to_np
 
@@ -185,6 +186,49 @@ def test_device_percentiles_of_grouped_histograms(api):
     torch.cuda.synchronize()
     assert pd.shape == (4, 45, 5)
     assert np.array_equal(to_np(pd), stats.percentiles(res.hist, -0.5, 3.5, (5, 17, 50, 83, 95)))
+
+
+@pytest.mark.parametrize("prec", ["f64", "f32"])
+@pytest.mark.parametrize("G", [0, 3, 9], ids=["pooled", "G3", "G9"])   # 3 groups: the 4-group tile; 9: the 8-group one
+def test_non_finite_temperatures_follow_the_rule(api, prec, G):
+    """T rows carrying NaN, +-inf, exactly lo / hi, one ulp below hi, bin edges and an all-NaN step, written between
+    the integrator and the statistics pass: NaN is neither binned nor in min / max and makes its row's sum and sumsq
+    NaN; the infinities land in the edge bins and enter every moment (include/ufair.h, statistics block)."""
+    import torch
+    from fiveeqscm_b200 import stats
+    M, n_t, lo, hi, bins = 1003, 8, -1.0, 6.0, 28
+    lab = _labels(M, G, True, 17) if G else None
+    spec = api.HistSpec(lo=lo, hi=hi, bins=bins, copies=3, groups=G)
+    plan, _ = _plan(api, M, n_t, prec, spec, lab)
+    plan.reset_stats()
+    plan.launch()
+    T = plant_non_finite(to_np(plan.result.T).copy(), lo, hi, bins)
+    plan.result.T.copy_(torch.from_numpy(T))                # the T rows the statistics pass reads
+    plan.stats_pass()
+    plan.finalize_stats()
+    torch.cuda.synchronize()
+    hist, mom = to_np(plan.result.hist), to_np(plan.result.moments)
+    if G:
+        h_ref, m_ref = grouped_temperature_stats(T, lo, hi, bins, lab, G)
+        absT = _abs_sums(T, lab, G)
+    else:
+        h_ref, m_ref = o.temperature_stats(T, lo, hi, bins)
+        absT = np.abs(T.astype(np.float64)).sum(axis=1)
+    assert np.array_equal(hist.astype(np.uint64), h_ref)
+    assert np.array_equal(mom[..., 2:], m_ref[..., 2:]), "min / max exact"
+    for j in (0, 1):                                      # sum, sumsq: NaN and inf where the reference has them
+        got, want = mom[..., j], m_ref[..., j]
+        fin = np.isfinite(want)
+        assert np.array_equal(np.isnan(got), np.isnan(want)) and np.array_equal(got[np.isinf(want)], want[np.isinf(want)])
+        tol = 1e-12 * (absT if j == 0 else want)
+        assert np.all(np.abs(got[fin] - want[fin]) <= tol[fin])
+    assert np.isnan(mom[..., 3, 0]).all() and (mom[..., 3, 2] == np.inf).all() and (mom[..., 3, 3] == -np.inf).all()
+    assert not hist[..., 3, :].any()
+    pcts = (0.0, 5.0, 50.0, 95.0, 100.0)
+    pd = to_np(stats.percentiles_device(plan.result.hist, lo, hi, pcts)).reshape(-1, n_t, len(pcts))
+    for g, h in enumerate(hist.reshape(-1, n_t, bins)):
+        assert np.array_equal(pd[g], o.percentiles_from_hist(h, lo, hi, pcts)), g
+        assert np.array_equal(pd[g, 3], o.percentiles_from_hist(h[3:4], lo, hi, pcts)[0])   # the all-NaN step
 
 
 @pytest.mark.parametrize("prec", ["f64", "f32"])

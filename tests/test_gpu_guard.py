@@ -19,7 +19,7 @@ import pytest
 
 from fiveeqscm_b200 import _abi
 from oracle import c_oracle as co
-from tests.util import ensemble, field_relerr
+from tests.util import ensemble, output_relerr
 
 pytestmark = pytest.mark.gpu
 
@@ -162,11 +162,12 @@ def test_device_outputs_stay_inside_their_rows(G, M, slack, n_t, prec, extra):
     if extra.get("fext_member"):
         fx = b["fx"].data().astype(np.float64)
     ref = co.oxfair(ens["E"], ens["gas_params"], ens["thermal_params"], f_ext=fx, fext_per_member=fx is not None,
-                    conc_driven=kw.get("conc_driven", 0))
+                    conc_driven=kw.get("conc_driven", 0), want_alpha=True)
     T = b["oT"].data().astype(np.float64)
     if prec == "f64":
-        assert field_relerr(T, ref["T"], floor=0.01) < 1e-10
-        assert field_relerr(b["oC"].data().reshape(G, n_t, M), ref["C"]) < 1e-10
+        for k in outputs:
+            assert output_relerr(k, b["o" + k].data().reshape(ref[k].shape), ref[k]) < 1e-10, k
+        assert output_relerr("state", b["state"].data(), ref["state"]) < 1e-10
     else:
         assert np.max(np.abs(T - ref["T"])) < 1e-4
 
@@ -208,7 +209,13 @@ def test_host_pipeline_with_a_chunk_that_does_not_divide_M(prec):
     assert (hist[0] == -7).all() and (hist[-1] == -7).all() and (hist[1:-1].sum(axis=1) == M).all()
     ref = co.oxfair(ens["E"], ens["gas_params"], ens["thermal_params"])
     T = b["oT"].data().astype(np.float64)
-    assert (field_relerr(T, ref["T"], floor=0.01) < 1e-10) if prec == "f64" else (np.max(np.abs(T - ref["T"])) < 1e-4)
+    if prec == "f64":
+        assert output_relerr("T", T, ref["T"]) < 1e-10
+        for k in ("C", "RF"):
+            assert output_relerr(k, b["o" + k].data().reshape(G, n_t, M), ref[k]) < 1e-10, k
+        assert output_relerr("state", b["state"].data(), ref["state"]) < 1e-10
+    else:
+        assert np.max(np.abs(T - ref["T"])) < 1e-4
 
 
 # ------------------------------------------------------------------ the checked build (libufair_dbg.so)

@@ -8,7 +8,7 @@ from fiveeqscm_b200 import _abi
 from fiveeqscm_b200 import params as P
 from oracle import c_oracle as co
 from oracle import ufair_oracle as o
-from tests.util import field_relerr, to_dev, to_np
+from tests.util import assert_parity, to_dev, to_np
 
 pytestmark = pytest.mark.gpu
 
@@ -64,8 +64,7 @@ def test_run_from_sampled_ensemble_matches_oracle(api):
     torch.cuda.synchronize()
     rgp, rtp, resc, rscen = o.sample_ensemble(seed, 0, M, n_scen=4, **t)
     ref = co.oxfair(scen_E, rgp, rtp, scen_idx=rscen, e_scale=resc)
-    for k in ("C", "RF", "T"):
-        assert field_relerr(to_np(getattr(res, k)), ref[k]) < 1e-10, k
+    assert_parity(res, ref, ("C", "RF", "T", "state"))
 
 
 def test_sampler_argument_errors(api):

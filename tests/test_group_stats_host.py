@@ -13,7 +13,7 @@ from fiveeqscm_b200 import _abi
 from fiveeqscm_b200 import concentrations as conc
 from fiveeqscm_b200 import stats as S
 from oracle import ufair_oracle as o
-from tests.group_stats_ref import grouped_temperature_stats
+from tests.group_stats_ref import grouped_temperature_stats, plant_non_finite
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -24,7 +24,9 @@ def _T(n_t, M, seed, dtype=np.float64):
 
 
 @pytest.mark.parametrize("dtype", [np.float64, np.float32])
-def test_grouped_reference_equals_a_loop_of_the_pooled_oracle(dtype):
+def test_grouped_reference_equals_a_loop_of_the_pooled_oracle_nan_outside_min_max(dtype):
+    """Group by group, the grouped reference is the pooled oracle on the group's members, and both keep a NaN out of
+    the histogram and out of min / max while it makes the sums NaN (the device's rule)."""
     n_t, M, G = 7, 5003, 13
     T = _T(n_t, M, 1, dtype)
     T[3, 17] = np.nan                                           # NaN is not binned
@@ -41,6 +43,11 @@ def test_grouped_reference_equals_a_loop_of_the_pooled_oracle(dtype):
         h, m = o.temperature_stats(T[:, sel], -1.0, 6.0, 300)
         assert np.array_equal(hist[g], h)
         np.testing.assert_array_equal(mom[g], m)
+    g17 = int(labels[17])
+    assert 0 <= g17 < G                                         # the NaN member is in a group
+    Tg = T[3, labels == g17].astype(np.float64)
+    assert np.isnan(mom[g17, 3, :2]).all()
+    assert mom[g17, 3, 2] == np.nanmin(Tg) and mom[g17, 3, 3] == np.nanmax(Tg)
     # every member with a label in range counted once per step, except the NaN
     n_in = int(((labels >= 0) & (labels < G)).sum())
     assert (hist.sum(axis=(0, 2)) == n_in - (np.arange(n_t) == 3) * int(0 <= labels[17] < G)).all()
@@ -99,7 +106,7 @@ import os, sys
 sys.path.insert(0, {root!r})
 import numpy as np, torch, torch.distributed as dist
 from fiveeqscm_b200 import dist as D
-from tests.group_stats_ref import grouped_temperature_stats
+from tests.group_stats_ref import grouped_temperature_stats, plant_non_finite
 rank, world = int(sys.argv[1]), int(sys.argv[2])
 os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=sys.argv[3], RANK=str(rank), WORLD_SIZE=str(world))
 dist.init_process_group("gloo", rank=rank, world_size=world)
@@ -184,3 +191,50 @@ def test_python_group_resolution():
     conc._check_labels(2, 3, "x")
     with pytest.raises(ValueError, match="label 3 >= groups 3"):
         conc._check_labels(3, 3, "x")
+
+
+def _same_moments(a, b):
+    """min / max exactly, sum / sumsq to summation order (assert_allclose: NaN where the other has NaN, inf equal)"""
+    np.testing.assert_array_equal(a[..., 2:], b[..., 2:])
+    np.testing.assert_allclose(a[..., :2], b[..., :2], rtol=1e-12)
+
+
+@pytest.mark.parametrize("dtype", [np.float64, np.float32])
+def test_one_rule_for_non_finite_temperatures(dtype):
+    """NaN: not binned, not in min / max, makes sum and sumsq NaN; +-inf: edge bins and every moment.  The numpy
+    oracle, the grouped reference and (for float64, which it bins in) the C oracle agree on it."""
+    from oracle import c_oracle as co
+    lo, hi, bins = -1.0, 6.0, 28
+    T = plant_non_finite(_T(6, 257, 5, dtype), lo, hi, bins)
+    n_t, M = T.shape
+    hist, mom = o.temperature_stats(T, lo, hi, bins)
+    fin = np.where(np.isfinite(T), T, np.nan).astype(np.float64)
+    nan = np.isnan(T)
+    assert (hist.sum(axis=1) == M - nan.sum(axis=1)).all()
+    assert hist[0, -1] >= 1 and hist[0, 0] >= 1 and hist[2, -1] >= 1 and hist[2, 0] >= 1     # infinities: edge bins
+    assert hist[1, 0] >= 1 and hist[1, -1] >= 2                             # lo -> bin 0; hi and hi - 1 ulp -> last bin
+    assert not hist[3].any()
+    assert np.array_equal(np.isnan(mom[:, 0]), nan.any(axis=1) | (np.isposinf(T).any(axis=1) & np.isneginf(T).any(axis=1)))
+    assert np.isnan(mom[[0, 3, 4], 1]).all() and mom[2, 1] == np.inf
+    assert mom[0, 2] == -np.inf and mom[0, 3] == np.inf and mom[4, 3] == np.inf
+    assert mom[3, 2] == np.inf and mom[3, 3] == -np.inf                     # all-NaN: the sentinels
+    assert mom[1, 2] == np.nanmin(fin[1]) and mom[1, 3] == np.nanmax(fin[1])
+    assert mom[5, 0] == -np.inf and mom[5, 1] == np.inf and mom[5, 2] == -np.inf and mom[5, 3] == np.nanmax(fin[5])
+    mean, _ = S.mean_std(mom, hist.sum(axis=1))
+    assert np.isnan(mean[[0, 2, 3, 4]]).all() and np.isfinite(mean[1]) and mean[5] == -np.inf
+    gh, gm = grouped_temperature_stats(T, lo, hi, bins, np.zeros(M, dtype=np.int32), 1)
+    assert np.array_equal(gh[0], hist)
+    _same_moments(gm[0], mom)
+    if dtype == np.float64:
+        ch, cm = co.temperature_stats(T, lo, hi, bins)
+        assert np.array_equal(ch, hist)
+        _same_moments(cm, mom)
+    # grouped: every group sees the rule, an empty group keeps the empty identities
+    lab = np.arange(M) % 4
+    lab[lab == 3] = -1
+    gh, gm = grouped_temperature_stats(T, lo, hi, bins, lab, 4)
+    for g in range(3):
+        h, m = o.temperature_stats(T[:, lab == g], lo, hi, bins)
+        assert np.array_equal(gh[g], h)
+        _same_moments(gm[g], m)
+    assert not gh[3].any() and (gm[3, :, :2] == 0).all() and (gm[3, :, 2] == np.inf).all() and (gm[3, :, 3] == -np.inf).all()

@@ -1,6 +1,7 @@
 """The numpy oracle against the C oracle on the same seeded random configurations the GPU fuzz test
 uses (tests/fuzz.py): the two independent restatements must agree on every layout / mode /
-concentration-driven combination, and the harness itself is exercised on CPU."""
+concentration-driven combination, gas by gas and state row by state row, and the harness itself is exercised
+on CPU."""
 from dataclasses import dataclass
 from types import SimpleNamespace
 
@@ -20,7 +21,8 @@ class _Spec:
     copies: int = 1
 
 
-def _numpy_oracle_as_api(E, gp, tp, *, dt, stats, outputs, alpha_mode, t_mode, conc_driven=None, **kw):
+def _numpy_oracle_as_api(E, gp, tp, *, dt, stats, outputs, alpha_mode, t_mode, precision, conc_driven=None, **kw):
+    assert precision == "f64"
     mask = sum(1 << g for g, f in enumerate(conc_driven or []) if f)
     out = o.oxfair(E, gp, tp, dt=dt, alpha_mode=fuzz._AM[alpha_mode], t_mode=o.T_END if t_mode == "end" else o.T_MID,
                    want_alpha=True, conc_driven=mask, **kw)
