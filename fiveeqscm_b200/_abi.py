@@ -7,7 +7,7 @@ from __future__ import annotations
 import ctypes as C
 import os
 
-ABI_VERSION = 3
+ABI_VERSION = 4
 MAX_GAS = 4
 N_POOL = 4
 MAX_STAT_GROUPS = 256
@@ -83,7 +83,7 @@ class UfairDesc(C.Structure):
         ("conc_driven", C.c_int32),
         ("out_E", C.c_void_p),
         ("n_stat_groups", C.c_int32),
-        ("reserved1", C.c_int32),
+        ("out_every", C.c_int32),
         ("stat_group", C.c_void_p),
     ]
 
@@ -99,7 +99,7 @@ class UfairDesc(C.Structure):
 
 
 DIST_FIXED, DIST_LOGNORMAL, DIST_NORMAL = 0, 1, 2
-LOOP_NAMES = ("general", "conc_driven", "plain", "plain_fext", "plain_subset")   # UFAIR_LOOP_*
+LOOP_NAMES = ("general", "conc_driven", "plain", "plain_fext", "plain_subset", "period_mean")   # UFAIR_LOOP_*
 
 
 class UfairSampler(C.Structure):

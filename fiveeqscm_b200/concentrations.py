@@ -45,7 +45,8 @@ def _require_cuda():
 
 @dataclass
 class HistSpec:
-    """Per-time-step temperature histogram: `bins` equal bins on [lo, hi) (edge bins absorb outliers).
+    """Per-output-row temperature histogram (per step, or per period with ``out_every``): `bins` equal bins on
+    [lo, hi) (edge bins absorb outliers).
 
     ``groups`` > 0 builds one histogram and one set of moments per member label (``stat_group=`` of
     :func:`run_ensemble`): results are then [groups][n_t][..].  0 pools every member (results [n_t][..]).
@@ -63,17 +64,18 @@ class HistSpec:
 
 @dataclass
 class EnsembleResult:
-    C: object = None        # [n_gas][n_t][n_member]
-    RF: object = None       # [n_gas][n_t][n_member]
-    T: object = None        # [n_t][n_member]
+    C: object = None        # [n_gas][n_out][n_member]; n_out = n_t, or n_t / out_every (period means)
+    RF: object = None       # [n_gas][n_out][n_member]
+    T: object = None        # [n_out][n_member]
     alpha: object = None    # [n_gas][n_t][n_member] (diagnostic)
     E: object = None        # [n_gas][n_t][n_member] emission rates (diagnosed for concentration-driven gases)
     state: object = None    # [5 n_gas + 3][n_member]  -> pass as state_in to continue the run
-    hist: object = None     # [n_t][bins] int64 counts (this rank's members); [groups][n_t][bins] when grouped
-    moments: object = None  # [n_t][4] float64: sum, sumsq, min, max of T over members; [groups][n_t][4] when grouped
+    hist: object = None     # [n_out][bins] int64 counts (this rank's members); [groups][n_out][bins] when grouped
+    moments: object = None  # [n_out][4] float64: sum, sumsq, min, max of T over members; [groups][n_out][4] when grouped
     spec: Optional[HistSpec] = None
     n_member: int = 0
     stat_group: Optional[str] = None  # what the statistics are grouped by: None (pooled), "scenario" or "labels"
+    out_every: int = 1      # steps per output row: 1 = every step, k >= 2 = means over periods of k steps
 
 
 # ------------------------------------------------------------------------------------------------
@@ -136,8 +138,25 @@ def _round_up(n, m):
     return (n + m - 1) // m * m
 
 
+def _out_rows(n_t, out_every=1, outputs=(), conc_driven=None) -> int:
+    """Output rows n_out of a run with ``out_every`` (include/ufair.h): n_t, or n_t / k for period means of k >= 2
+    steps -- which need n_t a multiple of k and support neither the alpha / E outputs nor concentration-driven
+    gases (the library rejects the same)."""
+    k = int(out_every)
+    if k != out_every or k < 0:
+        raise ValueError(f"out_every must be an integer >= 0, got {out_every!r}")
+    if k < 2:
+        return n_t
+    if n_t % k:
+        raise ValueError(f"out_every={k}: n_t = {n_t} steps is not a multiple of {k}")
+    if _any_driven(conc_driven) or "alpha" in outputs or "E" in outputs:
+        raise ValueError(f"out_every={k}: period means are not supported for the alpha / E outputs or "
+                         "concentration-driven gases")
+    return n_t // k
+
+
 def _build_desc(G, n_t, M, ld, n_scen, e_scen, fext_mode, alpha_mode, newton_iters, t_mode, outputs, dt, iirf_h,
-                iirf_max, stats: Optional[HistSpec], gas_form=None, conc_driven=None):
+                iirf_max, stats: Optional[HistSpec], gas_form=None, conc_driven=None, out_every=1):
     if alpha_mode not in _ALPHA:
         raise ValueError(f"alpha_mode must be one of {sorted(_ALPHA)}")
     if t_mode not in _TMODE:
@@ -155,9 +174,10 @@ def _build_desc(G, n_t, M, ld, n_scen, e_scen, fext_mode, alpha_mode, newton_ite
     if stats is not None:
         d.hist_bins, d.hist_copies = int(stats.bins), int(stats.copies)
         d.hist_lo, d.hist_hi = float(stats.lo), float(stats.hi)
-        d.hist_t0, d.hist_rows = 0, n_t
+        d.hist_t0, d.hist_rows = 0, _out_rows(n_t, out_every)
         d.n_stat_groups = int(stats.groups)
     d.conc_driven = _driven_mask(conc_driven, G)
+    d.out_every = int(out_every)
     if gas_form is not None and not isinstance(gas_form, str):
         if len(gas_form) != G:
             raise ValueError("gas_form must have one entry per gas")
@@ -210,14 +230,17 @@ def _driven_mask(conc_driven, G) -> int:
     return sum(1 << g for g, f in enumerate(flags) if f)
 
 
+def _any_driven(conc_driven) -> bool:
+    """Is any gas concentration-driven (``conc_driven=`` of :func:`run_ensemble`)?"""
+    if conc_driven is None or isinstance(conc_driven, bool):
+        return bool(conc_driven)
+    return any(bool(f) for f in conc_driven)
+
+
 def _with_E(outputs, conc_driven):
     """Concentration-driven runs always return the diagnosed emissions."""
     outputs = tuple(outputs)
-    if conc_driven is None or isinstance(conc_driven, bool):
-        driven = bool(conc_driven)
-    else:
-        driven = any(bool(f) for f in conc_driven)
-    return outputs + ("E",) if driven and "E" not in outputs else outputs
+    return outputs + ("E",) if _any_driven(conc_driven) and "E" not in outputs else outputs
 
 
 def _any_nonzero(row) -> bool:
@@ -241,19 +264,21 @@ def _detect_form_host(gp, state_in):
 
 
 def auto_chunk_members(n_gas, n_t, *, e_member, fext_member, outputs, return_state=True, state_in=False, e_scale=False,
-                       precision="f64") -> int:
+                       precision="f64", out_every=1) -> int:
     """Members per chunk of the host pipeline when the caller does not say.  What matters is which side of the
     pipeline a member keeps busy longer: the host link (bytes per member up or down at ~50 GB/s) or the integrator
     (~10 ns per member and 1000 gas-steps in FP64, a third of that in FP32).  Link-bound calls -- per-member emissions
     in, trajectories out -- want SMALL chunks (16 384: the fill and drain of the pipeline are one chunk each, and the
     link is busy whatever the kernel's efficiency); kernel-bound calls -- scenario-table inputs, statistics or T
     only out -- want chunks that fill the GPU for several waves (131 072; measured 1.8 / 2.2 / 2.2 / 1.9e10
-    member-steps/s at 32 768 / 131 072 / 262 144 / 786 432 on a 786 432-member call)."""
+    member-steps/s at 32 768 / 131 072 / 262 144 / 786 432 on a 786 432-member call).  Period means
+    (``out_every`` = k) bring back k times fewer rows, which can make a call with trajectories kernel-bound."""
     es = 8 if precision == "f64" else 4
     gt = n_gas * n_t
     up = (gt if e_member else 0) + (n_t if fext_member else 0) + n_gas * _abi.GP_COUNT + _abi.TP_COUNT + \
         (n_gas if e_scale else 0) + (_abi.state_rows(n_gas) if state_in else 0)
-    down = sum(math.prod(shape) for _, _, shape, _ in _result_layout(n_gas, n_t, 1, outputs, return_state, None))
+    down = sum(math.prod(shape) for _, _, shape, _ in _result_layout(n_gas, n_t, 1, outputs, return_state, None,
+                                                                      out_every))
     link_ns = max(up, down) * es / 50.0                       # ns per member at 50 GB/s, the busier direction
     kernel_ns = gt * (0.010 if precision == "f64" else 0.0035)   # ns per member: 27 ms / 9 ms per 1.25e6 x 736 x 3 on B200
     return 16384 if link_ns >= kernel_ns else 131072
@@ -283,7 +308,7 @@ def run_ensemble(emissions, gas_params, thermal_params, *, dt=1.0, scen_idx=None
                  fext_per_member=False, state_in=None, alpha_mode="exp", newton_iters=0, iirf_max=None,
                  iirf_h=100.0, t_mode="mid", outputs: Sequence[str] = ("C", "RF", "T"), stats: Optional[HistSpec] = None,
                  precision="f64", return_state=True, chunk_members=None, workspace=None, out=None,
-                 gas_form="auto", conc_driven=None, stat_group=None) -> EnsembleResult:
+                 gas_form="auto", conc_driven=None, stat_group=None, out_every=1) -> EnsembleResult:
     """Integrate the 5-equation model for an ensemble (oxfair, .coveragerc:19, as one kernel launch).
 
     emissions      [G][n_t][M] per-member emission RATES, or [G][n_t][S] scenario-shared with
@@ -299,6 +324,11 @@ def run_ensemble(emissions, gas_params, thermal_params, *, dt=1.0, scen_idx=None
                    scenario unless ``stats.groups`` says otherwise) or labels [M] int with ``stats.groups`` = G:
                    label g in [0, G) counts the member in group g, a negative label leaves it out of the
                    statistics.  ``.hist`` is then [G][n_t][bins] and ``.moments`` [G][n_t][4].
+    out_every      k >= 2: return one row of C, RF and T per period of k steps, the mean over its steps (a
+                   sequential sum in step order in the run's precision, times 1 / k); n_t must be a multiple of k.
+                   Results are then [G][n_t / k][M], [n_t / k][M], and the statistics bin the period-mean T
+                   rows.  Inputs stay per step.  Not with the alpha / E outputs or ``conc_driven``.  0 or 1: every
+                   step.  For labelled frames (frames.py) pass the period labels as ``years``.
     precision      "f64" (default; <= 1e-10 relative vs the float64 oracle) or "f32" (<= 1e-4 K in T).
     conc_driven    None, True (every gas) or one flag per gas: those gases' ``emissions`` rows are the
                    CONCENTRATION to reach at the end of each step; the emission rate that does so
@@ -321,7 +351,7 @@ def run_ensemble(emissions, gas_params, thermal_params, *, dt=1.0, scen_idx=None
     kw = dict(dt=dt, scen_idx=scen_idx, e_scale=e_scale, f_ext=f_ext, fext_per_member=fext_per_member, state_in=state_in,
               alpha_mode=alpha_mode, newton_iters=newton_iters, iirf_max=iirf_max, iirf_h=iirf_h, t_mode=t_mode,
               outputs=outputs, stats=stats, precision=precision, return_state=return_state, gas_form=gas_form,
-              conc_driven=conc_driven, stat_group=stat_group)
+              conc_driven=conc_driven, stat_group=stat_group, out_every=out_every)
     if isinstance(emissions, torch.Tensor) and emissions.is_cuda:
         return DevicePlan(emissions, gas_params, thermal_params, **kw).run()
     return _run_host(emissions, gas_params, thermal_params, chunk_members=chunk_members, workspace=workspace, out=out,
@@ -369,9 +399,11 @@ def _shapes(E_shape, gp_shape, tp_shape, scen_idx, fext_shape, fext_per_member, 
     return G, n_t, M, e_scen, n_scen, fext_mode
 
 
-def _result_layout(n_gas, n_t, M, outputs, return_state, stats: Optional[HistSpec]):
+def _result_layout(n_gas, n_t, M, outputs, return_state, stats: Optional[HistSpec], out_every=1):
     """(result field, descriptor field, shape, dtype) of every array a run returns.  dtype "real" is the run's
-    precision; hist and moments have no descriptor field (ufair_stats_finalize and ufair_run_host_* take them)."""
+    precision; hist and moments have no descriptor field (ufair_stats_finalize and ufair_run_host_* take them).
+    Output rows are per step, or per period of ``out_every`` steps."""
+    n_t = _out_rows(n_t, out_every, outputs)
     layout = [(o, "out_" + o, (n_t, M) if o == "T" else (n_gas, n_t, M), "real") for o in _OUT if o in outputs]
     if return_state:
         layout.append(("state", "state_out", (_abi.state_rows(n_gas), M), "real"))
@@ -439,7 +471,7 @@ class _HostArrays:
 
 def _prepare(arrays, E, gp, tp, *, dt=1.0, scen_idx=None, e_scale=None, f_ext=None, fext_per_member=False,
              state_in=None, alpha_mode="exp", newton_iters=0, iirf_max=None, iirf_h=100.0, t_mode="mid",
-             outputs=("C", "RF", "T"), stats=None, gas_form="auto", conc_driven=None, stat_group=None):
+             outputs=("C", "RF", "T"), stats=None, gas_form="auto", conc_driven=None, stat_group=None, out_every=1):
     """Checks a run's inputs (keywords of :func:`run_ensemble`) and places them with `arrays` (:class:`_DeviceArrays`
     or :class:`_HostArrays`).  Returns (descriptor with every input wired, the placed arrays by descriptor field,
     the outputs with "E" added for concentration-driven runs, the HistSpec with its group count settled, the label
@@ -453,9 +485,10 @@ def _prepare(arrays, E, gp, tp, *, dt=1.0, scen_idx=None, e_scale=None, f_ext=No
                                                    shape(e_scale), shape(state_in))
     stats, source = _resolve_groups(stats, stat_group, scen_idx is not None, n_scen)
     outputs = _with_E(outputs, conc_driven)
+    _out_rows(n_t, out_every, outputs, conc_driven)
     ld = arrays.ld(M)
     d = _build_desc(G, n_t, M, ld, n_scen, e_scen, fext_mode, alpha_mode, newton_iters, t_mode, outputs, dt, iirf_h,
-                    iirf_max, stats, gas_form, conc_driven)
+                    iirf_max, stats, gas_form, conc_driven, out_every)
     placed = dict(emissions=E if e_scen else arrays.rows(E, ld), gas_params=arrays.rows(gp, ld),
                   thermal_params=arrays.rows(tp, ld))
     if scen_idx is not None:
@@ -499,13 +532,15 @@ class DevicePlan:
         d, placed, outputs, stats, source = _prepare(_DeviceArrays(torch, dev, dtype), E, gp, tp, gas_form=gas_form,
                                                      **inputs)
         G, n_t, M, ld = d.n_gas, d.n_t, d.n_member, d.ld_member
+        k = max(int(d.out_every), 1)
         self.device, self.precision, self.stats = dev, precision, stats
         self.n_gas, self.n_t, self.n_member = G, n_t, M
+        self.out_every, self.n_out = k, n_t // k   # output rows: per step, or per period of k steps
         self.scen_idx = placed.get("scen_idx")   # the plan's own copy: callers that re-launch may overwrite it in place
         self.stat_group = placed.get("stat_group")
 
-        res = EnsembleResult(spec=stats, n_member=M, stat_group=source)
-        for name, field, shape, kind in _result_layout(G, n_t, M, outputs, return_state, stats):
+        res = EnsembleResult(spec=stats, n_member=M, stat_group=source, out_every=k)
+        for name, field, shape, kind in _result_layout(G, n_t, M, outputs, return_state, stats, k):
             if field is None:
                 setattr(res, name, torch.empty(shape, dtype=getattr(torch, kind), device=dev))
                 continue
@@ -514,9 +549,9 @@ class DevicePlan:
             setattr(res, name, buf[..., :M])
         if stats is not None:
             if "T" not in outputs:  # the moments pass reads the T rows: scratch the caller never sees
-                self._t_scratch = torch.empty(n_t, ld, dtype=dtype, device=dev)
+                self._t_scratch = torch.empty(self.n_out, ld, dtype=dtype, device=dev)
                 d.out_T = self._t_scratch.data_ptr()
-            rows = math.prod(stats.lead_shape(n_t))
+            rows = math.prod(stats.lead_shape(self.n_out))
             self._hp = torch.empty(stats.copies, rows, stats.bins, dtype=torch.int32, device=dev)
             self._mp = torch.empty(stats.copies, rows, _abi.MOM_COUNT, dtype=torch.float64, device=dev)
             d.hist_private, d.moments_private = self._hp.data_ptr(), self._mp.data_ptr()
@@ -598,13 +633,13 @@ def _run_host(E, gp, tp, *, precision="f64", return_state=True, gas_form="auto",
     torch = _torch()
     npdt = np.float64 if precision == "f64" else np.float32
     d, placed, outputs, stats, source = _prepare(_HostArrays(npdt), E, gp, tp, gas_form=gas_form, **inputs)
-    G, n_t, M = d.n_gas, d.n_t, d.n_member
+    G, n_t, M, k = d.n_gas, d.n_t, d.n_member, max(int(d.out_every), 1)
     if isinstance(gas_form, str) and M:
         for g, f in enumerate(_detect_form_host(placed["gas_params"], placed.get("state_in"))):
             d.gas_form[g] = f
     res = out if out is not None else EnsembleResult()
-    res.spec, res.n_member, res.stat_group = stats, M, source
-    for name, field, shape, kind in _result_layout(G, n_t, M, outputs, return_state, stats):
+    res.spec, res.n_member, res.stat_group, res.out_every = stats, M, source, k
+    for name, field, shape, kind in _result_layout(G, n_t, M, outputs, return_state, stats, k):
         cur = getattr(res, name)   # out= reuse: an array of the right shape and dtype is written in place
         if isinstance(cur, torch.Tensor):
             cur = cur.numpy()
@@ -620,7 +655,7 @@ def _run_host(E, gp, tp, *, precision="f64", return_state=True, gas_form="auto",
         chunk_members = auto_chunk_members(G, n_t, e_member=d.e_mode == _abi.E_MEMBER,
                                            fext_member=d.fext_mode == _abi.FEXT_MEMBER, outputs=outputs,
                                            return_state=return_state, state_in="state_in" in placed,
-                                           e_scale="e_scale" in placed, precision=precision)
+                                           e_scale="e_scale" in placed, precision=precision, out_every=k)
     ws = Workspace(torch.cuda.current_device(), chunk_members) if own else workspace
     try:
         L = _abi.lib()
@@ -633,13 +668,14 @@ def _run_host(E, gp, tp, *, precision="f64", return_state=True, gas_form="auto",
 
 
 def pinned_result(n_gas, n_t, n_member, outputs=("C", "RF", "T"), stats: Optional[HistSpec] = None, precision="f64",
-                  return_state=True) -> EnsembleResult:
+                  return_state=True, out_every=1) -> EnsembleResult:
     """Page-locked host output buffers for :func:`run_ensemble` ``out=`` (D2H at full PCIe speed).  Grouped
-    statistics need ``stats.groups`` set to the group count here (``HistSpec(groups=S)`` for per-scenario ones)."""
+    statistics need ``stats.groups`` set to the group count here (``HistSpec(groups=S)`` for per-scenario ones);
+    period means need the run's ``out_every``."""
     torch = _require_cuda()
     real = torch.float64 if precision == "f64" else torch.float32
-    r = EnsembleResult(spec=stats, n_member=n_member)
-    for name, _, shape, kind in _result_layout(n_gas, n_t, n_member, outputs, return_state, stats):
+    r = EnsembleResult(spec=stats, n_member=n_member, out_every=max(int(out_every), 1))
+    for name, _, shape, kind in _result_layout(n_gas, n_t, n_member, outputs, return_state, stats, out_every):
         dtype = real if kind == "real" else getattr(torch, kind)
         setattr(r, name, torch.empty(shape, dtype=dtype, pin_memory=True).numpy())
     return r

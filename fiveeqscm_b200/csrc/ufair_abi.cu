@@ -45,6 +45,19 @@ int check_stat_groups(const ufair_desc* d) {
   return UFAIR_OK;
 }
 
+// period means (out_every, include/ufair.h): the step count, and what the mean loop does not support
+int check_out_every(const ufair_desc* d) {
+  if (d->out_every < 0) return set_error(UFAIR_ERR_ARG, "out_every %d < 0", d->out_every);
+  if (d->out_every < 2) return UFAIR_OK;
+  if (d->n_t % d->out_every != 0)
+    return set_error(UFAIR_ERR_ARG, "n_t %d is not a multiple of out_every %d", d->n_t, d->out_every);
+  if (d->out_mask & (UFAIR_OUT_ALPHA | UFAIR_OUT_E))
+    return set_error(UFAIR_ERR_UNSUPPORTED, "out_every %d: the alpha and emissions outputs are per step only", d->out_every);
+  if (d->conc_driven != 0)
+    return set_error(UFAIR_ERR_UNSUPPORTED, "out_every %d: concentration-driven gases are not supported", d->out_every);
+  return UFAIR_OK;
+}
+
 int validate_desc(const ufair_desc* d, size_t elem) {
   if (!d) return set_error(UFAIR_ERR_ARG, "descriptor is NULL");
   if (d->struct_size != sizeof(ufair_desc))
@@ -68,8 +81,9 @@ int validate_desc(const ufair_desc* d, size_t elem) {
     return set_error(UFAIR_ERR_ARG, "newton_iters %d outside 0..8", d->newton_iters);
   if (d->n_scen < 1) return set_error(UFAIR_ERR_ARG, "n_scen must be >= 1");
   if (!(d->dt > 0.0) || !(d->iirf_h > 0.0)) return set_error(UFAIR_ERR_ARG, "dt and iirf_h must be > 0");
-  const int rc = check_stat_groups(d);
+  int rc = check_stat_groups(d);
   if (rc != UFAIR_OK) return rc;
+  if ((rc = check_out_every(d)) != UFAIR_OK) return rc;
   if (d->n_member == 0 || d->n_t == 0) return UFAIR_OK;
   if (!d->emissions || !d->gas_params || !d->thermal_params)
     return set_error(UFAIR_ERR_ARG, "emissions / gas_params / thermal_params must not be NULL");
@@ -90,8 +104,8 @@ int validate_desc(const ufair_desc* d, size_t elem) {
     if (d->hist_bins < 1 || d->hist_copies < 1 || !(d->hist_hi > d->hist_lo) || !d->hist_private || !d->moments_private)
       return set_error(UFAIR_ERR_ARG, "stats requested but histogram spec/buffers incomplete");
     if (!d->out_T) return set_error(UFAIR_ERR_ARG, "stats need out_T (the moments pass reads the T rows)");
-    if (d->hist_t0 < 0 || d->hist_rows < d->hist_t0 + d->n_t)
-      return set_error(UFAIR_ERR_ARG, "hist_rows %d < hist_t0 %d + n_t %d", d->hist_rows, d->hist_t0, d->n_t);
+    if (d->hist_t0 < 0 || d->hist_rows < d->hist_t0 + out_rows(d))
+      return set_error(UFAIR_ERR_ARG, "hist_rows %d < hist_t0 %d + output rows %d", d->hist_rows, d->hist_t0, out_rows(d));
   }
   return UFAIR_OK;
 }
@@ -138,6 +152,9 @@ template <typename Real> static KArgs<Real> make_args(const ufair_desc* d) {
   a.oE = (Real*)d->out_E;
   a.conc_driven = d->conc_driven;
   a.state_out = (Real*)d->state_out;
+  a.out_every = d->out_every >= 2 ? d->out_every : 1;
+  a.n_out = out_rows(d);
+  a.inv_every = (Real)(1.0 / a.out_every);
   return a;
 }
 
@@ -354,7 +371,8 @@ __global__ void __launch_bounds__(kStatsThreads)
 template <typename Real, int NGT, bool LABELS> static int launch_stats_pass(const ufair_desc* d, cudaStream_t stream) {
   const int G = LABELS ? stat_groups(d) : 1, n_tiles = (G + NGT - 1) / NGT;
   if (d->hist_copies > 65535) return set_error(UFAIR_ERR_ARG, "hist_copies %d > 65535", d->hist_copies);
-  if ((int64_t)d->n_t * n_tiles > (int64_t)INT32_MAX) return set_error(UFAIR_ERR_ARG, "n_t x group tiles too large");
+  const int rows = out_rows(d);  // the T rows the integrator wrote
+  if ((int64_t)rows * n_tiles > (int64_t)INT32_MAX) return set_error(UFAIR_ERR_ARG, "output rows x group tiles too large");
   const int smem_hist = (int64_t)NGT * d->hist_bins <= kStatsSmemBins ? 1 : 0;
   const size_t smem = smem_hist ? (size_t)NGT * d->hist_bins * sizeof(unsigned int) : 0;
   cudaError_t e = cudaSuccess;
@@ -363,7 +381,7 @@ template <typename Real, int NGT, bool LABELS> static int launch_stats_pass(cons
   if (e != cudaSuccess) return cuda_error(e, "cudaFuncSetAttribute(stats_pass_kernel)");
   const Real lo = (Real)d->hist_lo;
   const Real invw = (Real)((Real)d->hist_bins / ((Real)d->hist_hi - (Real)d->hist_lo));
-  stats_pass_kernel<Real, NGT, LABELS><<<dim3((unsigned)(d->n_t * n_tiles), (unsigned)d->hist_copies), kStatsThreads,
+  stats_pass_kernel<Real, NGT, LABELS><<<dim3((unsigned)(rows * n_tiles), (unsigned)d->hist_copies), kStatsThreads,
                                          smem, stream>>>((const Real*)d->out_T, d->ld_member, d->n_member, d->hist_t0,
                                                          d->hist_rows, d->hist_bins, lo, invw, smem_hist, d->hist_private,
                                                          d->moments_private, d->stat_group, G, n_tiles);

@@ -122,6 +122,7 @@ static int run_chunks(ufair_workspace* ws, const ufair_desc* h, const ufair_desc
   const int G = h->n_gas, n_t = h->n_t, out = h->out_mask;
   const int64_t M = h->n_member;
   const size_t gt = (size_t)G * n_t, srows = UFAIR_STATE_ROWS(G);
+  const size_t n_out = (size_t)out_rows(h), go = (size_t)G * n_out;  // output rows: per step or per period
   const bool e_member = h->e_mode == UFAIR_E_MEMBER;
   const bool labels_are_scen = h->stat_group != nullptr && h->stat_group == h->scen_idx;
   auto want = [&](int bit) { return (out & bit) != 0; };
@@ -139,9 +140,9 @@ static int run_chunks(ufair_workspace* ws, const ufair_desc* h, const ufair_desc
       {F(scen_idx), 1, i4, true, h->scen_idx != nullptr, false, true},
       {F(stat_group), 1, i4, true, h->stat_group != nullptr && !labels_are_scen, false, true,
        labels_are_scen ? F(scen_idx) : 0},
-      {F(out_C), gt, es, false, want(UFAIR_OUT_C), want(UFAIR_OUT_C), false},
-      {F(out_RF), gt, es, false, want(UFAIR_OUT_RF), want(UFAIR_OUT_RF), false},
-      {F(out_T), (size_t)n_t, es, false, want(UFAIR_OUT_T) || h->stats != 0, want(UFAIR_OUT_T), false},  // stats read T
+      {F(out_C), go, es, false, want(UFAIR_OUT_C), want(UFAIR_OUT_C), false},
+      {F(out_RF), go, es, false, want(UFAIR_OUT_RF), want(UFAIR_OUT_RF), false},
+      {F(out_T), n_out, es, false, want(UFAIR_OUT_T) || h->stats != 0, want(UFAIR_OUT_T), false},  // stats read T
       {F(out_alpha), gt, es, false, want(UFAIR_OUT_ALPHA), want(UFAIR_OUT_ALPHA), false},
       {F(out_E), gt, es, false, want(UFAIR_OUT_E), want(UFAIR_OUT_E), false},
       {F(state_out), srows, es, false, h->state_out != nullptr, h->state_out != nullptr, false},
@@ -233,7 +234,8 @@ template <typename Real> static int run_host(ufair_workspace* ws, const ufair_de
   if (h->n_gas < 1 || h->n_gas > UFAIR_MAX_GAS || h->n_t < 0 || h->n_member < 0 || h->ld_member < h->n_member)
     return set_error(UFAIR_ERR_ARG, "bad dimensions");
   if (h->stats && (!hist || !moments)) return set_error(UFAIR_ERR_ARG, "stats requested but hist/moments NULL");
-  const int rc0 = check_stat_groups(h);
+  int rc0 = check_stat_groups(h);
+  if (rc0 == UFAIR_OK) rc0 = check_out_every(h);
   if (rc0 != UFAIR_OK) return rc0;
   if (h->n_member == 0 || h->n_t == 0) return UFAIR_OK;
   if (!h->emissions || !h->gas_params || !h->thermal_params)
@@ -245,7 +247,7 @@ template <typename Real> static int run_host(ufair_workspace* ws, const ufair_de
 
   const size_t es = sizeof(Real);
   const int G = h->n_gas, n_t = h->n_t;
-  const size_t out_rows = (size_t)stat_groups(h) * n_t;  // statistics rows: [groups][n_t]
+  const size_t stat_rows = (size_t)stat_groups(h) * out_rows(h);  // statistics rows: [groups][n_out]
   ufair_desc d = *h;
   if (h->e_mode != UFAIR_E_MEMBER) {  // scenario-shared inputs go up once
     const size_t nb = (size_t)G * n_t * h->n_scen * es;
@@ -270,12 +272,12 @@ template <typename Real> static int run_host(ufair_workspace* ws, const ufair_de
     }
     d.hist_copies = h->hist_copies > 0 ? h->hist_copies : 16;
     d.hist_t0 = 0;
-    d.hist_rows = n_t;
-    const size_t rows = (size_t)d.hist_copies * out_rows;
+    d.hist_rows = out_rows(h);
+    const size_t rows = (size_t)d.hist_copies * stat_rows;
     CKS(ws->hist_private.reserve(rows * h->hist_bins * sizeof(uint32_t)), "cudaMalloc(hist_private)");
     CKS(ws->mom_private.reserve(rows * UFAIR_MOM_COUNT * sizeof(double)), "cudaMalloc(mom_private)");
-    CKS(ws->hist_out.reserve(out_rows * h->hist_bins * sizeof(uint64_t)), "cudaMalloc(hist)");
-    CKS(ws->mom_out.reserve(out_rows * UFAIR_MOM_COUNT * sizeof(double)), "cudaMalloc(moments)");
+    CKS(ws->hist_out.reserve(stat_rows * h->hist_bins * sizeof(uint64_t)), "cudaMalloc(hist)");
+    CKS(ws->mom_out.reserve(stat_rows * UFAIR_MOM_COUNT * sizeof(double)), "cudaMalloc(moments)");
     d.hist_private = (uint32_t*)ws->hist_private.p;
     d.moments_private = (double*)ws->mom_private.p;
     int rc = ufair_stats_reset(&d, ws->s_run);
@@ -294,8 +296,8 @@ template <typename Real> static int run_host(ufair_workspace* ws, const ufair_de
   if (rc == UFAIR_OK && h->stats) {
     rc = ufair_stats_finalize(&d, (uint64_t*)ws->hist_out.p, (double*)ws->mom_out.p, ws->s_run);
     if (rc == UFAIR_OK) {
-      cudaMemcpyAsync(hist, ws->hist_out.p, out_rows * h->hist_bins * sizeof(uint64_t), cudaMemcpyDeviceToHost, ws->s_run);
-      cudaMemcpyAsync(moments, ws->mom_out.p, out_rows * UFAIR_MOM_COUNT * sizeof(double), cudaMemcpyDeviceToHost, ws->s_run);
+      cudaMemcpyAsync(hist, ws->hist_out.p, stat_rows * h->hist_bins * sizeof(uint64_t), cudaMemcpyDeviceToHost, ws->s_run);
+      cudaMemcpyAsync(moments, ws->mom_out.p, stat_rows * UFAIR_MOM_COUNT * sizeof(double), cudaMemcpyDeviceToHost, ws->s_run);
     }
   }
   const cudaError_t e1 = cudaStreamSynchronize(ws->s_in), e2 = cudaStreamSynchronize(ws->s_run),

@@ -11,6 +11,9 @@ int validate_desc(const ufair_desc* d, size_t elem);
 int check_stat_groups(const ufair_desc* d);
 // statistics groups G: every statistics buffer holds G x hist_rows rows (include/ufair.h)
 inline int stat_groups(const ufair_desc* d) { return d->n_stat_groups > 1 ? d->n_stat_groups : 1; }
+// output rows of C, RF and T: one per step, or one per period of out_every >= 2 steps (include/ufair.h)
+inline int out_rows(const ufair_desc* d) { return d->out_every >= 2 ? d->n_t / d->out_every : d->n_t; }
+int check_out_every(const ufair_desc* d);
 template <typename Real> int run_device(const ufair_desc* d, cudaStream_t stream);
 template <typename Real> int run_stats_pass(const ufair_desc* d, cudaStream_t stream);
 }  // namespace ufair

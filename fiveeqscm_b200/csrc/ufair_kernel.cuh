@@ -137,7 +137,8 @@ constexpr int n_forms(int n_gas) {
 // code differs, so gases cannot share a warp's instruction stream).  The dense FP64 kernels of the default
 // alpha mode also exist with one gas per lane, for small ensembles (UFAIR_SMALL_ENSEMBLE).
 constexpr bool has_small_variant(int elem_size, int n_gas, int amode, int var) {
-  return elem_size == 8 && n_gas > 1 && amode == UFAIR_ALPHA_EXP && var != UFAIR_LOOP_CONC_DRIVEN;
+  return elem_size == 8 && n_gas > 1 && amode == UFAIR_ALPHA_EXP && var != UFAIR_LOOP_CONC_DRIVEN &&
+         var != UFAIR_LOOP_PERIOD_MEAN;
 }
 // members per warp: rows of MW elements must be a multiple of 16 bytes for the TMA box
 constexpr int members_per_warp(int elem_size, int n_gas, int gpl) {
@@ -171,6 +172,8 @@ template <typename Real> struct KArgs {
   unsigned long long* dbg_cut_hits;  // stores the check found in those rows (counted, not trapped)
 #endif
   Real* state_out;
+  int out_every, n_out;  // kVarMean: steps per output row (>= 2) and output rows
+  Real inv_every;        // (Real)(1.0 / out_every)
 };
 
 // ---- PTX wrappers: mbarrier, tensor-map TMA, shared-space loads/stores with 32-bit addresses ----
@@ -268,6 +271,18 @@ enum {
 };
 enum { T_QM0 = 0, T_QM1, T_DEC0, T_DEC1, T_COUNT };  // q_j (1 - e^{-dt/d_j}),  e^{-dt/d_j}
 
+// VAR, the instantiation of the time loop: kVarGeneral | kVarInverse (concentration-driven gases: diagnose the
+// emissions, emissions output) | kVarPlain (no external forcing, no iIRF ceiling, outputs among C, RF, T only: the
+// run-time switches for those cost ~38 of the general loop's 282 instructions, issued every step even when
+// predicated off -- measured 35.6 -> 34.1 ms) | kVarPlainFx (the same with external forcing, shared
+// or per member: the usual production configuration; default alpha mode only)
+// | kVarPlainSub (any subset of C, RF, T -- typically T + statistics only -- as three lane predicates
+// fixed before the loop; external forcing optional; default alpha mode only)
+// | kVarMean (out_every >= 2: the general loop's options but alpha / E outputs, with C, RF and T summed in
+// per-lane registers over a period of out_every steps and stored once per period, times 1 / out_every)
+enum { kVarGeneral = UFAIR_LOOP_GENERAL, kVarInverse = UFAIR_LOOP_CONC_DRIVEN, kVarPlain = UFAIR_LOOP_PLAIN,
+       kVarPlainFx = UFAIR_LOOP_PLAIN_FEXT, kVarPlainSub = UFAIR_LOOP_PLAIN_SUBSET, kVarMean = UFAIR_LOOP_PERIOD_MEAN };
+
 // ---- per-instantiation tuning: one row per class of kernel ---------------------------------------------
 // A class is a precision, dense or specialised form, and one gas or several per lane (GPL is 1 or NGAS, so the
 // one-gas kernels -- NGAS = 1, or the FP64 small-ensemble mapping -- share a row).  A row gives the time steps per
@@ -281,10 +296,13 @@ struct Tuning {
   bool alpha_reg, pool_reg, therm_reg;
   constexpr int min_blocks() const { return warps_per_sm / kWarps; }  // __launch_bounds__ counts CTAs
 };
-// classes by precision, then dense / specialised form, then several gases / one gas per lane
-enum { kF64Dense, kF64Dense1, kF64Form, kF64Form1, kF32Dense, kF32Dense1, kF32Form, kF32Form1, kClasses };
-constexpr int tuning_class(int elem_size, int gpl, unsigned form) {
-  return (elem_size == 8 ? 0 : 4) + (form != 0 ? 2 : 0) + (gpl == 1 ? 1 : 0);
+// classes by precision, then dense / specialised form, then several gases / one gas per lane; the period-mean loop
+// (seven more FP64 values per lane in the 3-gas kernel) has rows of its own where the register budget needs them
+enum { kF64Dense, kF64Dense1, kF64Form, kF64Form1, kF32Dense, kF32Dense1, kF32Form, kF32Form1, kF64DenseMean, kF64FormMean,
+       kClasses };
+constexpr int tuning_class(int elem_size, int gpl, unsigned form, int var) {
+  return (var == kVarMean && elem_size == 8 && gpl > 1) ? (form != 0 ? kF64FormMean : kF64DenseMean)
+                                                        : (elem_size == 8 ? 0 : 4) + (form != 0 ? 2 : 0) + (gpl == 1 ? 1 : 0);
 }
 constexpr Tuning kTuning[kClasses] = {
     // kF64Dense: all gases of a member in one lane, 2-4 gases.  Occupancy buys nothing here -- 16, 14, 12, 10 and
@@ -312,8 +330,17 @@ constexpr Tuning kTuning[kClasses] = {
     // kF32Form: specialised forms, 2-4 gases
     {8, 16, true, false, false},
     // kF32Form1: specialised forms of one gas: every constant in shared memory (not measured on its own)
-    {8, 16, false, false, false}};
-constexpr Tuning tuning(int elem_size, int gpl, unsigned form) { return kTuning[tuning_class(elem_size, gpl, form)]; }
+    {8, 16, false, false, false},
+    // kF64DenseMean: the period-mean loop, 2-4 gases: kF64Dense's row with the pool constants back in shared memory,
+    // which makes room for the accumulators (on the plain loop that move measured 2 %: [at,10] 27.5 ms, [apt,8] 27.0;
+    // 1.33x the plain loop's time at equal work, DESIGN.md 4.1)
+    {8, 8, true, false, true},
+    // kF64FormMean: the period-mean loop, specialised forms of 2-4 gases: kF64Form's row at 8 warps per SM (255
+    // registers instead of 168: the 4-gas kernel spills at 10)
+    {2, 8, true, true, true}};
+constexpr Tuning tuning(int elem_size, int gpl, unsigned form, int var) {
+  return kTuning[tuning_class(elem_size, gpl, form, var)];
+}
 
 constexpr int extra_rows(int amode) { return amode == UFAIR_ALPHA_NEWTON ? 3 : (amode == UFAIR_ALPHA_SINH ? 1 : 0); }
 constexpr size_t round128(size_t b) { return (b + 127) / 128 * 128; }
@@ -324,8 +351,8 @@ __host__ __device__ constexpr int gas_rows(int pg, int np) { return pg - 2 * (4 
 __host__ __device__ constexpr int compact_row(int np, int k) { return k < 4 ? k : (k < 8 ? np + (k - 4) : 2 * np + (k - 8)); }
 
 // per-WARP shared memory, in bytes (every piece 128-byte aligned: tensor-map TMA destinations)
-template <typename Real, int NGAS, int AMODE, int GPL, unsigned FORM = 0u> struct WarpSmem {
-  static constexpr Tuning TUNE = tuning(sizeof(Real), GPL, FORM);
+template <typename Real, int NGAS, int AMODE, int GPL, unsigned FORM, int VAR> struct WarpSmem {
+  static constexpr Tuning TUNE = tuning(sizeof(Real), GPL, FORM, VAR);
   static constexpr int TT = TUNE.tile_steps;  // time steps per tile
   static constexpr int MW = members_per_warp(sizeof(Real), NGAS, GPL);
   // rows per gas: register-resident alpha_val constants own none
@@ -373,8 +400,8 @@ template <typename Real, int NGAS, int AMODE, int GPL, unsigned FORM = 0u> struc
 // and change how the compiler unrolls the Newton iteration around them.  at() returns the place before the value
 // is computed, as a plain store computes its address first: a setter taking the value as an argument reorders the
 // prologue (and changes the code of the FP32 sinh kernels).
-template <typename Real, int NGAS, int AMODE, int GPL, unsigned FORM> struct LaneConsts {
-  using WS = WarpSmem<Real, NGAS, AMODE, GPL, FORM>;
+template <typename Real, int NGAS, int AMODE, int GPL, unsigned FORM, int VAR> struct LaneConsts {
+  using WS = WarpSmem<Real, NGAS, AMODE, GPL, FORM, VAR>;
   static constexpr bool kAlphaReg = WS::TUNE.alpha_reg, kPoolReg = WS::TUNE.pool_reg, kThermReg = WS::TUNE.therm_reg;
   uint32_t col;  // row 0 of this lane's column
   // register copies; only the rows in_reg() names are used, and of k0 / ka only the lane's pools (q < NP)
@@ -438,24 +465,17 @@ template <typename Real> __device__ __forceinline__ Real sum_pools(const Real (&
 }
 
 // GPL: gases per lane (1 or NGAS); FORM: per-gas specialisation (0 = dense; needs GPL == NGAS);
-// VAR: kVarGeneral | kVarInverse (concentration-driven gases: diagnose the emissions, emissions
-// output) | kVarPlain (no external forcing, no iIRF ceiling, outputs among C, RF, T only: the run-time
-// switches for those cost ~38 of the general loop's 282 instructions, issued every step even when
-// predicated off -- measured 35.6 -> 34.1 ms) | kVarPlainFx (the same with external forcing, shared
-// or per member: the usual production configuration; default alpha mode only)
-// | kVarPlainSub (any subset of C, RF, T -- typically T + statistics only -- as three lane predicates
-// fixed before the loop; external forcing optional; default alpha mode only)
-enum { kVarGeneral = UFAIR_LOOP_GENERAL, kVarInverse = UFAIR_LOOP_CONC_DRIVEN, kVarPlain = UFAIR_LOOP_PLAIN,
-       kVarPlainFx = UFAIR_LOOP_PLAIN_FEXT, kVarPlainSub = UFAIR_LOOP_PLAIN_SUBSET };
+// VAR: the loop (enum kVar* above the tuning table)
 template <typename Real, int NGAS, int AMODE, bool EMEM, int GPL, unsigned FORM, int VAR>
-__global__ void __launch_bounds__(kWarps * 32, tuning(sizeof(Real), GPL, FORM).min_blocks())
+__global__ void __launch_bounds__(kWarps * 32, tuning(sizeof(Real), GPL, FORM, VAR).min_blocks())
     ufair_integrate_kernel(const __grid_constant__ KArgs<Real> a, const __grid_constant__ CUtensorMap tmE,
                            const __grid_constant__ CUtensorMap tmF) {
   static_assert(FORM == 0 || GPL == NGAS, "a per-gas form needs all gases of a member in one lane");
-  constexpr bool INV = (VAR == kVarInverse), PLAIN = (VAR >= kVarPlain), NOFX = (VAR == kVarPlain),
-                 ALLOUT = (VAR == kVarPlain || VAR == kVarPlainFx);  // C, RF and T all written: no output predicates
+  constexpr bool INV = (VAR == kVarInverse), PLAIN = (VAR >= kVarPlain && VAR != kVarMean), NOFX = (VAR == kVarPlain),
+                 ALLOUT = (VAR == kVarPlain || VAR == kVarPlainFx),  // C, RF and T all written: no output predicates
+                 MEAN = (VAR == kVarMean);  // period means: sums in registers, one store per period and output
   using M = Math<Real>;
-  using WS = WarpSmem<Real, NGAS, AMODE, GPL, FORM>;
+  using WS = WarpSmem<Real, NGAS, AMODE, GPL, FORM, VAR>;
   constexpr int kTT = WS::TT;            // time steps per tile
   constexpr int GROUPS = NGAS / GPL;     // lanes per member
   constexpr int MW = WS::MW;             // members per warp
@@ -515,7 +535,7 @@ __global__ void __launch_bounds__(kWarps * 32, tuning(sizeof(Real), GPL, FORM).m
   // for the 10^6-year pool, so the one-off prologue always runs in FP64 and rounds once)
   Real R[GPL][4], Gcum[GPL], sumR[GPL];
   Real hot[GPL][H_COUNT], k0[GPL][4], ka[GPL][4], tr[T_COUNT];  // LaneConsts' register copies
-  LaneConsts<Real, NGAS, AMODE, GPL, FORM> cst{par, hot, k0, ka, tr};
+  LaneConsts<Real, NGAS, AMODE, GPL, FORM, VAR> cst{par, hot, k0, ka, tr};
   unsigned mk3[GPL];
   int nmin[GPL];  // lowest exponent alpha may take (Math::alpha_floor_exp)
   bool need_log[GPL], need_sqrt[GPL];
@@ -629,8 +649,8 @@ __global__ void __launch_bounds__(kWarps * 32, tuning(sizeof(Real), GPL, FORM).m
   const bool st_c = active && (a.out_mask & UFAIR_OUT_C) != 0, st_rf = active && (a.out_mask & UFAIR_OUT_RF) != 0,
              st_t = owner && ((a.out_mask & UFAIR_OUT_T) != 0 || a.stats != 0);
   pin(wm);
-  // running output pointers (gas g0; + gl * gstride)
-  const long long gstride = (long long)n_t * ld;
+  // running output pointers (gas g0; + gl * gstride); the mean loop's advance once per period
+  const long long gstride = (long long)(MEAN ? a.n_out : n_t) * ld;
   const long long o_gas = (long long)g0 * gstride + m_raw;
   Real* pC = a.oC + o_gas;
   Real* pRF = a.oRF + o_gas;
@@ -649,6 +669,16 @@ __global__ void __launch_bounds__(kWarps * 32, tuning(sizeof(Real), GPL, FORM).m
     e_next[gl] = (!EMEM && n_t > 0) ? __ldg(e_scen + gl * scen_gstride) : Real(0);
   }
   if (fx_scen && n_t > 0) fx_next = __ldg(fx_scen_p);
+  // the mean loop's period sums (s = 0; s = s + x every step; stored as s * (1 / out_every)) and its step counter
+  // inside the period, the same in every lane
+  Real sC[GPL], sRF[GPL], sT;
+  int kk;
+  if constexpr (MEAN) {
+    sT = Real(0);
+    kk = 0;
+#pragma unroll
+    for (int gl = 0; gl < GPL; ++gl) sC[gl] = sRF[gl] = Real(0);
+  }
 
   // ---------------- one time step ------------------------------------------------------------------
   auto step = [&](const int t, const uint32_t tt_off) {
@@ -749,11 +779,13 @@ __global__ void __launch_bounds__(kWarps * 32, tuning(sizeof(Real), GPL, FORM).m
       Gcum[gl] = fma(e[gl], dt, Gcum[gl]);
       sumR[gl] = sum_pools(R[gl], NP);
       Cg[gl] = cst.get(gl, G_C0) + sumR[gl];
-      if (ALLOUT ? active : PLAIN ? st_c : (wm & UFAIR_OUT_C) != 0) {
+      if constexpr (MEAN) {
+        sC[gl] = sC[gl] + Cg[gl];
+      } else if (ALLOUT ? active : PLAIN ? st_c : (wm & UFAIR_OUT_C) != 0) {
         UFAIR_CHECK_ST(a.oC, (long long)NGAS * n_t, pC + gl * gstride);
         st_stream(pC + gl * gstride, Cg[gl]);
       }
-      if (!PLAIN && (wm & UFAIR_OUT_ALPHA)) {
+      if (!PLAIN && !MEAN && (wm & UFAIR_OUT_ALPHA)) {
         UFAIR_CHECK_ST(a.oA, (long long)NGAS * n_t, pC + dA + gl * gstride);
         st_stream(pC + dA + gl * gstride, alpha[gl]);
       }
@@ -794,14 +826,18 @@ __global__ void __launch_bounds__(kWarps * 32, tuning(sizeof(Real), GPL, FORM).m
     Real Fsum = 0;
 #pragma unroll
     for (int gl = 0; gl < GPL; ++gl) {
-      if (ALLOUT ? active : PLAIN ? st_rf : (wm & UFAIR_OUT_RF) != 0) {
+      if constexpr (MEAN) {
+        sRF[gl] = sRF[gl] + Fg[gl];
+      } else if (ALLOUT ? active : PLAIN ? st_rf : (wm & UFAIR_OUT_RF) != 0) {
         UFAIR_CHECK_ST(a.oRF, (long long)NGAS * n_t, pRF + gl * gstride);
         st_stream(pRF + gl * gstride, Fg[gl]);
       }
       Fsum = (gl == 0) ? Fg[gl] : Fsum + Fg[gl];
     }
-    pC += ld;
-    pRF += ld;
+    if constexpr (!MEAN) {
+      pC += ld;
+      pRF += ld;
+    }
     // ---- total forcing of the member, gases in fixed order; external forcing last (as the oracle)
     Real Ftot;
     if (GROUPS == 1) {
@@ -821,11 +857,39 @@ __global__ void __launch_bounds__(kWarps * 32, tuning(sizeof(Real), GPL, FORM).m
     S1 = s1;
     Ssum = Snew;
     Tprev = T;
-    if (ALLOUT ? owner : PLAIN ? st_t : (wm & UFAIR_OUT_T) != 0) {
-      UFAIR_CHECK_ST(a.oT, (long long)n_t, pT);
-      st_stream(pT, T);
+    if constexpr (MEAN) {
+      sT = sT + T;
+      if (++kk == a.out_every) {  // uniform: the last step of a period stores its means and starts the next sums
+        kk = 0;
+        const Real w = a.inv_every;
+#pragma unroll
+        for (int gl = 0; gl < GPL; ++gl) {
+          if (st_c) {
+            UFAIR_CHECK_ST(a.oC, (long long)NGAS * a.n_out, pC + gl * gstride);
+            st_stream(pC + gl * gstride, sC[gl] * w);
+          }
+          if (st_rf) {
+            UFAIR_CHECK_ST(a.oRF, (long long)NGAS * a.n_out, pRF + gl * gstride);
+            st_stream(pRF + gl * gstride, sRF[gl] * w);
+          }
+          sC[gl] = sRF[gl] = Real(0);
+        }
+        if (st_t) {
+          UFAIR_CHECK_ST(a.oT, (long long)a.n_out, pT);
+          st_stream(pT, sT * w);
+        }
+        sT = Real(0);
+        pC += ld;
+        pRF += ld;
+        pT += ld;
+      }
+    } else {
+      if (ALLOUT ? owner : PLAIN ? st_t : (wm & UFAIR_OUT_T) != 0) {
+        UFAIR_CHECK_ST(a.oT, (long long)n_t, pT);
+        st_stream(pT, T);
+      }
+      pT += ld;
     }
-    pT += ld;
   };
 
   // ---------------- the time loop --------------------------------------------------------------------
@@ -874,7 +938,7 @@ int make_tensor_maps(const ufair_desc* d, size_t elem, int mw_members, int tile_
 
 template <typename Real, int NGAS, int AMODE, int GPL, unsigned FORM, int VAR>
 int launch_variant(const ufair_desc* d, const KArgs<Real>& a, cudaStream_t stream) {
-  using WS = WarpSmem<Real, NGAS, AMODE, GPL, FORM>;
+  using WS = WarpSmem<Real, NGAS, AMODE, GPL, FORM, VAR>;
   CUtensorMap tmE, tmF;  // box = WS::MW members x WS::TT steps (x NGAS gases): depends on the variant
   const int rc = make_tensor_maps(d, sizeof(Real), WS::MW, WS::TT, &tmE, &tmF);
   if (rc != UFAIR_OK) return rc;
@@ -919,7 +983,8 @@ struct Variant {
 inline Variant choose_variant(const ufair_desc* d, int elem_size) {
   // the plain loops: no iIRF ceiling, outputs among C, RF, T only, emission-driven
   const int crt = UFAIR_OUT_C | UFAIR_OUT_RF | UFAIR_OUT_T;
-  int loop = wants_inverse(d) ? kVarInverse
+  int loop = d->out_every >= 2 ? kVarMean
+             : wants_inverse(d) ? kVarInverse
              : ((d->iirf_max > 0.0 && isfinite(d->iirf_max)) || (d->out_mask & UFAIR_OUT_ALPHA)) ? kVarGeneral
              : (d->out_mask & crt) != crt ? kVarPlainSub
              : d->fext_mode == UFAIR_FEXT_NONE ? kVarPlain
@@ -977,7 +1042,8 @@ int launch_integrate(const ufair_desc* d, const KArgs<Real>& a, Variant v, cudaS
   template <>                                                                                               \
   int launch_integrate<Real, NGAS, AMODE>(const ufair_desc* d, const KArgs<Real>& a, Variant v, cudaStream_t s) { \
     return launch_chosen<Real, NGAS, AMODE>(                                                                \
-        d, a, v, s, std::integer_sequence<int, kVarGeneral, kVarInverse, kVarPlain, kVarPlainFx, kVarPlainSub>()); \
+        d, a, v, s,                                                                                         \
+        std::integer_sequence<int, kVarGeneral, kVarInverse, kVarPlain, kVarPlainFx, kVarPlainSub, kVarMean>()); \
   }
 #define UFAIR_INSTANTIATE(Real, NGAS)                                                                       \
   UFAIR_LAUNCHER(Real, NGAS, UFAIR_ALPHA_EXP)                                                               \

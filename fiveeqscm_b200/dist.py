@@ -58,7 +58,7 @@ class StatsReducer:
         self.plan, self.group = plan, group
         self.world = dist.get_world_size(group) if (dist.is_available() and dist.is_initialized()) else 1
         self._k = 0
-        self._rows = math.prod(plan.stats.lead_shape(plan.n_t)) if plan.stats is not None else 0
+        self._rows = math.prod(plan.stats.lead_shape(plan.n_out)) if plan.stats is not None else 0
         if self.world > 1 and plan.stats is not None:
             rows, bins = self._rows, plan.stats.bins
             dev = plan.device

@@ -40,7 +40,7 @@
 extern "C" {
 #endif
 
-#define UFAIR_ABI_VERSION 3
+#define UFAIR_ABI_VERSION 4
 
 #define UFAIR_MAX_GAS 4
 #define UFAIR_N_POOL 4
@@ -124,7 +124,7 @@ typedef struct ufair_desc {
   int32_t newton_iters; /* UFAIR_ALPHA_NEWTON only, 0..8 */
   int32_t t_mode;       /* UFAIR_T_* */
   int32_t out_mask;     /* UFAIR_OUT_* bits; outputs not selected may be NULL */
-  int32_t stats;        /* 0 = none, 1 = per-step T histogram + moments */
+  int32_t stats;        /* 0 = none, 1 = per-output-row T histogram + moments */
 
   double dt;       /* step length (yr) */
   double iirf_h;   /* iIRF horizon, 100 */
@@ -140,9 +140,9 @@ typedef struct ufair_desc {
   const void* state_in;       /* [UFAIR_STATE_ROWS][ld_member] or NULL (= all zero) */
 
   /* ---- outputs ---- */
-  void* out_C;     /* [n_gas][n_t][ld_member] */
-  void* out_RF;    /* [n_gas][n_t][ld_member] */
-  void* out_T;     /* [n_t][ld_member]        */
+  void* out_C;     /* [n_gas][n_out][ld_member]; n_out = n_t, or n_t / out_every (period means below) */
+  void* out_RF;    /* [n_gas][n_out][ld_member] */
+  void* out_T;     /* [n_out][ld_member]        */
   void* out_alpha; /* [n_gas][n_t][ld_member] (diagnostic) */
   void* state_out; /* [UFAIR_STATE_ROWS][ld_member] or NULL */
 
@@ -180,8 +180,8 @@ typedef struct ufair_desc {
   int32_t hist_bins;
   int32_t hist_copies;
   double hist_lo, hist_hi;
-  int32_t hist_t0;          /* row offset: step t of this call lands in row hist_t0 + t */
-  int32_t hist_rows;        /* rows allocated per copy (>= hist_t0 + n_t) */
+  int32_t hist_t0;          /* row offset: output row t of this call lands in row hist_t0 + t */
+  int32_t hist_rows;        /* rows allocated per copy (>= hist_t0 + n_out) */
   uint32_t* hist_private;   /* [hist_copies][hist_rows][hist_bins] */
   double* moments_private;  /* [hist_copies][hist_rows][UFAIR_MOM_COUNT]: member slice c of every
                                row is folded into copy c, in a fixed order (deterministic) */
@@ -200,7 +200,19 @@ typedef struct ufair_desc {
 
   /* ---- grouped statistics (see the statistics block above; stats == 1 only) ---- */
   int32_t n_stat_groups;      /* 0 or 1 = pooled; up to UFAIR_MAX_STAT_GROUPS */
-  int32_t reserved1;
+
+  /* ---- period means ----
+   * out_every = k: 0 or 1 writes one row of C, RF and T per step (n_out = n_t).  k >= 2 writes one row per
+   * period of k steps instead: n_t must be a multiple of k (else UFAIR_ERR_ARG), n_out = n_t / k, and row p of
+   * out_C, out_RF ([n_gas][n_out][ld_member]) and out_T ([n_out][ld_member]) is the mean of that output over
+   * steps p k .. p k + k - 1, defined bit for bit as
+   *   s = 0;  s = s + x_t for t = p k .. p k + k - 1 in step order (the run's precision);  mean = s * (Real)(1.0 / k)
+   * with no contraction into FMAs.  Inputs (emissions, f_ext) stay per step; state_out is the state at the end
+   * of the call.  A run split into calls of whole periods (state_in / state_out) gives the rows of one call.
+   * The statistics bin the period-mean T rows: hist_t0 counts output rows and hist_rows >= hist_t0 + n_out.
+   * With k >= 2 the diagnostics UFAIR_OUT_ALPHA and UFAIR_OUT_E and concentration-driven gases
+   * (conc_driven != 0) are not supported: UFAIR_ERR_UNSUPPORTED. */
+  int32_t out_every;
   const int32_t* stat_group;  /* [n_member] group labels, or NULL */
 } ufair_desc;
 
@@ -231,15 +243,17 @@ enum { UFAIR_LOOP_GENERAL = 0,      /* every run-time option                    
        UFAIR_LOOP_CONC_DRIVEN = 1,  /* concentration-driven gases / emissions output                 */
        UFAIR_LOOP_PLAIN = 2,        /* no f_ext, no iIRF ceiling, outputs exactly C + RF + T         */
        UFAIR_LOOP_PLAIN_FEXT = 3,   /* the same with external forcing (default alpha mode)           */
-       UFAIR_LOOP_PLAIN_SUBSET = 4  /* a subset of C, RF, T (e.g. T + statistics only), with or
-                                       without external forcing (default alpha mode)                */ };
+       UFAIR_LOOP_PLAIN_SUBSET = 4, /* a subset of C, RF, T (e.g. T + statistics only), with or
+                                       without external forcing (default alpha mode)                */
+       UFAIR_LOOP_PERIOD_MEAN = 5   /* out_every >= 2: period means of C, RF, T (every alpha mode)   */ };
 int ufair_kernel_variant(const ufair_desc* d, int32_t elem_size, uint32_t* form, int32_t* gases_per_lane,
                          int32_t* members_per_warp, int32_t* loop);
 
 /* Zero (and initialise the min/max sentinels of) the private statistics buffers. */
 int ufair_stats_reset(const ufair_desc* d, void* stream);
-/* The statistics pass: per-step histogram and moments of the T rows ufair_run_* just wrote
- * (d->out_T; same descriptor, same stream).  One call per ufair_run_* call when stats == 1. */
+/* The statistics pass: per-row histogram and moments of the T rows ufair_run_* just wrote
+ * (d->out_T, n_out rows: per step, or per period with out_every >= 2; same descriptor, same stream).
+ * One call per ufair_run_* call when stats == 1. */
 int ufair_stats_pass_f64(const ufair_desc* d, void* stream);
 int ufair_stats_pass_f32(const ufair_desc* d, void* stream);
 /* Fold the private copies: hist[G][hist_rows][hist_bins] (uint64 counts) and
