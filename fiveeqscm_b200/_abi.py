@@ -7,7 +7,7 @@ from __future__ import annotations
 import ctypes as C
 import os
 
-ABI_VERSION = 4
+ABI_VERSION = 5
 MAX_GAS = 4
 N_POOL = 4
 MAX_STAT_GROUPS = 256
@@ -30,6 +30,7 @@ FEXT_NONE, FEXT_SCENARIO, FEXT_MEMBER = 0, 1, 2
 ALPHA_EXP, ALPHA_SINH, ALPHA_NEWTON, ALPHA_ONE = 0, 1, 2, 3
 T_MID, T_END = 0, 1
 OUT_C, OUT_RF, OUT_T, OUT_ALPHA, OUT_E = 1, 2, 4, 8, 16
+OUTTYPE_RUN, OUTTYPE_F32 = 0, 1
 MOM_SUM, MOM_SUMSQ, MOM_MIN, MOM_MAX, MOM_COUNT = 0, 1, 2, 3, 4
 
 OK, ERR_ARG, ERR_ALIGN, ERR_CUDA, ERR_UNSUPPORTED, ERR_NOMEM = 0, -1, -2, -3, -4, -5
@@ -43,7 +44,7 @@ class UfairDesc(C.Structure):
     """Mirror of `struct ufair_desc` (include/ufair.h); field order and types must match."""
     _fields_ = [
         ("struct_size", C.c_uint32),
-        ("reserved0", C.c_uint32),
+        ("out_type", C.c_int32),
         ("n_gas", C.c_int32),
         ("n_t", C.c_int32),
         ("n_member", C.c_int64),

@@ -155,8 +155,24 @@ def _out_rows(n_t, out_every=1, outputs=(), conc_driven=None) -> int:
     return n_t // k
 
 
+def _out_kind(precision="f64", out_dtype=None, outputs=(), conc_driven=None) -> str:
+    """The element type of a run's C, RF and T (``out_dtype=`` of :func:`run_ensemble`) as a result-layout dtype:
+    "real" (the run's precision) or "float32" (float32 outputs of an FP64 run, which support neither the alpha / E
+    outputs nor concentration-driven gases: the library rejects the same).  No combination widens the outputs."""
+    if out_dtype not in (None, "f64", "f32"):
+        raise ValueError(f"out_dtype must be None, 'f64' or 'f32', got {out_dtype!r}")
+    if out_dtype is None or out_dtype == precision:
+        return "real"
+    if out_dtype == "f64":
+        raise ValueError("out_dtype='f64' with precision='f32': outputs are never wider than the run")
+    if _any_driven(conc_driven) or "alpha" in outputs or "E" in outputs:
+        raise ValueError("out_dtype='f32' of an FP64 run is not supported for the alpha / E outputs or "
+                         "concentration-driven gases")
+    return "float32"
+
+
 def _build_desc(G, n_t, M, ld, n_scen, e_scen, fext_mode, alpha_mode, newton_iters, t_mode, outputs, dt, iirf_h,
-                iirf_max, stats: Optional[HistSpec], gas_form=None, conc_driven=None, out_every=1):
+                iirf_max, stats: Optional[HistSpec], gas_form=None, conc_driven=None, out_every=1, out_kind="real"):
     if alpha_mode not in _ALPHA:
         raise ValueError(f"alpha_mode must be one of {sorted(_ALPHA)}")
     if t_mode not in _TMODE:
@@ -178,6 +194,7 @@ def _build_desc(G, n_t, M, ld, n_scen, e_scen, fext_mode, alpha_mode, newton_ite
         d.n_stat_groups = int(stats.groups)
     d.conc_driven = _driven_mask(conc_driven, G)
     d.out_every = int(out_every)
+    d.out_type = _abi.OUTTYPE_F32 if out_kind == "float32" else _abi.OUTTYPE_RUN
     if gas_form is not None and not isinstance(gas_form, str):
         if len(gas_form) != G:
             raise ValueError("gas_form must have one entry per gas")
@@ -264,7 +281,7 @@ def _detect_form_host(gp, state_in):
 
 
 def auto_chunk_members(n_gas, n_t, *, e_member, fext_member, outputs, return_state=True, state_in=False, e_scale=False,
-                       precision="f64", out_every=1) -> int:
+                       precision="f64", out_every=1, out_dtype=None) -> int:
     """Members per chunk of the host pipeline when the caller does not say.  What matters is which side of the
     pipeline a member keeps busy longer: the host link (bytes per member up or down at ~50 GB/s) or the integrator
     (~10 ns per member and 1000 gas-steps in FP64, a third of that in FP32).  Link-bound calls -- per-member emissions
@@ -272,14 +289,16 @@ def auto_chunk_members(n_gas, n_t, *, e_member, fext_member, outputs, return_sta
     link is busy whatever the kernel's efficiency); kernel-bound calls -- scenario-table inputs, statistics or T
     only out -- want chunks that fill the GPU for several waves (131 072; measured 1.8 / 2.2 / 2.2 / 1.9e10
     member-steps/s at 32 768 / 131 072 / 262 144 / 786 432 on a 786 432-member call).  Period means
-    (``out_every`` = k) bring back k times fewer rows, which can make a call with trajectories kernel-bound."""
+    (``out_every`` = k) bring back k times fewer rows, and float32 outputs (``out_dtype="f32"``) 4 bytes per element
+    instead of 8; either can make a call with trajectories kernel-bound."""
     es = 8 if precision == "f64" else 4
     gt = n_gas * n_t
     up = (gt if e_member else 0) + (n_t if fext_member else 0) + n_gas * _abi.GP_COUNT + _abi.TP_COUNT + \
         (n_gas if e_scale else 0) + (_abi.state_rows(n_gas) if state_in else 0)
-    down = sum(math.prod(shape) for _, _, shape, _ in _result_layout(n_gas, n_t, 1, outputs, return_state, None,
-                                                                      out_every))
-    link_ns = max(up, down) * es / 50.0                       # ns per member at 50 GB/s, the busier direction
+    kind = _out_kind(precision, out_dtype, outputs)
+    down = sum(math.prod(shape) * (es if k == "real" else np.dtype(k).itemsize)
+               for _, _, shape, k in _result_layout(n_gas, n_t, 1, outputs, return_state, None, out_every, kind))
+    link_ns = max(up * es, down) / 50.0                       # ns per member at 50 GB/s, the busier direction
     kernel_ns = gt * (0.010 if precision == "f64" else 0.0035)   # ns per member: 27 ms / 9 ms per 1.25e6 x 736 x 3 on B200
     return 16384 if link_ns >= kernel_ns else 131072
 
@@ -308,7 +327,7 @@ def run_ensemble(emissions, gas_params, thermal_params, *, dt=1.0, scen_idx=None
                  fext_per_member=False, state_in=None, alpha_mode="exp", newton_iters=0, iirf_max=None,
                  iirf_h=100.0, t_mode="mid", outputs: Sequence[str] = ("C", "RF", "T"), stats: Optional[HistSpec] = None,
                  precision="f64", return_state=True, chunk_members=None, workspace=None, out=None,
-                 gas_form="auto", conc_driven=None, stat_group=None, out_every=1) -> EnsembleResult:
+                 gas_form="auto", conc_driven=None, stat_group=None, out_every=1, out_dtype=None) -> EnsembleResult:
     """Integrate the 5-equation model for an ensemble (oxfair, .coveragerc:19, as one kernel launch).
 
     emissions      [G][n_t][M] per-member emission RATES, or [G][n_t][S] scenario-shared with
@@ -330,6 +349,11 @@ def run_ensemble(emissions, gas_params, thermal_params, *, dt=1.0, scen_idx=None
                    rows.  Inputs stay per step.  Not with the alpha / E outputs or ``conc_driven``.  0 or 1: every
                    step.  For labelled frames (frames.py) pass the period labels as ``years``.
     precision      "f64" (default; <= 1e-10 relative vs the float64 oracle) or "f32" (<= 1e-4 K in T).
+    out_dtype      element type of C, RF and T: None (the run's precision), "f64" or "f32".  "f32" with
+                   precision="f64" integrates in FP64 and stores each value rounded once to float32 (exactly the
+                   float32 cast of the FP64 run's value): half the bytes on the device and over the host link.
+                   ``.state`` stays float64; the statistics bin the stored float32 T.  Not with the alpha / E
+                   outputs or ``conc_driven``.  Never wider than ``precision``.
     conc_driven    None, True (every gas) or one flag per gas: those gases' ``emissions`` rows are the
                    CONCENTRATION to reach at the end of each step; the emission rate that does so
                    is diagnosed (step_conc inverted exactly) and returned as ``.E`` (all gases).
@@ -351,7 +375,7 @@ def run_ensemble(emissions, gas_params, thermal_params, *, dt=1.0, scen_idx=None
     kw = dict(dt=dt, scen_idx=scen_idx, e_scale=e_scale, f_ext=f_ext, fext_per_member=fext_per_member, state_in=state_in,
               alpha_mode=alpha_mode, newton_iters=newton_iters, iirf_max=iirf_max, iirf_h=iirf_h, t_mode=t_mode,
               outputs=outputs, stats=stats, precision=precision, return_state=return_state, gas_form=gas_form,
-              conc_driven=conc_driven, stat_group=stat_group, out_every=out_every)
+              conc_driven=conc_driven, stat_group=stat_group, out_every=out_every, out_dtype=out_dtype)
     if isinstance(emissions, torch.Tensor) and emissions.is_cuda:
         return DevicePlan(emissions, gas_params, thermal_params, **kw).run()
     return _run_host(emissions, gas_params, thermal_params, chunk_members=chunk_members, workspace=workspace, out=out,
@@ -399,12 +423,14 @@ def _shapes(E_shape, gp_shape, tp_shape, scen_idx, fext_shape, fext_per_member, 
     return G, n_t, M, e_scen, n_scen, fext_mode
 
 
-def _result_layout(n_gas, n_t, M, outputs, return_state, stats: Optional[HistSpec], out_every=1):
+def _result_layout(n_gas, n_t, M, outputs, return_state, stats: Optional[HistSpec], out_every=1, out_kind="real"):
     """(result field, descriptor field, shape, dtype) of every array a run returns.  dtype "real" is the run's
-    precision; hist and moments have no descriptor field (ufair_stats_finalize and ufair_run_host_* take them).
-    Output rows are per step, or per period of ``out_every`` steps."""
+    precision; C, RF and T have ``out_kind`` ("real" or "float32", :func:`_out_kind`), the state and the alpha / E
+    diagnostics "real"; hist and moments have no descriptor field (ufair_stats_finalize and ufair_run_host_* take
+    them).  Output rows are per step, or per period of ``out_every`` steps."""
     n_t = _out_rows(n_t, out_every, outputs)
-    layout = [(o, "out_" + o, (n_t, M) if o == "T" else (n_gas, n_t, M), "real") for o in _OUT if o in outputs]
+    layout = [(o, "out_" + o, (n_t, M) if o == "T" else (n_gas, n_t, M), out_kind if o in ("C", "RF", "T") else "real")
+              for o in _OUT if o in outputs]
     if return_state:
         layout.append(("state", "state_out", (_abi.state_rows(n_gas), M), "real"))
     if stats is not None:
@@ -471,11 +497,13 @@ class _HostArrays:
 
 def _prepare(arrays, E, gp, tp, *, dt=1.0, scen_idx=None, e_scale=None, f_ext=None, fext_per_member=False,
              state_in=None, alpha_mode="exp", newton_iters=0, iirf_max=None, iirf_h=100.0, t_mode="mid",
-             outputs=("C", "RF", "T"), stats=None, gas_form="auto", conc_driven=None, stat_group=None, out_every=1):
+             outputs=("C", "RF", "T"), stats=None, gas_form="auto", conc_driven=None, stat_group=None, out_every=1,
+             precision="f64", out_dtype=None):
     """Checks a run's inputs (keywords of :func:`run_ensemble`) and places them with `arrays` (:class:`_DeviceArrays`
     or :class:`_HostArrays`).  Returns (descriptor with every input wired, the placed arrays by descriptor field,
     the outputs with "E" added for concentration-driven runs, the HistSpec with its group count settled, the label
-    source of :func:`_resolve_groups`).  ``gas_form="auto"`` is left to the caller: it scans the placed arrays."""
+    source of :func:`_resolve_groups`); the descriptor's out_type gives the outputs' dtype (:func:`_desc_out_kind`).
+    ``gas_form="auto"`` is left to the caller: it scans the placed arrays."""
     if isinstance(gas_form, str) and gas_form != "auto":
         raise ValueError("gas_form must be 'auto', None or one entry per gas")
     E, gp, tp, e_scale, f_ext, state_in = (None if x is None else arrays.array(x)
@@ -486,9 +514,10 @@ def _prepare(arrays, E, gp, tp, *, dt=1.0, scen_idx=None, e_scale=None, f_ext=No
     stats, source = _resolve_groups(stats, stat_group, scen_idx is not None, n_scen)
     outputs = _with_E(outputs, conc_driven)
     _out_rows(n_t, out_every, outputs, conc_driven)
+    out_kind = _out_kind(precision, out_dtype, outputs, conc_driven)
     ld = arrays.ld(M)
     d = _build_desc(G, n_t, M, ld, n_scen, e_scen, fext_mode, alpha_mode, newton_iters, t_mode, outputs, dt, iirf_h,
-                    iirf_max, stats, gas_form, conc_driven, out_every)
+                    iirf_max, stats, gas_form, conc_driven, out_every, out_kind)
     placed = dict(emissions=E if e_scen else arrays.rows(E, ld), gas_params=arrays.rows(gp, ld),
                   thermal_params=arrays.rows(tp, ld))
     if scen_idx is not None:
@@ -518,6 +547,11 @@ def _prepare(arrays, E, gp, tp, *, dt=1.0, scen_idx=None, e_scale=None, f_ext=No
     return d, placed, outputs, stats, source
 
 
+def _desc_out_kind(d) -> str:
+    """The result-layout dtype of C, RF and T a prepared descriptor stores (:func:`_out_kind`)."""
+    return "float32" if d.out_type == _abi.OUTTYPE_F32 else "real"
+
+
 class DevicePlan:
     """A prepared device-resident run: descriptor + buffers.  ``run_ensemble`` on CUDA tensors is
     ``plan = DevicePlan(...); plan.reset_stats(); plan.launch(); plan.finalize_stats()``; callers
@@ -530,26 +564,28 @@ class DevicePlan:
         dtype = torch.float64 if precision == "f64" else torch.float32
         dev = E.device
         d, placed, outputs, stats, source = _prepare(_DeviceArrays(torch, dev, dtype), E, gp, tp, gas_form=gas_form,
-                                                     **inputs)
+                                                     precision=precision, **inputs)
+        out_kind = _desc_out_kind(d)
+        odtype = dtype if out_kind == "real" else getattr(torch, out_kind)   # C, RF and T (and the T scratch)
         G, n_t, M, ld = d.n_gas, d.n_t, d.n_member, d.ld_member
         k = max(int(d.out_every), 1)
-        self.device, self.precision, self.stats = dev, precision, stats
+        self.device, self.precision, self.stats, self.out_dtype = dev, precision, stats, odtype
         self.n_gas, self.n_t, self.n_member = G, n_t, M
         self.out_every, self.n_out = k, n_t // k   # output rows: per step, or per period of k steps
         self.scen_idx = placed.get("scen_idx")   # the plan's own copy: callers that re-launch may overwrite it in place
         self.stat_group = placed.get("stat_group")
 
         res = EnsembleResult(spec=stats, n_member=M, stat_group=source, out_every=k)
-        for name, field, shape, kind in _result_layout(G, n_t, M, outputs, return_state, stats, k):
+        for name, field, shape, kind in _result_layout(G, n_t, M, outputs, return_state, stats, k, out_kind):
             if field is None:
                 setattr(res, name, torch.empty(shape, dtype=getattr(torch, kind), device=dev))
                 continue
-            buf = torch.empty(shape[:-1] + (ld,), dtype=dtype, device=dev)
+            buf = torch.empty(shape[:-1] + (ld,), dtype=dtype if kind == "real" else getattr(torch, kind), device=dev)
             setattr(d, field, buf.data_ptr())
             setattr(res, name, buf[..., :M])
         if stats is not None:
             if "T" not in outputs:  # the moments pass reads the T rows: scratch the caller never sees
-                self._t_scratch = torch.empty(self.n_out, ld, dtype=dtype, device=dev)
+                self._t_scratch = torch.empty(self.n_out, ld, dtype=odtype, device=dev)
                 d.out_T = self._t_scratch.data_ptr()
             rows = math.prod(stats.lead_shape(self.n_out))
             self._hp = torch.empty(stats.copies, rows, stats.bins, dtype=torch.int32, device=dev)
@@ -632,14 +668,16 @@ def _run_host(E, gp, tp, *, precision="f64", return_state=True, gas_form="auto",
               out=None, **inputs):
     torch = _torch()
     npdt = np.float64 if precision == "f64" else np.float32
-    d, placed, outputs, stats, source = _prepare(_HostArrays(npdt), E, gp, tp, gas_form=gas_form, **inputs)
+    d, placed, outputs, stats, source = _prepare(_HostArrays(npdt), E, gp, tp, gas_form=gas_form, precision=precision,
+                                                 **inputs)
+    out_kind = _desc_out_kind(d)
     G, n_t, M, k = d.n_gas, d.n_t, d.n_member, max(int(d.out_every), 1)
     if isinstance(gas_form, str) and M:
         for g, f in enumerate(_detect_form_host(placed["gas_params"], placed.get("state_in"))):
             d.gas_form[g] = f
     res = out if out is not None else EnsembleResult()
     res.spec, res.n_member, res.stat_group, res.out_every = stats, M, source, k
-    for name, field, shape, kind in _result_layout(G, n_t, M, outputs, return_state, stats, k):
+    for name, field, shape, kind in _result_layout(G, n_t, M, outputs, return_state, stats, k, out_kind):
         cur = getattr(res, name)   # out= reuse: an array of the right shape and dtype is written in place
         if isinstance(cur, torch.Tensor):
             cur = cur.numpy()
@@ -655,7 +693,8 @@ def _run_host(E, gp, tp, *, precision="f64", return_state=True, gas_form="auto",
         chunk_members = auto_chunk_members(G, n_t, e_member=d.e_mode == _abi.E_MEMBER,
                                            fext_member=d.fext_mode == _abi.FEXT_MEMBER, outputs=outputs,
                                            return_state=return_state, state_in="state_in" in placed,
-                                           e_scale="e_scale" in placed, precision=precision, out_every=k)
+                                           e_scale="e_scale" in placed, precision=precision, out_every=k,
+                                           out_dtype=inputs.get("out_dtype"))
     ws = Workspace(torch.cuda.current_device(), chunk_members) if own else workspace
     try:
         L = _abi.lib()
@@ -668,14 +707,15 @@ def _run_host(E, gp, tp, *, precision="f64", return_state=True, gas_form="auto",
 
 
 def pinned_result(n_gas, n_t, n_member, outputs=("C", "RF", "T"), stats: Optional[HistSpec] = None, precision="f64",
-                  return_state=True, out_every=1) -> EnsembleResult:
+                  return_state=True, out_every=1, out_dtype=None) -> EnsembleResult:
     """Page-locked host output buffers for :func:`run_ensemble` ``out=`` (D2H at full PCIe speed).  Grouped
     statistics need ``stats.groups`` set to the group count here (``HistSpec(groups=S)`` for per-scenario ones);
-    period means need the run's ``out_every``."""
+    period means need the run's ``out_every``, float32 outputs its ``out_dtype``."""
     torch = _require_cuda()
     real = torch.float64 if precision == "f64" else torch.float32
     r = EnsembleResult(spec=stats, n_member=n_member, out_every=max(int(out_every), 1))
-    for name, _, shape, kind in _result_layout(n_gas, n_t, n_member, outputs, return_state, stats, out_every):
+    out_kind = _out_kind(precision, out_dtype, outputs)
+    for name, _, shape, kind in _result_layout(n_gas, n_t, n_member, outputs, return_state, stats, out_every, out_kind):
         dtype = real if kind == "real" else getattr(torch, kind)
         setattr(r, name, torch.empty(shape, dtype=dtype, pin_memory=True).numpy())
     return r

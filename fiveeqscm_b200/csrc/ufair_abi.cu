@@ -58,6 +58,18 @@ int check_out_every(const ufair_desc* d) {
   return UFAIR_OK;
 }
 
+// the outputs' element type (out_type, include/ufair.h), and what float32 outputs of an FP64 run do not support
+int check_out_type(const ufair_desc* d, size_t elem) {
+  if (d->out_type != UFAIR_OUTTYPE_RUN && d->out_type != UFAIR_OUTTYPE_F32)
+    return set_error(UFAIR_ERR_ARG, "out_type %d is not UFAIR_OUTTYPE_RUN (0) or UFAIR_OUTTYPE_F32 (1)", d->out_type);
+  if (out_elem(d, elem) == elem) return UFAIR_OK;
+  if (d->out_mask & (UFAIR_OUT_ALPHA | UFAIR_OUT_E))
+    return set_error(UFAIR_ERR_UNSUPPORTED, "float32 outputs: the alpha and emissions outputs are in the run's precision only");
+  if (d->conc_driven != 0)
+    return set_error(UFAIR_ERR_UNSUPPORTED, "float32 outputs: concentration-driven gases are not supported");
+  return UFAIR_OK;
+}
+
 int validate_desc(const ufair_desc* d, size_t elem) {
   if (!d) return set_error(UFAIR_ERR_ARG, "descriptor is NULL");
   if (d->struct_size != sizeof(ufair_desc))
@@ -84,6 +96,7 @@ int validate_desc(const ufair_desc* d, size_t elem) {
   int rc = check_stat_groups(d);
   if (rc != UFAIR_OK) return rc;
   if ((rc = check_out_every(d)) != UFAIR_OK) return rc;
+  if ((rc = check_out_type(d, elem)) != UFAIR_OK) return rc;
   if (d->n_member == 0 || d->n_t == 0) return UFAIR_OK;
   if (!d->emissions || !d->gas_params || !d->thermal_params)
     return set_error(UFAIR_ERR_ARG, "emissions / gas_params / thermal_params must not be NULL");
@@ -110,8 +123,8 @@ int validate_desc(const ufair_desc* d, size_t elem) {
   return UFAIR_OK;
 }
 
-template <typename Real> static KArgs<Real> make_args(const ufair_desc* d) {
-  KArgs<Real> a;
+template <typename Real, typename Out> static KArgs<Real, Out> make_args(const ufair_desc* d) {
+  KArgs<Real, Out> a;
   a.n_gas = d->n_gas;
   a.n_t = d->n_t;
   a.n_member = d->n_member;
@@ -145,9 +158,9 @@ template <typename Real> static KArgs<Real> make_args(const ufair_desc* d) {
   a.gp = (const Real*)d->gas_params;
   a.tp = (const Real*)d->thermal_params;
   a.state_in = (const Real*)d->state_in;
-  a.oC = (Real*)d->out_C;
-  a.oRF = (Real*)d->out_RF;
-  a.oT = (Real*)d->out_T;
+  a.oC = (Out*)d->out_C;
+  a.oRF = (Out*)d->out_RF;
+  a.oT = (Out*)d->out_T;
   a.oA = (Real*)d->out_alpha;
   a.oE = (Real*)d->out_E;
   a.conc_driven = d->conc_driven;
@@ -368,6 +381,7 @@ __global__ void __launch_bounds__(kStatsThreads)
   }
 }
 
+// Real here is the element type of the stored T rows (out_type), not necessarily the run's precision
 template <typename Real, int NGT, bool LABELS> static int launch_stats_pass(const ufair_desc* d, cudaStream_t stream) {
   const int G = LABELS ? stat_groups(d) : 1, n_tiles = (G + NGT - 1) / NGT;
   if (d->hist_copies > 65535) return set_error(UFAIR_ERR_ARG, "hist_copies %d > 65535", d->hist_copies);
@@ -390,13 +404,14 @@ template <typename Real, int NGT, bool LABELS> static int launch_stats_pass(cons
 }
 
 // the launcher of the descriptor's gas count and alpha mode (validate_desc bounds both); v picks the kernel
-template <typename Real> static int dispatch(const ufair_desc* d, const KArgs<Real>& a, Variant v, cudaStream_t s) {
+template <typename Real, typename Out>
+static int dispatch(const ufair_desc* d, const KArgs<Real, Out>& a, Variant v, cudaStream_t s) {
   switch (4 * d->n_gas + d->alpha_mode) {
-#define UFAIR_GAS(G)                                                                                 \
-  case 4 * G + UFAIR_ALPHA_EXP: return launch_integrate<Real, G, UFAIR_ALPHA_EXP>(d, a, v, s);       \
-  case 4 * G + UFAIR_ALPHA_SINH: return launch_integrate<Real, G, UFAIR_ALPHA_SINH>(d, a, v, s);     \
-  case 4 * G + UFAIR_ALPHA_NEWTON: return launch_integrate<Real, G, UFAIR_ALPHA_NEWTON>(d, a, v, s); \
-  case 4 * G + UFAIR_ALPHA_ONE: return launch_integrate<Real, G, UFAIR_ALPHA_ONE>(d, a, v, s);
+#define UFAIR_GAS(G)                                                                                      \
+  case 4 * G + UFAIR_ALPHA_EXP: return launch_integrate<Real, Out, G, UFAIR_ALPHA_EXP>(d, a, v, s);       \
+  case 4 * G + UFAIR_ALPHA_SINH: return launch_integrate<Real, Out, G, UFAIR_ALPHA_SINH>(d, a, v, s);     \
+  case 4 * G + UFAIR_ALPHA_NEWTON: return launch_integrate<Real, Out, G, UFAIR_ALPHA_NEWTON>(d, a, v, s); \
+  case 4 * G + UFAIR_ALPHA_ONE: return launch_integrate<Real, Out, G, UFAIR_ALPHA_ONE>(d, a, v, s);
     UFAIR_GAS(1) UFAIR_GAS(2) UFAIR_GAS(3) UFAIR_GAS(4)
 #undef UFAIR_GAS
   }
@@ -406,13 +421,14 @@ template <typename Real> static int dispatch(const ufair_desc* d, const KArgs<Re
 #ifdef UFAIR_DEBUG_BOUNDS
 // the negative control of the store check (a.dbg_cut > 0): run, then report every store the check found in the
 // rows it pretends are missing as an error of this call
-template <typename Real> static int run_cut_control(const ufair_desc* d, KArgs<Real> a, Variant v, cudaStream_t stream) {
+template <typename Real, typename Out>
+static int run_cut_control(const ufair_desc* d, KArgs<Real, Out> a, Variant v, cudaStream_t stream) {
   cudaError_t e = cudaMalloc(&a.dbg_cut_hits, sizeof(unsigned long long));
   if (e != cudaSuccess) return cuda_error(e, "cudaMalloc(dbg_cut_hits)");
   unsigned long long hits = 0;
   int rc = UFAIR_OK;
   if ((e = cudaMemsetAsync(a.dbg_cut_hits, 0, sizeof(hits), stream)) != cudaSuccess) rc = cuda_error(e, "cudaMemsetAsync(dbg_cut_hits)");
-  if (rc == UFAIR_OK) rc = dispatch<Real>(d, a, v, stream);
+  if (rc == UFAIR_OK) rc = dispatch<Real, Out>(d, a, v, stream);
   if (rc == UFAIR_OK && (e = cudaMemcpyAsync(&hits, a.dbg_cut_hits, sizeof(hits), cudaMemcpyDeviceToHost, stream)) != cudaSuccess)
     rc = cuda_error(e, "cudaMemcpyAsync(dbg_cut_hits)");
   if (rc == UFAIR_OK && (e = cudaStreamSynchronize(stream)) != cudaSuccess) rc = cuda_error(e, "cudaStreamSynchronize");
@@ -424,16 +440,23 @@ template <typename Real> static int run_cut_control(const ufair_desc* d, KArgs<R
 }
 #endif
 
+// the run with outputs of element type Out
+template <typename Real, typename Out> static int run_with(const ufair_desc* d, Variant v, cudaStream_t stream) {
+  const KArgs<Real, Out> a = make_args<Real, Out>(d);
+#ifdef UFAIR_DEBUG_BOUNDS
+  if (a.dbg_cut) return run_cut_control<Real, Out>(d, a, v, stream);
+#endif
+  return dispatch<Real, Out>(d, a, v, stream);
+}
+
 template <typename Real> int run_device(const ufair_desc* d, cudaStream_t stream) {
   int rc = validate_desc(d, sizeof(Real));
   if (rc != UFAIR_OK) return rc;
   if (d->n_member == 0 || d->n_t == 0) return UFAIR_OK;
-  const KArgs<Real> a = make_args<Real>(d);
   const Variant v = choose_variant(d, sizeof(Real));
-#ifdef UFAIR_DEBUG_BOUNDS
-  if (a.dbg_cut) return run_cut_control<Real>(d, a, v, stream);
-#endif
-  return dispatch<Real>(d, a, v, stream);
+  if constexpr (sizeof(Real) == 8)
+    if (v.out == UFAIR_OUTTYPE_F32) return run_with<Real, float>(d, v, stream);
+  return run_with<Real, Real>(d, v, stream);
 }
 
 // ---- gas_form detection: which pools carry mass, which forcing terms exist, over all members -------
@@ -482,14 +505,20 @@ template <typename Real> int detect_form(const ufair_desc* d, int32_t* scratch, 
   return UFAIR_OK;
 }
 
+// the pass over T rows of element type Rows
+template <typename Rows> static int stats_pass_rows(const ufair_desc* d, cudaStream_t stream) {
+  if (!d->stat_group) return launch_stats_pass<Rows, 1, false>(d, stream);
+  // up to four groups a tile of four: half the registers and predicated updates of a tile of eight
+  return stat_groups(d) <= 4 ? launch_stats_pass<Rows, 4, true>(d, stream) : launch_stats_pass<Rows, 8, true>(d, stream);
+}
+
 template <typename Real> int run_stats_pass(const ufair_desc* d, cudaStream_t stream) {
   int rc = validate_desc(d, sizeof(Real));
   if (rc != UFAIR_OK) return rc;
   if (!d->stats) return set_error(UFAIR_ERR_ARG, "ufair_stats_pass: descriptor has stats == 0");
   if (d->n_member == 0 || d->n_t == 0) return UFAIR_OK;
-  if (!d->stat_group) return launch_stats_pass<Real, 1, false>(d, stream);
-  // up to four groups a tile of four: half the registers and predicated updates of a tile of eight
-  return stat_groups(d) <= 4 ? launch_stats_pass<Real, 4, true>(d, stream) : launch_stats_pass<Real, 8, true>(d, stream);
+  // the T rows the integrator stored: float32 outputs of an FP64 run take the FP32 pass (include/ufair.h out_type)
+  return out_elem(d, sizeof(Real)) == sizeof(float) ? stats_pass_rows<float>(d, stream) : stats_pass_rows<Real>(d, stream);
 }
 template int run_stats_pass<double>(const ufair_desc*, cudaStream_t);
 template int run_stats_pass<float>(const ufair_desc*, cudaStream_t);

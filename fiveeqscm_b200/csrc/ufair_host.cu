@@ -118,7 +118,7 @@ static int copy_chunk(const Staged& t, const ufair_desc* h, void* dev, int64_t c
 
 template <typename Real>
 static int run_chunks(ufair_workspace* ws, const ufair_desc* h, const ufair_desc& d) {
-  const size_t es = sizeof(Real), i4 = sizeof(int32_t);
+  const size_t es = sizeof(Real), i4 = sizeof(int32_t), os = out_elem(h, es);  // os: C / RF / T (out_type)
   const int G = h->n_gas, n_t = h->n_t, out = h->out_mask;
   const int64_t M = h->n_member;
   const size_t gt = (size_t)G * n_t, srows = UFAIR_STATE_ROWS(G);
@@ -140,9 +140,9 @@ static int run_chunks(ufair_workspace* ws, const ufair_desc* h, const ufair_desc
       {F(scen_idx), 1, i4, true, h->scen_idx != nullptr, false, true},
       {F(stat_group), 1, i4, true, h->stat_group != nullptr && !labels_are_scen, false, true,
        labels_are_scen ? F(scen_idx) : 0},
-      {F(out_C), go, es, false, want(UFAIR_OUT_C), want(UFAIR_OUT_C), false},
-      {F(out_RF), go, es, false, want(UFAIR_OUT_RF), want(UFAIR_OUT_RF), false},
-      {F(out_T), n_out, es, false, want(UFAIR_OUT_T) || h->stats != 0, want(UFAIR_OUT_T), false},  // stats read T
+      {F(out_C), go, os, false, want(UFAIR_OUT_C), want(UFAIR_OUT_C), false},
+      {F(out_RF), go, os, false, want(UFAIR_OUT_RF), want(UFAIR_OUT_RF), false},
+      {F(out_T), n_out, os, false, want(UFAIR_OUT_T) || h->stats != 0, want(UFAIR_OUT_T), false},  // stats read T
       {F(out_alpha), gt, es, false, want(UFAIR_OUT_ALPHA), want(UFAIR_OUT_ALPHA), false},
       {F(out_E), gt, es, false, want(UFAIR_OUT_E), want(UFAIR_OUT_E), false},
       {F(state_out), srows, es, false, h->state_out != nullptr, h->state_out != nullptr, false},
@@ -236,6 +236,7 @@ template <typename Real> static int run_host(ufair_workspace* ws, const ufair_de
   if (h->stats && (!hist || !moments)) return set_error(UFAIR_ERR_ARG, "stats requested but hist/moments NULL");
   int rc0 = check_stat_groups(h);
   if (rc0 == UFAIR_OK) rc0 = check_out_every(h);
+  if (rc0 == UFAIR_OK) rc0 = check_out_type(h, sizeof(Real));
   if (rc0 != UFAIR_OK) return rc0;
   if (h->n_member == 0 || h->n_t == 0) return UFAIR_OK;
   if (!h->emissions || !h->gas_params || !h->thermal_params)

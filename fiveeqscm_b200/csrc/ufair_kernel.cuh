@@ -56,7 +56,8 @@
 //   * C / RF / T are written straight from registers with streaming 64-bit stores (STG.E.EF.64): with all
 //     gases of a member in one lane a warp writes one 256-byte run per row, with one gas per lane three
 //     80-byte runs; L2 merges them into full sectors (DRAM traffic 1.01x the algorithmic bytes, ncu) --
-//     nothing is re-read.
+//     nothing is re-read.  With float32 outputs of an FP64 run (UFAIR_OUTTYPE_F32, Out = float) each value is
+//     rounded once at its store (cvt.rn.f32.f64) and a warp writes one 128-byte run per row (32-bit stores).
 //   * optional statistics: the per-step histogram and the moments both come from a second,
 //     HBM-speed pass over the T rows this kernel writes (stats_pass_kernel, ufair_abi.cu; one kernel for
 //     pooled and per-label statistics, the pooled instantiation reading no labels): block-level
@@ -67,6 +68,7 @@
 #include <cuda.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <type_traits>
 #include <utility>
 
 #include "../../include/ufair.h"
@@ -136,9 +138,10 @@ constexpr int n_forms(int n_gas) {
 // the branch-free logarithm this wins in FP64 too, 31.3 -> 28.6 ms), and a specialised form must (its per-gas
 // code differs, so gases cannot share a warp's instruction stream).  The dense FP64 kernels of the default
 // alpha mode also exist with one gas per lane, for small ensembles (UFAIR_SMALL_ENSEMBLE).
-constexpr bool has_small_variant(int elem_size, int n_gas, int amode, int var) {
+// Float32 outputs (UFAIR_OUTTYPE_F32) have all gases per lane only: both mappings give the same bits.
+constexpr bool has_small_variant(int elem_size, int n_gas, int amode, int var, int out_type) {
   return elem_size == 8 && n_gas > 1 && amode == UFAIR_ALPHA_EXP && var != UFAIR_LOOP_CONC_DRIVEN &&
-         var != UFAIR_LOOP_PERIOD_MEAN;
+         var != UFAIR_LOOP_PERIOD_MEAN && out_type == UFAIR_OUTTYPE_RUN;
 }
 // members per warp: rows of MW elements must be a multiple of 16 bytes for the TMA box
 constexpr int members_per_warp(int elem_size, int n_gas, int gpl) {
@@ -147,7 +150,9 @@ constexpr int members_per_warp(int elem_size, int n_gas, int gpl) {
   return (32 / groups) / q * q;
 }
 
-template <typename Real> struct KArgs {
+// Out: the element type of the C / RF / T outputs (Real, or float for UFAIR_OUTTYPE_F32 outputs of an FP64 run);
+// every other array, the state included, is in the run's precision
+template <typename Real, typename Out = Real> struct KArgs {
   int n_gas, n_t;
   long long n_member, ld;
   int n_scen;
@@ -161,9 +166,9 @@ template <typename Real> struct KArgs {
   const Real* gp;
   const Real* tp;
   const Real* state_in;
-  Real* oC;
-  Real* oRF;
-  Real* oT;
+  Out* oC;
+  Out* oRF;
+  Out* oT;
   Real* oA;
   Real* oE;
   int conc_driven;  // bit g: gas g's input rows are target concentrations (INV kernels only)
@@ -229,7 +234,16 @@ __device__ __forceinline__ void sts(uint32_t a, float v) { asm volatile("st.shar
 // keep a loop-invariant value in a register (stops the compiler from re-deriving it every step)
 __device__ __forceinline__ void pin(uint32_t& x) { asm volatile("" : "+r"(x)); }
 
-template <typename Real> __device__ __forceinline__ void st_stream(Real* p, Real v) { __stcs(p, v); }
+// a streaming store of v as an Out: with Out = float and Real = double the one rounding, to nearest even
+template <typename Out, typename Real> __device__ __forceinline__ void st_stream(Out* p, Real v) { __stcs(p, (Out)v); }
+// p - q for the diagnostic outputs (alpha, E), which are addressed relative to out_C: they exist only when the
+// outputs have the run's element type (validate_desc rejects them otherwise)
+template <typename P, typename Q> __device__ __forceinline__ long long diag_offset(P* p, Q* q) {
+  if constexpr (std::is_same<P, Q>::value)
+    return p - q;
+  else
+    return 0;
+}
 
 // -DUFAIR_DEBUG_BOUNDS (libufair_dbg.so, `make debug`; tests/test_gpu_guard.py runs the ragged cases on it):
 // every output store must land inside its array, in a column below n_member, and every read of the
@@ -465,15 +479,17 @@ template <typename Real> __device__ __forceinline__ Real sum_pools(const Real (&
 }
 
 // GPL: gases per lane (1 or NGAS); FORM: per-gas specialisation (0 = dense; needs GPL == NGAS);
-// VAR: the loop (enum kVar* above the tuning table)
-template <typename Real, int NGAS, int AMODE, bool EMEM, int GPL, unsigned FORM, int VAR>
+// VAR: the loop (enum kVar* above the tuning table); Out: the element type of C / RF / T (KArgs)
+template <typename Real, int NGAS, int AMODE, bool EMEM, int GPL, unsigned FORM, int VAR, typename Out = Real>
 __global__ void __launch_bounds__(kWarps * 32, tuning(sizeof(Real), GPL, FORM, VAR).min_blocks())
-    ufair_integrate_kernel(const __grid_constant__ KArgs<Real> a, const __grid_constant__ CUtensorMap tmE,
+    ufair_integrate_kernel(const __grid_constant__ KArgs<Real, Out> a, const __grid_constant__ CUtensorMap tmE,
                            const __grid_constant__ CUtensorMap tmF) {
   static_assert(FORM == 0 || GPL == NGAS, "a per-gas form needs all gases of a member in one lane");
   constexpr bool INV = (VAR == kVarInverse), PLAIN = (VAR >= kVarPlain && VAR != kVarMean), NOFX = (VAR == kVarPlain),
                  ALLOUT = (VAR == kVarPlain || VAR == kVarPlainFx),  // C, RF and T all written: no output predicates
-                 MEAN = (VAR == kVarMean);  // period means: sums in registers, one store per period and output
+                 MEAN = (VAR == kVarMean),  // period means: sums in registers, one store per period and output
+                 DIAG = std::is_same<Out, Real>::value;  // the alpha / E outputs exist (outputs in the run's precision)
+  static_assert(DIAG || !INV, "the inverse loop has no float32-output instantiation");
   using M = Math<Real>;
   using WS = WarpSmem<Real, NGAS, AMODE, GPL, FORM, VAR>;
   constexpr int kTT = WS::TT;            // time steps per tile
@@ -652,11 +668,11 @@ __global__ void __launch_bounds__(kWarps * 32, tuning(sizeof(Real), GPL, FORM, V
   // running output pointers (gas g0; + gl * gstride); the mean loop's advance once per period
   const long long gstride = (long long)(MEAN ? a.n_out : n_t) * ld;
   const long long o_gas = (long long)g0 * gstride + m_raw;
-  Real* pC = a.oC + o_gas;
-  Real* pRF = a.oRF + o_gas;
-  const long long dA = a.oA - a.oC;  // the (diagnostic) alpha output is addressed relative to pC
-  const long long dE = INV ? (a.oE - a.oC) : 0;  // and so is the emissions output
-  Real* pT = a.oT + m_raw;
+  Out* pC = a.oC + o_gas;
+  Out* pRF = a.oRF + o_gas;
+  const long long dA = diag_offset(a.oA, a.oC);  // the (diagnostic) alpha output is addressed relative to pC
+  const long long dE = INV ? diag_offset(a.oE, a.oC) : 0;  // and so is the emissions output
+  Out* pT = a.oT + m_raw;
 
   // scenario-mode inputs: register prefetch one step ahead through the read-only path
   Real e_next[GPL], esc[GPL], fx_next = 0;
@@ -767,10 +783,11 @@ __global__ void __launch_bounds__(kWarps * 32, tuning(sizeof(Real), GPL, FORM, V
           }
         const Real e_inv = ((e[gl] - cst.get(gl, G_C0)) - keep) * M::rcp(gain * alpha[gl]);
         if ((a.conc_driven >> (g0 + gl)) & 1) e[gl] = e_inv;
-        if (wm & UFAIR_OUT_E) {
-          UFAIR_CHECK_ST(a.oE, (long long)NGAS * n_t, pC + dE + gl * gstride);
-          st_stream(pC + dE + gl * gstride, e[gl]);
-        }
+        if constexpr (DIAG)
+          if (wm & UFAIR_OUT_E) {
+            UFAIR_CHECK_ST(a.oE, (long long)NGAS * n_t, pC + dE + gl * gstride);
+            st_stream(pC + dE + gl * gstride, e[gl]);
+          }
       }
       const Real ea = e[gl] * alpha[gl];
 #pragma unroll
@@ -785,10 +802,11 @@ __global__ void __launch_bounds__(kWarps * 32, tuning(sizeof(Real), GPL, FORM, V
         UFAIR_CHECK_ST(a.oC, (long long)NGAS * n_t, pC + gl * gstride);
         st_stream(pC + gl * gstride, Cg[gl]);
       }
-      if (!PLAIN && !MEAN && (wm & UFAIR_OUT_ALPHA)) {
-        UFAIR_CHECK_ST(a.oA, (long long)NGAS * n_t, pC + dA + gl * gstride);
-        st_stream(pC + dA + gl * gstride, alpha[gl]);
-      }
+      if constexpr (DIAG && !PLAIN && !MEAN)
+        if (wm & UFAIR_OUT_ALPHA) {
+          UFAIR_CHECK_ST(a.oA, (long long)NGAS * n_t, pC + dA + gl * gstride);
+          st_stream(pC + dA + gl * gstride, alpha[gl]);
+        }
     }
     // ---- step_forc: F = f2 (C - C0) + f1 ln(C / C0) + f3 (sqrt C - sqrt C0), with C - C0 = sumR and
     // C / C0 = 1 + sumR / C0.  The logarithm runs its branch-free fast path for every gas (a special-case
@@ -936,15 +954,15 @@ __global__ void __launch_bounds__(kWarps * 32, tuning(sizeof(Real), GPL, FORM, V
 int make_tensor_maps(const ufair_desc* d, size_t elem, int mw_members, int tile_steps, CUtensorMap* tmE,
                      CUtensorMap* tmF);
 
-template <typename Real, int NGAS, int AMODE, int GPL, unsigned FORM, int VAR>
-int launch_variant(const ufair_desc* d, const KArgs<Real>& a, cudaStream_t stream) {
+template <typename Real, int NGAS, int AMODE, int GPL, unsigned FORM, int VAR, typename Out>
+int launch_variant(const ufair_desc* d, const KArgs<Real, Out>& a, cudaStream_t stream) {
   using WS = WarpSmem<Real, NGAS, AMODE, GPL, FORM, VAR>;
   CUtensorMap tmE, tmF;  // box = WS::MW members x WS::TT steps (x NGAS gases): depends on the variant
   const int rc = make_tensor_maps(d, sizeof(Real), WS::MW, WS::TT, &tmE, &tmF);
   if (rc != UFAIR_OK) return rc;
   const size_t smem = (size_t)WS::bytes(a.fext_mode == UFAIR_FEXT_MEMBER) * kWarps;
-  auto kern = (a.e_mode == UFAIR_E_MEMBER) ? ufair_integrate_kernel<Real, NGAS, AMODE, true, GPL, FORM, VAR>
-                                            : ufair_integrate_kernel<Real, NGAS, AMODE, false, GPL, FORM, VAR>;
+  auto kern = (a.e_mode == UFAIR_E_MEMBER) ? ufair_integrate_kernel<Real, NGAS, AMODE, true, GPL, FORM, VAR, Out>
+                                            : ufair_integrate_kernel<Real, NGAS, AMODE, false, GPL, FORM, VAR, Out>;
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return cuda_error(e, "cudaFuncSetAttribute(ufair_integrate_kernel)");
   const long long n_warp = (a.n_member + WS::MW - 1) / WS::MW;
@@ -964,10 +982,16 @@ inline unsigned requested_form(const ufair_desc* d) {
 // concentration-driven gases / the emissions output run on the INV instantiation of the general kernel
 inline bool wants_inverse(const ufair_desc* d) { return d->conc_driven != 0 || (d->out_mask & UFAIR_OUT_E) != 0; }
 
+// the element type of the C / RF / T outputs an instantiation stores
+template <typename Real, typename Out>
+constexpr int kOutType = std::is_same<Out, Real>::value ? UFAIR_OUTTYPE_RUN : UFAIR_OUTTYPE_F32;
+
 // the loops each alpha mode has: the plain loops with external forcing (kVarPlainFx) or with a subset of
-// the outputs (kVarPlainSub) exist in the default alpha mode only ...
-constexpr bool loop_instantiated(int amode, int loop) {
-  return amode == UFAIR_ALPHA_EXP || (loop != kVarPlainFx && loop != kVarPlainSub);
+// the outputs (kVarPlainSub) exist in the default alpha mode only, and float32 outputs have every loop but
+// the inverse one (validate_desc rejects what needs it) ...
+constexpr bool loop_instantiated(int amode, int loop, int out_type) {
+  return (amode == UFAIR_ALPHA_EXP || (loop != kVarPlainFx && loop != kVarPlainSub)) &&
+         (out_type == UFAIR_OUTTYPE_RUN || loop != kVarInverse);
 }
 // ... and so do the specialised forms, for every loop but the inverse one
 constexpr bool forms_instantiated(int amode, int loop) { return amode == UFAIR_ALPHA_EXP && loop != kVarInverse; }
@@ -977,10 +1001,13 @@ struct Variant {
   unsigned form;  // FORM: an entry of kForms[n_gas], 0 = the dense kernel
   int loop;       // VAR: kVar* = UFAIR_LOOP_*
   int gpl;        // GPL: gases per lane, 1 or n_gas
+  int out;        // Out: UFAIR_OUTTYPE_RUN (Out = Real) or UFAIR_OUTTYPE_F32 (Out = float, FP64 runs only)
 };
 
 // The only statement of the choice: run_device launches it and ufair_kernel_variant reports it.
 inline Variant choose_variant(const ufair_desc* d, int elem_size) {
+  // float32 outputs of an FP32 run are its own outputs
+  const int out = (elem_size == 8 && d->out_type == UFAIR_OUTTYPE_F32) ? UFAIR_OUTTYPE_F32 : UFAIR_OUTTYPE_RUN;
   // the plain loops: no iIRF ceiling, outputs among C, RF, T only, emission-driven
   const int crt = UFAIR_OUT_C | UFAIR_OUT_RF | UFAIR_OUT_T;
   int loop = d->out_every >= 2 ? kVarMean
@@ -989,66 +1016,72 @@ inline Variant choose_variant(const ufair_desc* d, int elem_size) {
              : (d->out_mask & crt) != crt ? kVarPlainSub
              : d->fext_mode == UFAIR_FEXT_NONE ? kVarPlain
                                               : kVarPlainFx;
-  if (!loop_instantiated(d->alpha_mode, loop)) loop = kVarGeneral;
+  if (!loop_instantiated(d->alpha_mode, loop, out)) loop = kVarGeneral;
   unsigned form = 0;  // the first instantiated form that covers the requested one
   const unsigned want = requested_form(d);
   if (want != 0 && forms_instantiated(d->alpha_mode, loop))
     for (int k = 0; k < n_forms(d->n_gas) && form == 0; ++k)
       if (form_covers(kForms[d->n_gas][k], want, d->n_gas)) form = kForms[d->n_gas][k];
-  const bool small = form == 0 && has_small_variant(elem_size, d->n_gas, d->alpha_mode, loop) &&
+  const bool small = form == 0 && has_small_variant(elem_size, d->n_gas, d->alpha_mode, loop, out) &&
                      d->n_member <= UFAIR_SMALL_ENSEMBLE;
-  return {form, loop, small ? 1 : d->n_gas};
+  return {form, loop, small ? 1 : d->n_gas, out};
 }
 
-// launches <GPL, FORM, LOOP> if that is v
-template <typename Real, int NGAS, int AMODE, int LOOP, int GPL, unsigned FORM>
-bool launch_if(const ufair_desc* d, const KArgs<Real>& a, Variant v, cudaStream_t stream, int& rc) {
-  if (v.loop != LOOP || v.gpl != GPL || v.form != FORM) return false;
-  rc = launch_variant<Real, NGAS, AMODE, GPL, FORM, LOOP>(d, a, stream);
+// launches <GPL, FORM, LOOP, Out> if that is v
+template <typename Real, typename Out, int NGAS, int AMODE, int LOOP, int GPL, unsigned FORM>
+bool launch_if(const ufair_desc* d, const KArgs<Real, Out>& a, Variant v, cudaStream_t stream, int& rc) {
+  if (v.loop != LOOP || v.gpl != GPL || v.form != FORM || v.out != kOutType<Real, Out>) return false;
+  rc = launch_variant<Real, NGAS, AMODE, GPL, FORM, LOOP, Out>(d, a, stream);
   return true;
 }
 // the instantiations of one loop: dense with one gas per lane, dense with all of them, and the forms kForms[NGAS][K]
-template <typename Real, int NGAS, int AMODE, int LOOP, size_t... K>
-bool launch_loop(const ufair_desc* d, const KArgs<Real>& a, Variant v, cudaStream_t stream, int& rc,
+template <typename Real, typename Out, int NGAS, int AMODE, int LOOP, size_t... K>
+bool launch_loop(const ufair_desc* d, const KArgs<Real, Out>& a, Variant v, cudaStream_t stream, int& rc,
                  std::index_sequence<K...>) {
-  if constexpr (loop_instantiated(AMODE, LOOP)) {
-    if constexpr (has_small_variant(sizeof(Real), NGAS, AMODE, LOOP))
-      if (launch_if<Real, NGAS, AMODE, LOOP, 1, 0u>(d, a, v, stream, rc)) return true;
-    return launch_if<Real, NGAS, AMODE, LOOP, NGAS, 0u>(d, a, v, stream, rc) ||
-           (launch_if<Real, NGAS, AMODE, LOOP, NGAS, kForms[NGAS][K]>(d, a, v, stream, rc) || ...);
+  constexpr int OUT = kOutType<Real, Out>;
+  if constexpr (loop_instantiated(AMODE, LOOP, OUT)) {
+    if constexpr (has_small_variant(sizeof(Real), NGAS, AMODE, LOOP, OUT))
+      if (launch_if<Real, Out, NGAS, AMODE, LOOP, 1, 0u>(d, a, v, stream, rc)) return true;
+    return launch_if<Real, Out, NGAS, AMODE, LOOP, NGAS, 0u>(d, a, v, stream, rc) ||
+           (launch_if<Real, Out, NGAS, AMODE, LOOP, NGAS, kForms[NGAS][K]>(d, a, v, stream, rc) || ...);
   }
   return false;
 }
-// every instantiation of one (Real, NGAS, AMODE) in turn: exactly those choose_variant can return; one that is
+// every instantiation of one (Real, Out, NGAS, AMODE) in turn: exactly those choose_variant can return; one that is
 // not there is an error, never another kernel
-template <typename Real, int NGAS, int AMODE, int... LOOP>
-int launch_chosen(const ufair_desc* d, const KArgs<Real>& a, Variant v, cudaStream_t stream,
+template <typename Real, typename Out, int NGAS, int AMODE, int... LOOP>
+int launch_chosen(const ufair_desc* d, const KArgs<Real, Out>& a, Variant v, cudaStream_t stream,
                   std::integer_sequence<int, LOOP...>) {
   int rc = UFAIR_OK;
-  if ((launch_loop<Real, NGAS, AMODE, LOOP>(
+  if ((launch_loop<Real, Out, NGAS, AMODE, LOOP>(
            d, a, v, stream, rc, std::make_index_sequence<forms_instantiated(AMODE, LOOP) ? n_forms(NGAS) : 0>()) ||
        ...))
     return rc;
-  return set_error(UFAIR_ERR_UNSUPPORTED, "no integrator for %d gases, alpha mode %d, form 0x%x, %d gases per lane, loop %d",
-                   NGAS, AMODE, v.form, v.gpl, v.loop);
+  return set_error(UFAIR_ERR_UNSUPPORTED,
+                   "no integrator for %d gases, alpha mode %d, form 0x%x, %d gases per lane, loop %d, output type %d", NGAS,
+                   AMODE, v.form, v.gpl, v.loop, v.out);
 }
 
-// The launcher of one (precision, gas count, alpha mode): runs the instantiation v names.  UFAIR_INSTANTIATE
-// defines the four of a (precision, gas count), one ufair_inst_*.cu each, so the kernels compile in parallel.
-template <typename Real, int NGAS, int AMODE>
-int launch_integrate(const ufair_desc* d, const KArgs<Real>& a, Variant v, cudaStream_t stream);
+// The launcher of one (precision, output type, gas count, alpha mode): runs the instantiation v names.
+// UFAIR_INSTANTIATE defines the four of a (precision, gas count) with outputs in the run's precision, and
+// UFAIR_INSTANTIATE_OUT those of another output type (float32 outputs of FP64 runs), one ufair_inst_*.cu per
+// (precision, gas count), so the kernels compile in parallel.
+template <typename Real, typename Out, int NGAS, int AMODE>
+int launch_integrate(const ufair_desc* d, const KArgs<Real, Out>& a, Variant v, cudaStream_t stream);
 
-#define UFAIR_LAUNCHER(Real, NGAS, AMODE)                                                                   \
-  template <>                                                                                               \
-  int launch_integrate<Real, NGAS, AMODE>(const ufair_desc* d, const KArgs<Real>& a, Variant v, cudaStream_t s) { \
-    return launch_chosen<Real, NGAS, AMODE>(                                                                \
-        d, a, v, s,                                                                                         \
+#define UFAIR_LAUNCHER(Real, Out, NGAS, AMODE)                                                                  \
+  template <>                                                                                                   \
+  int launch_integrate<Real, Out, NGAS, AMODE>(const ufair_desc* d, const KArgs<Real, Out>& a, Variant v,      \
+                                               cudaStream_t s) {                                                \
+    return launch_chosen<Real, Out, NGAS, AMODE>(                                                               \
+        d, a, v, s,                                                                                             \
         std::integer_sequence<int, kVarGeneral, kVarInverse, kVarPlain, kVarPlainFx, kVarPlainSub, kVarMean>()); \
   }
-#define UFAIR_INSTANTIATE(Real, NGAS)                                                                       \
-  UFAIR_LAUNCHER(Real, NGAS, UFAIR_ALPHA_EXP)                                                               \
-  UFAIR_LAUNCHER(Real, NGAS, UFAIR_ALPHA_SINH)                                                              \
-  UFAIR_LAUNCHER(Real, NGAS, UFAIR_ALPHA_NEWTON)                                                            \
-  UFAIR_LAUNCHER(Real, NGAS, UFAIR_ALPHA_ONE)
+#define UFAIR_INSTANTIATE_OUT(Real, Out, NGAS)                                                                  \
+  UFAIR_LAUNCHER(Real, Out, NGAS, UFAIR_ALPHA_EXP)                                                              \
+  UFAIR_LAUNCHER(Real, Out, NGAS, UFAIR_ALPHA_SINH)                                                             \
+  UFAIR_LAUNCHER(Real, Out, NGAS, UFAIR_ALPHA_NEWTON)                                                           \
+  UFAIR_LAUNCHER(Real, Out, NGAS, UFAIR_ALPHA_ONE)
+#define UFAIR_INSTANTIATE(Real, NGAS) UFAIR_INSTANTIATE_OUT(Real, Real, NGAS)
 
 }  // namespace ufair

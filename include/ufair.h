@@ -23,7 +23,9 @@
  *     (reference: time is axis 0 of `emissions`, U_FaIR/concentrations.py:5).
  *   - rows must be 16-byte aligned: base pointers 16-B aligned and ld_member a
  *     multiple of 2 (f64) / 4 (f32). Violations return UFAIR_ERR_ALIGN -- the
- *     kernel streams emission rows with TMA bulk copies.
+ *     kernel streams emission rows with TMA bulk copies.  The rule is on the
+ *     run's element size also with float32 outputs (out_type below), whose rows
+ *     are then only 8-byte aligned; nothing that reads or writes them needs more.
  *   - every entry point returns 0 on success or a negative UFAIR_ERR_*;
  *     ufair_last_error() gives the message (thread-local). Nothing aborts.
  *   - `stream` is a cudaStream_t passed as void*. Calls are asynchronous on it.
@@ -40,7 +42,7 @@
 extern "C" {
 #endif
 
-#define UFAIR_ABI_VERSION 4
+#define UFAIR_ABI_VERSION 5
 
 #define UFAIR_MAX_GAS 4
 #define UFAIR_N_POOL 4
@@ -84,6 +86,24 @@ enum { UFAIR_T_MID = 0,  /* T = sum_j (S_j + S_j')/2 */
        UFAIR_T_END = 1   /* T = sum_j S_j'           */ };
 enum { UFAIR_OUT_C = 1, UFAIR_OUT_RF = 2, UFAIR_OUT_T = 4, UFAIR_OUT_ALPHA = 8, UFAIR_OUT_E = 16 };
 
+/* out_type: the element type of out_C, out_RF and out_T.
+ *   UFAIR_OUTTYPE_RUN (0, the default): the run's precision, as ufair_run_f64 / ufair_run_f32 say.
+ *   UFAIR_OUTTYPE_F32 (1): float32.  The integration stays in the run's precision; with ufair_run_f64 every
+ *     element of out_C, out_RF and out_T is the round-to-nearest-even float32 (cvt.rn.f32.f64) of the double
+ *     the same descriptor stores with UFAIR_OUTTYPE_RUN -- bit for bit, period means (out_every >= 2) included:
+ *     their sum and their product with (Real)(1.0 / k) stay in FP64, and the mean is rounded once, at the store.
+ *     Half the bytes cross HBM and the host link, and the outputs take half the device memory.
+ *     state_out stays in the run's precision, so a run split into time chunks gives the float32 rows of one call.
+ *     The statistics (stats == 1) bin the T rows the integrator stored: here float32 T, with ufair_stats_pass_f64
+ *     running the FP32 pass -- FP32 binning rule, FP64 moments of the float32 values.  The histogram is thus a
+ *     recount of the stored float32 T, not of the FP64 T: a member within about 1e-7 relative of a bin edge can
+ *     land in the neighbouring bin.  A statistics-only call (stats == 1 without UFAIR_OUT_T) needs a float32
+ *     out_T scratch of n_out rows.
+ *     Not supported (UFAIR_ERR_UNSUPPORTED) with ufair_run_f64: the UFAIR_OUT_ALPHA and UFAIR_OUT_E diagnostics
+ *     and concentration-driven gases (conc_driven != 0).  With ufair_run_f32 it is accepted and changes nothing.
+ *   Any other value: UFAIR_ERR_ARG.  No combination widens the outputs. */
+enum { UFAIR_OUTTYPE_RUN = 0, UFAIR_OUTTYPE_F32 = 1 };
+
 /* gas_form[g]: what gas g actually uses, so that the library may pick a kernel that skips the rest.
  * 0 = unspecified (four pools, all three forcing terms).  Otherwise UFAIR_FORM(n_pool, terms):
  * only pools 1..n_pool carry mass (a_i == 0 and zero initial state for the others) and only the
@@ -108,7 +128,7 @@ enum {
 
 typedef struct ufair_desc {
   uint32_t struct_size; /* = sizeof(ufair_desc); checked */
-  uint32_t reserved0;
+  int32_t out_type;     /* UFAIR_OUTTYPE_*: element type of out_C / out_RF / out_T (see above) */
 
   /* ---- dimensions ---- */
   int32_t n_gas;     /* 1..UFAIR_MAX_GAS */
@@ -140,15 +160,15 @@ typedef struct ufair_desc {
   const void* state_in;       /* [UFAIR_STATE_ROWS][ld_member] or NULL (= all zero) */
 
   /* ---- outputs ---- */
-  void* out_C;     /* [n_gas][n_out][ld_member]; n_out = n_t, or n_t / out_every (period means below) */
-  void* out_RF;    /* [n_gas][n_out][ld_member] */
-  void* out_T;     /* [n_out][ld_member]        */
+  void* out_C;     /* [n_gas][n_out][ld_member]; n_out = n_t, or n_t / out_every (period means below); out_type */
+  void* out_RF;    /* [n_gas][n_out][ld_member]; out_type */
+  void* out_T;     /* [n_out][ld_member]; out_type */
   void* out_alpha; /* [n_gas][n_t][ld_member] (diagnostic) */
-  void* state_out; /* [UFAIR_STATE_ROWS][ld_member] or NULL */
+  void* state_out; /* [UFAIR_STATE_ROWS][ld_member] or NULL; always the run's precision */
 
   /* ---- ensemble statistics (stats == 1) ----
    * bin(T) = clamp(floor((T - hist_lo) * (hist_bins / (hist_hi - hist_lo))), 0, hist_bins-1),
-   * evaluated in the run's precision.  Non-finite T: NaN is neither counted in the histogram nor
+   * evaluated in the precision of the stored T rows: the run's, or float32 with UFAIR_OUTTYPE_F32.  Non-finite T: NaN is neither counted in the histogram nor
    * taken into min / max, but it makes its row's sum and sum of squares NaN (a mean / std computed
    * from them flags the step); +inf and -inf are counted in the last and first bin and enter every
    * moment.  A row with no value other than NaN keeps the min / max sentinels +inf / -inf.
@@ -238,7 +258,8 @@ int ufair_detect_form_f32(const ufair_desc* d, int32_t* scratch, uint8_t* form, 
  * *form = the specialised per-gas form in use, packed one UFAIR_FORM byte per gas (0 = the general
  * kernel), *gases_per_lane and *members_per_warp = the lane mapping, *loop = UFAIR_LOOP_*: which
  * instantiation of the time loop (all of them give bit-identical results; the plain ones carry no
- * run-time switches for features that are off).  elem_size: 8 (f64) or 4 (f32).  Out-pointers may be NULL. */
+ * run-time switches for features that are off).  elem_size: 8 (f64) or 4 (f32).  Out-pointers may be NULL.
+ * Float32 outputs of an FP64 run (UFAIR_OUTTYPE_F32) always run all gases per lane. */
 enum { UFAIR_LOOP_GENERAL = 0,      /* every run-time option                                         */
        UFAIR_LOOP_CONC_DRIVEN = 1,  /* concentration-driven gases / emissions output                 */
        UFAIR_LOOP_PLAIN = 2,        /* no f_ext, no iIRF ceiling, outputs exactly C + RF + T         */
@@ -253,7 +274,8 @@ int ufair_kernel_variant(const ufair_desc* d, int32_t elem_size, uint32_t* form,
 int ufair_stats_reset(const ufair_desc* d, void* stream);
 /* The statistics pass: per-row histogram and moments of the T rows ufair_run_* just wrote
  * (d->out_T, n_out rows: per step, or per period with out_every >= 2; same descriptor, same stream).
- * One call per ufair_run_* call when stats == 1. */
+ * One call per ufair_run_* call when stats == 1.  The _f64 / _f32 suffix names the run's precision; the
+ * rows are read in the descriptor's out_type (float32 rows of an FP64 run take the FP32 pass). */
 int ufair_stats_pass_f64(const ufair_desc* d, void* stream);
 int ufair_stats_pass_f32(const ufair_desc* d, void* stream);
 /* Fold the private copies: hist[G][hist_rows][hist_bins] (uint64 counts) and
