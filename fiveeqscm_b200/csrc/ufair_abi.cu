@@ -33,7 +33,7 @@ int cuda_error(cudaError_t e, const char* what) {
 static bool misaligned(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) != 0; }
 
 // the grouped-statistics fields (shared by the run / pass validation and the statistics-buffer entry points)
-int check_stat_groups(const ufair_desc* d) {
+static int check_stat_groups(const ufair_desc* d) {
   if (d->n_stat_groups < 0 || d->n_stat_groups > UFAIR_MAX_STAT_GROUPS)
     return set_error(UFAIR_ERR_ARG, "n_stat_groups %d outside 0..%d", d->n_stat_groups, UFAIR_MAX_STAT_GROUPS);
   if (d->n_stat_groups > 1 && !d->stat_group)
@@ -46,7 +46,7 @@ int check_stat_groups(const ufair_desc* d) {
 }
 
 // period means (out_every, include/ufair.h): the step count, and what the mean loop does not support
-int check_out_every(const ufair_desc* d) {
+static int check_out_every(const ufair_desc* d) {
   if (d->out_every < 0) return set_error(UFAIR_ERR_ARG, "out_every %d < 0", d->out_every);
   if (d->out_every < 2) return UFAIR_OK;
   if (d->n_t % d->out_every != 0)
@@ -59,7 +59,7 @@ int check_out_every(const ufair_desc* d) {
 }
 
 // the outputs' element type (out_type, include/ufair.h), and what float32 outputs of an FP64 run do not support
-int check_out_type(const ufair_desc* d, size_t elem) {
+static int check_out_type(const ufair_desc* d, size_t elem) {
   if (d->out_type != UFAIR_OUTTYPE_RUN && d->out_type != UFAIR_OUTTYPE_F32)
     return set_error(UFAIR_ERR_ARG, "out_type %d is not UFAIR_OUTTYPE_RUN (0) or UFAIR_OUTTYPE_F32 (1)", d->out_type);
   if (out_elem(d, elem) == elem) return UFAIR_OK;
@@ -70,7 +70,19 @@ int check_out_type(const ufair_desc* d, size_t elem) {
   return UFAIR_OK;
 }
 
-int validate_desc(const ufair_desc* d, size_t elem) {
+// the private statistics buffers: what the statistics pass adds into, and what ufair_stats_reset / _finalize /
+// _finalize_packed work on
+static int check_stat_buffers(const ufair_desc* d) {
+  if (d->hist_copies < 1 || !d->hist_private || !d->moments_private)
+    return set_error(UFAIR_ERR_ARG, "stats requested but histogram spec/buffers incomplete");
+  return UFAIR_OK;
+}
+
+// The run rules say what the caller asked for; they hold for host and device arrays alike.  The placement rules
+// (placement == true) say how device arrays must be laid out for this library's kernels: the 16-byte rows of the TMA
+// bulk copies, and the statistics buffers, row offset and T rows of the statistics pass.  The pitch rule comes before
+// the other run rules, so that misaligned rows are reported before missing arrays.
+static int check_desc(const ufair_desc* d, size_t elem, bool placement) {
   if (!d) return set_error(UFAIR_ERR_ARG, "descriptor is NULL");
   if (d->struct_size != sizeof(ufair_desc))
     return set_error(UFAIR_ERR_ARG, "struct_size %u != sizeof(ufair_desc) %zu (header/binding mismatch)",
@@ -83,7 +95,7 @@ int validate_desc(const ufair_desc* d, size_t elem) {
   if (d->ld_member > (int64_t)INT32_MAX)
     return set_error(UFAIR_ERR_ARG, "ld_member %lld > %d: split the member axis over several calls", (long long)d->ld_member,
                      INT32_MAX);
-  if (d->n_member > 0 && (d->ld_member * (int64_t)elem) % 16 != 0)
+  if (placement && d->n_member > 0 && (d->ld_member * (int64_t)elem) % 16 != 0)
     return set_error(UFAIR_ERR_ALIGN, "ld_member %lld: rows must be a multiple of 16 bytes", (long long)d->ld_member);
   if (d->e_mode != UFAIR_E_MEMBER && d->e_mode != UFAIR_E_SCENARIO) return set_error(UFAIR_ERR_ARG, "bad e_mode");
   if (d->fext_mode < UFAIR_FEXT_NONE || d->fext_mode > UFAIR_FEXT_MEMBER) return set_error(UFAIR_ERR_ARG, "bad fext_mode");
@@ -108,20 +120,24 @@ int validate_desc(const ufair_desc* d, size_t elem) {
   if ((d->out_mask & UFAIR_OUT_E) && !d->out_E) return set_error(UFAIR_ERR_ARG, "out_E requested but NULL");
   if (d->conc_driven < 0 || d->conc_driven >= (1 << d->n_gas))
     return set_error(UFAIR_ERR_ARG, "conc_driven 0x%x names a gas >= n_gas %d", d->conc_driven, d->n_gas);
+  if (d->stats && (d->hist_bins < 1 || !(d->hist_hi > d->hist_lo)))
+    return set_error(UFAIR_ERR_ARG, "stats requested but histogram spec/buffers incomplete");
+  if (!placement) return UFAIR_OK;
   // TMA bulk-copy sources
   if (d->e_mode == UFAIR_E_MEMBER && misaligned(d->emissions))
     return set_error(UFAIR_ERR_ALIGN, "emissions must be 16-byte aligned");
   if (d->fext_mode == UFAIR_FEXT_MEMBER && misaligned(d->f_ext))
     return set_error(UFAIR_ERR_ALIGN, "f_ext must be 16-byte aligned");
   if (d->stats) {
-    if (d->hist_bins < 1 || d->hist_copies < 1 || !(d->hist_hi > d->hist_lo) || !d->hist_private || !d->moments_private)
-      return set_error(UFAIR_ERR_ARG, "stats requested but histogram spec/buffers incomplete");
+    if ((rc = check_stat_buffers(d)) != UFAIR_OK) return rc;
     if (!d->out_T) return set_error(UFAIR_ERR_ARG, "stats need out_T (the moments pass reads the T rows)");
     if (d->hist_t0 < 0 || d->hist_rows < d->hist_t0 + out_rows(d))
       return set_error(UFAIR_ERR_ARG, "hist_rows %d < hist_t0 %d + output rows %d", d->hist_rows, d->hist_t0, out_rows(d));
   }
   return UFAIR_OK;
 }
+int validate_desc(const ufair_desc* d, size_t elem) { return check_desc(d, elem, true); }
+int check_run(const ufair_desc* d, size_t elem) { return check_desc(d, elem, false); }
 
 template <typename Real, typename Out> static KArgs<Real, Out> make_args(const ufair_desc* d) {
   KArgs<Real, Out> a;
@@ -624,9 +640,9 @@ __global__ void percentiles_kernel(const unsigned long long* __restrict__ hist, 
 
 static int check_stats_desc(const ufair_desc* d) {
   if (!d || d->struct_size != sizeof(ufair_desc)) return set_error(UFAIR_ERR_ARG, "bad descriptor");
-  if (d->hist_bins < 1 || d->hist_copies < 1 || d->hist_rows < 1 || !d->hist_private || !d->moments_private)
-    return set_error(UFAIR_ERR_ARG, "histogram spec/buffers incomplete");
-  return check_stat_groups(d);
+  if (d->hist_bins < 1 || d->hist_rows < 1) return set_error(UFAIR_ERR_ARG, "histogram spec/buffers incomplete");
+  const int rc = check_stat_buffers(d);
+  return rc != UFAIR_OK ? rc : check_stat_groups(d);
 }
 
 // ---- parameter preparation ------------------------------------------------------------------------

@@ -230,19 +230,11 @@ static int run_chunks(ufair_workspace* ws, const ufair_desc* h, const ufair_desc
 
 template <typename Real> static int run_host(ufair_workspace* ws, const ufair_desc* h, uint64_t* hist, double* moments) {
   if (!ws) return set_error(UFAIR_ERR_ARG, "workspace is NULL");
-  if (!h || h->struct_size != sizeof(ufair_desc)) return set_error(UFAIR_ERR_ARG, "bad descriptor");
-  if (h->n_gas < 1 || h->n_gas > UFAIR_MAX_GAS || h->n_t < 0 || h->n_member < 0 || h->ld_member < h->n_member)
-    return set_error(UFAIR_ERR_ARG, "bad dimensions");
-  if (h->stats && (!hist || !moments)) return set_error(UFAIR_ERR_ARG, "stats requested but hist/moments NULL");
-  int rc0 = check_stat_groups(h);
-  if (rc0 == UFAIR_OK) rc0 = check_out_every(h);
-  if (rc0 == UFAIR_OK) rc0 = check_out_type(h, sizeof(Real));
+  // the device path's run rules; its placement rules apply to the staged chunks (run_device, run_stats_pass)
+  const int rc0 = check_run(h, sizeof(Real));
   if (rc0 != UFAIR_OK) return rc0;
+  if (h->stats && (!hist || !moments)) return set_error(UFAIR_ERR_ARG, "stats requested but hist/moments NULL");
   if (h->n_member == 0 || h->n_t == 0) return UFAIR_OK;
-  if (!h->emissions || !h->gas_params || !h->thermal_params)
-    return set_error(UFAIR_ERR_ARG, "emissions / gas_params / thermal_params must not be NULL");
-  if (h->ld_member > (int64_t)INT32_MAX || (uint64_t)h->ld_member * sizeof(Real) > (uint64_t)INT32_MAX * 8u)
-    return set_error(UFAIR_ERR_ARG, "ld_member %lld is too large for one call: split the member axis", (long long)h->ld_member);
   DeviceGuard guard(ws->device);  // the caller's current device is restored on every return path
   if (guard.err != cudaSuccess) return cuda_error(guard.err, "cudaSetDevice");
 
@@ -257,20 +249,12 @@ template <typename Real> static int run_host(ufair_workspace* ws, const ufair_de
     d.emissions = ws->e_scen.p;
   }
   if (h->fext_mode == UFAIR_FEXT_SCENARIO) {
-    if (!h->f_ext) {
-      cudaStreamSynchronize(ws->s_in);
-      return set_error(UFAIR_ERR_ARG, "fext_mode set but f_ext is NULL");
-    }
     const size_t nb = (size_t)n_t * h->n_scen * es;
     CKS(ws->fext_scen.reserve(nb), "cudaMalloc(fext_scen)");
     CKS(cudaMemcpyAsync(ws->fext_scen.p, h->f_ext, nb, cudaMemcpyHostToDevice, ws->s_in), "H2D scenario forcing");
     d.f_ext = ws->fext_scen.p;
   }
   if (h->stats) {
-    if (h->hist_bins < 1 || !(h->hist_hi > h->hist_lo)) {
-      cudaStreamSynchronize(ws->s_in);
-      return set_error(UFAIR_ERR_ARG, "bad histogram spec");
-    }
     d.hist_copies = h->hist_copies > 0 ? h->hist_copies : 16;
     d.hist_t0 = 0;
     d.hist_rows = out_rows(h);

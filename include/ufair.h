@@ -21,9 +21,10 @@
  *   - every [..][member] array has the member axis fastest, with one common row
  *     pitch `ld_member` (elements). Time is the axis above it
  *     (reference: time is axis 0 of `emissions`, U_FaIR/concentrations.py:5).
- *   - rows must be 16-byte aligned: base pointers 16-B aligned and ld_member a
- *     multiple of 2 (f64) / 4 (f32). Violations return UFAIR_ERR_ALIGN -- the
- *     kernel streams emission rows with TMA bulk copies.  The rule is on the
+ *   - device rows must be 16-byte aligned: base pointers 16-B aligned and
+ *     ld_member a multiple of 2 (f64) / 4 (f32). Violations return
+ *     UFAIR_ERR_ALIGN -- the kernel streams emission rows with TMA bulk copies.
+ *     The host pipeline's arrays have no such rule (see there).  The rule is on the
  *     run's element size also with float32 outputs (out_type below), whose rows
  *     are then only 8-byte aligned; nothing that reads or writes them needs more.
  *   - every entry point returns 0 on success or a negative UFAIR_ERR_*;
@@ -353,7 +354,13 @@ int ufair_hfc_pulse_f64(const double* e0, const double* time, double* out, int64
 /* ---- host-buffer pipeline (HOST pointers inside `d`, same meaning otherwise) ----
  * Splits the member axis into chunks, and overlaps H2D copies, the kernel and
  * D2H copies on three streams with double-buffered device staging.
- * Statistics, when requested, are finalised into host `hist`/`moments`. */
+ * Statistics, when requested, are finalised into host `hist`/`moments`.
+ * Host arrays may have any row pitch and any alignment: the 16-byte rule above
+ * is for device arrays, and the pipeline stages each chunk into aligned ones.
+ * The pipeline owns hist_copies (0 means 16), hist_t0, hist_rows, hist_private
+ * and moments_private, and stages T itself when stats == 1 without
+ * UFAIR_OUT_T, so out_T may then be NULL.  Every other rule of ufair_run_* is
+ * checked on `d`, with the same code and message, before anything is copied. */
 typedef struct ufair_workspace ufair_workspace;
 int ufair_workspace_create(int device, int64_t chunk_members, ufair_workspace** ws);
 int ufair_workspace_destroy(ufair_workspace* ws);
