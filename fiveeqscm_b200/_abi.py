@@ -154,6 +154,8 @@ SIGNATURES = {
     "ufair_stats_reset": (C.c_int, [C.POINTER(UfairDesc), _vp]),
     "ufair_stats_pass_f64": (C.c_int, [C.POINTER(UfairDesc), _vp]),
     "ufair_stats_pass_f32": (C.c_int, [C.POINTER(UfairDesc), _vp]),
+    "ufair_stats_pass_weighted_f64": (C.c_int, [C.POINTER(UfairDesc), _vp, _vp]),
+    "ufair_stats_pass_weighted_f32": (C.c_int, [C.POINTER(UfairDesc), _vp, _vp]),
     "ufair_stats_finalize": (C.c_int, [C.POINTER(UfairDesc), _vp, _vp, _vp]),
     "ufair_stats_finalize_packed": (C.c_int, [C.POINTER(UfairDesc), _vp, _vp, _vp]),
     "ufair_stats_unpack": (C.c_int, [_vp, _vp, _i32, _i32, _vp, _vp, _vp]),
@@ -167,6 +169,8 @@ SIGNATURES = {
     "ufair_workspace_destroy": (C.c_int, [_vp]),
     "ufair_run_host_f64": (C.c_int, [_vp, C.POINTER(UfairDesc), _vp, _vp]),
     "ufair_run_host_f32": (C.c_int, [_vp, C.POINTER(UfairDesc), _vp, _vp]),
+    "ufair_run_host_weighted_f64": (C.c_int, [_vp, C.POINTER(UfairDesc), _vp, _vp, _vp]),
+    "ufair_run_host_weighted_f32": (C.c_int, [_vp, C.POINTER(UfairDesc), _vp, _vp, _vp]),
     "ufair_link_probe": (C.c_int, [C.c_int, _i64, _i64, _i32, _i32, _pd, _pd]),
     "ufair_math_probe_f64": (C.c_int, [C.c_int, _vp, _vp, _i64, _vp]),
     "ufair_math_probe_f32": (C.c_int, [C.c_int, _vp, _vp, _i64, _vp]),

@@ -25,6 +25,7 @@ from typing import Optional, Sequence
 import numpy as np
 
 from . import _abi
+from .stats import WEIGHT_MAX
 
 _ALPHA = {"exp": _abi.ALPHA_EXP, "sinh": _abi.ALPHA_SINH, "newton": _abi.ALPHA_NEWTON, "one": _abi.ALPHA_ONE}
 _TMODE = {"mid": _abi.T_MID, "end": _abi.T_END}
@@ -76,6 +77,7 @@ class EnsembleResult:
     n_member: int = 0
     stat_group: Optional[str] = None  # what the statistics are grouped by: None (pooled), "scenario" or "labels"
     out_every: int = 1      # steps per output row: 1 = every step, k >= 2 = means over periods of k steps
+    weighted: bool = False  # statistics with member weights (stat_weight=): hist counts weight units, moments weighted
 
 
 # ------------------------------------------------------------------------------------------------
@@ -235,6 +237,50 @@ def _check_labels(top: int, groups: int, name: str):
         raise ValueError(f"{name} has a label {top} >= groups {groups}")
 
 
+def _check_weights(w, M: int, stats):
+    """The checks of ``stat_weight=`` on an integer array [M] (numpy or torch, any device), in exact integer
+    arithmetic: every weight in 0 .. 2^32 - 1 and their sum <= 2^32 - 1, the bound under which the library's uint32
+    private histograms count exactly (the library does not check it).  Returns ``w`` as int64 of the same kind; a
+    device tensor costs one synchronise."""
+    if stats is None:
+        raise ValueError("stat_weight needs stats=HistSpec(...)")
+    torch = _torch() if not isinstance(w, np.ndarray) else None
+    is_int = (np.issubdtype(w.dtype, np.integer) if torch is None else
+              not (w.dtype.is_floating_point or w.dtype.is_complex or w.dtype == torch.bool))
+    if not is_int:
+        raise ValueError(f"stat_weight must hold integers, got dtype {w.dtype}")
+    if w.ndim != 1 or w.shape[0] != M:
+        raise ValueError(f"stat_weight must have one weight per member: shape ({M},), got {tuple(w.shape)}")
+    if M == 0:
+        return w.astype(np.int64) if torch is None else w.to(torch.int64)
+    too_large = f"stat_weight has a weight > 2^32 - 1 = {WEIGHT_MAX}"
+    # min, max and partial sums of 2^30 weights (exact in int64 once every weight is below 2^32)
+    if torch is None:
+        if w.dtype == np.uint64 and int(w.max()) > WEIGHT_MAX:
+            raise ValueError(too_large)
+        w = w.astype(np.int64)
+        lo, hi, *sums = (int(x) for x in [w.min(), w.max()] + [w[i:i + 2 ** 30].sum() for i in range(0, M, 2 ** 30)])
+    else:
+        # unsigned tensors are read through their signed twin (casts of unsigned types are not available everywhere)
+        wide = w.dtype == torch.uint64   # seen through int64, values >= 2^63 are negative
+        if w.dtype in (torch.uint16, torch.uint32):
+            bits = 16 if w.dtype == torch.uint16 else 32
+            w = w.view(torch.int16 if bits == 16 else torch.int32).to(torch.int64) & ((1 << bits) - 1)
+        w = (w.view(torch.int64) if wide else w).to(torch.int64)
+        lo, hi, *sums = torch.stack([w.min(), w.max()] + [w[i:i + 2 ** 30].sum() for i in range(0, M, 2 ** 30)]).tolist()
+        if wide and lo < 0:
+            raise ValueError(too_large)
+    if lo < 0:
+        raise ValueError(f"stat_weight has a negative weight ({lo})")
+    if hi > WEIGHT_MAX:
+        raise ValueError(too_large)
+    total = sum(sums)
+    if total > WEIGHT_MAX:
+        raise ValueError(f"stat_weight sums to {total} > 2^32 - 1 = {WEIGHT_MAX}: the statistics count in 32 bits "
+                         "(scale the weights down, e.g. with stats.integer_weights)")
+    return w
+
+
 def _driven_mask(conc_driven, G) -> int:
     """None / False -> 0; True -> every gas; else one truth value per gas."""
     if conc_driven is None or conc_driven is False:
@@ -327,7 +373,8 @@ def run_ensemble(emissions, gas_params, thermal_params, *, dt=1.0, scen_idx=None
                  fext_per_member=False, state_in=None, alpha_mode="exp", newton_iters=0, iirf_max=None,
                  iirf_h=100.0, t_mode="mid", outputs: Sequence[str] = ("C", "RF", "T"), stats: Optional[HistSpec] = None,
                  precision="f64", return_state=True, chunk_members=None, workspace=None, out=None,
-                 gas_form="auto", conc_driven=None, stat_group=None, out_every=1, out_dtype=None) -> EnsembleResult:
+                 gas_form="auto", conc_driven=None, stat_group=None, out_every=1, out_dtype=None,
+                 stat_weight=None) -> EnsembleResult:
     """Integrate the 5-equation model for an ensemble (oxfair, .coveragerc:19, as one kernel launch).
 
     emissions      [G][n_t][M] per-member emission RATES, or [G][n_t][S] scenario-shared with
@@ -343,6 +390,13 @@ def run_ensemble(emissions, gas_params, thermal_params, *, dt=1.0, scen_idx=None
                    scenario unless ``stats.groups`` says otherwise) or labels [M] int with ``stats.groups`` = G:
                    label g in [0, G) counts the member in group g, a negative label leaves it out of the
                    statistics.  ``.hist`` is then [G][n_t][bins] and ``.moments`` [G][n_t][4].
+    stat_weight    integer weights [M] for the statistics (e.g. likelihood weights from
+                   :func:`fiveeqscm_b200.stats.integer_weights`): member m adds stat_weight[m] to its bin instead of 1,
+                   its moments are weighted (sum of w T, sum of w T^2), and weight 0 leaves it out of every statistic,
+                   like a negative label.  Combines with ``stat_group``.  A CUDA tensor for device inputs, numpy / a CPU
+                   tensor for the host pipeline.  Every weight must be in 0 .. 2^32 - 1 and their sum <= 2^32 - 1
+                   (ValueError otherwise; on the device the check synchronises once).  ``.hist`` and ``.moments``
+                   keep their shapes and dtypes, counting weight units; ``.weighted`` is True.
     out_every      k >= 2: return one row of C, RF and T per period of k steps, the mean over its steps (a
                    sequential sum in step order in the run's precision, times 1 / k); n_t must be a multiple of k.
                    Results are then [G][n_t / k][M], [n_t / k][M], and the statistics bin the period-mean T
@@ -375,7 +429,8 @@ def run_ensemble(emissions, gas_params, thermal_params, *, dt=1.0, scen_idx=None
     kw = dict(dt=dt, scen_idx=scen_idx, e_scale=e_scale, f_ext=f_ext, fext_per_member=fext_per_member, state_in=state_in,
               alpha_mode=alpha_mode, newton_iters=newton_iters, iirf_max=iirf_max, iirf_h=iirf_h, t_mode=t_mode,
               outputs=outputs, stats=stats, precision=precision, return_state=return_state, gas_form=gas_form,
-              conc_driven=conc_driven, stat_group=stat_group, out_every=out_every, out_dtype=out_dtype)
+              conc_driven=conc_driven, stat_group=stat_group, out_every=out_every, out_dtype=out_dtype,
+              stat_weight=stat_weight)
     if isinstance(emissions, torch.Tensor) and emissions.is_cuda:
         return DevicePlan(emissions, gas_params, thermal_params, **kw).run()
     return _run_host(emissions, gas_params, thermal_params, chunk_members=chunk_members, workspace=workspace, out=out,
@@ -464,6 +519,13 @@ class _DeviceArrays:
     def labels(self, x):
         return self.torch.as_tensor(x, device=self.device).to(self.torch.int32).contiguous().reshape(-1)
 
+    def weights(self, x, M, stats):
+        """The checked member weights as a new uint32 tensor [M] (:func:`_check_weights`: one synchronise), written
+        through its int32 view."""
+        torch = self.torch
+        w = _check_weights(torch.as_tensor(x, device=self.device), M, stats)
+        return torch.where(w >= 2 ** 31, w - 2 ** 32, w).to(torch.int32).view(torch.uint32)
+
     @staticmethod
     def ptr(x):
         return x.data_ptr()
@@ -491,6 +553,11 @@ class _HostArrays:
         return np.ascontiguousarray(_numpy(x), dtype=np.int32).reshape(-1)
 
     @staticmethod
+    def weights(x, M, stats):
+        """The checked member weights as a new uint32 array [M] (:func:`_check_weights`)."""
+        return _check_weights(np.asarray(_numpy(x)), M, stats).astype(np.uint32)
+
+    @staticmethod
     def ptr(x):
         return x.ctypes.data
 
@@ -498,11 +565,12 @@ class _HostArrays:
 def _prepare(arrays, E, gp, tp, *, dt=1.0, scen_idx=None, e_scale=None, f_ext=None, fext_per_member=False,
              state_in=None, alpha_mode="exp", newton_iters=0, iirf_max=None, iirf_h=100.0, t_mode="mid",
              outputs=("C", "RF", "T"), stats=None, gas_form="auto", conc_driven=None, stat_group=None, out_every=1,
-             precision="f64", out_dtype=None):
+             precision="f64", out_dtype=None, stat_weight=None):
     """Checks a run's inputs (keywords of :func:`run_ensemble`) and places them with `arrays` (:class:`_DeviceArrays`
-    or :class:`_HostArrays`).  Returns (descriptor with every input wired, the placed arrays by descriptor field,
-    the outputs with "E" added for concentration-driven runs, the HistSpec with its group count settled, the label
-    source of :func:`_resolve_groups`); the descriptor's out_type gives the outputs' dtype (:func:`_desc_out_kind`).
+    or :class:`_HostArrays`).  Returns (descriptor with every input wired, the placed arrays by descriptor field --
+    and the member weights under "stat_weight", which is no descriptor field --, the outputs with "E" added for
+    concentration-driven runs, the HistSpec with its group count settled, the label source of
+    :func:`_resolve_groups`); the descriptor's out_type gives the outputs' dtype (:func:`_desc_out_kind`).
     ``gas_form="auto"`` is left to the caller: it scans the placed arrays."""
     if isinstance(gas_form, str) and gas_form != "auto":
         raise ValueError("gas_form must be 'auto', None or one entry per gas")
@@ -532,6 +600,7 @@ def _prepare(arrays, E, gp, tp, *, dt=1.0, scen_idx=None, e_scale=None, f_ext=No
             raise ValueError("stat_group must have one label per member")
         if M:
             _check_labels(int(lab.max()), stats.groups, "scen_idx" if source == "scenario" else "stat_group")
+    weights = None if stat_weight is None else arrays.weights(stat_weight, M, stats)
     if e_scale is not None:
         placed["e_scale"] = arrays.rows(e_scale, ld)
     if f_ext is not None:
@@ -544,6 +613,8 @@ def _prepare(arrays, E, gp, tp, *, dt=1.0, scen_idx=None, e_scale=None, f_ext=No
         placed["state_in"] = arrays.rows(state_in, ld)
     for field, x in placed.items():
         setattr(d, field, arrays.ptr(x))
+    if weights is not None:
+        placed["stat_weight"] = weights
     return d, placed, outputs, stats, source
 
 
@@ -574,8 +645,9 @@ class DevicePlan:
         self.out_every, self.n_out = k, n_t // k   # output rows: per step, or per period of k steps
         self.scen_idx = placed.get("scen_idx")   # the plan's own copy: callers that re-launch may overwrite it in place
         self.stat_group = placed.get("stat_group")
+        self.stat_weight = placed.get("stat_weight")   # the plan's own uint32 copy, like scen_idx
 
-        res = EnsembleResult(spec=stats, n_member=M, stat_group=source, out_every=k)
+        res = EnsembleResult(spec=stats, n_member=M, stat_group=source, out_every=k, weighted=self.stat_weight is not None)
         for name, field, shape, kind in _result_layout(G, n_t, M, outputs, return_state, stats, k, out_kind):
             if field is None:
                 setattr(res, name, torch.empty(shape, dtype=getattr(torch, kind), device=dev))
@@ -625,10 +697,17 @@ class DevicePlan:
         _abi.check(self._run(C.byref(self.desc), self._stream()))
 
     def stats_pass(self):
-        """Statistics pass: histogram and moments of the T rows the integrator just wrote."""
-        if self.stats is not None:
-            fn = self._L.ufair_stats_pass_f64 if self.precision == "f64" else self._L.ufair_stats_pass_f32
+        """Statistics pass: histogram and moments of the T rows the integrator just wrote (weighted by
+        ``stat_weight`` when the plan has one)."""
+        if self.stats is None:
+            return
+        L, f64 = self._L, self.precision == "f64"
+        if self.stat_weight is None:
+            fn = L.ufair_stats_pass_f64 if f64 else L.ufair_stats_pass_f32
             _abi.check(fn(C.byref(self.desc), self._stream()))
+        else:
+            fn = L.ufair_stats_pass_weighted_f64 if f64 else L.ufair_stats_pass_weighted_f32
+            _abi.check(fn(C.byref(self.desc), self.stat_weight.data_ptr(), self._stream()))
 
     def finalize_stats(self):
         if self.stats is not None:
@@ -676,7 +755,8 @@ def _run_host(E, gp, tp, *, precision="f64", return_state=True, gas_form="auto",
         for g, f in enumerate(_detect_form_host(placed["gas_params"], placed.get("state_in"))):
             d.gas_form[g] = f
     res = out if out is not None else EnsembleResult()
-    res.spec, res.n_member, res.stat_group, res.out_every = stats, M, source, k
+    weights = placed.get("stat_weight")
+    res.spec, res.n_member, res.stat_group, res.out_every, res.weighted = stats, M, source, k, weights is not None
     for name, field, shape, kind in _result_layout(G, n_t, M, outputs, return_state, stats, k, out_kind):
         cur = getattr(res, name)   # out= reuse: an array of the right shape and dtype is written in place
         if isinstance(cur, torch.Tensor):
@@ -698,8 +778,12 @@ def _run_host(E, gp, tp, *, precision="f64", return_state=True, gas_form="auto",
     ws = Workspace(torch.cuda.current_device(), chunk_members) if own else workspace
     try:
         L = _abi.lib()
-        run = L.ufair_run_host_f64 if precision == "f64" else L.ufair_run_host_f32
-        _abi.check(run(ws._h, C.byref(d), *stat_out))
+        if weights is None:
+            run = L.ufair_run_host_f64 if precision == "f64" else L.ufair_run_host_f32
+            _abi.check(run(ws._h, C.byref(d), *stat_out))
+        else:
+            run = L.ufair_run_host_weighted_f64 if precision == "f64" else L.ufair_run_host_weighted_f32
+            _abi.check(run(ws._h, C.byref(d), weights.ctypes.data, *stat_out))
     finally:
         if own:
             ws.close()

@@ -252,6 +252,13 @@ struct Moments {
     min = fmin(min, v);
     max = fmax(max, v);
   }
+  // a value of integer weight w > 0, with wv = (double)w * v: with w == 1 the operations of take(v)
+  __device__ void take(double v, double wv) {
+    sum += wv;
+    sumsq = fma(wv, v, sumsq);
+    min = fmin(min, v);
+    max = fmax(max, v);
+  }
   __device__ void merge(const Moments& o) {
     sum += o.sum;
     sumsq += o.sumsq;
@@ -285,16 +292,20 @@ static_assert(offsetof(Moments, sum) == UFAIR_MOM_SUM * sizeof(double) &&
 //   moments: strided per-thread partials (per group in registers: unrolled predicated updates), shuffle tree, warps in
 //   order, merged into the same row of moments_private: no atomics, deterministic.  One group with every label 0
 //   performs the pooled pass's operations in the same order, so it reproduces the pooled pass bit for bit.
+//   WEIGHTS (ufair_stats_pass_weighted_*): member m adds weight[m] to its bin instead of 1 and takes
+//   Moments::take(v, w * v); weight 0 counts the member nowhere, like a negative label.  Weights of 1 perform the
+//   unweighted operations, so they reproduce the unweighted pass bit for bit.
 constexpr int kStatsThreads = 256;
 constexpr int kStatsSmemBins = 16384;  // 64 KB of dynamic shared memory at most
 
-// The label arguments come last: the pooled instantiation then keeps the pooled pass's parameter offsets, and with
-// them its instruction schedule.
-template <typename Real, int NGT, bool LABELS>
+// The label arguments come after the pooled pass's, and the weights after them: each instantiation then keeps the
+// parameter offsets of the arguments it shares with the pooled pass, and with them its instruction schedule.
+template <typename Real, int NGT, bool LABELS, bool WEIGHTS>
 __global__ void __launch_bounds__(kStatsThreads)
     stats_pass_kernel(const Real* __restrict__ T, long long ld, long long n_member, int t0_row, int rows, int bins,
                       Real lo, Real invw, int smem_hist, unsigned int* __restrict__ hp, double* mp,
-                      const int32_t* __restrict__ labels, int n_groups, int n_tiles) {
+                      const int32_t* __restrict__ labels, int n_groups, int n_tiles,
+                      const uint32_t* __restrict__ weight) {
   static_assert(LABELS || NGT == 1, "without labels every member is in the one group");
   using M = Math<Real>;
   extern __shared__ unsigned int sh[];
@@ -332,16 +343,25 @@ __global__ void __launch_bounds__(kStatsThreads)
     else
       atomicAdd(hdst + last_b, run);
   };
-  auto take = [&](Real x, int label) {
+  auto take = [&](Real x, int label, unsigned wt) {
     int sel = 0;  // the member's group in this tile, -1 for none
     if constexpr (LABELS) {
       const int gl = label - g0;
       sel = (unsigned)gl < (unsigned)ngt ? gl : -1;
     }
+    if constexpr (WEIGHTS)
+      if (wt == 0u) sel = -1;  // skipped, not multiplied by 0: 0 * NaN and 0 * inf are NaN
     const double v = (double)x;
+    if constexpr (WEIGHTS) {
+      const double wv = (double)wt * v;
 #pragma unroll
-    for (int j = 0; j < NGT; ++j)
-      if (sel == j) mom[j].take(v);
+      for (int j = 0; j < NGT; ++j)
+        if (sel == j) mom[j].take(v, wv);
+    } else {
+#pragma unroll
+      for (int j = 0; j < NGT; ++j)
+        if (sel == j) mom[j].take(v);
+    }
     const Real q = M::bin_x(x, lo, invw);
     const int b = (sel >= 0 && q == q) ? max(0, min(bins_m1, M::floor_to_int(q))) : -1;
     if (b != last_b || (LABELS && sel != last_g)) {
@@ -350,7 +370,10 @@ __global__ void __launch_bounds__(kStatsThreads)
       last_b = b;
       run = 0;
     }
-    run += (b >= 0);
+    if constexpr (WEIGHTS)
+      run += b >= 0 ? wt : 0u;  // the sum of a call's weights fits in 32 bits (include/ufair.h)
+    else
+      run += (b >= 0);
   };
   // one tile: stream T past L2; several: keep it for the sibling tiles.  The addresses are src + k + offset: with
   // src + (k + offset) nvcc unrolls the pooled FP64 loop differently (40 registers and 14 loads instead of 48 and 30).
@@ -362,18 +385,27 @@ __global__ void __launch_bounds__(kStatsThreads)
     else
       return 0;
   };
+  // the weight slice, like the label slice, is shared by every row of copy c: __ldg keeps it in L2
+  auto wgt = [&](long long i) {
+    if constexpr (WEIGHTS)
+      return __ldg(weight + m_lo + i);
+    else
+      return 1u;
+  };
   long long k = threadIdx.x;
   for (; k + 3 * kStatsThreads < span; k += 4 * kStatsThreads) {
     const Real x0 = load(src + k), x1 = load(src + k + kStatsThreads), x2 = load(src + k + 2 * kStatsThreads),
                x3 = load(src + k + 3 * kStatsThreads);
     const int l0 = label(k), l1 = label(k + kStatsThreads), l2 = label(k + 2 * kStatsThreads),
               l3 = label(k + 3 * kStatsThreads);
-    take(x0, l0);
-    take(x1, l1);
-    take(x2, l2);
-    take(x3, l3);
+    const unsigned w0 = wgt(k), w1 = wgt(k + kStatsThreads), w2 = wgt(k + 2 * kStatsThreads),
+                   w3 = wgt(k + 3 * kStatsThreads);
+    take(x0, l0, w0);
+    take(x1, l1, w1);
+    take(x2, l2, w2);
+    take(x3, l3, w3);
   }
-  for (; k < span; k += kStatsThreads) take(load(src + k), label(k));
+  for (; k < span; k += kStatsThreads) take(load(src + k), label(k), wgt(k));
   flush();
 #pragma unroll
   for (int j = 0; j < NGT; ++j)
@@ -398,7 +430,8 @@ __global__ void __launch_bounds__(kStatsThreads)
 }
 
 // Real here is the element type of the stored T rows (out_type), not necessarily the run's precision
-template <typename Real, int NGT, bool LABELS> static int launch_stats_pass(const ufair_desc* d, cudaStream_t stream) {
+template <typename Real, int NGT, bool LABELS, bool WEIGHTS>
+static int launch_stats_pass(const ufair_desc* d, const uint32_t* weight, cudaStream_t stream) {
   const int G = LABELS ? stat_groups(d) : 1, n_tiles = (G + NGT - 1) / NGT;
   if (d->hist_copies > 65535) return set_error(UFAIR_ERR_ARG, "hist_copies %d > 65535", d->hist_copies);
   const int rows = out_rows(d);  // the T rows the integrator wrote
@@ -407,14 +440,15 @@ template <typename Real, int NGT, bool LABELS> static int launch_stats_pass(cons
   const size_t smem = smem_hist ? (size_t)NGT * d->hist_bins * sizeof(unsigned int) : 0;
   cudaError_t e = cudaSuccess;
   if (smem > 48 * 1024)
-    e = cudaFuncSetAttribute(stats_pass_kernel<Real, NGT, LABELS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    e = cudaFuncSetAttribute(stats_pass_kernel<Real, NGT, LABELS, WEIGHTS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             (int)smem);
   if (e != cudaSuccess) return cuda_error(e, "cudaFuncSetAttribute(stats_pass_kernel)");
   const Real lo = (Real)d->hist_lo;
   const Real invw = (Real)((Real)d->hist_bins / ((Real)d->hist_hi - (Real)d->hist_lo));
-  stats_pass_kernel<Real, NGT, LABELS><<<dim3((unsigned)(rows * n_tiles), (unsigned)d->hist_copies), kStatsThreads,
-                                         smem, stream>>>((const Real*)d->out_T, d->ld_member, d->n_member, d->hist_t0,
-                                                         d->hist_rows, d->hist_bins, lo, invw, smem_hist, d->hist_private,
-                                                         d->moments_private, d->stat_group, G, n_tiles);
+  stats_pass_kernel<Real, NGT, LABELS, WEIGHTS>
+      <<<dim3((unsigned)(rows * n_tiles), (unsigned)d->hist_copies), kStatsThreads, smem, stream>>>(
+          (const Real*)d->out_T, d->ld_member, d->n_member, d->hist_t0, d->hist_rows, d->hist_bins, lo, invw, smem_hist,
+          d->hist_private, d->moments_private, d->stat_group, G, n_tiles, weight);
   e = cudaGetLastError();
   return e == cudaSuccess ? UFAIR_OK : cuda_error(e, "stats_pass_kernel launch");
 }
@@ -521,23 +555,30 @@ template <typename Real> int detect_form(const ufair_desc* d, int32_t* scratch, 
   return UFAIR_OK;
 }
 
-// the pass over T rows of element type Rows
-template <typename Rows> static int stats_pass_rows(const ufair_desc* d, cudaStream_t stream) {
-  if (!d->stat_group) return launch_stats_pass<Rows, 1, false>(d, stream);
+// the pass over T rows of element type Rows, with or without member weights
+template <typename Rows, bool WEIGHTS>
+static int stats_pass_rows(const ufair_desc* d, const uint32_t* weight, cudaStream_t stream) {
+  if (!d->stat_group) return launch_stats_pass<Rows, 1, false, WEIGHTS>(d, weight, stream);
   // up to four groups a tile of four: half the registers and predicated updates of a tile of eight
-  return stat_groups(d) <= 4 ? launch_stats_pass<Rows, 4, true>(d, stream) : launch_stats_pass<Rows, 8, true>(d, stream);
+  return stat_groups(d) <= 4 ? launch_stats_pass<Rows, 4, true, WEIGHTS>(d, weight, stream)
+                             : launch_stats_pass<Rows, 8, true, WEIGHTS>(d, weight, stream);
+}
+template <typename Rows> static int stats_pass_rows(const ufair_desc* d, const uint32_t* weight, cudaStream_t stream) {
+  return weight ? stats_pass_rows<Rows, true>(d, weight, stream) : stats_pass_rows<Rows, false>(d, nullptr, stream);
 }
 
-template <typename Real> int run_stats_pass(const ufair_desc* d, cudaStream_t stream) {
+// weight: the member weights of the weighted pass, NULL for the unweighted one
+template <typename Real> int run_stats_pass(const ufair_desc* d, const uint32_t* weight, cudaStream_t stream) {
   int rc = validate_desc(d, sizeof(Real));
   if (rc != UFAIR_OK) return rc;
   if (!d->stats) return set_error(UFAIR_ERR_ARG, "ufair_stats_pass: descriptor has stats == 0");
   if (d->n_member == 0 || d->n_t == 0) return UFAIR_OK;
   // the T rows the integrator stored: float32 outputs of an FP64 run take the FP32 pass (include/ufair.h out_type)
-  return out_elem(d, sizeof(Real)) == sizeof(float) ? stats_pass_rows<float>(d, stream) : stats_pass_rows<Real>(d, stream);
+  return out_elem(d, sizeof(Real)) == sizeof(float) ? stats_pass_rows<float>(d, weight, stream)
+                                                    : stats_pass_rows<Real>(d, weight, stream);
 }
-template int run_stats_pass<double>(const ufair_desc*, cudaStream_t);
-template int run_stats_pass<float>(const ufair_desc*, cudaStream_t);
+template int run_stats_pass<double>(const ufair_desc*, const uint32_t*, cudaStream_t);
+template int run_stats_pass<float>(const ufair_desc*, const uint32_t*, cudaStream_t);
 template int run_device<double>(const ufair_desc*, cudaStream_t);
 template int run_device<float>(const ufair_desc*, cudaStream_t);
 
@@ -770,8 +811,20 @@ int64_t ufair_block_members(void) { return kWarps * 32; }
 int ufair_run_f64(const ufair_desc* d, void* stream) { return run_device<double>(d, (cudaStream_t)stream); }
 int ufair_run_f32(const ufair_desc* d, void* stream) { return run_device<float>(d, (cudaStream_t)stream); }
 
-int ufair_stats_pass_f64(const ufair_desc* d, void* stream) { return run_stats_pass<double>(d, (cudaStream_t)stream); }
-int ufair_stats_pass_f32(const ufair_desc* d, void* stream) { return run_stats_pass<float>(d, (cudaStream_t)stream); }
+int ufair_stats_pass_f64(const ufair_desc* d, void* stream) {
+  return run_stats_pass<double>(d, nullptr, (cudaStream_t)stream);
+}
+int ufair_stats_pass_f32(const ufair_desc* d, void* stream) {
+  return run_stats_pass<float>(d, nullptr, (cudaStream_t)stream);
+}
+int ufair_stats_pass_weighted_f64(const ufair_desc* d, const uint32_t* weight, void* stream) {
+  if (!weight) return set_error(UFAIR_ERR_ARG, "ufair_stats_pass_weighted: weight is NULL");
+  return run_stats_pass<double>(d, weight, (cudaStream_t)stream);
+}
+int ufair_stats_pass_weighted_f32(const ufair_desc* d, const uint32_t* weight, void* stream) {
+  if (!weight) return set_error(UFAIR_ERR_ARG, "ufair_stats_pass_weighted: weight is NULL");
+  return run_stats_pass<float>(d, weight, (cudaStream_t)stream);
+}
 
 int ufair_detect_form_f64(const ufair_desc* d, int32_t* scratch, uint8_t* form, void* stream) {
   return detect_form<double>(d, scratch, form, (cudaStream_t)stream);

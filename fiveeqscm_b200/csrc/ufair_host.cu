@@ -5,7 +5,8 @@
 // streams with two device staging buffers so copy-in(c+1), kernel(c) and copy-out(c-1) overlap.
 // Scenario-shared inputs go up once.  Statistics accumulate across chunks in the private
 // histogram copies and are finalised once at the end; statistics labels (stat_group) are staged per
-// chunk next to scen_idx, or not at all when they are scen_idx itself.
+// chunk next to scen_idx, or not at all when they are scen_idx itself, and member weights
+// (ufair_run_host_weighted_*) next to them.
 #include <cuda_runtime.h>
 #include <stddef.h>
 #include <stdint.h>
@@ -52,10 +53,17 @@ struct DevBuf {
   }
 };
 
+// The arrays of one call: the descriptor's, and the statistics weights of ufair_run_host_weighted_*, which are not a
+// descriptor field.  The staging table addresses each array by the offset of its pointer in this struct.
+struct RunArrays {
+  ufair_desc d;
+  const uint32_t* weight;  // [n_member], or NULL: unweighted statistics
+};
+
 // One array the pipeline stages per chunk: `rows` rows of the chunk's members, `elem` bytes each, in a device buffer
-// that takes the place of descriptor field `field` in the chunk's descriptor.
+// that takes the place of field `field` in the chunk's arrays.
 struct Staged {
-  size_t field;      // offsetof(ufair_desc, <the array's pointer>)
+  size_t field;      // offsetof(RunArrays, <the array's pointer>)
   size_t rows;       // rows per member
   size_t elem;       // bytes per element
   bool in;           // copied up before the kernel; else written by the kernel
@@ -64,7 +72,7 @@ struct Staged {
   bool flat;         // an [n_member] array without row pitch: one 1-D copy
   size_t alias = 0;  // not staged but the staged array of this field instead (labels that are scen_idx itself)
 };
-constexpr int kStaged = 14;  // entries of run_chunks' table
+constexpr int kStaged = 15;  // entries of run_chunks' table
 
 struct Stage {
   DevBuf b[kStaged];
@@ -90,23 +98,23 @@ namespace ufair {
     if (e__ != cudaSuccess) return cuda_error(e__, what); \
   } while (0)
 
-// the descriptor's pointer field at byte offset `field` (every array field is a plain pointer)
-static const void* get_field(const ufair_desc& d, size_t field) {
+// the pointer field at byte offset `field` of a call's arrays (every array field is a plain pointer)
+static const void* get_field(const RunArrays& a, size_t field) {
   const void* p;
-  memcpy(&p, (const char*)&d + field, sizeof p);
+  memcpy(&p, (const char*)&a + field, sizeof p);
   return p;
 }
-static void set_field(ufair_desc& d, size_t field, const void* p) { memcpy((char*)&d + field, &p, sizeof p); }
+static void set_field(RunArrays& a, size_t field, const void* p) { memcpy((char*)&a + field, &p, sizeof p); }
 
 // members [c0, c0 + cm) of staged array t, between the caller's array (row pitch ld_member) and its device buffer
 // (row pitch chunk)
-static int copy_chunk(const Staged& t, const ufair_desc* h, void* dev, int64_t c0, int64_t cm, int64_t chunk,
+static int copy_chunk(const Staged& t, const RunArrays& h, void* dev, int64_t c0, int64_t cm, int64_t chunk,
                       cudaMemcpyKind kind, cudaStream_t s) {
-  char* host = (char*)get_field(*h, t.field) + (size_t)c0 * t.elem;
+  char* host = (char*)get_field(h, t.field) + (size_t)c0 * t.elem;
   const bool up = kind == cudaMemcpyHostToDevice;
   void* dst = up ? dev : (void*)host;
   const void* src = up ? (const void*)host : dev;
-  const size_t w = (size_t)cm * t.elem, hp = (size_t)h->ld_member * t.elem, dp = (size_t)chunk * t.elem;
+  const size_t w = (size_t)cm * t.elem, hp = (size_t)h.d.ld_member * t.elem, dp = (size_t)chunk * t.elem;
   if (t.flat) {
     CK(cudaMemcpyAsync(dst, src, w, kind, s), "cudaMemcpyAsync");
     return UFAIR_OK;
@@ -116,8 +124,10 @@ static int copy_chunk(const Staged& t, const ufair_desc* h, void* dev, int64_t c
   return UFAIR_OK;
 }
 
+// ha: the caller's host arrays; da: the same with the scenario-shared inputs and statistics buffers on the device
 template <typename Real>
-static int run_chunks(ufair_workspace* ws, const ufair_desc* h, const ufair_desc& d) {
+static int run_chunks(ufair_workspace* ws, const RunArrays& ha, const RunArrays& da) {
+  const ufair_desc* h = &ha.d;
   const size_t es = sizeof(Real), i4 = sizeof(int32_t), os = out_elem(h, es);  // os: C / RF / T (out_type)
   const int G = h->n_gas, n_t = h->n_t, out = h->out_mask;
   const int64_t M = h->n_member;
@@ -127,9 +137,9 @@ static int run_chunks(ufair_workspace* ws, const ufair_desc* h, const ufair_desc
   const bool labels_are_scen = h->stat_group != nullptr && h->stat_group == h->scen_idx;
   auto want = [&](int bit) { return (out & bit) != 0; };
   // Every array staged per chunk, in the order its copies are issued: field, rows per member, element bytes, in, on,
-  // back, flat[, alias].  Arrays that are not staged keep their field of `d`: NULL, or the scenario-shared copy
+  // back, flat[, alias].  Arrays that are not staged keep their field of `da`: NULL, or the scenario-shared copy
   // run_host put on the device.
-#define F(x) offsetof(ufair_desc, x)
+#define F(x) offsetof(RunArrays, d.x)
   const Staged table[] = {
       {F(emissions), gt, es, true, e_member, false, false},
       {F(f_ext), (size_t)n_t, es, true, h->fext_mode == UFAIR_FEXT_MEMBER, false, false},
@@ -140,6 +150,7 @@ static int run_chunks(ufair_workspace* ws, const ufair_desc* h, const ufair_desc
       {F(scen_idx), 1, i4, true, h->scen_idx != nullptr, false, true},
       {F(stat_group), 1, i4, true, h->stat_group != nullptr && !labels_are_scen, false, true,
        labels_are_scen ? F(scen_idx) : 0},
+      {offsetof(RunArrays, weight), 1, sizeof(uint32_t), true, ha.weight != nullptr, false, true},
       {F(out_C), go, os, false, want(UFAIR_OUT_C), want(UFAIR_OUT_C), false},
       {F(out_RF), go, os, false, want(UFAIR_OUT_RF), want(UFAIR_OUT_RF), false},
       {F(out_T), n_out, os, false, want(UFAIR_OUT_T) || h->stats != 0, want(UFAIR_OUT_T), false},  // stats read T
@@ -183,30 +194,30 @@ static int run_chunks(ufair_workspace* ws, const ufair_desc* h, const ufair_desc
     // ---- H2D
     for (int i = 0; i < kStaged; ++i) {
       if (!table[i].on || !table[i].in) continue;
-      const int rc = copy_chunk(table[i], h, S.b[i].p, c0, cm, chunk, cudaMemcpyHostToDevice, ws->s_in);
+      const int rc = copy_chunk(table[i], ha, S.b[i].p, c0, cm, chunk, cudaMemcpyHostToDevice, ws->s_in);
       if (rc != UFAIR_OK) return rc;
     }
     CK(cudaEventRecord(S.in_done, ws->s_in), "cudaEventRecord");
     // ---- kernel
     CK(cudaStreamWaitEvent(ws->s_run, S.in_done, 0), "cudaStreamWaitEvent");
-    ufair_desc k = d;
-    k.n_member = cm;
-    k.ld_member = chunk;
+    RunArrays k = da;
+    k.d.n_member = cm;
+    k.d.ld_member = chunk;
     for (int i = 0; i < kStaged; ++i) {
       if (table[i].on)
         set_field(k, table[i].field, S.b[i].p);
       else if (table[i].alias)
         set_field(k, table[i].field, get_field(k, table[i].alias));
     }
-    int rc = run_device<Real>(&k, ws->s_run);
-    if (rc == UFAIR_OK && h->stats) rc = run_stats_pass<Real>(&k, ws->s_run);
+    int rc = run_device<Real>(&k.d, ws->s_run);
+    if (rc == UFAIR_OK && h->stats) rc = run_stats_pass<Real>(&k.d, k.weight, ws->s_run);
     if (rc != UFAIR_OK) return rc;
     CK(cudaEventRecord(S.run_done, ws->s_run), "cudaEventRecord");
     // ---- D2H
     CK(cudaStreamWaitEvent(ws->s_out, S.run_done, 0), "cudaStreamWaitEvent");
     for (int i = 0; i < kStaged; ++i) {
       if (!table[i].back) continue;
-      rc = copy_chunk(table[i], h, S.b[i].p, c0, cm, chunk, cudaMemcpyDeviceToHost, ws->s_out);
+      rc = copy_chunk(table[i], ha, S.b[i].p, c0, cm, chunk, cudaMemcpyDeviceToHost, ws->s_out);
       if (rc != UFAIR_OK) return rc;
     }
     CK(cudaEventRecord(S.out_done, ws->s_out), "cudaEventRecord");
@@ -228,12 +239,17 @@ static int run_chunks(ufair_workspace* ws, const ufair_desc* h, const ufair_desc
     }                                        \
   } while (0)
 
-template <typename Real> static int run_host(ufair_workspace* ws, const ufair_desc* h, uint64_t* hist, double* moments) {
+// weighted: ufair_run_host_weighted_*, whose statistics take the member weights `weight`
+template <typename Real>
+static int run_host(ufair_workspace* ws, const ufair_desc* h, bool weighted, const uint32_t* weight, uint64_t* hist,
+                    double* moments) {
   if (!ws) return set_error(UFAIR_ERR_ARG, "workspace is NULL");
+  if (weighted && !weight) return set_error(UFAIR_ERR_ARG, "ufair_run_host_weighted: weight is NULL");
   // the device path's run rules; its placement rules apply to the staged chunks (run_device, run_stats_pass)
   const int rc0 = check_run(h, sizeof(Real));
   if (rc0 != UFAIR_OK) return rc0;
   if (h->stats && (!hist || !moments)) return set_error(UFAIR_ERR_ARG, "stats requested but hist/moments NULL");
+  if (weighted && !h->stats) return set_error(UFAIR_ERR_ARG, "ufair_run_host_weighted: weights need stats == 1");
   if (h->n_member == 0 || h->n_t == 0) return UFAIR_OK;
   DeviceGuard guard(ws->device);  // the caller's current device is restored on every return path
   if (guard.err != cudaSuccess) return cuda_error(guard.err, "cudaSetDevice");
@@ -276,7 +292,7 @@ template <typename Real> static int run_host(ufair_workspace* ws, const ufair_de
   cudaEventRecord(shared_up, ws->s_in);
   cudaStreamWaitEvent(ws->s_run, shared_up, 0);
 
-  int rc = run_chunks<Real>(ws, h, d);
+  int rc = run_chunks<Real>(ws, RunArrays{*h, weight}, RunArrays{d, nullptr});
 
   if (rc == UFAIR_OK && h->stats) {
     rc = ufair_stats_finalize(&d, (uint64_t*)ws->hist_out.p, (double*)ws->mom_out.p, ws->s_run);
@@ -351,10 +367,18 @@ int ufair_workspace_destroy(ufair_workspace* ws) {
 }
 
 int ufair_run_host_f64(ufair_workspace* ws, const ufair_desc* d, uint64_t* hist, double* moments) {
-  return run_host<double>(ws, d, hist, moments);
+  return run_host<double>(ws, d, false, nullptr, hist, moments);
 }
 int ufair_run_host_f32(ufair_workspace* ws, const ufair_desc* d, uint64_t* hist, double* moments) {
-  return run_host<float>(ws, d, hist, moments);
+  return run_host<float>(ws, d, false, nullptr, hist, moments);
+}
+int ufair_run_host_weighted_f64(ufair_workspace* ws, const ufair_desc* d, const uint32_t* weight, uint64_t* hist,
+                                double* moments) {
+  return run_host<double>(ws, d, true, weight, hist, moments);
+}
+int ufair_run_host_weighted_f32(ufair_workspace* ws, const ufair_desc* d, const uint32_t* weight, uint64_t* hist,
+                                double* moments) {
+  return run_host<float>(ws, d, true, weight, hist, moments);
 }
 
 }  // extern "C"

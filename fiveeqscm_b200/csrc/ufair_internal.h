@@ -18,5 +18,6 @@ inline int out_rows(const ufair_desc* d) { return d->out_every >= 2 ? d->n_t / d
 // bytes per element of out_C / out_RF / out_T in a run of element size elem (out_type, include/ufair.h)
 inline size_t out_elem(const ufair_desc* d, size_t elem) { return d->out_type == UFAIR_OUTTYPE_F32 ? sizeof(float) : elem; }
 template <typename Real> int run_device(const ufair_desc* d, cudaStream_t stream);
-template <typename Real> int run_stats_pass(const ufair_desc* d, cudaStream_t stream);
+// the statistics pass; weight: [n_member] member weights (ufair_stats_pass_weighted_*), NULL for the unweighted pass
+template <typename Real> int run_stats_pass(const ufair_desc* d, const uint32_t* weight, cudaStream_t stream);
 }  // namespace ufair

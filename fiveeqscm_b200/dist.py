@@ -27,7 +27,9 @@ def allreduce_stats(hist, moments, group=None):
     collectives: one SUM over [counts as float64 | sum T | sum T^2] (integer counts below 2^53 add
     exactly in any order, so the reduced histogram is bitwise independent of the GPU count) and one
     MAX over [max T, -min T].  Generic torch version (any backend, CPU or CUDA tensors);
-    :class:`StatsReducer` is the device fast path that packs inside the library and overlaps."""
+    :class:`StatsReducer` is the device fast path that packs inside the library and overlaps.
+    Weighted statistics (``stat_weight=``) reduce the same way: the counts are integer weight totals, exact as long
+    as each rank's total stays <= 2^32 - 1 (and so the reduced one far below 2^53)."""
     import torch
     import torch.distributed as dist
     if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) == 1:

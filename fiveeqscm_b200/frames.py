@@ -64,7 +64,9 @@ def summary_frame(result, years, pcts: Sequence[float] = (5.0, 17.0, 50.0, 83.0,
     (after the cross-GPU all-reduce, if any): mean, std, min, max and percentiles off the histogram.
     Grouped statistics (``stat_group=``) give a long frame, one block of years per group, led by a
     ``scenario`` column (grouped by scenario) or a ``group`` column (by labels) holding ``group_names[g]``
-    (default: the group index).  A group's member count is its histogram row sum."""
+    (default: the group index).  A group's member count is its histogram row sum.  For a weighted run
+    (``stat_weight=``) that row sum is the weight total: the ``members`` column then holds the weight total, and
+    mean, std and percentiles are the weighted ones."""
     import pandas as pd
     if result.hist is None or result.moments is None or result.spec is None:
         raise ValueError("summary_frame needs a result computed with stats=HistSpec(...)")

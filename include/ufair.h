@@ -279,6 +279,24 @@ int ufair_stats_reset(const ufair_desc* d, void* stream);
  * rows are read in the descriptor's out_type (float32 rows of an FP64 run take the FP32 pass). */
 int ufair_stats_pass_f64(const ufair_desc* d, void* stream);
 int ufair_stats_pass_f32(const ufair_desc* d, void* stream);
+/* Weighted statistics: the same pass with an integer weight per member (e.g. integer likelihood weights of a
+ * constrained ensemble).  weight: DEVICE [n_member] uint32, member m of this call at weight[m].
+ *   weight[m] == 0   member m is counted nowhere: not in the histogram, not in any moment (min / max included),
+ *                    exactly like a negative stat_group label; its T is never multiplied, so a NaN or inf there
+ *                    changes nothing.
+ *   weight[m] == w   the member adds w to its bin instead of 1, and its moments are, bit for bit,
+ *                    wv = (double)w * v;  sum += wv;  sumsq = fma(wv, v, sumsq);  min / max over members with
+ *                    w > 0, in the pass's fixed order.  All-ones weights give the unweighted pass bit for bit.
+ * Weights combine with stat_group: member m adds weight[m] in group stat_group[m].  The binning rule, the
+ * non-finite rule, the row layout and the finalize / packed / unpack / percentile calls are unchanged: a weighted
+ * histogram is a histogram in units of weight.
+ * Overflow contract: the private histograms are uint32, so the sum of all weights of one call must be
+ * <= 2^32 - 1 -- over every member chunk and host-pipeline chunk accumulated into the same private buffers.  Then
+ * every count is exact, and so is the packed cross-GPU reduction (exact below 2^53).  The library does not check
+ * this (it would need a synchronise); the Python layer does.  A NULL weight is UFAIR_ERR_ARG; every other rule,
+ * code and message is that of ufair_stats_pass_f64 / _f32, and the suffix has the same meaning. */
+int ufair_stats_pass_weighted_f64(const ufair_desc* d, const uint32_t* weight, void* stream);
+int ufair_stats_pass_weighted_f32(const ufair_desc* d, const uint32_t* weight, void* stream);
 /* Fold the private copies: hist[G][hist_rows][hist_bins] (uint64 counts) and
  * moments[G][hist_rows][UFAIR_MOM_COUNT] (sum, sumsq, min, max as doubles); G = max(1, n_stat_groups).
  * Here and in ufair_stats_finalize_packed, "hist_rows" below stands for G * hist_rows. */
@@ -366,6 +384,13 @@ int ufair_workspace_create(int device, int64_t chunk_members, ufair_workspace** 
 int ufair_workspace_destroy(ufair_workspace* ws);
 int ufair_run_host_f64(ufair_workspace* ws, const ufair_desc* d, uint64_t* hist, double* moments);
 int ufair_run_host_f32(ufair_workspace* ws, const ufair_desc* d, uint64_t* hist, double* moments);
+/* The same with weighted statistics (ufair_stats_pass_weighted_*): weight is HOST [n_member] uint32, staged per
+ * chunk with the other per-member arrays.  Needs stats == 1; a NULL weight or stats == 0 is UFAIR_ERR_ARG,
+ * reported before anything is copied.  The sum of all weights must be <= 2^32 - 1 (not checked). */
+int ufair_run_host_weighted_f64(ufair_workspace* ws, const ufair_desc* d, const uint32_t* weight, uint64_t* hist,
+                                double* moments);
+int ufair_run_host_weighted_f32(ufair_workspace* ws, const ufair_desc* d, const uint32_t* weight, uint64_t* hist,
+                                double* moments);
 
 /* ---- host-link probe (measurement support: the ceiling bench.py states e2e against) ----
  * Times `reps` rounds of copies between a page-locked host buffer (allocated and kept by the probe) and
